@@ -3,6 +3,9 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo (libinfltm, sm_100a)
   python bench.py --impl reference ...                     # the reference algorithm on the host cores
+  python bench.py ... --dump-outputs DIR                   # also save what the last timed step returned, DIR/*.npy
+
+Inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 Workload (config.workload): the NExT-QA shape of BASELINE.json configs[1] -- chunks of L=256 frames x 32
 Q-former tokens x 768, num_basis=256, tau=0.75, sticky re-sampling, 32 queries -- for `--videos` independent
@@ -300,6 +303,14 @@ def parity_check(dev, chunks, videos=4, precision="tf32", shape=None):
             "ok": bool(worst_ctx < 1e-3 and worst_B < 1e-3 and flips <= 0.01 * max(draws, 1))}
 
 
+def write_outputs(directory, arrays):
+    """--dump-outputs: one float32 .npy per output array."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(a, dtype=np.float32))
+
+
 def run_reference_impl(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -314,12 +325,15 @@ def run_reference_impl(args):
     per_call = []
     t0 = time.perf_counter()
     for _ in range(args.steps):
+        step_outs = []
         for c in range(chunks):
             t1 = time.perf_counter()
             with torch.no_grad():
-                orc.forward(ks[c], qs[c], c == 0, us[c])
+                step_outs.append(orc.forward(ks[c], qs[c], c == 0, us[c]))
             per_call.append(time.perf_counter() - t1)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {f"ctx_chunk{c}": o.numpy() for c, o in enumerate(step_outs)})
     calls = args.steps * chunks
     val = calls / dt
     as_is = None
@@ -410,6 +424,12 @@ def run_b200(args):
     names = ["pool", "resample", "consolidate", "project_kv", "attention"]
 
     host_ms = [0.0]
+    dumped = {}          # --dump-outputs: the contexts of the last timed step of the headline pass, on the host
+    dump_videos = None
+    if args.dump_outputs:
+        # every chunk's ctx[Bv,Q,D] of the step, for a fixed seeded sample of the videos when all would exceed 64 MB
+        n = min(Bv, int(64e6) // (C * Q * D * 4))
+        dump_videos = torch.randperm(Bv, generator=torch.Generator().manual_seed(0))[:n].sort().values.to(dev)
 
     def graph_pass():
         """The same K steps as `timed_pass(True, ...)`, replayed from ONE CUDA graph per step (the C chunk-steps of a
@@ -490,8 +510,10 @@ def run_b200(args):
         t_host = time.perf_counter()
         i = 0
         gathers = []
+        keep = dump_videos is not None and with_overlap == overlap
         for _ in range(args.steps):
             out = None
+            step_outs = []
             for c in range(C):
                 eng.prof_events = ev_sets[i]
                 i += 1
@@ -502,6 +524,8 @@ def run_b200(args):
                                               k_next=ks[(c + 1) % C], next_new_doc=((c + 1) % C == 0))
                 else:
                     out = eng.step(ks[c], qs[c], us[c] if c else None, new_doc=(c == 0))
+                if keep:
+                    step_outs.append(out)
             if world > 1:
                 # gather of this step's outputs: asynchronous, so that the next step's kernels are not held up;
                 # every gather is complete before the end of the timed region
@@ -518,6 +542,8 @@ def run_b200(args):
         D_.barrier(dev)
         clk = sampler.stop() if sampler else None
         ms_ = D_.max_over_ranks(e0.elapsed_time(e1), dev)
+        for c, o in enumerate(step_outs):
+            dumped[f"ctx_chunk{c}"] = o.index_select(0, dump_videos).cpu().numpy()
         stage_ms = {n: [] for n in names}
         f = Ct.c_float()
         for si, evs in enumerate(ev_sets):
@@ -543,6 +569,8 @@ def run_b200(args):
     for _r in range(max(1, args.repeats)):
         reps.append(timed_pass(overlap, True) + (host_ms[0],))
     ms, stage_avg, clocks, host_enqueue_ms = min(reps, key=lambda t: t[0])
+    if dump_videos is not None and rank == 0:
+        write_outputs(args.dump_outputs, dumped)
     calls_total = Bv * C * args.steps * world
     value_eager = calls_total / (ms * 1e-3)
 
@@ -1065,7 +1093,12 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the other BASELINE shapes (cfg1 / cfg3 / cfg4)")
     ap.add_argument("--gauss-videos", type=int, default=128)
     ap.add_argument("--gauss-frames", type=int, default=256, help="Lk of the Gaussian arm (k is consumed un-pooled)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the contexts the last timed step returned as DIR/ctx_chunk<c>.npy (float32 [videos,Q,D]"
+                         "; a fixed seeded sample of the videos when all would exceed 64 MB), for comparing two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference_impl(args)
