@@ -49,7 +49,8 @@ struct GemmDev {
   long long c_group_stride, bias_stride;
   int ab_half;                              // operands are fp16 (kind::f16, 64 K-elements per 128-byte row)
   int round_tf32;                           // round stored row-major results to the tf32 grid
-  int c_vec;                                // row-major stores may be 128-bit (alignment checked on the host)
+  int c_vec;                                // row-major fp32 stores may be 128-bit (alignment checked on the host)
+  int c_vec8;                               // fp16 stores may be 128-bit: 8 halves (alignment checked on the host)
   int a_group;                              // two-level row mapping of A (0 = off): tile rows span 128 / a_group groups
   int c_half;                               // C is fp16 storage (row-major path only)
   void* C_lo;                               // fp16 output only: second array for the residual x - float(half(x))
@@ -216,7 +217,7 @@ __device__ __forceinline__ void epilogue_tile(const GemmDev& g, uint32_t tmem_ac
       // fp16 rows: lane -> (row 8 i + lane / 4, columns 8 (lane % 4) .. + 7): two staged 16-byte chunks -> one 16-byte
       // store of 8 halves (rows of 64 B per warp-wide store)
       const int col8 = n0 + c0 + 8 * lchunk;
-      const bool vec8 = g.c_vec && (g.ldc % 8 == 0) && (col8 + 7 < g.Nc);
+      const bool vec8 = g.c_vec8 && (col8 + 7 < g.Nc);
       float bb[8];
 #pragma unroll
       for (int t = 0; t < 8; ++t) bb[t] = (bias != nullptr && col8 + t < g.Nc) ? __ldg(bias + col8 + t) : 0.f;
@@ -1039,6 +1040,10 @@ static int gemm_tcgen05_launch(const ltm_gemm_args& a, cudaStream_t stream) {
   d.ab_half = half;
   d.c_vec = (a.ldc % 4 == 0 && a.strideC % 4 == 0 && a.c_group_stride % 4 == 0 && aligned16(a.C) &&
              (a.CT == nullptr || a.ct_cols % 4 == 0)) ? 1 : 0;
+  // fp16 output: a 16-byte store holds 8 halves, so every term of its address (row pitch, batch stride, group stride,
+  // the base of C and of C_lo) must be a multiple of 8 halves; otherwise the epilogue stores halves one by one
+  d.c_vec8 = (a.c_fp16 && a.ldc % 8 == 0 && a.strideC % 8 == 0 && a.c_group_stride % 8 == 0 && aligned16(a.C) &&
+              (a.C_lo == nullptr || aligned16(a.C_lo))) ? 1 : 0;
   d.a_group = a.a_group;
   d.c_half = a.c_fp16 ? 1 : 0;
   d.C_lo = a.c_fp16 ? a.C_lo : nullptr;
