@@ -58,6 +58,14 @@ int ltm_pool_bins(const float* k, float* xbin, const int32_t* fbin_ptr, int Bv, 
 int ltm_pool_mean_16(const void* k, int is_bf16, float* xpart, int Bv, int L, int T, int e, int splits,
                      void* stream);
 
+/* ---- frame pooling of a ragged batch: k[Bv, L, T, e] is padded, video v uses its first lengths[v] frames
+ * (0 = none), given as offs[Bv+1] = the exclusive prefix sum of the lengths (frames = offs[Bv]).
+ * xpart[frames, splits, e] receives the pooled frames packed in video order, each bit-identical to ltm_pool_mean with
+ * the same splits.  Only the frames listed are read.  max_ctas > 0 bounds the grid (persistent CTAs).
+ * dtype: 0 fp32, 1 fp16, 2 bfloat16 (16-bit: e % 8 == 0, ltm_pool_mean_16's summation). */
+int ltm_pool_mean_ragged(const void* k, int dtype, float* xpart, const int32_t* offs, int Bv, int L, int T, int e,
+                         int splits, int frames, int max_ctas, void* stream);
+
 /* ---- R6: sticky histogram of the previous call's density.  gibbs:196-203 (+score :224-230,
  * compute_probability :232-249).  scores[Bv,H,Q,N] -> hist_part[Bv,H,127] (sum over q; the sum
  * over heads happens in ltm_resample).  Normally fused into ltm_cont_attn_rect. */
@@ -352,6 +360,22 @@ typedef struct {
   /* grid bound of the K/V projection GEMM (ltm_gemm_args.max_ctas; 0 = one CTA per SM): set when the next chunk's
    * pooling runs beside this step */
   int gemm_ctas;
+  /* ragged batch (lengths != NULL): video v uses the first lengths[v] frames of its padded chunk k[v, L*T, e]
+   * (lengths[v] == 0: the video is idle this call).  frame_offs[Bv+1] is the exclusive prefix sum of lengths and
+   * `frames` its total; `xpart` holds the pooled frames packed in that order, [frames, splits, e].  The tables of a
+   * video are selected from the bank by its length: bank_seg_ptr0/1 [L+1, N+1] (absolute offsets into the
+   * concatenated bank_seg_mem0/1), bank_g0/1 [L+1, N] (infinite_video_b200/tables.py RectBank).  `jf` must be the
+   * smallest jf among the lengths of the videos that update.  new_doc flags apply to the videos that are present.
+   * An idle video keeps its state bit for bit: its coefficient rows (zeros when B_past == NULL), K|V rows (when
+   * KV_past is set; otherwise they are projected from the kept coefficients) and sticky histogram partials (saved in
+   * hist_keep[Bv, H*ceil(Q/32), 127] during the call) carry over, its re-sampling is skipped (its row of u is not
+   * read), and its ctx rows are zero.  n_idle: number of idle videos.  u may be NULL
+   * when no video continues its memory.  Frame pooling per
+   * bin (binned) does not apply.  lengths == NULL: lock-step, every field below is ignored. */
+  const int32_t* lengths; const int32_t* frame_offs; int frames; int n_idle;
+  const int32_t *bank_seg_ptr0, *bank_seg_mem0; const float* bank_g0;
+  const int32_t *bank_seg_ptr1, *bank_seg_mem1; const float* bank_g1;
+  float* hist_keep;
 } ltm_rect_step_args;
 int ltm_rect_step(const ltm_rect_step_args* a, const float* k, const float* q, const double* u,
                   const uint8_t* new_doc, float* ctx, void* stream);
@@ -372,6 +396,9 @@ typedef struct {
   void *ev_fork_pool, *ev_pooled_cur, *ev_pooled_next, *ev_fork, *ev_join;
   const float* k_next; float* xpart_next; int pool_ctas;
   int next_binned;     /* pool k_next with ltm_pool_bins (the call that consumes it must set args.binned) */
+  /* ragged next chunk (next_lengths != NULL): pool the first next_lengths[v] frames of each video of k_next (padded
+   * to args.L frames) into xpart_next packed as [next_frames, next_splits, e] (ltm_pool_mean_ragged) */
+  const int32_t* next_lengths; const int32_t* next_offs; int next_frames; int next_splits;
 } ltm_overlap;
 int ltm_rect_step_overlap(const ltm_rect_step_args* a, const ltm_overlap* o, const float* q, const double* u,
                           const uint8_t* new_doc, float* ctx);

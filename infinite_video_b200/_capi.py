@@ -59,6 +59,10 @@ class RectStepArgs(C.Structure):
         ("binned", C.c_int), ("xb_rows", C.c_int),
         ("fbin_ptr", C.c_void_p), ("seg_ptr1b", C.c_void_p), ("seg_mem1b", C.c_void_p),
         ("gemm_ctas", C.c_int),
+        ("lengths", C.c_void_p), ("frame_offs", C.c_void_p), ("frames", C.c_int), ("n_idle", C.c_int),
+        ("bank_seg_ptr0", C.c_void_p), ("bank_seg_mem0", C.c_void_p), ("bank_g0", C.c_void_p),
+        ("bank_seg_ptr1", C.c_void_p), ("bank_seg_mem1", C.c_void_p), ("bank_g1", C.c_void_p),
+        ("hist_keep", C.c_void_p),
     ]
 
 
@@ -69,6 +73,7 @@ class Overlap(C.Structure):
         ("ev_fork", C.c_void_p), ("ev_join", C.c_void_p),
         ("k_next", C.c_void_p), ("xpart_next", C.c_void_p), ("pool_ctas", C.c_int),
         ("next_binned", C.c_int),
+        ("next_lengths", C.c_void_p), ("next_offs", C.c_void_p), ("next_frames", C.c_int), ("next_splits", C.c_int),
     ]
 
 
@@ -85,6 +90,7 @@ _SIGS = {
     "ltm_pool_bins": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "ltm_pool_mean_16": (C.c_int, [_P, _I, _P, _I, _I, _I, _I, _I, _P]),
     "ltm_pool_mean_grid": (C.c_int, [_P, _P, _I, _I, _I, _I, _I, _I, _P]),
+    "ltm_pool_mean_ragged": (C.c_int, [_P, _I, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "ltm_sticky_hist_rect": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "ltm_sticky_hist_rect_tiles": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "ltm_density_rect": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),

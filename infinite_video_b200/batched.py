@@ -14,6 +14,7 @@ import functools
 import math
 import weakref
 
+import numpy as np
 import torch
 
 from . import ops, tables
@@ -46,6 +47,27 @@ def _as_flags(new_doc, Bv, device):
         raise ValueError("new_doc must be a bool or one flag per video")
     t = t.to(device=device, dtype=torch.uint8).contiguous()
     return None, t
+
+
+def _as_lengths(lengths, Bv, Lmax):
+    """Per-video chunk lengths of a ragged step -> int tuple; 0 (idle) or within [2, Lmax].  Host values only: the
+    tables are selected from them on the host, and reading a CUDA tensor would be a hidden synchronisation."""
+    if isinstance(lengths, torch.Tensor):
+        if lengths.device.type != "cpu":
+            raise ValueError("lengths must be host integers (a list or a CPU tensor), not a CUDA tensor")
+        if lengths.is_floating_point() or lengths.is_complex():
+            raise ValueError("lengths must be integers")
+        lengths = lengths.reshape(-1).tolist()
+    vals = tuple(int(x) for x in lengths)
+    if any(float(x) != float(y) for x, y in zip(vals, lengths)):
+        raise ValueError("lengths must be integers")
+    if len(vals) != Bv:
+        raise ValueError(f"lengths must hold one value per video ({Bv}), got {len(vals)}")
+    for x in vals:
+        if x != 0 and not 2 <= x <= Lmax:
+            raise ValueError(f"chunk length {x} is outside [2, {Lmax}] (0 = idle; chunks of one frame are not "
+                             "supported)")
+    return vals
 
 
 def _pad_rows(m):
@@ -165,6 +187,9 @@ class BatchedRectLTM(_BatchedBase):
         self._B = None
         self._cur = 0
         self.last = {}
+        self._slots = None            # per-slot memory after ragged steps (bool [Bv]); None: every slot has_state
+        self._banks = {}              # Lmax -> tables.RectBank
+        self._last_ragged = False
 
     # ------------------------------------------------------------------ buffers
     def _workspace(self, Bv, L, Q):
@@ -226,6 +251,7 @@ class BatchedRectLTM(_BatchedBase):
     def reset(self):
         """Forget every video (new_doc for all) and every pending prefetch."""
         super().reset()
+        self._slots = None
         self._pref.clear()
 
     def cancel_prefetch(self):
@@ -235,9 +261,9 @@ class BatchedRectLTM(_BatchedBase):
     # pending prefetches are identified by the tensor OBJECT (weak reference) and its version counter: a data pointer
     # is not a key, the caching allocator hands the same address to the next chunk (and an in-place write changes
     # the contents behind an unchanged pointer)
-    def _pref_take(self, k):
+    def _pref_take(self, k, lens=None):
         for i, ent in enumerate(self._pref):
-            if ent["ref"]() is k and ent["ver"] == k._version:
+            if ent["ref"]() is k and ent["ver"] == k._version and ent["lens"] == lens:
                 return self._pref.pop(i)
         return None
 
@@ -260,13 +286,14 @@ class BatchedRectLTM(_BatchedBase):
             self._cur = 0
             self.Bv = Bv
             self.has_state = False
+            self._slots = None
 
     @property
     def B_past(self):
         return self._B[self._cur] if (self._B is not None and self.has_state) else None
 
     # ------------------------------------------------------------------ one chunk
-    def _args(self, Bv, L, Q, ws, tab, tdev, beside_pool=False):
+    def _args(self, Bv, L, Q, ws, tab, tdev, beside_pool=False, rag=None):
         # the argument block is built once per workspace / table set / weights and only its per-call fields are
         # rewritten afterwards (the ~40 ctypes assignments were a third of the host time of a chunk)
         sig = (id(tdev), self.Wkv.data_ptr(), self.bkv.data_ptr(), self._hist.data_ptr(), self.sticky,
@@ -289,6 +316,17 @@ class BatchedRectLTM(_BatchedBase):
         if ws["KVs"] is not None and len(ws["KVs"]) == 2:      # K|V ping-pong, in phase with the coefficient buffers
             a.KV = ws["KVs"][1 - self._cur].data_ptr()
             a.KV_past = ws["KVs"][self._cur].data_ptr() if (self.has_state and ws.get("kv_valid")) else None
+        if rag is None:
+            a.lengths, a.frame_offs, a.n_idle, a.jf = None, None, 0, tab.jf
+        else:
+            lt, bank = rag["dev"], rag["bank"]
+            a.lengths, a.frame_offs = lt.data_ptr(), lt.data_ptr() + 4 * Bv
+            a.frames, a.n_idle, a.jf, a.splits, a.binned = rag["frames"], rag["n_idle"], rag["jf"], rag["splits"], 0
+            a.bank_seg_ptr0, a.bank_seg_mem0, a.bank_g0 = (bank["seg_ptr0"].data_ptr(), bank["seg_mem0"].data_ptr(),
+                                                           bank["g0"].data_ptr())
+            a.bank_seg_ptr1, a.bank_seg_mem1, a.bank_g1 = (bank["seg_ptr1"].data_ptr(), bank["seg_mem1"].data_ptr(),
+                                                           bank["g1"].data_ptr())
+            a.hist_keep = rag["hist_keep"].data_ptr() if rag["hist_keep"] is not None else None
         if self.prof_events is not None:
             for i, ev in enumerate(self.prof_events):
                 a.prof_events[i] = ev
@@ -358,6 +396,10 @@ class BatchedRectLTM(_BatchedBase):
             # the sticky histogram of the previous call is kept per (head, tile of 32 queries): a different number
             # of query tiles inside a video would silently restart the memory
             raise ValueError(f"the number of queries changed inside a video ({Q} now): pass new_doc=True or keep Q")
+        if self._slots is not None and self.has_state and not all_new and self.Bv == Bv and not self._slots.all():
+            # (only after a ragged step left slots without memory)
+            nd = torch.as_tensor(new_doc).reshape(-1).to("cpu", torch.bool).numpy() if all_new is None else False
+            self._no_memory_check(~np.asarray(nd, bool) & ~self._slots)
         self._state(Bv, Q)
         if all_new:
             self.has_state = False
@@ -366,7 +408,88 @@ class BatchedRectLTM(_BatchedBase):
         tab = tables.rect_tables(L, self.N, self.tau, self.S, spacing=self.spacing)
         return Bv, L, Q, tab, tab.to(self.device), flags
 
-    def _finish(self, ws, xp=None, k=None):
+    def _no_memory_check(self, bad):
+        if np.any(bad):
+            raise ValueError(f"video slot(s) {np.flatnonzero(bad).tolist()} hold no memory and receive a chunk without "
+                             "new_doc: pass new_doc for their first chunk")
+
+    def _bank(self, L):
+        bank = self._banks.get(L)
+        if bank is None:
+            bank = self._banks[L] = tables.RectBank(L, self.N, self.tau, self.S, spacing=self.spacing)
+        return bank
+
+    def _lengths_dev(self, lens):
+        """[lengths (Bv) | exclusive prefix sum (Bv+1)] as one int32 device tensor, copied on the current stream."""
+        Bv = len(lens)
+        host = np.zeros(2 * Bv + 1, np.int32)
+        host[:Bv] = lens
+        np.cumsum(host[:Bv], out=host[Bv + 1:])
+        return torch.from_numpy(host).pin_memory().to(self.device, non_blocking=True)
+
+    def _ragged_ws(self, ws, Bv, L):
+        """Packed pooled frames of a ragged step take sum(lengths) * splits rows: at most Bv * L (one split) or, when
+        the frames alone do not fill the GPU, fewer than twice the `_splits` target.  Grows the frame buffers of a
+        workspace once to hold either (pending prefetches into the old buffers are dropped)."""
+        need = max(Bv * L, 2 * 4 * 8 * self.sm_count) * self.e
+        if ws["xbufs"][0].numel() >= need:
+            return
+        if self._side is not None:
+            for b in ws["xbufs"]:
+                b.record_stream(self._side)
+        self._pref.clear()
+        splits = ws["splits"]
+        ws["xbufs"] = [torch.empty(need, device=self.device, dtype=torch.float32) for _ in range(2)]
+        ws["xparts"] = [b[:Bv * L * splits * self.e].view(Bv, L, splits, self.e) for b in ws["xbufs"]]
+        ws["xtag"] = [False, False]
+
+    def _prepare_ragged(self, kshape, qshape, new_doc, lengths):
+        """Host side of a ragged step: validation, per-slot bookkeeping, table bank, device lengths / offsets."""
+        Bv, LT, e = kshape
+        if e != self.e:
+            raise ValueError(f"k has width {e}, projections expect {self.e}")
+        if LT % self.T or LT // self.T < 2:
+            raise ValueError(f"k has {LT} tokens: a ragged chunk is padded to L*{self.T} tokens, L >= 2")
+        L, Q = LT // self.T, qshape[1]
+        if qshape[0] != Bv or qshape[2] != self.D:
+            raise ValueError(f"q must be [{Bv}, Q, {self.D}]")
+        ln = np.asarray(_as_lengths(lengths, Bv, L), np.int64)
+        if isinstance(new_doc, (bool, int)):
+            nd = np.full(Bv, bool(new_doc))
+        else:
+            t = torch.as_tensor(new_doc)
+            if t.device.type != "cpu" or t.numel() != Bv:
+                raise ValueError("a ragged step takes new_doc as a bool or one host flag per video")
+            nd = t.reshape(-1).to(torch.bool).numpy()
+        present = ln > 0
+        same = self._B is not None and self.Bv == Bv and self.has_state
+        mem = (self._slots if self._slots is not None else np.full(Bv, self.has_state)) if same else np.zeros(Bv, bool)
+        if same and self._hist.shape[1] != self.H * ((Q + 31) // 32) and (mem & ~nd).any():
+            raise ValueError(f"the number of queries changed inside a video ({Q} now): pass new_doc=True or keep Q")
+        cont = present & ~nd
+        self._no_memory_check(cont & ~mem)
+        self._state(Bv, Q)
+        first = present & nd
+        flags = None
+        if self.has_state and first.any():
+            flags = torch.from_numpy(first.astype(np.uint8)).pin_memory().to(self.device, non_blocking=True)
+        bank = self._bank(L)
+        bdev = bank.to(self.device, set(ln.tolist()))
+        frames, n_idle = int(ln.sum()), int((~present).sum())
+        hist_keep = None
+        if n_idle and self.sticky:
+            if getattr(self, "_hist_keep", None) is None or self._hist_keep.shape != self._hist.shape:
+                self._hist_keep = torch.empty_like(self._hist)
+            hist_keep = self._hist_keep
+        tab = tables.rect_tables(L, self.N, self.tau, self.S, spacing=self.spacing)   # (its L-independent tables)
+        rag = dict(lens=tuple(ln.tolist()), dev=self._lengths_dev(ln), bank=bdev, frames=frames,
+                   splits=self._splits(frames) if frames else 1, n_idle=n_idle,
+                   jf=int(bank.jf[ln[cont]].min()) if (self.has_state and cont.any()) else self.N,
+                   need_u=bool(self.has_state and self.sticky and cont.any()), hist_keep=hist_keep,
+                   slots=np.where(nd, present, mem))
+        return Bv, L, Q, tab, tab.to(self.device), flags, rag
+
+    def _finish(self, ws, xp=None, k=None, rag=None):
         # pooled frames of this call (for `x_past`); a call that pooled per bin keeps a weak reference to the chunk
         # instead and pools it again on demand
         binned = xp is None and ws["xtag"][ws["xi"]]
@@ -375,6 +498,13 @@ class BatchedRectLTM(_BatchedBase):
         self._last_updated = self.has_state          # False: the call just made was a first chunk
         self._cur = 1 - self._cur
         self.has_state = True
+        self._last_ragged = rag is not None
+        if rag is not None:
+            self._last_xpart = self._last_k = None
+            self._slots = rag["slots"]
+            self.has_state = bool(rag["slots"].any())
+        else:
+            self._slots = None
         self._last_L = ws["xparts"][0].shape[1]
         kv = None
         if ws["KVs"] is not None:
@@ -384,10 +514,11 @@ class BatchedRectLTM(_BatchedBase):
         self.last = dict(b=ws["b_draw"], ts=ws["ts"], idx=ws["idx"], p=ws["p"], scores=ws["scores"], V=V, KV=kv)
 
     @_on_device
-    def prefetch(self, k_next, Q, events=None, update=False):
+    def prefetch(self, k_next, Q, lengths=None, events=None, update=False):
         """Pool the frames of the NEXT chunk now, on a side stream, into the alternate buffer.
         `update=True`: the chunk will continue every video (no new_doc), so it may be pooled per bin (`bin_pool`); a
-        step that turns out to start a new document pools it again.
+        step that turns out to start a new document pools it again.  `lengths`: the chunk is ragged (see `step`); the
+        step that consumes it must pass the same lengths, or it is pooled again.
 
         Frame pooling (gibbs:304) does not depend on the memory state, and it is the HBM-bound 93 % of a
         call's bytes, while regression / projection / attention of the current chunk are compute-bound; issuing
@@ -398,6 +529,11 @@ class BatchedRectLTM(_BatchedBase):
         Bv, LT, e = k_next.shape
         L = LT // self.T
         ws = self._workspace(Bv, L, Q)
+        lens = lt = None
+        if lengths is not None:
+            lens = _as_lengths(lengths, Bv, L)
+            self._ragged_ws(ws, Bv, L)
+            lt = self._lengths_dev(lens)
         if self._side is None:
             # pooling runs at the lowest priority, the compute-bound kernels of `step` on a high-priority stream:
             # the block scheduler then places regression / projection / attention CTAs as soon as resources free
@@ -420,8 +556,14 @@ class BatchedRectLTM(_BatchedBase):
         if events is not None:
             check(lib().ltm_event_record(events[0], sp), "event_record")
         tab = tables.rect_tables(L, self.N, self.tau, self.S, spacing=self.spacing)
-        binned = bool(update) and self._bin_ok(Bv, L, tab)
-        if binned:
+        binned = lens is None and bool(update) and self._bin_ok(Bv, L, tab)
+        if lens is not None:
+            frames = sum(lens)
+            lt.record_stream(self._side)
+            check(lib().ltm_pool_mean_ragged(ptr(k_next), 0, ptr(ws["xbufs"][b]), C.c_void_p(lt.data_ptr() + 4 * Bv),
+                                             Bv, L, self.T, self.e, self._splits(frames) if frames else 1, frames,
+                                             int(self.pool_ctas), sp), "pool_mean_ragged")
+        elif binned:
             check(lib().ltm_pool_bins(ptr(k_next), ptr(ws["xbufs"][b]), ptr(tab.to(self.device)["fbin_ptr"]), Bv, L,
                                       self.T, self.e, tab.xb_rows, sp), "pool_bins")
         else:
@@ -431,7 +573,7 @@ class BatchedRectLTM(_BatchedBase):
             check(lib().ltm_event_record(events[1], sp), "event_record")
         check(lib().ltm_event_record(ev["pooled"][b], sp), "event_record")
         self._pref.append(dict(ref=weakref.ref(k_next), ver=k_next._version, buf=b, event=ev["pooled"][b],
-                               captured=torch.cuda.is_current_stream_capturing(), binned=binned))
+                               captured=torch.cuda.is_current_stream_capturing(), binned=binned, lens=lens))
 
     def _sync_events(self):
         if self._evs is None:
@@ -446,6 +588,9 @@ class BatchedRectLTM(_BatchedBase):
     def x_past(self):
         """[Bv, e, S+L] ([Bv, e, L] after a first chunk): what the reference keeps as `x_past` (gibbs:215,221) -- the
         re-sampled rows of the previous coefficients followed by the pooled frames of the most recent call."""
+        if self._last_ragged:
+            raise RuntimeError("x_past: the last call was a ragged step (per-video lengths); its pooled frames are not "
+                               "kept -- x_past is defined for lock-step calls only")
         xp = self._last_xpart
         if xp is None:                      # the last call pooled per bin: pool the chunk again, per frame
             k = self._last_k() if getattr(self, "_last_k", None) is not None else None
@@ -474,59 +619,97 @@ class BatchedRectLTM(_BatchedBase):
         return ops.density_rect(sc, td["jd"], td["wd"])
 
     @_on_device
-    def pool(self, k, with_half=False):
+    def pool(self, k, with_half=False, lengths=None):
         """Frame pooling alone (gibbs:304): k[Bv, L*T, e] -> pooled frames [Bv, L, splits, e].  The result can be
         handed to `step(..., pooled=...)` of SEVERAL engines: every LTM layer of a Q-former receives the same
         `encoder_hidden_states` per chunk (2 layers in Video-LLaMA, 6 in VideoChat2; SURVEY section 8f N2), so the
         25 MB/video chunk needs to be streamed from HBM once, not once per layer.
         `with_half=True` (fp32 chunks): the same pass also writes the chunk as float16 and returns
-        (pooled, k16[Bv, L*T, e]) -- the operand of the caller's short-term attention (SURVEY 8f N1)."""
+        (pooled, k16[Bv, L*T, e]) -- the operand of the caller's short-term attention (SURVEY 8f N1).
+        `lengths` (ragged chunk, see `step`): only the first lengths[v] frames of video v are pooled and read; the
+        result is packed video after video, [sum(lengths), splits, e] with splits = `_splits(sum(lengths))`, and is
+        handed to `step(..., pooled=..., lengths=...)` with the same lengths."""
         require_cuda(k)
         k = k.contiguous()
         Bv, LT, e = k.shape
         if e != self.e or LT % self.T:
             raise ValueError(f"k must be [Bv, L*{self.T}, {self.e}]")
         L = LT // self.T
+        if lengths is not None:
+            dtype = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}.get(k.dtype)
+            if with_half or dtype is None:
+                raise ValueError("a ragged chunk is pooled from float32 / float16 / bfloat16 storage, without with_half")
+            lens = _as_lengths(lengths, Bv, L)
+            frames = sum(lens)
+            splits = self._splits(frames) if frames else 1
+            out = torch.empty(frames, splits, e, device=self.device, dtype=torch.float32)
+            if frames:
+                lt = self._lengths_dev(lens)
+                check(lib().ltm_pool_mean_ragged(ptr(k), dtype, ptr(out), C.c_void_p(lt.data_ptr() + 4 * Bv), Bv, L,
+                                                 self.T, e, splits, frames, 0, stream_ptr(self.device)),
+                      "pool_mean_ragged")
+            return out
         if with_half:
             x, k16 = ops.pool_mean_convert(k.view(Bv, L, self.T, e), self._splits(Bv * L))
             return x, k16.view(Bv, LT, e)
         return ops.pool_mean(k.view(Bv, L, self.T, e), self._splits(Bv * L))
 
     @_on_device
-    def step(self, k, q, u=None, new_doc=False, pooled=None, beside_pooling=False):
+    def step(self, k, q, u=None, new_doc=False, pooled=None, beside_pooling=False, lengths=None):
         """k[Bv, L*T, e], q[Bv,Q,D] fp32 CUDA; u[Bv,S] fp64 uniforms (needed from the second chunk on when
         sticky); new_doc: bool or per-video flags; pooled: result of `pool(k)` (then `k` is only used for its
         shape); beside_pooling: the caller pools another chunk on a second stream while this step runs (the K/V
-        projection then keeps to part of the SMs, see `gemm_ctas_overlap`).  Returns ctx[Bv,Q,D]."""
+        projection then keeps to part of the SMs, see `gemm_ctas_overlap`).  Returns ctx[Bv,Q,D].
+
+        lengths (ragged batch): Bv host integers, each 0 or in [2, L].  Video v uses the first lengths[v] frames of
+        its padded chunk (the rest is never read and may hold anything); lengths[v] == 0 leaves video v idle: its
+        memory is kept bit for bit, its row of u is not read and its ctx rows are zero (with new_doc[v] the slot is
+        cleared instead).  new_doc is then a bool or host flags; a slot without memory must receive new_doc with its
+        first chunk.  Passing lengths always takes the ragged kernels, even when all lengths are equal."""
         require_cuda(k, q, u)
         if k.dtype in (torch.float16, torch.bfloat16) and pooled is None:
-            pooled = self.pool(k)                  # 16-bit chunk: pooled straight from its 16-bit storage
+            pooled = self.pool(k, lengths=lengths)  # 16-bit chunk: pooled straight from its 16-bit storage
         if (k.dtype != torch.float32 and pooled is None) or q.dtype != torch.float32:
             raise ValueError("k must be float32 / float16 / bfloat16 and q float32")
         k, q = k.contiguous(), q.contiguous()
-        Bv, L, Q, tab, tdev, flags = self._prepare(k.shape, q.shape, new_doc)
+        rag = None
+        if lengths is None:
+            Bv, L, Q, tab, tdev, flags = self._prepare(k.shape, q.shape, new_doc)
+            need_u = self.has_state and self.sticky
+        else:
+            Bv, L, Q, tab, tdev, flags, rag = self._prepare_ragged(k.shape, q.shape, new_doc, lengths)
+            need_u = rag["need_u"]
         ws = self._workspace(Bv, L, Q)
+        if rag is not None:
+            self._ragged_ws(ws, Bv, L)
         if pooled is not None:
-            if tuple(pooled.shape[:2]) != (Bv, L) or pooled.shape[3] != self.e or not pooled.is_contiguous():
+            if rag is None and (tuple(pooled.shape[:2]) != (Bv, L) or pooled.shape[3] != self.e):
                 raise ValueError("pooled frames do not match k")
-            if self.has_state and self.sticky:
+            if rag is not None and (pooled.dim() != 3 or pooled.shape[0] != rag["frames"] or pooled.shape[2] != self.e):
+                raise ValueError(f"pooled frames of a ragged chunk must be [{rag['frames']}, splits, {self.e}]")
+            if not pooled.is_contiguous():
+                raise ValueError("pooled frames do not match k")
+            if need_u:
                 if u is None or u.dtype != torch.float64 or tuple(u.shape) != (Bv, self.S):
                     raise ValueError(f"sticky re-sampling needs u: float64 [{Bv},{self.S}]")
                 u = u.contiguous()
             ctx = torch.empty(Bv, Q, self.D, device=self.device, dtype=torch.float32)
-            a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=bool(beside_pooling))
-            a.xpart, a.splits, a.binned = pooled.data_ptr(), pooled.shape[2], 0
-            check(lib().ltm_rect_step(C.byref(a), None, ptr(q), ptr(u), ptr(flags), ptr(ctx),
-                                      stream_ptr(self.device)), "rect_step")
-            self._finish(ws, pooled)
+            a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=bool(beside_pooling), rag=rag)
+            a.xpart, a.splits, a.binned = pooled.data_ptr(), pooled.shape[-2], 0
+            check(lib().ltm_rect_step(C.byref(a), None, ptr(q), ptr(u if rag is None or need_u else None),
+                                      ptr(flags), ptr(ctx), stream_ptr(self.device)), "rect_step")
+            self._finish(ws, pooled, rag=rag)
             return ctx
-        if self.has_state and self.sticky:
+        if need_u:
             if u is None or u.dtype != torch.float64 or tuple(u.shape) != (Bv, self.S):
                 raise ValueError(f"sticky re-sampling needs u: float64 [{Bv},{self.S}]")
             u = u.contiguous()
+        elif rag is not None:
+            u = None
         ctx = torch.empty(Bv, Q, self.D, device=self.device, dtype=torch.float32)
-        hit = self._pref_take(k)
-        update = self.has_state and flags is None       # every video continues: per-bin pooling is possible
+        hit = self._pref_take(k, None if rag is None else rag["lens"])
+        # every video continues: per-bin pooling is possible (lock-step only)
+        update = rag is None and self.has_state and flags is None
         if hit is not None and hit["binned"] and not update:
             hit = None                                   # pooled per bin for an update that did not come: pool again
         pooled = hit is not None
@@ -551,40 +734,56 @@ class BatchedRectLTM(_BatchedBase):
                 self._pref[:] = [e for e in self._pref if e["buf"] != ws["xi"]]
             ws["xtag"][ws["xi"]] = update and self._bin_ok(Bv, L, tab)
         # (a pending prefetch = the next chunk is being pooled on the side stream while this step runs)
-        a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=bool(self._pref) or bool(beside_pooling))
+        a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=bool(self._pref) or bool(beside_pooling), rag=rag)
+        if rag is not None and run is not main:
+            rag["dev"].record_stream(run)
         check(lib().ltm_rect_step(C.byref(a), None if pooled else ptr(k), ptr(q), ptr(u), ptr(flags), ptr(ctx),
                                   C.c_void_p(run.cuda_stream)), "rect_step")
         if pooled:
             check(lib().ltm_event_record(ev["join"], rp), "event_record")
             check(lib().ltm_stream_wait_event(mp, ev["join"]), "stream_wait_event")
-        self._finish(ws, k=k)
+        self._finish(ws, k=k, rag=rag)
         return ctx
 
     @_on_device
-    def step_overlapped(self, k, q, u=None, new_doc=False, k_next=None, next_new_doc=False):
+    def step_overlapped(self, k, q, u=None, new_doc=False, k_next=None, next_new_doc=False, lengths=None,
+                        next_lengths=None):
         """`step(k, ...)` with the frame pooling of `k_next` issued beside it, in ONE library call
         (`ltm_rect_step_overlap`: side stream pools the next chunk, a high-priority stream runs this chunk's
         regression / projection / attention, the current stream joins both).  `k` must be the tensor handed over as
         `k_next` by the previous call (or to `prefetch`); the first chunk of a stream is pooled here.  Same results as
         `step`, bit for bit.  `next_new_doc=True` says that `k_next` will start new documents (then it is pooled per
-        frame; a chunk expected to continue the videos may be pooled per bin, see `bin_pool`)."""
+        frame; a chunk expected to continue the videos may be pooled per bin, see `bin_pool`).
+        `lengths` / `next_lengths`: per-video lengths of `k` / `k_next` (ragged chunks, see `step`); `k` is matched
+        with its prefetch by lengths too."""
         require_cuda(k, q, u, k_next)
         if k.dtype != torch.float32 or q.dtype != torch.float32 or (k_next is not None and k_next.dtype != torch.float32):
             raise ValueError("step_overlapped takes float32 tensors")
         k, q = k.contiguous(), q.contiguous()
-        Bv, L, Q, tab, tdev, flags = self._prepare(k.shape, q.shape, new_doc)
+        rag = None
+        if lengths is None:
+            Bv, L, Q, tab, tdev, flags = self._prepare(k.shape, q.shape, new_doc)
+            need_u = self.has_state and self.sticky
+        else:
+            Bv, L, Q, tab, tdev, flags, rag = self._prepare_ragged(k.shape, q.shape, new_doc, lengths)
+            need_u = rag["need_u"]
         ws = self._workspace(Bv, L, Q)
-        if self.has_state and self.sticky:
+        if rag is not None or next_lengths is not None:
+            self._ragged_ws(ws, Bv, L)
+        if need_u:
             if u is None or u.dtype != torch.float64 or tuple(u.shape) != (Bv, self.S):
                 raise ValueError(f"sticky re-sampling needs u: float64 [{Bv},{self.S}]")
             u = u.contiguous()
-        hit = self._pref_take(k)
-        update = self.has_state and flags is None
+        elif rag is not None:
+            u = None
+        lens = None if rag is None else rag["lens"]
+        hit = self._pref_take(k, lens)
+        update = rag is None and self.has_state and flags is None
         if hit is not None and hit["binned"] and not update:
             hit = None                                   # pooled per bin for an update that did not come: pool again
         if hit is None:
-            self.prefetch(k, Q, update=update)
-            hit = self._pref_take(k)
+            self.prefetch(k, Q, lengths=lens, update=update)
+            hit = self._pref_take(k, lens)
         ev = self._sync_events()
         main = torch.cuda.current_stream(self.device)
         capturing = torch.cuda.is_current_stream_capturing()
@@ -599,17 +798,29 @@ class BatchedRectLTM(_BatchedBase):
             if not k_next.is_contiguous() or tuple(k_next.shape) != tuple(k.shape):
                 raise ValueError("k_next must be contiguous and have the shape of k")
             b = self._pref_buffer(ws)
-            nb = (not next_new_doc) and self._bin_ok(Bv, L, tab)
+            nl = None
+            if next_lengths is not None:
+                nl = _as_lengths(next_lengths, Bv, L)
+                nt = self._lengths_dev(nl)
+                nt.record_stream(self._side)
+                nf = sum(nl)
+                o.next_lengths, o.next_offs = nt.data_ptr(), nt.data_ptr() + 4 * Bv
+                o.next_frames, o.next_splits = nf, self._splits(nf) if nf else 1
+                nb = False
+            else:
+                nb = (not next_new_doc) and self._bin_ok(Bv, L, tab)
             o.k_next, o.xpart_next, o.next_binned = k_next.data_ptr(), ws["xbufs"][b].data_ptr(), int(nb)
             o.ev_fork_pool, o.ev_pooled_next = ev["fork_pool"][b], ev["pooled"][b]
             k_next.record_stream(self._side)
             self._pref.append(dict(ref=weakref.ref(k_next), ver=k_next._version, buf=b, event=ev["pooled"][b],
-                                   captured=capturing, binned=nb))
+                                   captured=capturing, binned=nb, lens=nl))
         ctx = torch.empty(Bv, Q, self.D, device=self.device, dtype=torch.float32)   # main joins the compute stream
-        a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=k_next is not None)
+        a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=k_next is not None, rag=rag)
+        if rag is not None:
+            rag["dev"].record_stream(self._compute)
         check(lib().ltm_rect_step_overlap(C.byref(a), C.byref(o), ptr(q), ptr(u), ptr(flags), ptr(ctx)),
               "rect_step_overlap")
-        self._finish(ws, k=k)
+        self._finish(ws, k=k, rag=rag)
         return ctx
 
     @_on_device

@@ -63,23 +63,46 @@ extern "C" int ltm_rect_step(const ltm_rect_step_args* a, const float* k, const 
     LTM_REQUIRE(B_past != nullptr && new_doc == nullptr, "rect_step: bin sums only exist for update calls of all videos");
     LTM_REQUIRE(a->xb_rows > 0 && a->fbin_ptr && a->seg_ptr1b && a->seg_mem1b, "rect_step: binned tables missing");
   }
+  // ragged batch: per-video lengths (0 = idle), tables from the bank, pooled frames packed by the frame offsets
+  const int32_t* lengths = a->lengths;
+  const bool ragged = lengths != nullptr;
+  const size_t hist_bytes = sizeof(float) * a->H * qtiles * (LTM_STICKY_EDGES - 2);
+  if (ragged) {
+    LTM_REQUIRE(!binned, "rect_step: per-bin pooling does not apply to ragged batches");
+    LTM_REQUIRE(a->frame_offs && a->bank_seg_ptr0 && a->bank_seg_mem0 && a->bank_g0 && a->bank_seg_ptr1 &&
+                a->bank_seg_mem1 && a->bank_g1, "rect_step: ragged batch without frame offsets / table bank");
+    LTM_REQUIRE(a->n_idle == 0 || !a->sticky || a->hist_keep, "rect_step: idle videos need hist_keep");
+    if (a->n_idle > 0 && a->sticky) {
+      rc = carry_idle(lengths, a->hist_part, a->hist_keep, hist_bytes, a->Bv, stream);
+      if (rc) return rc;
+    }
+  }
   if (k != nullptr) {          // k == NULL: a->xpart was already filled (frame pooling is stateless and may be
     LTM_PROF(0);               // issued ahead of time on another stream, see BatchedRectLTM.prefetch)
-    rc = binned ? ltm_pool_bins(k, a->xpart, a->fbin_ptr, a->Bv, a->L, a->T, a->e, a->xb_rows, stream)
-                : ltm_pool_mean(k, a->xpart, a->Bv, a->L, a->T, a->e, a->splits, stream);
+    rc = ragged ? ltm_pool_mean_ragged(k, 0, a->xpart, a->frame_offs, a->Bv, a->L, a->T, a->e, a->splits, a->frames, 0,
+                                       stream)
+         : binned ? ltm_pool_bins(k, a->xpart, a->fbin_ptr, a->Bv, a->L, a->T, a->e, a->xb_rows, stream)
+                  : ltm_pool_mean(k, a->xpart, a->Bv, a->L, a->T, a->e, a->splits, stream);
     if (rc) return rc;
     LTM_PROF(1);
   }
   const int xL = binned ? a->xb_rows : a->L, xsplits = binned ? 1 : a->splits;
-  const int32_t* seg_ptr1 = binned ? a->seg_ptr1b : a->seg_ptr1;
-  const int32_t* seg_mem1 = binned ? a->seg_mem1b : a->seg_mem1;
+  const int32_t* seg_ptr0 = ragged ? a->bank_seg_ptr0 : a->seg_ptr0;
+  const int32_t* seg_mem0 = ragged ? a->bank_seg_mem0 : a->seg_mem0;
+  const float* g0 = ragged ? a->bank_g0 : a->g0;
+  const int32_t* seg_ptr1 = ragged ? a->bank_seg_ptr1 : binned ? a->seg_ptr1b : a->seg_ptr1;
+  const int32_t* seg_mem1 = ragged ? a->bank_seg_mem1 : binned ? a->seg_mem1b : a->seg_mem1;
+  const float* g1 = ragged ? a->bank_g1 : a->g1;
   const int32_t* idx = a->idx_uniform;     // non-sticky: fixed table shared by all videos (index stride 0)
   long long idx_stride = 0;
-  if (B_past != nullptr && a->sticky) {
+  // (ragged: u == NULL when no video continues its memory in this call)
+  if (B_past != nullptr && a->sticky && !(ragged && u == nullptr)) {
     LTM_REQUIRE(u != nullptr, "rect_step: sticky re-sampling needs the uniform draws");
     LTM_PROF(2);
-    rc = ltm_resample(a->hist_part, a->H * qtiles, LTM_STICKY_EDGES - 2, 1, u, a->bins, a->bin2basis, 0, a->p,
-                      a->b_draw, nullptr, a->ts, a->idx, a->Bv, a->S, stream);
+    rc = ragged ? resample_ragged(a->hist_part, a->H * qtiles, LTM_STICKY_EDGES - 2, 1, u, a->bins, a->bin2basis, 0,
+                                  a->p, a->b_draw, nullptr, a->ts, a->idx, a->Bv, a->S, lengths, stream)
+                : ltm_resample(a->hist_part, a->H * qtiles, LTM_STICKY_EDGES - 2, 1, u, a->bins, a->bin2basis, 0, a->p,
+                               a->b_draw, nullptr, a->ts, a->idx, a->Bv, a->S, stream);
     if (rc) return rc;
     LTM_PROF(3);
     idx = a->idx;
@@ -125,10 +148,12 @@ extern "C" int ltm_rect_step(const ltm_rect_step_args* a, const float* k, const 
     const float* KVp = kvstate ? a->KV_past + kvo : nullptr;
     void* Bh = half_ops ? (void*)((uint16_t*)a->B_half + v0 * sB) : nullptr;
     if (!blocked) LTM_PROF(4);
-    rc = ltm_consolidate_rect_kv(Bp, a->xpart + v0 * sX, idx_stride ? idx + (size_t)v0 * idx_stride : idx, idx_stride,
-                                 new_doc ? new_doc + v0 : nullptr, a->seg_ptr0, a->seg_mem0, a->g0, seg_ptr1,
-                                 seg_mem1, a->g1, Bn, Bh, KVp, KVn, a->bkv, 2 * D, jg, kvh ? 2 : (tcp ? 1 : 0), nv, a->N,
-                                 a->e, xL, xsplits, a->S, stream);
+    // (ragged: the packed frames are addressed through the absolute frame offsets of the block's videos)
+    rc = consolidate_rect_ragged(Bp, ragged ? a->xpart : a->xpart + v0 * sX,
+                                 idx_stride ? idx + (size_t)v0 * idx_stride : idx, idx_stride,
+                                 new_doc ? new_doc + v0 : nullptr, seg_ptr0, seg_mem0, g0, seg_ptr1, seg_mem1, g1, Bn,
+                                 Bh, KVp, KVn, a->bkv, 2 * D, jg, kvh ? 2 : (tcp ? 1 : 0), nv, a->N, a->e, xL, xsplits,
+                                 a->S, ragged ? lengths + v0 : nullptr, ragged ? a->frame_offs + v0 : nullptr, stream);
     if (rc) return rc;
     if (!blocked) { LTM_PROF(5); LTM_PROF(6); }
     if (kvstate) {
@@ -213,6 +238,15 @@ extern "C" int ltm_rect_step(const ltm_rect_step_args* a, const float* k, const 
   }
   if (blocked) LTM_PROF(9);
 #undef LTM_PROF
+  if (ragged && a->n_idle > 0) {
+    // idle videos: the consolidation copied their coefficients into B_new, and the projection and attention ran over
+    // them; what those overwrote goes back to what it was -- the carried K|V into the buffer of the next call, the saved
+    // histogram partials -- and their context rows are zero.  (Without KV_past the K|V rows just projected from the
+    // kept coefficients stay.)
+    if (a->KV_past && a->KV) rc = carry_idle(lengths, a->KV_past, a->KV, (kvh ? 2 : 4) * sKV, a->Bv, stream);
+    if (!rc && a->sticky) rc = carry_idle(lengths, a->hist_keep, a->hist_part, hist_bytes, a->Bv, stream);
+    if (!rc) rc = carry_idle(lengths, nullptr, ctx, sizeof(float) * a->Q * D, a->Bv, stream);
+  }
   return rc;
 }
 
@@ -275,7 +309,11 @@ extern "C" int ltm_rect_step_overlap(const ltm_rect_step_args* a, const ltm_over
     LTM_CUDA(cudaStreamWaitEvent(ss, (cudaEvent_t)o->ev_fork_pool, 0));
     LTM_OV_MARK(0);
     if (a->prof_events[0]) cudaEventRecord((cudaEvent_t)a->prof_events[0], ss);
-    int rc = o->next_binned
+    LTM_REQUIRE(!o->next_lengths || (o->next_offs && !o->next_binned), "rect_step_overlap: ragged next chunk");
+    int rc = o->next_lengths
+                 ? ltm_pool_mean_ragged(o->k_next, 0, o->xpart_next, o->next_offs, a->Bv, a->L, a->T, a->e,
+                                        o->next_splits, o->next_frames, o->pool_ctas, ss)
+             : o->next_binned
                  ? ltm_pool_bins(o->k_next, o->xpart_next, a->fbin_ptr, a->Bv, a->L, a->T, a->e, a->xb_rows, ss)
                  : ltm_pool_mean_grid(o->k_next, o->xpart_next, a->Bv, a->L, a->T, a->e, a->splits, o->pool_ctas, ss);
     if (rc) return rc;

@@ -39,6 +39,21 @@ void set_error(const char* fmt, ...);
 
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
+// ---- ragged batches (ltm_rect_step_args.lengths), internal to the library
+// ltm_consolidate_rect_kv with per-video lengths (0 = idle) and frame offsets; NULL lengths = lock-step
+int consolidate_rect_ragged(const float* B_past, const float* xpart, const int32_t* idx, int64_t idx_stride,
+                            const uint8_t* new_doc, const int32_t* seg_ptr0, const int32_t* seg_mem0, const float* g0,
+                            const int32_t* seg_ptr1, const int32_t* seg_mem1, const float* g1, float* B_new,
+                            void* B_half, const float* KV_past, float* KV_new, const float* bkv, int ldkv, int jf,
+                            int round_tf32, int Bv, int N, int e, int L, int splits, int S, const int32_t* lengths,
+                            const int32_t* offs, void* stream);
+// dst[v] = src[v] (src NULL: zeros) over bytes_per_video for the videos with lengths[v] == 0
+int carry_idle(const int32_t* lengths, const void* src, void* dst, size_t bytes_per_video, int Bv, void* stream);
+// ltm_resample that skips (reads no uniforms of, writes nothing for) the videos with lengths[v] == 0
+int resample_ragged(const float* hist_part, int parts, int ncat, int normalize, const double* u, const float* bins,
+                    const int32_t* bin2basis, int sort, float* p_out, int32_t* b_draw, int32_t* b_used, float* ts,
+                    int32_t* idx, int Bv, int S, const int32_t* lengths, void* stream);
+
 // The dynamic-shared-memory opt-in of a kernel and the SM count are properties of a DEVICE, so their one-time setup
 // is cached per device ordinal (a process may drive several GPUs: a Q-former sharded with device_map).
 constexpr int LTM_MAX_DEVICES = 64;

@@ -27,7 +27,16 @@ __device__ __forceinline__ float tf32_round(float x) {
   return __uint_as_float(r);
 }
 
-template <int ROWS>
+// Ragged batch (RAGGED kernels only): video v has lengths[v] frames, packed from frame offs[v] in xpart; its tables are
+// entry lengths[v] of the table bank (seg_ptr0/1 [L+1, N+1] with absolute member offsets, g0/1 [L+1, N]).  An idle
+// video (lengths[v] == 0) keeps its coefficients: B_past is copied to B_new (zeros for a slot that holds no memory,
+// B_past == NULL) together with the fp16 copy, so that every later kernel of the call sees defined operands for it.
+struct Ragged {
+  const int32_t* lengths;
+  const int32_t* offs;
+};
+
+template <int ROWS, bool RAGGED>
 __global__ void __launch_bounds__(256)
 consolidate_rect_kernel(const float4* __restrict__ B_past, const float4* __restrict__ xpart,
                         const int32_t* __restrict__ idx, const long long idx_stride,
@@ -37,8 +46,32 @@ consolidate_rect_kernel(const float4* __restrict__ B_past, const float4* __restr
                         const int32_t* __restrict__ seg_ptr1, const int32_t* __restrict__ seg_mem1,
                         const float* __restrict__ g1,
                         float4* __restrict__ B_new, uint2* __restrict__ B_half, const KvState kv, int N, int e4, int L,
-                        int splits, int S) {
+                        int splits, int S, const Ragged rg) {
   const int v = blockIdx.y;
+  long long xrow = (long long)v * L;          // first pooled frame of this video in xpart
+  if (RAGGED) {
+    const int Lv = rg.lengths[v];
+    if (Lv == 0) {
+#pragma unroll 1
+      for (int jr = 0; jr < ROWS; ++jr) {
+        const int j = blockIdx.x * ROWS + jr;
+        if (j >= N) break;
+        for (int c = threadIdx.x; c < e4; c += blockDim.x) {
+          const size_t o = ((size_t)v * N + j) * e4 + c;
+          const float4 b = B_past != nullptr ? B_past[o] : make_float4(0.f, 0.f, 0.f, 0.f);
+          B_new[o] = b;
+          if (B_half != nullptr) {
+            const __half2 lo = __floats2half2_rn(b.x, b.y), hi = __floats2half2_rn(b.z, b.w);
+            B_half[o] = make_uint2(*reinterpret_cast<const uint32_t*>(&lo), *reinterpret_cast<const uint32_t*>(&hi));
+          }
+        }
+      }
+      return;
+    }
+    xrow = rg.offs[v];
+    seg_ptr0 += (size_t)Lv * (N + 1); g0 += (size_t)Lv * N;
+    seg_ptr1 += (size_t)Lv * (N + 1); g1 += (size_t)Lv * N;
+  }
   // ROWS coefficient rows per CTA (1: the loop folds away and the kernel is the one-row kernel, 32 registers)
 #pragma unroll 1
   for (int jr = 0; jr < ROWS; ++jr) {
@@ -50,7 +83,7 @@ consolidate_rect_kernel(const float4* __restrict__ B_past, const float4* __restr
   const float g = first ? g0[j] : g1[j];
   const int m0 = seg_ptr[j], m1 = seg_ptr[j + 1];
   const int frame_base = first ? 0 : S;       // member ids >= frame_base are frames
-  const float4* xv = xpart + (size_t)v * L * splits * e4;
+  const float4* xv = xpart + (size_t)xrow * splits * e4;
   const float4* bv = first ? nullptr : B_past + (size_t)v * N * e4;
   const int32_t* iv = first ? nullptr : idx + (size_t)v * idx_stride;
   for (int c = threadIdx.x; c < e4; c += blockDim.x) {
@@ -192,6 +225,37 @@ fold_sample_columns_kernel(const float* __restrict__ GT, long long ldg, const in
   }
 }
 
+// Idle videos of a ragged batch: dst[v] = src[v] (zero when src == NULL) for every v with lengths[v] == 0, as n words
+// of type W per video.  Keeps what an idle video owns -- coefficient rows, K|V rows, sticky histogram partials -- bit
+// for bit across a call whose kernels run over every video, and zeroes its ctx rows.
+template <class W>
+__global__ void __launch_bounds__(256)
+carry_idle_kernel(const int32_t* __restrict__ lengths, const W* __restrict__ src, W* __restrict__ dst, long long n) {
+  const int v = blockIdx.y;
+  if (lengths[v] != 0) return;
+  const W* s = src ? src + (size_t)v * n : nullptr;
+  W* d = dst + (size_t)v * n;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+    d[i] = s ? s[i] : W{};
+}
+
+int carry_idle(const int32_t* lengths, const void* src, void* dst, size_t bytes_per_video, int Bv, void* stream) {
+  LTM_REQUIRE(lengths && dst && bytes_per_video % 4 == 0 && Bv <= 65535, "carry_idle: bad arguments");
+  // 16-byte words where every video's slice is 16-byte aligned, else 4-byte words
+  const bool wide = bytes_per_video % 16 == 0 && aligned16(src) && aligned16(dst);
+  const long long n = (long long)(bytes_per_video / (wide ? 16 : 4));
+  const int blocks = (int)((n + 255) / 256 < 64 ? (n + 255) / 256 : 64);
+  if (n == 0) return 0;
+  if (wide)
+    carry_idle_kernel<uint4><<<dim3(blocks, Bv), 256, 0, (cudaStream_t)stream>>>(
+        lengths, reinterpret_cast<const uint4*>(src), reinterpret_cast<uint4*>(dst), n);
+  else
+    carry_idle_kernel<uint32_t><<<dim3(blocks, Bv), 256, 0, (cudaStream_t)stream>>>(
+        lengths, reinterpret_cast<const uint32_t*>(src), reinterpret_cast<uint32_t*>(dst), n);
+  LTM_CHECK_LAUNCH("carry_idle");
+  return 0;
+}
+
 // out[v,s,:] = src[v, idx[v,s], :]
 __global__ void __launch_bounds__(256)
 gather_rows_kernel(const float4* __restrict__ src, const int32_t* __restrict__ idx, float4* __restrict__ out,
@@ -233,6 +297,18 @@ extern "C" int ltm_consolidate_rect_kv(const float* B_past, const float* xpart, 
                                        float* B_new, void* B_half,
                                        const float* KV_past, float* KV_new, const float* bkv, int ldkv, int jf,
                                        int round_tf32, int Bv, int N, int e, int L, int splits, int S, void* stream) {
+  return ltm::consolidate_rect_ragged(B_past, xpart, idx, idx_stride, new_doc, seg_ptr0, seg_mem0, g0, seg_ptr1,
+                                      seg_mem1, g1, B_new, B_half, KV_past, KV_new, bkv, ldkv, jf, round_tf32, Bv, N,
+                                      e, L, splits, S, nullptr, nullptr, stream);
+}
+
+// lengths == NULL: the lock-step kernels.  Otherwise the ragged ones (see Ragged); the tables are the bank's.
+int ltm::consolidate_rect_ragged(const float* B_past, const float* xpart, const int32_t* idx, int64_t idx_stride,
+                                 const uint8_t* new_doc, const int32_t* seg_ptr0, const int32_t* seg_mem0,
+                                 const float* g0, const int32_t* seg_ptr1, const int32_t* seg_mem1, const float* g1,
+                                 float* B_new, void* B_half, const float* KV_past, float* KV_new, const float* bkv,
+                                 int ldkv, int jf, int round_tf32, int Bv, int N, int e, int L, int splits, int S,
+                                 const int32_t* lengths, const int32_t* offs, void* stream) {
   using namespace ltm;
   // round_tf32 == 2: KV_past / KV_new point to fp16 storage [Bv, N, ldkv] (ldkv % 8 == 0)
   const int kv_half = round_tf32 == 2 ? 1 : 0;
@@ -266,16 +342,19 @@ extern "C" int ltm_consolidate_rect_kv(const float* B_past, const float* xpart, 
   // (num_basis 64 x 1024 videos: 5 % slower with four rows under the overlap -- its rows are longer, 8-10 members each)
   const int rows_per_cta = (N >= 128 && (long long)N * Bv >= 16384) ? 4 : 1;
   dim3 grid((N + rows_per_cta - 1) / rows_per_cta, Bv);
-  if (rows_per_cta == 4)
-    consolidate_rect_kernel<4><<<grid, threads, 0, (cudaStream_t)stream>>>(
-        reinterpret_cast<const float4*>(B_past), reinterpret_cast<const float4*>(xpart), idx, (long long)idx_stride,
-        new_doc, seg_ptr0, seg_mem0, g0, seg_ptr1, seg_mem1, g1, reinterpret_cast<float4*>(B_new),
-        reinterpret_cast<uint2*>(B_half), kv, N, e4, L, splits, S);
-  else
-    consolidate_rect_kernel<1><<<grid, threads, 0, (cudaStream_t)stream>>>(
-        reinterpret_cast<const float4*>(B_past), reinterpret_cast<const float4*>(xpart), idx, (long long)idx_stride,
-        new_doc, seg_ptr0, seg_mem0, g0, seg_ptr1, seg_mem1, g1, reinterpret_cast<float4*>(B_new),
-        reinterpret_cast<uint2*>(B_half), kv, N, e4, L, splits, S);
+  LTM_REQUIRE((lengths == nullptr) == (offs == nullptr), "consolidate_rect: ragged batches need lengths and offsets");
+  const Ragged rg{lengths, offs};
+#define LTM_CONSOLIDATE(ROWS, RAGGED)                                                                                 \
+  consolidate_rect_kernel<ROWS, RAGGED><<<grid, threads, 0, (cudaStream_t)stream>>>(                                  \
+      reinterpret_cast<const float4*>(B_past), reinterpret_cast<const float4*>(xpart), idx, (long long)idx_stride,   \
+      new_doc, seg_ptr0, seg_mem0, g0, seg_ptr1, seg_mem1, g1, reinterpret_cast<float4*>(B_new),                     \
+      reinterpret_cast<uint2*>(B_half), kv, N, e4, L, splits, S, rg)
+  if (rows_per_cta == 4) {
+    if (lengths) LTM_CONSOLIDATE(4, true); else LTM_CONSOLIDATE(4, false);
+  } else {
+    if (lengths) LTM_CONSOLIDATE(1, true); else LTM_CONSOLIDATE(1, false);
+  }
+#undef LTM_CONSOLIDATE
   LTM_CHECK_LAUNCH("consolidate_rect");
   return 0;
 }

@@ -40,14 +40,13 @@ __device__ __forceinline__ float4 pool_rows(const float4* __restrict__ base, int
   return acc[0];
 }
 
-// One (frame, token-split) work item: the threads of the CTA each own 128-bit column groups.
-__device__ __forceinline__ void pool_unit(const float4* __restrict__ k, float4* __restrict__ xpart, int T, int e4,
-                                          int splits, float Tf, unsigned work, uint64_t pol) {
-  const int unit = work / splits;                // (v*L + l)
-  const int sp = work - unit * splits;
+// Token-split `sp` of frame `src` of the chunk, written to row (unit * splits + sp) of xpart: the threads of the CTA
+// each own 128-bit column groups.
+__device__ __forceinline__ void pool_unit_at(const float4* __restrict__ k, float4* __restrict__ xpart, int T, int e4,
+                                             int splits, float Tf, unsigned unit, int sp, size_t src, uint64_t pol) {
   const int r0 = (int)(((long long)T * sp) / splits);
   const int r1 = (int)(((long long)T * (sp + 1)) / splits);
-  const float4* base = k + (size_t)unit * T * e4;
+  const float4* base = k + src * T * e4;
   for (int c = threadIdx.x; c < e4; c += blockDim.x) {
     float4 o = pool_rows(base, r0, r1, e4, c, pol);
     // torch.mean == sum / T (true division, so T = 196 rounds like the reference).  With splits > 1 (small batches
@@ -56,6 +55,13 @@ __device__ __forceinline__ void pool_unit(const float4* __restrict__ k, float4* 
     o.x = __fdiv_rn(o.x, Tf); o.y = __fdiv_rn(o.y, Tf); o.z = __fdiv_rn(o.z, Tf); o.w = __fdiv_rn(o.w, Tf);
     xpart[((size_t)unit * splits + sp) * e4 + c] = o;
   }
+}
+
+// One (frame, token-split) work item of a lock-step chunk: frame unit = v*L + l in and out.
+__device__ __forceinline__ void pool_unit(const float4* __restrict__ k, float4* __restrict__ xpart, int T, int e4,
+                                          int splits, float Tf, unsigned work, uint64_t pol) {
+  const unsigned unit = work / splits;
+  pool_unit_at(k, xpart, T, e4, splits, Tf, unit, (int)(work - unit * splits), unit, pol);
 }
 
 // Frame pooling folded with the first half of the regression (VERDICT r1, "bin sums instead of xpart"): the frames of
@@ -197,16 +203,13 @@ __device__ __forceinline__ uint4 ldg_stream_u4(const uint4* p, uint64_t policy) 
   return r;
 }
 
+// 16-bit twin of pool_unit_at
 template <bool BF16>
-__global__ void __launch_bounds__(256)
-pool_mean16_kernel(const uint4* __restrict__ k, float4* __restrict__ xpart, int T, int e8, int splits, float Tf) {
-  const uint64_t pol = policy_evict_first();
-  const unsigned work = blockIdx.x;
-  const int unit = work / splits;
-  const int sp = work - unit * splits;
+__device__ __forceinline__ void pool_unit16_at(const uint4* __restrict__ k, float4* __restrict__ xpart, int T, int e8,
+                                               int splits, float Tf, unsigned unit, int sp, size_t src, uint64_t pol) {
   const int r0 = (int)(((long long)T * sp) / splits);
   const int r1 = (int)(((long long)T * (sp + 1)) / splits);
-  const uint4* base = k + (size_t)unit * T * e8;
+  const uint4* base = k + src * T * e8;
   for (int c = threadIdx.x; c < e8; c += blockDim.x) {
     float acc[8];
 #pragma unroll
@@ -236,7 +239,80 @@ pool_mean16_kernel(const uint4* __restrict__ k, float4* __restrict__ xpart, int 
   }
 }
 
+template <bool BF16>
+__global__ void __launch_bounds__(256)
+pool_mean16_kernel(const uint4* __restrict__ k, float4* __restrict__ xpart, int T, int e8, int splits, float Tf) {
+  const unsigned unit = blockIdx.x / splits;
+  pool_unit16_at<BF16>(k, xpart, T, e8, splits, Tf, unit, (int)(blockIdx.x - unit * splits), unit, policy_evict_first());
+}
+
+// ---- ragged batch: the grid covers exactly the (frame, token-split) items of the frames in use, packed video after
+// video (frame f of the packing is frame f - offs[v] of video v, offs[v] <= f < offs[v+1]); the padding of the chunk
+// is never read.  Each item runs the lock-step code above, so a pooled frame carries the same bits.  PERSIST: bounded
+// grid walking the item list (the side-stream pooling of step_overlapped).
+__device__ __forceinline__ size_t ragged_src(const int32_t* __restrict__ offs, int Bv, int L, unsigned f) {
+  int lo = 0, hi = Bv;                                  // offs[lo] <= f < offs[hi]
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if ((unsigned)__ldg(offs + mid) <= f) lo = mid; else hi = mid;
+  }
+  return (size_t)lo * L + (f - (unsigned)__ldg(offs + lo));
+}
+
+template <int DT, bool PERSIST>        // DT: 0 fp32, 1 fp16, 2 bfloat16
+__global__ void __launch_bounds__(256)
+pool_ragged_kernel(const void* __restrict__ k, float4* __restrict__ xpart, const int32_t* __restrict__ offs, int Bv,
+                   int L, int T, int ev, int splits, float Tf, unsigned total) {
+  const uint64_t pol = policy_evict_first();
+  for (unsigned work = blockIdx.x; work < total; work += gridDim.x) {
+    const unsigned f = work / splits;
+    const int sp = (int)(work - f * splits);
+    const size_t src = ragged_src(offs, Bv, L, f);
+    if (DT == 0)
+      pool_unit_at(reinterpret_cast<const float4*>(k), xpart, T, ev, splits, Tf, f, sp, src, pol);
+    else
+      pool_unit16_at<DT == 2>(reinterpret_cast<const uint4*>(k), xpart, T, ev, splits, Tf, f, sp, src, pol);
+    if (!PERSIST) break;
+  }
+}
+
+template <int DT>
+static void launch_pool_ragged(const void* k, float* xpart, const int32_t* offs, int Bv, int L, int T, int ev,
+                               int splits, float Tf, unsigned total, int max_ctas, cudaStream_t st) {
+  const int threads = ev >= 256 ? 256 : ((ev + 31) / 32) * 32;
+  float4* x = reinterpret_cast<float4*>(xpart);
+  if (max_ctas > 0 && (unsigned)max_ctas < total)
+    pool_ragged_kernel<DT, true><<<(unsigned)max_ctas, threads, 0, st>>>(k, x, offs, Bv, L, T, ev, splits, Tf, total);
+  else
+    pool_ragged_kernel<DT, false><<<total, threads, 0, st>>>(k, x, offs, Bv, L, T, ev, splits, Tf, total);
+}
+
 }  // namespace ltm
+
+extern "C" int ltm_pool_mean_ragged(const void* k, int dtype, float* xpart, const int32_t* offs, int Bv, int L, int T,
+                                    int e, int splits, int frames, int max_ctas, void* stream) {
+  using namespace ltm;
+  LTM_REQUIRE(k && xpart && offs, "pool_mean_ragged: null pointer");
+  LTM_REQUIRE(Bv > 0 && L > 0 && T > 0 && e > 0 && frames >= 0 && frames <= (long long)Bv * L,
+              "pool_mean_ragged: bad shape Bv=%d L=%d T=%d e=%d frames=%d", Bv, L, T, e, frames);
+  LTM_REQUIRE(dtype >= 0 && dtype <= 2, "pool_mean_ragged: dtype=%d", dtype);
+  LTM_REQUIRE(e % (dtype ? 8 : 4) == 0, "pool_mean_ragged: e=%d must be a multiple of %d", e, dtype ? 8 : 4);
+  LTM_REQUIRE(splits >= 1 && splits <= T, "pool_mean_ragged: splits=%d out of range [1,%d]", splits, T);
+  LTM_REQUIRE(aligned16(k) && aligned16(xpart), "pool_mean_ragged: pointers must be 16-byte aligned");
+  const long long units = (long long)frames * splits;
+  LTM_REQUIRE(units < (1ll << 31), "pool_mean_ragged: too many frames");
+  if (units == 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int ev = dtype ? e / 8 : e / 4;
+  if (dtype == 0)
+    launch_pool_ragged<0>(k, xpart, offs, Bv, L, T, ev, splits, (float)T, (unsigned)units, max_ctas, st);
+  else if (dtype == 1)
+    launch_pool_ragged<1>(k, xpart, offs, Bv, L, T, ev, splits, (float)T, (unsigned)units, max_ctas, st);
+  else
+    launch_pool_ragged<2>(k, xpart, offs, Bv, L, T, ev, splits, (float)T, (unsigned)units, max_ctas, st);
+  LTM_CHECK_LAUNCH("pool_mean_ragged");
+  return 0;
+}
 
 extern "C" int ltm_pool_mean_16(const void* k, int is_bf16, float* xpart, int Bv, int L, int T, int e, int splits,
                                 void* stream) {

@@ -102,18 +102,21 @@ __device__ __forceinline__ float block_sum_128(float v, float* red) {
   return t;
 }
 
+// RAGGED: videos with lengths[v] == 0 (idle in a ragged batch) are skipped
+template <bool RAGGED>
 __global__ void __launch_bounds__(RS_THREADS)
 resample_kernel(const float* __restrict__ hist_part, int parts, int ncat, int normalize,
                 const double* __restrict__ u, const float* __restrict__ bins,
                 const int32_t* __restrict__ bin2basis, int sort,
                 float* __restrict__ p_out, int32_t* __restrict__ b_draw, int32_t* __restrict__ b_used,
-                float* __restrict__ ts, int32_t* __restrict__ idx, int S) {
+                float* __restrict__ ts, int32_t* __restrict__ idx, int S, const int32_t* __restrict__ lengths) {
   __shared__ float cdf[MAX_CAT];
   __shared__ int cnt[MAX_CAT];
   __shared__ int start_s[MAX_CAT];
   __shared__ float red[4];
   __shared__ float total_s;
   const int v = blockIdx.x, tid = threadIdx.x;
+  if (RAGGED && lengths[v] == 0) return;
 
   // 1. assemble p
   float a = 0.f;
@@ -330,8 +333,22 @@ extern "C" int ltm_resample(const float* hist_part, int parts, int ncat, int nor
   LTM_REQUIRE(hist_part && u && bins, "resample: null pointer");
   LTM_REQUIRE(ncat >= 1 && ncat <= MAX_CAT, "resample: ncat=%d out of range [1,%d]", ncat, MAX_CAT);
   LTM_REQUIRE(parts >= 1 && Bv > 0 && S > 0, "resample: bad shape");
-  resample_kernel<<<Bv, RS_THREADS, 0, (cudaStream_t)stream>>>(hist_part, parts, ncat, normalize, u, bins,
-                                                            bin2basis, sort, p_out, b_draw, b_used, ts, idx, S);
+  resample_kernel<false><<<Bv, RS_THREADS, 0, (cudaStream_t)stream>>>(hist_part, parts, ncat, normalize, u, bins,
+                                                                   bin2basis, sort, p_out, b_draw, b_used, ts, idx, S,
+                                                                   nullptr);
+  LTM_CHECK_LAUNCH("resample");
+  return 0;
+}
+
+int ltm::resample_ragged(const float* hist_part, int parts, int ncat, int normalize, const double* u, const float* bins,
+                         const int32_t* bin2basis, int sort, float* p_out, int32_t* b_draw, int32_t* b_used, float* ts,
+                         int32_t* idx, int Bv, int S, const int32_t* lengths, void* stream) {
+  LTM_REQUIRE(hist_part && u && bins && lengths, "resample: null pointer");
+  LTM_REQUIRE(ncat >= 1 && ncat <= MAX_CAT, "resample: ncat=%d out of range [1,%d]", ncat, MAX_CAT);
+  LTM_REQUIRE(parts >= 1 && Bv > 0 && S > 0, "resample: bad shape");
+  resample_kernel<true><<<Bv, RS_THREADS, 0, (cudaStream_t)stream>>>(hist_part, parts, ncat, normalize, u, bins,
+                                                                  bin2basis, sort, p_out, b_draw, b_used, ts, idx, S,
+                                                                  lengths);
   LTM_CHECK_LAUNCH("resample");
   return 0;
 }

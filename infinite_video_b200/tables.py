@@ -312,6 +312,94 @@ def rect_tables(L: int, N: int, tau: float, S: int = NB_SAMPLES, num_quad: int =
     return t
 
 
+class RectBank:
+    """The chunk-length dependent tables of variant R -- first-chunk and update segment tables, weights and jf -- for
+    every chunk length up to `Lmax`, at fixed strides, so that a kernel selects the tables of a video from its length
+    alone (ragged batches, `BatchedRectLTM.step(..., lengths=...)`):
+
+      seg_ptr0 / seg_ptr1  int32 [Lmax+1, N+1]  absolute offsets into the concatenated seg_mem0 / seg_mem1
+      seg_mem0 / seg_mem1  int32                entry L at mem0_off(L) = L(L-1)/2, mem1_off(L) = L*S + L(L-1)/2
+      g0 / g1              fp32  [Lmax+1, N]
+      jf                   int32 [Lmax+1]       (host only: the step derives its projected-row split from it)
+
+    Entries are filled on first use from `rect_tables(L, ...)`, which stays the single source of bin membership, and
+    uploaded to a device stream-ordered on the current stream, once per (device, L).  Every other table of variant R
+    (sticky edges, quadrature, uniform re-sampling, density grid) does not depend on L."""
+
+    def __init__(self, Lmax, N, tau, S=NB_SAMPLES, spacing="linear"):
+        self.Lmax, self.N, self.tau, self.S, self.spacing = int(Lmax), int(N), float(tau), int(S), spacing
+        n = self.Lmax + 1
+        self.seg_ptr0 = np.zeros((n, N + 1), np.int32)
+        self.seg_ptr1 = np.zeros((n, N + 1), np.int32)
+        self.seg_mem0 = np.zeros(self.mem0_off(n), np.int32)
+        self.seg_mem1 = np.zeros(self.mem1_off(n), np.int32)
+        self.g0 = np.zeros((n, N), np.float32)
+        self.g1 = np.zeros((n, N), np.float32)
+        self.jf = np.zeros(n, np.int32)
+        self.filled = set()
+        self._dev = {}
+
+    @staticmethod
+    def mem0_off(L):
+        return L * (L - 1) // 2                          # a first chunk of l frames has at most l members
+
+    def mem1_off(self, L):
+        return L * self.S + L * (L - 1) // 2             # an update of l frames has at most S + l members
+
+    def fill(self, lengths):
+        """Host entries for every length in `lengths` (0 = idle, skipped); returns the lengths newly filled."""
+        new = sorted({int(L) for L in lengths} - self.filled - {0})
+        for L in new:
+            if not 2 <= L <= self.Lmax:
+                raise ValueError(f"chunk length {L} outside [2, {self.Lmax}]")
+            t = rect_tables(L, self.N, self.tau, self.S, spacing=self.spacing)
+            o0, o1 = self.mem0_off(L), self.mem1_off(L)
+            self.seg_ptr0[L] = t.seg_ptr0 + o0
+            self.seg_mem0[o0:o0 + t.seg_mem0.size] = t.seg_mem0
+            self.seg_ptr1[L] = t.seg_ptr1 + o1
+            self.seg_mem1[o1:o1 + t.seg_mem1.size] = t.seg_mem1
+            self.g0[L], self.g1[L], self.jf[L] = t.g0, t.g1, t.jf
+            self.filled.add(L)
+        return new
+
+    def entry(self, L):
+        """The tables of length L sliced back out of the bank (host): (seg_ptr0, seg_mem0, g0, seg_ptr1, seg_mem1, g1,
+        jf), in the layout of `rect_tables`."""
+        o0, o1 = self.mem0_off(L), self.mem1_off(L)
+        p0, p1 = self.seg_ptr0[L] - o0, self.seg_ptr1[L] - o1
+        return (p0, self.seg_mem0[o0:o0 + p0[-1]], self.g0[L], p1, self.seg_mem1[o1:o1 + p1[-1]], self.g1[L],
+                int(self.jf[L]))
+
+    def to(self, device, lengths):
+        """Device arrays holding (at least) the entries of `lengths`.  Entries not on this device yet are copied on the
+        current stream, consecutive lengths in one copy per array."""
+        key = str(device)
+        d = self._dev.get(key)
+        if d is None:
+            d = dict(done=set())
+            for name in ("seg_ptr0", "seg_mem0", "g0", "seg_ptr1", "seg_mem1", "g1"):
+                d[name] = torch.zeros(getattr(self, name).shape, dtype=torch.float32 if name[0] == "g" else torch.int32,
+                                      device=device)
+            self._dev[key] = d
+        self.fill(lengths)
+        todo = sorted({int(L) for L in lengths} - d["done"] - {0})
+        runs = []
+        for L in todo:
+            if runs and runs[-1][1] == L:
+                runs[-1][1] = L + 1
+            else:
+                runs.append([L, L + 1])
+        for a, b in runs:
+            for name in ("seg_ptr0", "g0", "seg_ptr1", "g1"):
+                d[name][a:b].copy_(torch.from_numpy(getattr(self, name)[a:b]))
+            d["seg_mem0"][self.mem0_off(a):self.mem0_off(b)].copy_(
+                torch.from_numpy(self.seg_mem0[self.mem0_off(a):self.mem0_off(b)]))
+            d["seg_mem1"][self.mem1_off(a):self.mem1_off(b)].copy_(
+                torch.from_numpy(self.seg_mem1[self.mem1_off(a):self.mem1_off(b)]))
+        d["done"].update(todo)
+        return d
+
+
 # ----------------------------------------------------------------------------------------------
 # Variant G (Gaussian RBF): host side only provides positions / basis parameters; the design matrix
 # and the ridge solve run on the device (csrc/ridge.cu).

@@ -18,7 +18,7 @@ from .batched import BatchedRectLTM
 
 
 @torch.no_grad()
-def consolidate_video(engines, chunks, queries, uniforms=None, new_doc=True, reduce=None):
+def consolidate_video(engines, chunks, queries, uniforms=None, new_doc=True, reduce=None, lengths=None):
     """engines:  one `BatchedRectLTM` per LTM layer (same device, same chunk geometry).
     chunks:   C tensors [Bv, L*T, e] -- the `encoder_hidden_states` of each chunk, in order.
     queries:  `queries[layer][c]` tensors [Bv, Q, D], or a callable `queries(layer, c, prev)` returning that tensor
@@ -27,6 +27,9 @@ def consolidate_video(engines, chunks, queries, uniforms=None, new_doc=True, red
     uniforms: `uniforms[layer][c]` float64 [Bv, 512] for c >= 1 (sticky engines); None entries allowed at c == 0.
     new_doc:  whether chunk 0 starts a new document for every video.
     reduce:   None -> `ctx[layer][c]`;  "mean" -> running mean over the chunks, `ctx[layer]` [Bv, Q, D].
+    lengths:  videos of different lengths: `lengths[c]` holds Bv host ints, the frames video v has in chunk c (its
+              chunk padded to L frames; 0 once the video has ended -- its memory is kept and its ctx rows are zero).
+              "mean" then divides each video by the number of chunks it actually had.
     """
     if not engines or any(not isinstance(e, BatchedRectLTM) for e in engines):
         raise ValueError("consolidate_video takes a list of BatchedRectLTM engines (one per LTM layer)")
@@ -36,6 +39,9 @@ def consolidate_video(engines, chunks, queries, uniforms=None, new_doc=True, red
     if reduce not in (None, "mean"):
         raise ValueError("reduce must be None or 'mean'")
     C = len(chunks)
+    if lengths is not None and len(lengths) != C:
+        raise ValueError("lengths must hold one entry per chunk")
+    lens = [None] * C if lengths is None else lengths
     pool_eng = engines[0]
     with torch.cuda.device(dev):
         main = torch.cuda.current_stream(dev)
@@ -45,7 +51,7 @@ def consolidate_video(engines, chunks, queries, uniforms=None, new_doc=True, red
 
         def pool_ahead(c):
             with torch.cuda.stream(side):
-                pooled[c] = pool_eng.pool(chunks[c])
+                pooled[c] = pool_eng.pool(chunks[c], lengths=lens[c])
                 ready[c] = torch.cuda.Event()
                 ready[c].record(side)
 
@@ -62,7 +68,7 @@ def consolidate_video(engines, chunks, queries, uniforms=None, new_doc=True, red
                 q = queries(li, c, prev) if callable(queries) else queries[li][c]
                 u = None if uniforms is None else uniforms[li][c]
                 ctx = eng.step(chunks[c], q, u if c > 0 or not new_doc else None, new_doc=(new_doc and c == 0),
-                               pooled=pooled[c], beside_pooling=(c + 1 < C))
+                               pooled=pooled[c], beside_pooling=(c + 1 < C), lengths=lens[c])
                 prev = ctx
                 if reduce == "mean":
                     acc[li] = ctx.clone() if acc[li] is None else acc[li].add_(ctx)
@@ -70,5 +76,8 @@ def consolidate_video(engines, chunks, queries, uniforms=None, new_doc=True, red
                     out[li].append(ctx)
             pooled[c] = None
         if reduce == "mean":
-            return [a / C for a in acc]
+            if lengths is None:
+                return [a / C for a in acc]
+            had = torch.as_tensor([[int(x) > 0 for x in lc] for lc in lengths]).sum(0).clamp_min(1)
+            return [a / had.to(dev, a.dtype).view(-1, 1, 1) for a in acc]
         return out
