@@ -234,10 +234,10 @@ class BatchedRectLTM(_BatchedBase):
         """Token-splits of the frame pooling: one CTA per frame when that already gives the GPU four waves of CTAs
         (8 resident per SM), otherwise each frame's tokens are split so that it does -- a grid of barely more than one
         wave leaves the second one almost empty (VideoChat2 shape, 64 videos x 16 frames = 1024 CTAs for 1184 slots:
-        146 us for 822 MB)."""
+        146 us for 822 MB).  No units (a ragged chunk of idle videos): 1."""
         want = 4 * 8 * self.sm_count
         # (at most T/8 splits: the partial sums are written and read back, T/splits rows of input per row of output)
-        return 1 if units >= want else max(1, min(max(1, self.T // 8), -(-want // units)))
+        return 1 if units >= want or units == 0 else max(1, min(max(1, self.T // 8), -(-want // units)))
 
     def _bin_ok(self, Bv, L, tab):
         """Whether an update chunk of this shape is pooled per bin (see `bin_pool`)."""
@@ -276,6 +276,32 @@ class BatchedRectLTM(_BatchedBase):
         held = {e["buf"] for e in self._pref}
         pref = 1 - ws["xi"]
         return pref if pref not in held else 1 - pref
+
+    def _frames_source(self, k, Q, ws, tab, flags, rag, pooled=None, prefetch=False):
+        """Where the pooled frames of chunk k come from, for `step` and `step_overlapped`: `pooled` when given (returns
+        None); else a pending prefetch of k, whose entry is returned with ws["xi"] on its buffer; else, with
+        `prefetch`, one issued here; else the step pools k itself (returns None), into a buffer that no pending
+        prefetch holds."""
+        if pooled is not None:
+            return None
+        lens = None if rag is None else rag["lens"]
+        update = rag is None and self.has_state and flags is None   # every video continues: per-bin pooling possible
+        hit = self._pref_take(k, lens)
+        if hit is not None and hit["binned"] and not update:
+            hit = None                                   # pooled per bin for an update that did not come: pool again
+        if hit is None and prefetch:
+            self.prefetch(k, Q, lengths=lens, update=update)
+            hit = self._pref_take(k, lens)
+        if hit is not None:
+            ws["xi"] = hit["buf"]
+            ws["xtag"][hit["buf"]] = hit["binned"]
+            return hit
+        held = {e["buf"] for e in self._pref}          # never pool over frames a pending prefetch still owns
+        ws["xi"] = (1 - ws["xi"]) if (1 - ws["xi"]) not in held else ws["xi"]
+        if ws["xi"] in held:
+            self._pref[:] = [e for e in self._pref if e["buf"] != ws["xi"]]
+        ws["xtag"][ws["xi"]] = update and self._bin_ok(k.shape[0], k.shape[1] // self.T, tab)
+        return None
 
     def _state(self, Bv, Q):
         qt = (Q + 31) // 32
@@ -319,8 +345,8 @@ class BatchedRectLTM(_BatchedBase):
         if rag is None:
             a.lengths, a.frame_offs, a.n_idle, a.jf = None, None, 0, tab.jf
         else:
-            lt, bank = rag["dev"], rag["bank"]
-            a.lengths, a.frame_offs = lt.data_ptr(), lt.data_ptr() + 4 * Bv
+            bank = rag["bank"]
+            a.lengths, a.frame_offs = rag["lens_dev"].data_ptr(), rag["offs_dev"].data_ptr()
             a.frames, a.n_idle, a.jf, a.splits, a.binned = rag["frames"], rag["n_idle"], rag["jf"], rag["splits"], 0
             a.bank_seg_ptr0, a.bank_seg_mem0, a.bank_g0 = (bank["seg_ptr0"].data_ptr(), bank["seg_mem0"].data_ptr(),
                                                            bank["g0"].data_ptr())
@@ -380,33 +406,89 @@ class BatchedRectLTM(_BatchedBase):
             setattr(a, f, ws[n].data_ptr() if ws[n] is not None else None)
         return a
 
-    def _prepare(self, kshape, qshape, new_doc):
-        Bv, LT, e = kshape
+    def _prepare(self, k, q, new_doc, u, lengths=None, pooled=None, u_name="u"):
+        """Host side of a step: validation, per-slot bookkeeping, tables.  Every ValueError fires before any state
+        changes.  Returns (Bv, L, Q, tab, tdev, flags, u, rag): the device new_doc flags the step applies (None: none),
+        the contiguous uniforms (None: the step reads none) and, for a ragged step, its table bank and device lengths /
+        offsets (rag; None: lock-step).  A lock-step call takes new_doc as a device tensor too, a ragged one as host
+        flags (it selects tables from them)."""
+        Bv, LT, e = k.shape
         if e != self.e:
             raise ValueError(f"k has width {e}, projections expect {self.e}")
-        if LT % self.T:
+        if lengths is None and LT % self.T:
             raise ValueError(f"k has {LT} tokens, not a multiple of tokens_per_frame={self.T}")
-        L = LT // self.T
-        Q = qshape[1]
-        if qshape[0] != Bv or qshape[2] != self.D:
+        if lengths is not None and (LT % self.T or LT // self.T < 2):
+            raise ValueError(f"k has {LT} tokens: a ragged chunk is padded to L*{self.T} tokens, L >= 2")
+        L, Q = LT // self.T, q.shape[1]
+        if q.shape[0] != Bv or q.shape[2] != self.D:
             raise ValueError(f"q must be [{Bv}, Q, {self.D}]")
-        all_new, flags = _as_flags(new_doc, Bv, self.device)
-        if (self.has_state and not all_new and self._B is not None and self.Bv == Bv
-                and self._hist.shape[1] != self.H * ((Q + 31) // 32)):
-            # the sticky histogram of the previous call is kept per (head, tile of 32 queries): a different number
-            # of query tiles inside a video would silently restart the memory
-            raise ValueError(f"the number of queries changed inside a video ({Q} now): pass new_doc=True or keep Q")
-        if self._slots is not None and self.has_state and not all_new and self.Bv == Bv and not self._slots.all():
-            # (only after a ragged step left slots without memory)
-            nd = torch.as_tensor(new_doc).reshape(-1).to("cpu", torch.bool).numpy() if all_new is None else False
-            self._no_memory_check(~np.asarray(nd, bool) & ~self._slots)
+        same = self.has_state and self._B is not None and self.Bv == Bv        # this batch has memory to continue
+        # the sticky histogram of the previous call is kept per (head, tile of 32 queries): a different number of
+        # query tiles inside a video would silently restart the memory
+        retiled = same and self._hist.shape[1] != self.H * ((Q + 31) // 32)
+        retiled_msg = f"the number of queries changed inside a video ({Q} now): pass new_doc=True or keep Q"
+        if lengths is None:
+            all_new, flags = _as_flags(new_doc, Bv, self.device)
+            keep = same and not all_new
+            if keep and retiled:
+                raise ValueError(retiled_msg)
+            if keep and self._slots is not None and not self._slots.all():
+                # (only after a ragged step left slots without memory)
+                nd = torch.as_tensor(new_doc).reshape(-1).to("cpu", torch.bool).numpy() if all_new is None else False
+                self._no_memory_check(~np.asarray(nd, bool) & ~self._slots)
+            need_u = keep and self.sticky
+        else:
+            ln = np.asarray(_as_lengths(lengths, Bv, L), np.int64)
+            if isinstance(new_doc, (bool, int)):
+                nd = np.full(Bv, bool(new_doc))
+            else:
+                t = torch.as_tensor(new_doc)
+                if t.device.type != "cpu" or t.numel() != Bv:
+                    raise ValueError("a ragged step takes new_doc as a bool or one host flag per video")
+                nd = t.reshape(-1).to(torch.bool).numpy()
+            present = ln > 0
+            mem = (self._slots if self._slots is not None else np.ones(Bv, bool)) if same else np.zeros(Bv, bool)
+            if retiled and (mem & ~nd).any():
+                raise ValueError(retiled_msg)
+            cont = present & ~nd
+            self._no_memory_check(cont & ~mem)
+            keep = same and not retiled
+            need_u = keep and self.sticky and bool(cont.any())
+            frames = int(ln.sum())
+            if pooled is not None and (pooled.dim() != 3 or pooled.shape[0] != frames or pooled.shape[2] != self.e):
+                raise ValueError(f"pooled frames of a ragged chunk must be [{frames}, splits, {self.e}]")
+        if pooled is not None and (not pooled.is_contiguous() or lengths is None and (
+                tuple(pooled.shape[:2]) != (Bv, L) or pooled.shape[3] != self.e)):
+            raise ValueError("pooled frames do not match k")
+        if need_u:
+            if u is None or u.dtype != torch.float64 or tuple(u.shape) != (Bv, self.S):
+                raise ValueError(f"sticky re-sampling needs {u_name}: float64 [{Bv},{self.S}]")
+            u = u.contiguous()
+        else:
+            u = None
         self._state(Bv, Q)
-        if all_new:
-            self.has_state = False
-        elif flags is not None and not self.has_state:
-            flags = None                     # nothing to keep anyway: everything is a first chunk
+        self.has_state = keep                # False: every video starts with this chunk
         tab = tables.rect_tables(L, self.N, self.tau, self.S, spacing=self.spacing)
-        return Bv, L, Q, tab, tab.to(self.device), flags
+        if lengths is None:
+            return Bv, L, Q, tab, tab.to(self.device), flags if keep else None, u, None
+        first = present & nd
+        flags = None
+        if keep and first.any():
+            flags = torch.from_numpy(first.astype(np.uint8)).pin_memory().to(self.device, non_blocking=True)
+        bank = self._bank(L)
+        bdev = bank.to(self.device, set(ln.tolist()))
+        n_idle = int((~present).sum())
+        hist_keep = None
+        if n_idle and self.sticky:
+            if getattr(self, "_hist_keep", None) is None or self._hist_keep.shape != self._hist.shape:
+                self._hist_keep = torch.empty_like(self._hist)
+            hist_keep = self._hist_keep
+        lens_dev, offs_dev = self._lengths_dev(ln)
+        rag = dict(lens=tuple(ln.tolist()), lens_dev=lens_dev, offs_dev=offs_dev, bank=bdev, frames=frames,
+                   splits=self._splits(frames), n_idle=n_idle,
+                   jf=int(bank.jf[ln[cont]].min()) if (keep and cont.any()) else self.N, hist_keep=hist_keep,
+                   slots=np.where(nd, present, mem))
+        return Bv, L, Q, tab, tab.to(self.device), flags, u, rag
 
     def _no_memory_check(self, bad):
         if np.any(bad):
@@ -420,12 +502,13 @@ class BatchedRectLTM(_BatchedBase):
         return bank
 
     def _lengths_dev(self, lens):
-        """[lengths (Bv) | exclusive prefix sum (Bv+1)] as one int32 device tensor, copied on the current stream."""
+        """(lengths [Bv], exclusive prefix sum [Bv+1]): int32 views of one device buffer, copied on the current stream."""
         Bv = len(lens)
         host = np.zeros(2 * Bv + 1, np.int32)
         host[:Bv] = lens
         np.cumsum(host[:Bv], out=host[Bv + 1:])
-        return torch.from_numpy(host).pin_memory().to(self.device, non_blocking=True)
+        t = torch.from_numpy(host).pin_memory().to(self.device, non_blocking=True)
+        return t[:Bv], t[Bv:]
 
     def _ragged_ws(self, ws, Bv, L):
         """Packed pooled frames of a ragged step take sum(lengths) * splits rows: at most Bv * L (one split) or, when
@@ -442,52 +525,6 @@ class BatchedRectLTM(_BatchedBase):
         ws["xbufs"] = [torch.empty(need, device=self.device, dtype=torch.float32) for _ in range(2)]
         ws["xparts"] = [b[:Bv * L * splits * self.e].view(Bv, L, splits, self.e) for b in ws["xbufs"]]
         ws["xtag"] = [False, False]
-
-    def _prepare_ragged(self, kshape, qshape, new_doc, lengths):
-        """Host side of a ragged step: validation, per-slot bookkeeping, table bank, device lengths / offsets."""
-        Bv, LT, e = kshape
-        if e != self.e:
-            raise ValueError(f"k has width {e}, projections expect {self.e}")
-        if LT % self.T or LT // self.T < 2:
-            raise ValueError(f"k has {LT} tokens: a ragged chunk is padded to L*{self.T} tokens, L >= 2")
-        L, Q = LT // self.T, qshape[1]
-        if qshape[0] != Bv or qshape[2] != self.D:
-            raise ValueError(f"q must be [{Bv}, Q, {self.D}]")
-        ln = np.asarray(_as_lengths(lengths, Bv, L), np.int64)
-        if isinstance(new_doc, (bool, int)):
-            nd = np.full(Bv, bool(new_doc))
-        else:
-            t = torch.as_tensor(new_doc)
-            if t.device.type != "cpu" or t.numel() != Bv:
-                raise ValueError("a ragged step takes new_doc as a bool or one host flag per video")
-            nd = t.reshape(-1).to(torch.bool).numpy()
-        present = ln > 0
-        same = self._B is not None and self.Bv == Bv and self.has_state
-        mem = (self._slots if self._slots is not None else np.full(Bv, self.has_state)) if same else np.zeros(Bv, bool)
-        if same and self._hist.shape[1] != self.H * ((Q + 31) // 32) and (mem & ~nd).any():
-            raise ValueError(f"the number of queries changed inside a video ({Q} now): pass new_doc=True or keep Q")
-        cont = present & ~nd
-        self._no_memory_check(cont & ~mem)
-        self._state(Bv, Q)
-        first = present & nd
-        flags = None
-        if self.has_state and first.any():
-            flags = torch.from_numpy(first.astype(np.uint8)).pin_memory().to(self.device, non_blocking=True)
-        bank = self._bank(L)
-        bdev = bank.to(self.device, set(ln.tolist()))
-        frames, n_idle = int(ln.sum()), int((~present).sum())
-        hist_keep = None
-        if n_idle and self.sticky:
-            if getattr(self, "_hist_keep", None) is None or self._hist_keep.shape != self._hist.shape:
-                self._hist_keep = torch.empty_like(self._hist)
-            hist_keep = self._hist_keep
-        tab = tables.rect_tables(L, self.N, self.tau, self.S, spacing=self.spacing)   # (its L-independent tables)
-        rag = dict(lens=tuple(ln.tolist()), dev=self._lengths_dev(ln), bank=bdev, frames=frames,
-                   splits=self._splits(frames) if frames else 1, n_idle=n_idle,
-                   jf=int(bank.jf[ln[cont]].min()) if (self.has_state and cont.any()) else self.N,
-                   need_u=bool(self.has_state and self.sticky and cont.any()), hist_keep=hist_keep,
-                   slots=np.where(nd, present, mem))
-        return Bv, L, Q, tab, tab.to(self.device), flags, rag
 
     def _finish(self, ws, xp=None, k=None, rag=None):
         # pooled frames of this call (for `x_past`); a call that pooled per bin keeps a weak reference to the chunk
@@ -529,11 +566,14 @@ class BatchedRectLTM(_BatchedBase):
         Bv, LT, e = k_next.shape
         L = LT // self.T
         ws = self._workspace(Bv, L, Q)
-        lens = lt = None
+        lens = offs = None
+        frames, splits = 0, ws["splits"]
         if lengths is not None:
             lens = _as_lengths(lengths, Bv, L)
             self._ragged_ws(ws, Bv, L)
-            lt = self._lengths_dev(lens)
+            offs = self._lengths_dev(lens)[1]
+            frames = sum(lens)
+            splits = self._splits(frames)
         if self._side is None:
             # pooling runs at the lowest priority, the compute-bound kernels of `step` on a high-priority stream:
             # the block scheduler then places regression / projection / attention CTAs as soon as resources free
@@ -557,23 +597,29 @@ class BatchedRectLTM(_BatchedBase):
             check(lib().ltm_event_record(events[0], sp), "event_record")
         tab = tables.rect_tables(L, self.N, self.tau, self.S, spacing=self.spacing)
         binned = lens is None and bool(update) and self._bin_ok(Bv, L, tab)
-        if lens is not None:
-            frames = sum(lens)
-            lt.record_stream(self._side)
-            check(lib().ltm_pool_mean_ragged(ptr(k_next), 0, ptr(ws["xbufs"][b]), C.c_void_p(lt.data_ptr() + 4 * Bv),
-                                             Bv, L, self.T, self.e, self._splits(frames) if frames else 1, frames,
-                                             int(self.pool_ctas), sp), "pool_mean_ragged")
-        elif binned:
-            check(lib().ltm_pool_bins(ptr(k_next), ptr(ws["xbufs"][b]), ptr(tab.to(self.device)["fbin_ptr"]), Bv, L,
-                                      self.T, self.e, tab.xb_rows, sp), "pool_bins")
-        else:
-            check(lib().ltm_pool_mean_grid(ptr(k_next), ptr(ws["xbufs"][b]), Bv, L, self.T, self.e, ws["splits"],
-                                           int(self.pool_ctas), sp), "pool_mean")
+        if offs is not None:
+            offs.record_stream(self._side)
+        self._pool_launch(k_next, ws["xbufs"][b], Bv, L, splits, int(self.pool_ctas), sp, offs=offs, frames=frames,
+                          bins=tab if binned else None)
         if events is not None:
             check(lib().ltm_event_record(events[1], sp), "event_record")
         check(lib().ltm_event_record(ev["pooled"][b], sp), "event_record")
         self._pref.append(dict(ref=weakref.ref(k_next), ver=k_next._version, buf=b, event=ev["pooled"][b],
                                captured=torch.cuda.is_current_stream_capturing(), binned=binned, lens=lens))
+
+    def _pool_launch(self, k, out, Bv, L, splits, max_ctas, stream, offs=None, frames=0, bins=None, dtype=0):
+        """Pool chunk k[Bv, L*T, e] into `out` on `stream`: the packed frames of a ragged chunk (offs: device frame
+        offsets, `frames` in all; dtype 0 / 1 / 2: float32 / float16 / bfloat16 storage), the per-bin sums of an update
+        chunk (bins: its tables) or per-frame means.  max_ctas bounds the grid (0 = one CTA per unit)."""
+        if offs is not None:
+            check(lib().ltm_pool_mean_ragged(ptr(k), dtype, ptr(out), ptr(offs), Bv, L, self.T, self.e, splits, frames,
+                                             max_ctas, stream), "pool_mean_ragged")
+        elif bins is not None:
+            check(lib().ltm_pool_bins(ptr(k), ptr(out), ptr(bins.to(self.device)["fbin_ptr"]), Bv, L, self.T, self.e,
+                                      bins.xb_rows, stream), "pool_bins")
+        else:
+            check(lib().ltm_pool_mean_grid(ptr(k), ptr(out), Bv, L, self.T, self.e, splits, max_ctas, stream),
+                  "pool_mean")
 
     def _sync_events(self):
         if self._evs is None:
@@ -641,13 +687,11 @@ class BatchedRectLTM(_BatchedBase):
                 raise ValueError("a ragged chunk is pooled from float32 / float16 / bfloat16 storage, without with_half")
             lens = _as_lengths(lengths, Bv, L)
             frames = sum(lens)
-            splits = self._splits(frames) if frames else 1
+            splits = self._splits(frames)
             out = torch.empty(frames, splits, e, device=self.device, dtype=torch.float32)
             if frames:
-                lt = self._lengths_dev(lens)
-                check(lib().ltm_pool_mean_ragged(ptr(k), dtype, ptr(out), C.c_void_p(lt.data_ptr() + 4 * Bv), Bv, L,
-                                                 self.T, e, splits, frames, 0, stream_ptr(self.device)),
-                      "pool_mean_ragged")
+                self._pool_launch(k, out, Bv, L, splits, 0, stream_ptr(self.device), offs=self._lengths_dev(lens)[1],
+                                  frames=frames, dtype=dtype)
             return out
         if with_half:
             x, k16 = ops.pool_mean_convert(k.view(Bv, L, self.T, e), self._splits(Bv * L))
@@ -672,52 +716,15 @@ class BatchedRectLTM(_BatchedBase):
         if (k.dtype != torch.float32 and pooled is None) or q.dtype != torch.float32:
             raise ValueError("k must be float32 / float16 / bfloat16 and q float32")
         k, q = k.contiguous(), q.contiguous()
-        rag = None
-        if lengths is None:
-            Bv, L, Q, tab, tdev, flags = self._prepare(k.shape, q.shape, new_doc)
-            need_u = self.has_state and self.sticky
-        else:
-            Bv, L, Q, tab, tdev, flags, rag = self._prepare_ragged(k.shape, q.shape, new_doc, lengths)
-            need_u = rag["need_u"]
+        Bv, L, Q, tab, tdev, flags, u, rag = self._prepare(k, q, new_doc, u, lengths, pooled)
         ws = self._workspace(Bv, L, Q)
         if rag is not None:
             self._ragged_ws(ws, Bv, L)
-        if pooled is not None:
-            if rag is None and (tuple(pooled.shape[:2]) != (Bv, L) or pooled.shape[3] != self.e):
-                raise ValueError("pooled frames do not match k")
-            if rag is not None and (pooled.dim() != 3 or pooled.shape[0] != rag["frames"] or pooled.shape[2] != self.e):
-                raise ValueError(f"pooled frames of a ragged chunk must be [{rag['frames']}, splits, {self.e}]")
-            if not pooled.is_contiguous():
-                raise ValueError("pooled frames do not match k")
-            if need_u:
-                if u is None or u.dtype != torch.float64 or tuple(u.shape) != (Bv, self.S):
-                    raise ValueError(f"sticky re-sampling needs u: float64 [{Bv},{self.S}]")
-                u = u.contiguous()
-            ctx = torch.empty(Bv, Q, self.D, device=self.device, dtype=torch.float32)
-            a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=bool(beside_pooling), rag=rag)
-            a.xpart, a.splits, a.binned = pooled.data_ptr(), pooled.shape[-2], 0
-            check(lib().ltm_rect_step(C.byref(a), None, ptr(q), ptr(u if rag is None or need_u else None),
-                                      ptr(flags), ptr(ctx), stream_ptr(self.device)), "rect_step")
-            self._finish(ws, pooled, rag=rag)
-            return ctx
-        if need_u:
-            if u is None or u.dtype != torch.float64 or tuple(u.shape) != (Bv, self.S):
-                raise ValueError(f"sticky re-sampling needs u: float64 [{Bv},{self.S}]")
-            u = u.contiguous()
-        elif rag is not None:
-            u = None
         ctx = torch.empty(Bv, Q, self.D, device=self.device, dtype=torch.float32)
-        hit = self._pref_take(k, None if rag is None else rag["lens"])
-        # every video continues: per-bin pooling is possible (lock-step only)
-        update = rag is None and self.has_state and flags is None
-        if hit is not None and hit["binned"] and not update:
-            hit = None                                   # pooled per bin for an update that did not come: pool again
-        pooled = hit is not None
+        hit = self._frames_source(k, Q, ws, tab, flags, rag, pooled)
         main = torch.cuda.current_stream(self.device)
         run = main
-        if pooled:
-            ws["xi"] = hit["buf"]
-            ws["xtag"][hit["buf"]] = hit["binned"]
+        if hit is not None:
             run = self._compute                      # fork: high-priority compute stream, joined below
             ev = self._sync_events()
             rp, mp = C.c_void_p(run.cuda_stream), C.c_void_p(main.cuda_stream)
@@ -727,22 +734,20 @@ class BatchedRectLTM(_BatchedBase):
             # and on replay the buffer is the one the previous replay's last prefetch filled)
             if hit["captured"] or not torch.cuda.is_current_stream_capturing():
                 check(lib().ltm_stream_wait_event(rp, hit["event"]), "stream_wait_event")
-        else:
-            held = {e["buf"] for e in self._pref}          # never pool over frames a pending prefetch still owns
-            ws["xi"] = (1 - ws["xi"]) if (1 - ws["xi"]) not in held else ws["xi"]
-            if ws["xi"] in held:
-                self._pref[:] = [e for e in self._pref if e["buf"] != ws["xi"]]
-            ws["xtag"][ws["xi"]] = update and self._bin_ok(Bv, L, tab)
         # (a pending prefetch = the next chunk is being pooled on the side stream while this step runs)
-        a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=bool(self._pref) or bool(beside_pooling), rag=rag)
+        beside = bool(beside_pooling) or (pooled is None and bool(self._pref))
+        a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=beside, rag=rag)
+        if pooled is not None:
+            a.xpart, a.splits, a.binned = pooled.data_ptr(), pooled.shape[-2], 0
         if rag is not None and run is not main:
-            rag["dev"].record_stream(run)
-        check(lib().ltm_rect_step(C.byref(a), None if pooled else ptr(k), ptr(q), ptr(u), ptr(flags), ptr(ctx),
+            rag["lens_dev"].record_stream(run)
+        pool_here = pooled is None and hit is None
+        check(lib().ltm_rect_step(C.byref(a), ptr(k) if pool_here else None, ptr(q), ptr(u), ptr(flags), ptr(ctx),
                                   C.c_void_p(run.cuda_stream)), "rect_step")
-        if pooled:
+        if hit is not None:
             check(lib().ltm_event_record(ev["join"], rp), "event_record")
             check(lib().ltm_stream_wait_event(mp, ev["join"]), "stream_wait_event")
-        self._finish(ws, k=k, rag=rag)
+        self._finish(ws, pooled, k=k, rag=rag)
         return ctx
 
     @_on_device
@@ -760,35 +765,14 @@ class BatchedRectLTM(_BatchedBase):
         if k.dtype != torch.float32 or q.dtype != torch.float32 or (k_next is not None and k_next.dtype != torch.float32):
             raise ValueError("step_overlapped takes float32 tensors")
         k, q = k.contiguous(), q.contiguous()
-        rag = None
-        if lengths is None:
-            Bv, L, Q, tab, tdev, flags = self._prepare(k.shape, q.shape, new_doc)
-            need_u = self.has_state and self.sticky
-        else:
-            Bv, L, Q, tab, tdev, flags, rag = self._prepare_ragged(k.shape, q.shape, new_doc, lengths)
-            need_u = rag["need_u"]
+        Bv, L, Q, tab, tdev, flags, u, rag = self._prepare(k, q, new_doc, u, lengths)
         ws = self._workspace(Bv, L, Q)
         if rag is not None or next_lengths is not None:
             self._ragged_ws(ws, Bv, L)
-        if need_u:
-            if u is None or u.dtype != torch.float64 or tuple(u.shape) != (Bv, self.S):
-                raise ValueError(f"sticky re-sampling needs u: float64 [{Bv},{self.S}]")
-            u = u.contiguous()
-        elif rag is not None:
-            u = None
-        lens = None if rag is None else rag["lens"]
-        hit = self._pref_take(k, lens)
-        update = rag is None and self.has_state and flags is None
-        if hit is not None and hit["binned"] and not update:
-            hit = None                                   # pooled per bin for an update that did not come: pool again
-        if hit is None:
-            self.prefetch(k, Q, lengths=lens, update=update)
-            hit = self._pref_take(k, lens)
+        hit = self._frames_source(k, Q, ws, tab, flags, rag, prefetch=True)
         ev = self._sync_events()
         main = torch.cuda.current_stream(self.device)
         capturing = torch.cuda.is_current_stream_capturing()
-        ws["xi"] = hit["buf"]
-        ws["xtag"][hit["buf"]] = hit["binned"]
         o = Overlap()
         o.main_stream, o.side_stream, o.compute_stream = main.cuda_stream, self._side.cuda_stream, self._compute.cuda_stream
         o.ev_fork, o.ev_join = ev["fork"], ev["join"]
@@ -801,11 +785,11 @@ class BatchedRectLTM(_BatchedBase):
             nl = None
             if next_lengths is not None:
                 nl = _as_lengths(next_lengths, Bv, L)
-                nt = self._lengths_dev(nl)
-                nt.record_stream(self._side)
+                nl_dev, noffs_dev = self._lengths_dev(nl)
+                nl_dev.record_stream(self._side)
                 nf = sum(nl)
-                o.next_lengths, o.next_offs = nt.data_ptr(), nt.data_ptr() + 4 * Bv
-                o.next_frames, o.next_splits = nf, self._splits(nf) if nf else 1
+                o.next_lengths, o.next_offs = nl_dev.data_ptr(), noffs_dev.data_ptr()
+                o.next_frames, o.next_splits = nf, self._splits(nf)
                 nb = False
             else:
                 nb = (not next_new_doc) and self._bin_ok(Bv, L, tab)
@@ -817,7 +801,7 @@ class BatchedRectLTM(_BatchedBase):
         ctx = torch.empty(Bv, Q, self.D, device=self.device, dtype=torch.float32)   # main joins the compute stream
         a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=k_next is not None, rag=rag)
         if rag is not None:
-            rag["dev"].record_stream(self._compute)
+            rag["lens_dev"].record_stream(self._compute)
         check(lib().ltm_rect_step_overlap(C.byref(a), C.byref(o), ptr(q), ptr(u), ptr(flags), ptr(ctx)),
               "rect_step_overlap")
         self._finish(ws, k=k, rag=rag)
@@ -830,7 +814,9 @@ class BatchedRectLTM(_BatchedBase):
         synchronises the stream before reading it."""
         if k_host.is_cuda or q_host.is_cuda:
             raise ValueError("step_host takes host tensors")
-        Bv, L, Q, tab, tdev, flags = self._prepare(k_host.shape, q_host.shape, new_doc)
+        if k_host.dtype != torch.float32 or q_host.dtype != torch.float32:
+            raise ValueError("step_host takes float32 k and q")
+        Bv, L, Q, tab, tdev, flags, u_host, _ = self._prepare(k_host, q_host, new_doc, u_host, u_name="u_host")
         ws = self._workspace(Bv, L, Q)
         dev = self.device
         if ws["k_dev"] is None:
@@ -841,18 +827,12 @@ class BatchedRectLTM(_BatchedBase):
             ws["ctx_dev"] = torch.empty(Bv, Q, self.D, device=dev, dtype=torch.float32)
         if out is None:
             out = torch.empty(Bv, Q, self.D, dtype=torch.float32, pin_memory=True)
-        need_u = self.has_state and self.sticky
-        if need_u and (u_host is None or u_host.dtype != torch.float64 or tuple(u_host.shape) != (Bv, self.S)):
-            raise ValueError(f"sticky re-sampling needs u_host: float64 [{Bv},{self.S}]")
-        if k_host.dtype != torch.float32 or q_host.dtype != torch.float32:
-            raise ValueError("step_host takes float32 k and q")
         ws["xtag"][ws["xi"]] = False          # the host path pools per frame
         a = self._args(Bv, L, Q, ws, tab, tdev)
         nd_host = None
         if flags is not None:
             nd_host = torch.as_tensor(new_doc).to(torch.uint8).contiguous()
-        check(lib().ltm_rect_step_host(C.byref(a), ptr(k_host.contiguous()), ptr(q_host.contiguous()),
-                                       ptr(u_host.contiguous()) if need_u else None,
+        check(lib().ltm_rect_step_host(C.byref(a), ptr(k_host.contiguous()), ptr(q_host.contiguous()), ptr(u_host),
                                        ptr(nd_host), ptr(out), stream_ptr(dev)), "rect_step_host")
         self._keep = (k_host, q_host, u_host, nd_host)      # keep host buffers alive until the stream drains
         self._finish(ws)

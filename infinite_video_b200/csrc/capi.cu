@@ -43,6 +43,15 @@ extern "C" int ltm_device_check(void) {
   return 0;
 }
 
+// Frame pooling of one chunk of the geometry of `a` into xpart: packed frames of a ragged chunk (offs != NULL: frame
+// offsets, `frames` in all), per-bin sums (binned) or per-frame means.  max_ctas bounds the grid (0 = one CTA per unit).
+static int pool_chunk(const ltm_rect_step_args* a, const float* k, float* xpart, const int32_t* offs, int frames,
+                      int splits, bool binned, int max_ctas, void* stream) {
+  if (offs) return ltm_pool_mean_ragged(k, 0, xpart, offs, a->Bv, a->L, a->T, a->e, splits, frames, max_ctas, stream);
+  if (binned) return ltm_pool_bins(k, xpart, a->fbin_ptr, a->Bv, a->L, a->T, a->e, a->xb_rows, stream);
+  return ltm_pool_mean_grid(k, xpart, a->Bv, a->L, a->T, a->e, splits, max_ctas, stream);
+}
+
 // ------------------------------------------------------------------------------------------------
 // One chunk of variant R for Bv videos:  pool -> (re-sample) -> consolidate -> project K,V ->
 // continuous attention (+ next call's sticky histogram).  long_term_attention_gibbs.py:288-346.
@@ -79,10 +88,7 @@ extern "C" int ltm_rect_step(const ltm_rect_step_args* a, const float* k, const 
   }
   if (k != nullptr) {          // k == NULL: a->xpart was already filled (frame pooling is stateless and may be
     LTM_PROF(0);               // issued ahead of time on another stream, see BatchedRectLTM.prefetch)
-    rc = ragged ? ltm_pool_mean_ragged(k, 0, a->xpart, a->frame_offs, a->Bv, a->L, a->T, a->e, a->splits, a->frames, 0,
-                                       stream)
-         : binned ? ltm_pool_bins(k, a->xpart, a->fbin_ptr, a->Bv, a->L, a->T, a->e, a->xb_rows, stream)
-                  : ltm_pool_mean(k, a->xpart, a->Bv, a->L, a->T, a->e, a->splits, stream);
+    rc = pool_chunk(a, k, a->xpart, ragged ? a->frame_offs : nullptr, a->frames, a->splits, binned, 0, stream);
     if (rc) return rc;
     LTM_PROF(1);
   }
@@ -156,56 +162,36 @@ extern "C" int ltm_rect_step(const ltm_rect_step_args* a, const float* k, const 
                                  a->S, ragged ? lengths + v0 : nullptr, ragged ? a->frame_offs + v0 : nullptr, stream);
     if (rc) return rc;
     if (!blocked) { LTM_PROF(5); LTM_PROF(6); }
+    // K|V projection KV = B_new W_kv^T + b_kv (fp16 operands: the fp16 copy of the new coefficient rows and of the
+    // weights, kind::f16 UMMAs; K|V for the tensor-core attention is stored as fp16 or rounded to the tf32 grid)
+    ltm_gemm_args ga;
+    memset(&ga, 0, sizeof(ga));
+    ga.A = half_ops ? reinterpret_cast<const float*>(Bh) : Bn; ga.lda = a->e; ga.a_kmajor = 1;
+    ga.B = half_ops ? reinterpret_cast<const float*>(a->Wkv_half) : a->Wkv; ga.ldb = a->e; ga.b_kmajor = 1;
+    ga.ab_fp16 = half_ops ? 1 : 0;
+    ga.K1 = a->e; ga.bias = a->bkv;
+    ga.C = KVn; ga.ldc = 2 * D;
+    ga.M = nv * a->N; ga.Nc = 2 * D; ga.K = a->e; ga.batch = 1;
+    // (the transposed-key and generic projections ignore proj_precision, except for the generic projected-memory rows)
+    ga.precision = half_ops ? 1 : (tcp || kvstate) ? pprec : a->precision;
+    ga.impl = a->gemm_impl; ga.round_tf32 = (tcp && !kvh) ? 1 : 0; ga.c_fp16 = kvh ? 1 : 0;
+    // (only the fp16-operand, fp16-K|V and projected-memory projections take the grid bound)
+    ga.max_ctas = (half_ops || kvh || kvstate) ? a->gemm_ctas : 0;
     if (kvstate) {
-      // rows [jf, N) of every video as one flat problem: A = B_new + jf * e grouped per video, C = KV + jf * 2D
-      ltm_gemm_args ga;
-      memset(&ga, 0, sizeof(ga));
-      // (fp16 operands: the fp16 copy of the new coefficient rows and of the weights, kind::f16 UMMAs)
+      // rows [jg, N) of every video as one flat problem: A = B_new + jg * e grouped per video, C = KV + jg * 2D
       ga.A = half_ops ? reinterpret_cast<const float*>(reinterpret_cast<const uint16_t*>(Bh) + (size_t)jg * a->e)
                       : Bn + (size_t)jg * a->e;
-      ga.lda = a->e; ga.a_kmajor = 1;
       ga.a_group = n_new; ga.a_group_stride = (int64_t)a->N * a->e;
-      ga.B = half_ops ? reinterpret_cast<const float*>(a->Wkv_half) : a->Wkv; ga.ldb = a->e; ga.b_kmajor = 1;
-      ga.ab_fp16 = half_ops ? 1 : 0;
-      ga.K1 = a->e; ga.bias = a->bkv;
       ga.C = kvh ? reinterpret_cast<float*>(reinterpret_cast<uint16_t*>(KVn) + (size_t)jg * 2 * D)
                  : KVn + (size_t)jg * 2 * D;
-      ga.ldc = 2 * D;
       ga.c_group = n_new; ga.c_group_stride = (int64_t)a->N * 2 * D;
-      ga.M = nv * n_new; ga.Nc = 2 * D; ga.K = a->e; ga.batch = 1;
-      ga.precision = half_ops ? 1 : pprec; ga.impl = a->gemm_impl; ga.round_tf32 = (tcp && !kvh) ? 1 : 0;
-      ga.c_fp16 = kvh ? 1 : 0;
-      ga.max_ctas = a->gemm_ctas;
-      rc = ltm_gemm(&ga, stream);
-    } else if (half_ops) {
-      ltm_gemm_args ga;
-      memset(&ga, 0, sizeof(ga));
-      ga.A = reinterpret_cast<const float*>(Bh); ga.lda = a->e; ga.a_kmajor = 1;
-      ga.B = reinterpret_cast<const float*>(a->Wkv_half); ga.ldb = a->e; ga.b_kmajor = 1;
-      ga.K1 = a->e; ga.bias = a->bkv;
-      ga.C = KVn; ga.ldc = 2 * D;
-      ga.M = nv * a->N; ga.Nc = 2 * D; ga.K = a->e; ga.batch = 1;
-      ga.precision = 1; ga.impl = 0; ga.round_tf32 = kvh ? 0 : 1; ga.ab_fp16 = 1; ga.c_fp16 = kvh ? 1 : 0;
-      ga.max_ctas = a->gemm_ctas;
-      rc = ltm_gemm(&ga, stream);
-    } else if (kvh) {
-      ltm_gemm_args ga;
-      memset(&ga, 0, sizeof(ga));
-      ga.A = Bn; ga.lda = a->e; ga.a_kmajor = 1;
-      ga.B = a->Wkv; ga.ldb = a->e; ga.b_kmajor = 1;
-      ga.K1 = a->e; ga.bias = a->bkv;
-      ga.C = KVn; ga.ldc = 2 * D;
-      ga.M = nv * a->N; ga.Nc = 2 * D; ga.K = a->e; ga.batch = 1;
-      ga.precision = pprec; ga.impl = a->gemm_impl; ga.c_fp16 = 1;
-      ga.max_ctas = a->gemm_ctas;
-      rc = ltm_gemm(&ga, stream);
-    } else if (tcp)
-      rc = ltm_project_kv_r(Bn, a->Wkv, a->bkv, KVn, nv * a->N, a->e, 2 * D, pprec, a->gemm_impl, stream);
-    else if (fast)
-      rc = ltm_project_kv_t(Bn, a->Wkv, a->bkv, a->Kt, a->V, nv * a->N, a->e, D, a->N, a->precision, a->gemm_impl,
-                            stream);
-    else
-      rc = ltm_project_kv(Bn, a->Wkv, a->bkv, KVn, nv * a->N, a->e, 2 * D, a->precision, a->gemm_impl, stream);
+      ga.M = nv * n_new;
+    } else if (fast) {
+      // keys transposed per head for the fast attention: Kt[Bv, H, d, N], values V[Bv, N, D]
+      ga.C = a->V; ga.ldc = D;
+      ga.CT = a->Kt; ga.ct_cols = D; ga.ct_group = a->N;
+    }
+    rc = ltm_gemm(&ga, stream);
     if (rc) return rc;
     if (!blocked) { LTM_PROF(7); LTM_PROF(8); }
     const float* qb = q + (size_t)v0 * a->Q * D;
@@ -310,12 +296,9 @@ extern "C" int ltm_rect_step_overlap(const ltm_rect_step_args* a, const ltm_over
     LTM_OV_MARK(0);
     if (a->prof_events[0]) cudaEventRecord((cudaEvent_t)a->prof_events[0], ss);
     LTM_REQUIRE(!o->next_lengths || (o->next_offs && !o->next_binned), "rect_step_overlap: ragged next chunk");
-    int rc = o->next_lengths
-                 ? ltm_pool_mean_ragged(o->k_next, 0, o->xpart_next, o->next_offs, a->Bv, a->L, a->T, a->e,
-                                        o->next_splits, o->next_frames, o->pool_ctas, ss)
-             : o->next_binned
-                 ? ltm_pool_bins(o->k_next, o->xpart_next, a->fbin_ptr, a->Bv, a->L, a->T, a->e, a->xb_rows, ss)
-                 : ltm_pool_mean_grid(o->k_next, o->xpart_next, a->Bv, a->L, a->T, a->e, a->splits, o->pool_ctas, ss);
+    const bool ragged_next = o->next_lengths != nullptr;
+    int rc = pool_chunk(a, o->k_next, o->xpart_next, ragged_next ? o->next_offs : nullptr, o->next_frames,
+                        ragged_next ? o->next_splits : a->splits, o->next_binned != 0, o->pool_ctas, ss);
     if (rc) return rc;
     if (a->prof_events[1]) cudaEventRecord((cudaEvent_t)a->prof_events[1], ss);
     LTM_OV_MARK(1);
