@@ -25,13 +25,32 @@ from . import ops
 from .ltm import LongTermAttention
 
 
+def encoder_mask_rows(mask, B, LT, device=None):
+    """The caller's additive encoder mask as a contiguous float32 [B, LT] (one row per video, shared by every head and
+    query), or None.  Accepted: [B, LT], [B, 1, LT] and [B, 1, 1, LT] in any float dtype -- the last is what HF's
+    `invert_attention_mask` makes of a 2-D mask over the encoder tokens, in the model's dtype (fp16 under autocast).
+    Anything else raises ValueError: a mask of batch 1 broadcast over B > 1 videos, a mask that varies per query or
+    per head, a wrong LT, an integer or boolean mask, or (with `device`) a mask on another device."""
+    if mask is None:
+        return None
+    shape = tuple(mask.shape)
+    if shape not in ((B, LT), (B, 1, LT), (B, 1, 1, LT)):
+        raise ValueError(f"encoder_attention_mask of shape {list(shape)}: expected [B, LT], [B, 1, LT] or "
+                         f"[B, 1, 1, LT] with B = {B}, LT = {LT} (per-query and per-head masks are not supported)")
+    if not mask.is_floating_point():
+        raise ValueError(f"encoder_attention_mask must be an additive float mask, got {mask.dtype}")
+    if device is not None and mask.device != torch.device(device):
+        raise ValueError(f"encoder_attention_mask is on {mask.device}, the chunk on {device}")
+    return mask.reshape(B, LT).float().contiguous()
+
+
 class CrossAttentionLTM(nn.Module):
     """Drop-in for the cross-attention use of `BertSelfAttention` (eval mode, absolute position embeddings, no head
     mask).  Construct from the caller's own `query` / `key` / `value` `nn.Linear`s and its config values."""
 
     def __init__(self, query: nn.Linear, key: nn.Linear, value: nn.Linear, alpha: float, num_basis: int, tau: float,
                  sticky: bool = True, n_heads: int = 12, tokens_per_frame: int = 32, videos_per_pass: int = 32,
-                 precision: str = "tf32", score_precision: str = None, value_precision: str = None,
+                 precision: str = "tf32x3", score_precision: str = None, value_precision: str = None,
                  operands: str = "fp16", **ltm_kwargs):
         super().__init__()
         self.query, self.key, self.value = query, key, value
@@ -44,11 +63,14 @@ class CrossAttentionLTM(nn.Module):
         self.precision = precision
         # the two large contractions (scores = Qt enc^T, Y = probs enc); the three small ones always run split-TF32.
         # Measured (scripts/stm_probe.py, error vs fp64 at L*T = 8192 / 256, time at 16 videos):
-        #   scores x1 (Qt rounded to tf32) / values x3   2.6e-4 / 2.1e-4   0.80 ms   <- default
+        #   scores x1 (Qt rounded to tf32) / values x3   2.6e-4 / 2.1e-4   0.80 ms
         #   scores x3 / values x1                         4.5e-4 / 9.4e-4   0.87 ms
         #   x1 / x1                                       5.8e-4 / 9.2e-4   0.59 ms
-        #   x3 / x3                                       3.9e-5 / 1.2e-5   1.08 ms
-        # (the value contraction reads the raw chunk, which the tensor core truncates: its bias is the larger error)
+        #   x3 / x3                                       3.9e-5 / 1.2e-5   1.08 ms   <- default
+        # (a single pass reads the raw chunk, which the tensor core truncates: a bias that shrinks every score by about
+        # 2^-11 of itself, so its error grows with the logits.  Single-pass scores reach 1.1e-3 at logits of std 1.2,
+        # VideoChat2 widths (tests/test_gpu_cross_attention.py): split-TF32 scores are the default.  This is also the
+        # path "fp16" operands fall back to, where it must not be less accurate than the fp16 path it stands in for)
         self.score_precision = score_precision or precision
         self.value_precision = value_precision or "tf32x3"
         # operands of the two large contractions.  "fp16" (default): the chunk tokens are converted ONCE per chunk to
@@ -78,12 +100,14 @@ class CrossAttentionLTM(nn.Module):
     @torch.no_grad()
     def short_term(self, q, enc, mask=None, enc16=None):
         """softmax(q_h K_h^T / sqrt(d) + mask) V_h for all heads.  q[B,Q,D] (already projected), enc[B,LT,e] fp32,
-        mask: additive [B, LT] or None; enc16: the chunk as float16 when the caller already has it (the pooling pass of
-        the LTM writes it, `LongTermAttention.pool_for_caller`).  Returns [B,Q,D]."""
+        mask: additive, one row per video ([B, LT], [B, 1, LT] or [B, 1, 1, LT], `encoder_mask_rows`) or None; enc16:
+        the chunk as float16 when the caller already has it (the pooling pass of the LTM writes it,
+        `LongTermAttention.pool_for_caller`).  Returns [B,Q,D]."""
         B, Q, D = q.shape
         LT, e = enc.shape[1], enc.shape[2]
         H, d = self.H, self.d
         dev = q.device
+        mask = encoder_mask_rows(mask, B, LT, dev)
         wk = self.key.weight.detach().float().contiguous()          # [D, e]
         wv = self.value.weight.detach().float().contiguous()
         bv = self.value.bias.detach().float().contiguous() if self.value.bias is not None else None
@@ -104,7 +128,7 @@ class CrossAttentionLTM(nn.Module):
                 ops.gemm_raw(Qt, e, H * Q * e, True, e16, e, LT * e, True, S, LT, H * Q * LT, H * Q, LT, e, nb,
                              precision="tf32", ab_fp16=True)
                 # (3) probabilities as fp16
-                m = None if mask is None else mask[v0:v0 + nb].float().contiguous()
+                m = None if mask is None else mask[v0:v0 + nb]
                 P = ops.softmax_rows_half(S, 1.0 / math.sqrt(d), m, H * Q)
                 # (4) Yh[h][v][q][:] = probs enc[v] : A fp16 K-major, B = enc16[v] read as [K = LT][N = e] (MN-major)
                 Yh = torch.empty(H, nb, Q, e, device=dev, dtype=torch.float32)
@@ -125,7 +149,7 @@ class CrossAttentionLTM(nn.Module):
             ops.gemm_raw(Qt, e, H * Q * e, True, ev, e, LT * e, True, S, LT, H * Q * LT, H * Q, LT, e, nb,
                          precision=self.score_precision)
             # (3) probs = softmax(scores / sqrt(d) + mask), in place
-            m = None if mask is None else mask[v0:v0 + nb].float().contiguous()
+            m = None if mask is None else mask[v0:v0 + nb]
             ops.softmax_rows(S, 1.0 / math.sqrt(d), m, H * Q)
             # (4) Yh[h][v][q][:] = probs[v][(h,q)] enc[v] : B operand = enc[v] read as [K = LT][N = e] (MN-major)
             Yh = torch.empty(H, nb, Q, e, device=dev, dtype=torch.float32)
@@ -143,12 +167,12 @@ class CrossAttentionLTM(nn.Module):
         if not hidden_states.is_cuda:
             raise RuntimeError("CrossAttentionLTM runs on CUDA tensors only (no CPU fallback)")
         B, Q, _ = hidden_states.shape
-        enc = encoder_hidden_states.float().contiguous()
+        # HF additive mask [B,1,1,LT] -> [B,LT], validated before anything is launched
+        enc = encoder_hidden_states
+        mask = encoder_mask_rows(encoder_attention_mask, B, enc.shape[1], enc.device)
+        enc = enc.float().contiguous()
         q = self._linear(hidden_states.float().reshape(B * Q, -1).contiguous(), self.query, "tf32x3")
         q = q.view(B, Q, -1)
-        mask = None
-        if encoder_attention_mask is not None:                       # HF additive mask [B,1,1,LT] -> [B,LT]
-            mask = encoder_attention_mask.reshape(B, -1)
         ltm = self.long_term_attention
         enc16 = None
         if (self.alpha != 1.0 and self.operands == "fp16" and ltm.variant == "gibbs" and ltm.share_pooling

@@ -275,6 +275,19 @@ def gemm_fp16(A, B, bias=None, out=None, round_tf32=False):
     return out
 
 
+def _check_softmax_mask(S, mask, rows, n, rows_per_mask, what):
+    """The kernels read mask row `row // rows_per_mask` at pitch n, unchecked: the mask must hold exactly those rows."""
+    if mask is None:
+        return
+    if mask.dtype != torch.float32 or not mask.is_contiguous() or mask.device != S.device:
+        raise ValueError(f"{what}: the mask must be a contiguous float32 tensor on {S.device}, got {mask.dtype} "
+                         f"on {mask.device}")
+    if rows_per_mask <= 0 or rows % rows_per_mask:
+        raise ValueError(f"{what}: rows_per_mask={rows_per_mask} must divide rows={rows}")
+    if mask.numel() != (rows // rows_per_mask) * n:
+        raise ValueError(f"{what}: the mask has {mask.numel()} elements, {rows // rows_per_mask} rows of {n} expected")
+
+
 def softmax_rows(S, scale=1.0, mask=None, rows_per_mask=1):
     """In place: S[rows, n] <- softmax(S * scale + mask[row // rows_per_mask]).  Qformer.py:279-285."""
     require_cuda(S, mask)
@@ -282,6 +295,7 @@ def softmax_rows(S, scale=1.0, mask=None, rows_per_mask=1):
         raise ValueError("softmax_rows needs a contiguous float32 tensor")
     n = S.shape[-1]
     rows = S.numel() // n
+    _check_softmax_mask(S, mask, rows, n, rows_per_mask, "softmax_rows")
     check(lib().ltm_softmax_rows(ptr(S), ptr(mask), rows, n, rows_per_mask, float(scale), stream_ptr(S.device)),
           "softmax_rows")
     return S
@@ -294,6 +308,7 @@ def softmax_rows_half(S, scale=1.0, mask=None, rows_per_mask=1):
         raise ValueError("softmax_rows_half needs a contiguous float32 tensor")
     n = S.shape[-1]
     rows = S.numel() // n
+    _check_softmax_mask(S, mask, rows, n, rows_per_mask, "softmax_rows_half")
     P = torch.empty(S.shape, device=S.device, dtype=torch.float16)
     check(lib().ltm_softmax_rows_h(ptr(S), ptr(mask), ptr(P), rows, n, rows_per_mask, float(scale),
                                    stream_ptr(S.device)), "softmax_rows_h")

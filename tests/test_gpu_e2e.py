@@ -872,34 +872,67 @@ def test_fp16_chunk_through_the_drop_in(dev):
             assert relerr(got.float(), want) < 2e-3          # output rounded to fp16 (2^-11) on top of TOL_CTX
 
 
+# Video-LLaMA: T = 32 tokens per frame, e = D = 768, Q = 32;  VideoChat2 (BASELINE cfg3): T = 196, e = 1024, Q = 96
+CALLER_SHAPES = {"videollama": (32, 768, 32), "videochat2": (196, 1024, 96)}
+CALLER_MASKS = ("none", "last40", "every_third_frame", "one_frame_left", "all")
+
+
+def _caller_mask(B, L, T, c):
+    """HF's extended encoder mask [B,1,1,LT]: a different masking pattern per video and chunk, -10000 on even chunks
+    and finfo(float32).min on odd ones."""
+    value = -10000.0 if c % 2 == 0 else torch.finfo(torch.float32).min
+    m = torch.zeros(B, L, T)
+    for v in range(B):
+        kind = CALLER_MASKS[(v + 2 * c) % len(CALLER_MASKS)]
+        if kind == "last40":
+            m[v].view(-1)[int(round(.6 * L * T)):] = value
+        elif kind == "every_third_frame":
+            m[v, ::3] = value
+        elif kind == "one_frame_left":
+            m[v] = value
+            m[v, L // 2] = 0.0
+        elif kind == "all":
+            m[v] = value
+    return m.view(B, 1, 1, L * T)
+
+
 @pytest.mark.parametrize("operands", ["fp16", "fp32"])
-@pytest.mark.parametrize("alpha,N,L,B", [(0.5, 64, 8, 2), (0.9, 256, 64, 1), (0.7, 256, 256, 2)])
-def test_caller_cross_attention_with_ltm_blend_on_gpu(dev, alpha, N, L, B, operands):
+@pytest.mark.parametrize("mask", [False, True], ids=["nomask", "mask"])
+@pytest.mark.parametrize("shape,alpha,N,L,B", [("videollama", 0.5, 64, 8, 2), ("videollama", 0.9, 256, 64, 1),
+                                               ("videollama", 0.7, 256, 256, 2), ("videochat2", 0.5, 64, 16, 2)])
+def test_caller_cross_attention_with_ltm_blend_on_gpu(dev, shape, alpha, N, L, B, mask, operands):
     """N1: short-term softmax attention over the chunk + (1-alpha) LTM, against the oracle of the caller
-    (bit-identical to the real BertSelfAttention, tests/test_oracle_vs_reference.py)."""
+    (bit-identical to the real BertSelfAttention, tests/test_oracle_vs_reference.py), with and without an encoder
+    mask."""
     from infinite_video_b200.cross_attention import CrossAttentionLTM
+    T, e, Q = CALLER_SHAPES[shape]
     torch.manual_seed(21)
-    lq, lk, lv = torch.nn.Linear(768, 768), torch.nn.Linear(768, 768), torch.nn.Linear(768, 768)
+    lq, lk, lv = torch.nn.Linear(768, 768), torch.nn.Linear(e, 768), torch.nn.Linear(e, 768)
     orcs = [O.CrossAttentionLTM(N, .75, alpha, lq.weight.detach(), lq.bias.detach(), lk.weight.detach(),
-                                lk.bias.detach(), lv.weight.detach(), lv.bias.detach(), rebuild_tables=False)
+                                lk.bias.detach(), lv.weight.detach(), lv.bias.detach(), tokens_per_frame=T,
+                                rebuild_tables=False)
             for _ in range(B)]
     import copy
     m = CrossAttentionLTM(copy.deepcopy(lq).to(dev), copy.deepcopy(lk).to(dev), copy.deepcopy(lv).to(dev), alpha, N,
-                          .75, operands=operands)
+                          .75, tokens_per_frame=T, operands=operands)
     g = torch.Generator().manual_seed(22)
     with torch.no_grad():
         for c in range(3):
-            hidden = torch.randn(B, 32, 768, generator=g)
-            enc = torch.randn(B, L * 32, 768, generator=g)
+            hidden = torch.randn(B, Q, 768, generator=g)
+            enc = torch.randn(B, L * T, e, generator=g)
             u = torch.rand(B, 512, dtype=torch.float64, generator=g)
-            got = m(hidden.to(dev), enc.to(dev), new_video=(c == 0), layer=0, u=u)
+            am = _caller_mask(B, L, T, c) if mask else None
+            got = m(hidden.to(dev), enc.to(dev), new_video=(c == 0), layer=0, u=u,
+                    encoder_attention_mask=None if am is None else am.to(dev))
             b_got = m.long_term_attention._engine.last["b"].cpu().long() if c else None
             want = torch.cat([orcs[v].forward(hidden[v:v + 1], enc[v:v + 1], c == 0, u[v:v + 1],
+                                              mask=None if am is None else am[v:v + 1],
                                               b_override=b_got[v:v + 1] if c else None) for v in range(B)])
             if c:
                 compare_draws(b_got, torch.cat([o.ltm.last["b_own"] for o in orcs]), u,
                               torch.cat([o.ltm.last["p"] for o in orcs]), TIE["tf32"])
-            stm = m.short_term(torch.nn.functional.linear(hidden, lq.weight, lq.bias).to(dev), enc.to(dev))
+            stm = m.short_term(torch.nn.functional.linear(hidden, lq.weight, lq.bias).to(dev), enc.to(dev),
+                               None if am is None else am.to(dev))
             assert relerr(stm, torch.cat([o.last_stm for o in orcs])) < TOL_CTX, f"short-term, chunk {c}"
             assert relerr(got, want) < TOL_CTX, f"blend, chunk {c}"
 
