@@ -341,10 +341,6 @@ typedef struct {
    * jf > 0, every video takes the update branch (B_past != NULL, new_doc == NULL) and N - jf tiles 128 rows evenly;
    * otherwise all N rows are projected.  proj_precision: precision of the K/V projection GEMM (0 = `precision`). */
   const float* KV_past; int jf; int proj_precision;
-  /* > 0: consolidate / project / attend in blocks of this many videos, so that what a block writes (K|V, coefficient
-   * rows) is read back from L2; 0 or >= Bv: every kernel covers all videos.  In blocked mode only prof_events[4]
-   * (before the first block) and [9] (after the last) are recorded besides the pooling / re-sampling pairs. */
-  int video_block;
   /* workspace of the two-half tensor-core attention (num_basis 512): ltm_attn_tc_split_workspace_floats(Bv,Q,H)
    * floats; with it (and `scores`) set, num_basis 512 takes ltm_cont_attn_rect_tc_split */
   float* attn_part;

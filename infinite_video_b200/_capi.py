@@ -53,7 +53,7 @@ class RectStepArgs(C.Structure):
         ("prof_events", C.c_void_p * 10),
         ("X", C.c_void_p), ("c_none", C.c_float),
         ("B_half", C.c_void_p), ("Wkv_half", C.c_void_p),
-        ("KV_past", C.c_void_p), ("jf", C.c_int), ("proj_precision", C.c_int), ("video_block", C.c_int),
+        ("KV_past", C.c_void_p), ("jf", C.c_int), ("proj_precision", C.c_int),
         ("attn_part", C.c_void_p),
         ("kv_half", C.c_int), ("X16", C.c_void_p),
         ("binned", C.c_int), ("xb_rows", C.c_int),

@@ -174,9 +174,6 @@ class BatchedRectLTM(_BatchedBase):
         if kv_dtype not in ("fp32", "fp16"):
             raise ValueError("kv_dtype must be 'fp32' or 'fp16'")
         self.kv_half = kv_dtype == "fp16" and self.tc_attn
-        # consolidate / project / attend in blocks of this many videos (L2 reuse of what a block writes); 0 = off
-        # (measured at 128 videos: 16 / 32 / 43 / 64-video blocks all lose 4-14 % to the smaller kernels' tails)
-        self.video_block = 0
         self._Wkv_h = None
         self.prof_events = None       # optional list of 10 cudaEvent_t handles (bench.py stage timing)
         self._side = None             # side stream for pooling the next chunk ahead of time
@@ -330,7 +327,6 @@ class BatchedRectLTM(_BatchedBase):
             ws["_args"], ws["_args_sig"], ws["_args_prof"] = a, sig, False
             ws["_args_keep"] = (tdev, self.Wkv, self.bkv, self._hist)     # the block holds raw pointers into these
         a.splits = ws["splits"]
-        a.video_block = int(self.video_block)
         a.B_past = self._B[self._cur].data_ptr() if self.has_state else None
         a.B_new = self._B[1 - self._cur].data_ptr()
         a.xpart = ws["xbufs"][ws["xi"]].data_ptr()
@@ -412,6 +408,10 @@ class BatchedRectLTM(_BatchedBase):
         the contiguous uniforms (None: the step reads none) and, for a ragged step, its table bank and device lengths /
         offsets (rag; None: lock-step).  A lock-step call takes new_doc as a device tensor too, a ragged one as host
         flags (it selects tables from them)."""
+        if getattr(self, "video_block", 0):
+            # the step in blocks of videos (4-14 % slower at every block size) was removed; refusing the setting keeps
+            # a caller from running, and recording, a block size that has no effect
+            raise ValueError("video_block: the blocked step was removed; every kernel covers all videos")
         Bv, LT, e = k.shape
         if e != self.e:
             raise ValueError(f"k has width {e}, projections expect {self.e}")
@@ -578,10 +578,8 @@ class BatchedRectLTM(_BatchedBase):
             # pooling runs at the lowest priority, the compute-bound kernels of `step` on a high-priority stream:
             # the block scheduler then places regression / projection / attention CTAs as soon as resources free
             # up and the streaming kernel fills whatever is left
-            import os
-            flat = os.environ.get("LTM_FLAT_PRIORITY") == "1"        # bring-up: both streams at the default priority
             self._side = torch.cuda.Stream(device=self.device, priority=0)
-            self._compute = torch.cuda.Stream(device=self.device, priority=0 if flat else -1)
+            self._compute = torch.cuda.Stream(device=self.device, priority=-1)
         main = torch.cuda.current_stream(self.device)
         ev = self._sync_events()
         b = self._pref_buffer(ws)

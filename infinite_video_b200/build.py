@@ -10,10 +10,6 @@ SOURCES = ["pool.cu", "consolidate.cu", "sticky.cu", "attn.cu", "attn_fast.cu", 
            "capi.cu"]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC"]
-# INFLTM_BRINGUP=1: also compile the ltm_debug_* hooks the probes under scripts/ use (kernel variant switches, store /
-# load suppression, per-item timelines).  The product library is built without them.
-if os.environ.get("INFLTM_BRINGUP") == "1":
-    FLAGS = FLAGS + ["-DLTM_BRINGUP"]
 
 
 def _stale():

@@ -51,7 +51,6 @@ struct Params {
   // and attn_tc_combine_kernel merges the two halves (exp(m_half - m) rescaling, as in a two-block online softmax).
   int halves, NT;
   float* part;
-  unsigned long long* trace;   // bring-up: CTA 0 writes globaltimer stamps [item][16] (NULL = off)
 };
 constexpr int PART_ROWS = 68;
 
@@ -67,17 +66,6 @@ struct Lay {
   static constexpr int BYTES = MISC_OFF + MISC_FLOATS * 4 + 64 + 1024;   // + 6 barriers, TMEM slot, alignment slack
 };
 
-__device__ __forceinline__ void stamp(unsigned long long* trace, uint32_t it, int slot) {
-#ifndef LTM_BRINGUP
-  (void)trace; (void)it; (void)slot;          // the per-item timeline exists in bring-up builds only
-  return;
-#endif
-  if (trace != nullptr && blockIdx.x == 0 && it < 16) {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    trace[it * 16 + slot] = t;
-  }
-}
 __device__ __forceinline__ void cw_sync() { asm volatile("bar.sync 1, 256;" ::: "memory"); }   // the 8 compute warps
 
 // q tile of one work item, scaled by 1/sqrt(d) (gibbs:226; a power of two, exact) and rounded to tf32, in the
@@ -207,11 +195,10 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
       const uint64_t dV = umma_desc(sV, L_::SLAB, 512, 1u), dR = umma_desc(sR, 16, 1024, 2u);
       const uint32_t dk_lo = (uint32_t)dK, dk_hi = (uint32_t)(dK >> 32), dq_lo = (uint32_t)dQ;
       const uint32_t dv_lo = (uint32_t)dV, dv_hi = (uint32_t)(dV >> 32), dr_lo = (uint32_t)dR;
-      auto issue_scores = [&](uint32_t ph, uint32_t sit) {            // S^T of the item whose K tile / q tile carry parity ph
+      auto issue_scores = [&](uint32_t ph) {            // S^T of the item whose K tile / q tile carry parity ph
         mbar_wait(bar_q, ph);                          // q tile written, S read out of TMEM
         mbar_wait(bar_k, ph);
         tcgen05_fence_after();
-        if (threadIdx.x == 256) stamp(p.trace, sit, 5);
 #pragma unroll
         for (int hf = 0; hf < HALVES; ++hf) {
 #pragma unroll
@@ -224,23 +211,20 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
         tcgen05_commit(bar_s);
       };
       uint32_t it = 0;
-      issue_scores(0u, 0u);
+      issue_scores(0u);
       for (int w = w0; w < total; w += wstride, ++it) {
         const uint32_t ph = it & 1u;
         const int wn = w + wstride;
         int qtn = 0, hn = 0, vn = 0;
         if (wn < total) decode(wn, qtn, hn, vn);
         mbar_wait(bar_s, ph);                          // the K buffer has been read
-        stamp(p.trace, it, 0);
         if (wn < total) {
           mbar_arrive_expect_tx(bar_k, 2 * L_::SLAB);
           tma_load_2d(&mapK, sK, bar_k, hn * DH, jrow(wn, vn));
           tma_load_2d(&mapK, sK + L_::SLAB, bar_k, hn * DH + 32, jrow(wn, vn));
         }
         mbar_wait(bar_r, ph);                          // e^T written, D free
-        stamp(p.trace, it, 1);
         mbar_wait(bar_v, ph);
-        stamp(p.trace, it, 2);
         tcgen05_fence_after();
         // this warp contracts the first half of the basis range into D0, warp 9 the second half into D1: the issue
         // of 32 small MMAs by one thread (~33 ns each) was 1.05 us of the item's 4.7 us
@@ -250,12 +234,10 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
                            dr_lo + (uint32_t)(((ks >> 2) * 4096 + (ks & 3) * 32) >> 4), dk_hi, IDESC_PV,
                            ks != 0 ? 1u : 0u);
         tcgen05_commit(bar_pv);
-        stamp(p.trace, it, 3);
         // the next item's scores go out right behind: its keys landed during this item's weight phase, so S is
         // ready by the time the compute warps have written this item's outputs
-        if (wn < total) issue_scores(ph ^ 1u, it + 1);
+        if (wn < total) issue_scores(ph ^ 1u);
         mbar_wait(bar_pv, ph);                         // the V buffer (and e^T) have been read
-        stamp(p.trace, it, 4);
         if (wn < total) {
           // (the per-basis operand rows X change with the basis half: re-fetched with V when there are two)
           mbar_arrive_expect_tx(bar_v, (halves > 1 ? 3 : 2) * L_::SLAB);
@@ -332,7 +314,6 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
         rWj = 1.0f / Wj;
       }
       mbar_wait(bar_s, ph);
-      if (tid == 0) stamp(p.trace, it, 8);
       tcgen05_fence_after();
       if (active) {
         uint32_t r[32];
@@ -372,7 +353,6 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
         }
       }
       cw_sync();                                                                           // column maxima
-      if (tid == 0) stamp(p.trace, it, 9);
       if (active) {
         float M = 0.f;                                 // per-row shift m = max(0, max_j S_j): it cancels exactly
 #pragma unroll
@@ -390,7 +370,6 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
       }
       tcgen05_fence_before();
       mbar_arrive(bar_r);
-      if (tid == 0) stamp(p.trace, it, 10);
       if (wn + wstride < total) {                      // queries of item it + 2: consumed after the next bar_s
         int qtn, hn, vn;
         decode(wn + wstride, qtn, hn, vn);
@@ -399,7 +378,6 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
 
       // ---- outputs: D[lane m][q]; warp (quarter, chalf) reads 16 columns
       mbar_wait(bar_pv, ph);
-      if (tid == 0) stamp(p.trace, it, 11);
       tcgen05_fence_after();
       float dv[16];
       {
@@ -457,7 +435,6 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
         }
       }
       cw_sync();                                                                           // normalisers
-      if (tid == 0) stamp(p.trace, it, 12);
       if (quarter < 2) {
         const int dd = quarter * 32 + lane;
         float* dst = p.ctx + ((size_t)v * Q + q0 + chalf * 16) * D + h * DH + dd;
@@ -483,7 +460,6 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
               hdt * (Gs[hja] + Gs[hjb]);
         // no barrier before the next item: everything above is rewritten only behind the next item's first
         // cw_sync, which no thread passes before all of them have finished this item
-        if (tid == 0) stamp(p.trace, it, 13);
       }
     }
   }
@@ -547,12 +523,8 @@ static int launch(const CUtensorMap& mK, const CUtensorMap& mV, const CUtensorMa
   return 0;
 }
 
-static unsigned long long* g_trace = nullptr;
 }  // namespace tc
 }  // namespace ltm
-#ifdef LTM_BRINGUP
-extern "C" void ltm_debug_set_attn_trace(void* p) { ltm::tc::g_trace = (unsigned long long*)p; }
-#endif
 
 extern "C" int ltm_attn_tc_supported(int N, int d) { return (d == 64 && (N == 64 || N == 128 || N == 256)) ? 1 : 0; }
 extern "C" int ltm_attn_tc_split_supported(int N, int d) { return (d == 64 && N == 512) ? 1 : 0; }
@@ -583,7 +555,6 @@ static int cont_attn_rect_tc_impl(const float* q, const float* K, const float* V
   p.q = q; p.W = W; p.tb = tb; p.jb = jb; p.W_out = W_out; p.c_none = c_none; p.ctx = ctx;
   p.scores_out = scores_out; p.hist_part = hist_part; p.Q = Q; p.H = H;
   p.halves = halves; p.NT = N; p.part = part;
-  p.trace = tc::g_trace;
   if (NBk == 256) return tc::launch<256>(mK, mV, mX, p, Bv, (cudaStream_t)stream);
   if (NBk == 128) return tc::launch<128>(mK, mV, mX, p, Bv, (cudaStream_t)stream);
   return tc::launch<64>(mK, mV, mX, p, Bv, (cudaStream_t)stream);

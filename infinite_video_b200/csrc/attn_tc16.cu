@@ -48,7 +48,6 @@ struct Params {
   // and attn_tc_combine_kernel merges the two halves (exp(m_half - m) rescaling, as in a two-block online softmax).
   int halves, NT;
   float* part;
-  unsigned long long* trace;   // bring-up: CTA 0 writes globaltimer stamps [item][16] (NULL = off)
 };
 constexpr int PART_ROWS = 68;
 
@@ -67,17 +66,6 @@ struct Lay {
   static constexpr int BYTES = MISC_OFF + MISC_FLOATS * 4 + 64 + 1024;   // + 6 barriers, TMEM slot, alignment slack
 };
 
-__device__ __forceinline__ void stamp(unsigned long long* trace, uint32_t it, int slot) {
-#ifndef LTM_BRINGUP
-  (void)trace; (void)it; (void)slot;          // the per-item timeline exists in bring-up builds only
-  return;
-#endif
-  if (trace != nullptr && blockIdx.x == 0 && it < 16) {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    trace[it * 16 + slot] = t;
-  }
-}
 __device__ __forceinline__ void cw_sync() { asm volatile("bar.sync 1, 256;" ::: "memory"); }   // the 8 compute warps
 
 // q tile of one work item, scaled by 1/sqrt(d) (gibbs:226; a power of two, exact) and rounded to fp16, in the K-major
@@ -207,11 +195,10 @@ cont_attn_tc16_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_con
       const uint64_t dV = umma_desc(sV, L_::SLAB, 1024, 2u), dR = umma_desc(sR, 16, 1024, 2u);
       const uint32_t dk_lo = (uint32_t)dK, dk_hi = (uint32_t)(dK >> 32), dq_lo = (uint32_t)dQ;
       const uint32_t dv_lo = (uint32_t)dV, dv_hi = (uint32_t)(dV >> 32), dr_lo = (uint32_t)dR;
-      auto issue_scores = [&](uint32_t ph, uint32_t sit) {            // S^T of the item whose K tile / q tile carry parity ph
+      auto issue_scores = [&](uint32_t ph) {            // S^T of the item whose K tile / q tile carry parity ph
         mbar_wait(bar_q, ph);                          // q tile written, S read out of TMEM
         mbar_wait(bar_k, ph);
         tcgen05_fence_after();
-        if (threadIdx.x == 256) stamp(p.trace, sit, 5);
 #pragma unroll
         for (int hf = 0; hf < HALVES; ++hf) {
 #pragma unroll
@@ -222,22 +209,19 @@ cont_attn_tc16_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_con
         tcgen05_commit(bar_s);
       };
       uint32_t it = 0;
-      issue_scores(0u, 0u);
+      issue_scores(0u);
       for (int w = w0; w < total; w += wstride, ++it) {
         const uint32_t ph = it & 1u;
         const int wn = w + wstride;
         int qtn = 0, hn = 0, vn = 0;
         if (wn < total) decode(wn, qtn, hn, vn);
         mbar_wait(bar_s, ph);                          // the K buffer has been read
-        stamp(p.trace, it, 0);
         if (wn < total) {
           mbar_arrive_expect_tx(bar_k, L_::SLAB);
           tma_load_2d(&mapK, sK, bar_k, hn * DH, jrow(wn, vn));
         }
         mbar_wait(bar_r, ph);                          // e^T written, D free
-        stamp(p.trace, it, 1);
         mbar_wait(bar_v, ph);
-        stamp(p.trace, it, 2);
         tcgen05_fence_after();
         // this warp contracts the first half of the basis range into D0, warp 9 the second half into D1: the issue
         // of 32 small MMAs by one thread (~33 ns each) was 1.05 us of the item's 4.7 us
@@ -247,12 +231,10 @@ cont_attn_tc16_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_con
                           dr_lo + (uint32_t)(((ks >> 2) * 4096 + (ks & 3) * 32) >> 4), dk_hi, IDESC_PV,
                           ks != 0 ? 1u : 0u);
         tcgen05_commit(bar_pv);
-        stamp(p.trace, it, 3);
         // the next item's scores go out right behind: its keys landed during this item's weight phase, so S is
         // ready by the time the compute warps have written this item's outputs
-        if (wn < total) issue_scores(ph ^ 1u, it + 1);
+        if (wn < total) issue_scores(ph ^ 1u);
         mbar_wait(bar_pv, ph);                         // the V buffer (and e^T) have been read
-        stamp(p.trace, it, 4);
         if (wn < total) {
           // (the per-basis operand rows X change with the basis half: re-fetched with V when there are two)
           mbar_arrive_expect_tx(bar_v, (halves > 1 ? 2 : 1) * L_::SLAB);
@@ -328,7 +310,6 @@ cont_attn_tc16_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_con
         rWj = 1.0f / Wj;
       }
       mbar_wait(bar_s, ph);
-      if (tid == 0) stamp(p.trace, it, 8);
       tcgen05_fence_after();
       if (active) {
         uint32_t r[32];
@@ -368,7 +349,6 @@ cont_attn_tc16_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_con
         }
       }
       cw_sync();                                                                           // column maxima
-      if (tid == 0) stamp(p.trace, it, 9);
       if (active) {
         float M = 0.f;                                 // per-row shift m = max(0, max_j S_j): it cancels exactly
 #pragma unroll
@@ -387,7 +367,6 @@ cont_attn_tc16_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_con
       }
       tcgen05_fence_before();
       mbar_arrive(bar_r);
-      if (tid == 0) stamp(p.trace, it, 10);
       if (wn + wstride < total) {                      // queries of item it + 2: consumed after the next bar_s
         int qtn, hn, vn;
         decode(wn + wstride, qtn, hn, vn);
@@ -396,7 +375,6 @@ cont_attn_tc16_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_con
 
       // ---- outputs: D[lane m][q]; warp (quarter, chalf) reads 16 columns
       mbar_wait(bar_pv, ph);
-      if (tid == 0) stamp(p.trace, it, 11);
       tcgen05_fence_after();
       float dv[16];
       {
@@ -454,7 +432,6 @@ cont_attn_tc16_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_con
         }
       }
       cw_sync();                                                                           // normalisers
-      if (tid == 0) stamp(p.trace, it, 12);
       if (quarter < 2) {
         const int dd = quarter * 32 + lane;
         float* dst = p.ctx + ((size_t)v * Q + q0 + chalf * 16) * D + h * DH + dd;
@@ -480,7 +457,6 @@ cont_attn_tc16_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_con
               hdt * (Gs[hja] + Gs[hjb]);
         // no barrier before the next item: everything above is rewritten only behind the next item's first
         // cw_sync, which no thread passes before all of them have finished this item
-        if (tid == 0) stamp(p.trace, it, 13);
       }
     }
   }
@@ -596,7 +572,6 @@ static int cont_attn_rect_tc16_impl(const float* q, const void* K, const void* V
   p.q = q; p.W = W; p.tb = tb; p.jb = jb; p.W_out = W_out; p.c_none = c_none; p.ctx = ctx;
   p.scores_out = scores_out; p.hist_part = hist_part; p.Q = Q; p.H = H;
   p.halves = halves; p.NT = N; p.part = part;
-  p.trace = nullptr;
   if (NBk == 256) return tc16::launch<256>(mK, mV, mX, p, Bv, (cudaStream_t)stream);
   if (NBk == 128) return tc16::launch<128>(mK, mV, mX, p, Bv, (cudaStream_t)stream);
   return tc16::launch<64>(mK, mV, mX, p, Bv, (cudaStream_t)stream);

@@ -1,8 +1,6 @@
 // C-ABI glue: error reporting, device check, and the fused per-chunk step of variant R.
 #include <stdarg.h>
 
-#include <time.h>
-
 #include "common.cuh"
 
 namespace ltm {
@@ -137,92 +135,72 @@ extern "C" int ltm_rect_step(const ltm_rect_step_args* a, const float* k, const 
                        new_doc == nullptr && a->jf > 0 && n_new > 0 && jg > 0 && a->e % 4 == 0;
   const int pprec = a->proj_precision ? a->proj_precision : a->precision;
   const bool kvh = a->kv_half != 0 && tcp && a->X16 != nullptr;                    // K|V stored as fp16
-  // Blocks of videos run consolidate -> project -> attention back to back, so that the K|V (and coefficient) rows a
-  // block has just written are still in L2 when its attention (projection) reads them: with all videos per kernel
-  // the 201 MB of K|V at 128 videos go out to HBM and come back.  video_block: 0 = all videos in one block.
-  int vblock = (a->video_block > 0 && a->video_block < a->Bv && !fast) ? a->video_block : a->Bv;
-  const size_t sB = (size_t)a->N * a->e, sKV = (size_t)a->N * 2 * D, sX = (size_t)xL * xsplits * a->e;
-  const bool blocked = vblock < a->Bv;
-  if (blocked) LTM_PROF(4);
-  for (int v0 = 0; v0 < a->Bv; v0 += vblock) {
-    const int nv = (a->Bv - v0 < vblock) ? a->Bv - v0 : vblock;
-    const float* Bp = B_past ? B_past + v0 * sB : nullptr;
-    float* Bn = a->B_new + v0 * sB;
-    // (fp16 K|V: the same pointers, offsets counted in 2-byte elements)
-    const size_t kvo = kvh ? v0 * sKV / 2 : v0 * sKV;
-    float* KVn = a->KV ? a->KV + kvo : nullptr;
-    const float* KVp = kvstate ? a->KV_past + kvo : nullptr;
-    void* Bh = half_ops ? (void*)((uint16_t*)a->B_half + v0 * sB) : nullptr;
-    if (!blocked) LTM_PROF(4);
-    // (ragged: the packed frames are addressed through the absolute frame offsets of the block's videos)
-    rc = consolidate_rect_ragged(Bp, ragged ? a->xpart : a->xpart + v0 * sX,
-                                 idx_stride ? idx + (size_t)v0 * idx_stride : idx, idx_stride,
-                                 new_doc ? new_doc + v0 : nullptr, seg_ptr0, seg_mem0, g0, seg_ptr1, seg_mem1, g1, Bn,
-                                 Bh, KVp, KVn, a->bkv, 2 * D, jg, kvh ? 2 : (tcp ? 1 : 0), nv, a->N, a->e, xL, xsplits,
-                                 a->S, ragged ? lengths + v0 : nullptr, ragged ? a->frame_offs + v0 : nullptr, stream);
-    if (rc) return rc;
-    if (!blocked) { LTM_PROF(5); LTM_PROF(6); }
-    // K|V projection KV = B_new W_kv^T + b_kv (fp16 operands: the fp16 copy of the new coefficient rows and of the
-    // weights, kind::f16 UMMAs; K|V for the tensor-core attention is stored as fp16 or rounded to the tf32 grid)
-    ltm_gemm_args ga;
-    memset(&ga, 0, sizeof(ga));
-    ga.A = half_ops ? reinterpret_cast<const float*>(Bh) : Bn; ga.lda = a->e; ga.a_kmajor = 1;
-    ga.B = half_ops ? reinterpret_cast<const float*>(a->Wkv_half) : a->Wkv; ga.ldb = a->e; ga.b_kmajor = 1;
-    ga.ab_fp16 = half_ops ? 1 : 0;
-    ga.K1 = a->e; ga.bias = a->bkv;
-    ga.C = KVn; ga.ldc = 2 * D;
-    ga.M = nv * a->N; ga.Nc = 2 * D; ga.K = a->e; ga.batch = 1;
-    // (the transposed-key and generic projections ignore proj_precision, except for the generic projected-memory rows)
-    ga.precision = half_ops ? 1 : (tcp || kvstate) ? pprec : a->precision;
-    ga.impl = a->gemm_impl; ga.round_tf32 = (tcp && !kvh) ? 1 : 0; ga.c_fp16 = kvh ? 1 : 0;
-    // (only the fp16-operand, fp16-K|V and projected-memory projections take the grid bound)
-    ga.max_ctas = (half_ops || kvh || kvstate) ? a->gemm_ctas : 0;
-    if (kvstate) {
-      // rows [jg, N) of every video as one flat problem: A = B_new + jg * e grouped per video, C = KV + jg * 2D
-      ga.A = half_ops ? reinterpret_cast<const float*>(reinterpret_cast<const uint16_t*>(Bh) + (size_t)jg * a->e)
-                      : Bn + (size_t)jg * a->e;
-      ga.a_group = n_new; ga.a_group_stride = (int64_t)a->N * a->e;
-      ga.C = kvh ? reinterpret_cast<float*>(reinterpret_cast<uint16_t*>(KVn) + (size_t)jg * 2 * D)
-                 : KVn + (size_t)jg * 2 * D;
-      ga.c_group = n_new; ga.c_group_stride = (int64_t)a->N * 2 * D;
-      ga.M = nv * n_new;
-    } else if (fast) {
-      // keys transposed per head for the fast attention: Kt[Bv, H, d, N], values V[Bv, N, D]
-      ga.C = a->V; ga.ldc = D;
-      ga.CT = a->Kt; ga.ct_cols = D; ga.ct_group = a->N;
-    }
-    rc = ltm_gemm(&ga, stream);
-    if (rc) return rc;
-    if (!blocked) { LTM_PROF(7); LTM_PROF(8); }
-    const float* qb = q + (size_t)v0 * a->Q * D;
-    float* cb = ctx + (size_t)v0 * a->Q * D;
-    float* sc = a->scores ? a->scores + (size_t)v0 * a->H * a->Q * a->N : nullptr;
-    float* hp = a->sticky ? a->hist_part + (size_t)v0 * a->H * qtiles * (LTM_STICKY_EDGES - 2) : nullptr;
-    if (kvh) {
-      const uint16_t* Kh = reinterpret_cast<const uint16_t*>(KVn);
-      if (tc512)
-        rc = ltm_cont_attn_rect_tc16_split(qb, Kh, Kh + D, 2 * D, a->X16, a->W, a->W_out, a->jb, a->tb, cb, sc,
-                                           a->attn_part + ltm_attn_tc_split_workspace_floats(v0, a->Q, a->H), hp, nv,
-                                           a->Q, a->N, a->H, a->d, stream);
-      else
-        rc = ltm_cont_attn_rect_tc16(qb, Kh, Kh + D, 2 * D, a->X16, a->W, a->W_out, a->c_none, a->jb, a->tb, cb, sc, hp,
-                                     nv, a->Q, a->N, a->H, a->d, stream);
-    } else if (tcp && tc512)
-      rc = ltm_cont_attn_rect_tc_split(qb, KVn, KVn + D, 2 * D, a->X, a->W, a->W_out, a->jb, a->tb, cb, sc,
-                                       a->attn_part + ltm_attn_tc_split_workspace_floats(v0, a->Q, a->H), hp, nv, a->Q,
-                                       a->N, a->H, a->d, stream);
-    else if (tcp)
-      rc = ltm_cont_attn_rect_tc(qb, KVn, KVn + D, 2 * D, a->X, a->W, a->W_out, a->c_none, a->jb, a->tb, cb, sc, hp,
-                                 nv, a->Q, a->N, a->H, a->d, stream);
-    else if (fast)
-      rc = ltm_cont_attn_rect_t(qb, a->Kt, a->V, D, a->W, a->W_out, a->jb, a->tb, cb, sc, hp, nv, a->Q, a->N, a->H,
-                                a->d, stream);
-    else
-      rc = ltm_cont_attn_rect(qb, KVn, a->W, a->W_out, a->jb, a->tb, cb, sc, hp, nv, a->Q, a->N, a->H, a->d, stream);
-    if (rc) return rc;
-    if (!blocked) LTM_PROF(9);
+  const size_t sKV = (size_t)a->N * 2 * D;
+  void* Bh = half_ops ? a->B_half : nullptr;
+  LTM_PROF(4);
+  rc = consolidate_rect_ragged(B_past, a->xpart, idx, idx_stride, new_doc, seg_ptr0, seg_mem0, g0, seg_ptr1, seg_mem1,
+                               g1, a->B_new, Bh, kvstate ? a->KV_past : nullptr, a->KV, a->bkv, 2 * D, jg,
+                               kvh ? 2 : (tcp ? 1 : 0), a->Bv, a->N, a->e, xL, xsplits, a->S,
+                               ragged ? lengths : nullptr, ragged ? a->frame_offs : nullptr, stream);
+  if (rc) return rc;
+  LTM_PROF(5);
+  LTM_PROF(6);
+  // K|V projection KV = B_new W_kv^T + b_kv (fp16 operands: the fp16 copy of the new coefficient rows and of the
+  // weights, kind::f16 UMMAs; K|V for the tensor-core attention is stored as fp16 or rounded to the tf32 grid)
+  ltm_gemm_args ga;
+  memset(&ga, 0, sizeof(ga));
+  ga.A = half_ops ? reinterpret_cast<const float*>(Bh) : a->B_new; ga.lda = a->e; ga.a_kmajor = 1;
+  ga.B = half_ops ? reinterpret_cast<const float*>(a->Wkv_half) : a->Wkv; ga.ldb = a->e; ga.b_kmajor = 1;
+  ga.ab_fp16 = half_ops ? 1 : 0;
+  ga.K1 = a->e; ga.bias = a->bkv;
+  ga.C = a->KV; ga.ldc = 2 * D;
+  ga.M = a->Bv * a->N; ga.Nc = 2 * D; ga.K = a->e; ga.batch = 1;
+  // (the transposed-key and generic projections ignore proj_precision, except for the generic projected-memory rows)
+  ga.precision = half_ops ? 1 : (tcp || kvstate) ? pprec : a->precision;
+  ga.impl = a->gemm_impl; ga.round_tf32 = (tcp && !kvh) ? 1 : 0; ga.c_fp16 = kvh ? 1 : 0;
+  // (only the fp16-operand, fp16-K|V and projected-memory projections take the grid bound)
+  ga.max_ctas = (half_ops || kvh || kvstate) ? a->gemm_ctas : 0;
+  if (kvstate) {
+    // rows [jg, N) of every video as one flat problem: A = B_new + jg * e grouped per video, C = KV + jg * 2D
+    ga.A = half_ops ? reinterpret_cast<const float*>(reinterpret_cast<const uint16_t*>(Bh) + (size_t)jg * a->e)
+                    : a->B_new + (size_t)jg * a->e;
+    ga.a_group = n_new; ga.a_group_stride = (int64_t)a->N * a->e;
+    ga.C = kvh ? reinterpret_cast<float*>(reinterpret_cast<uint16_t*>(a->KV) + (size_t)jg * 2 * D)
+               : a->KV + (size_t)jg * 2 * D;
+    ga.c_group = n_new; ga.c_group_stride = (int64_t)a->N * 2 * D;
+    ga.M = a->Bv * n_new;
+  } else if (fast) {
+    // keys transposed per head for the fast attention: Kt[Bv, H, d, N], values V[Bv, N, D]
+    ga.C = a->V; ga.ldc = D;
+    ga.CT = a->Kt; ga.ct_cols = D; ga.ct_group = a->N;
   }
-  if (blocked) LTM_PROF(9);
+  rc = ltm_gemm(&ga, stream);
+  if (rc) return rc;
+  LTM_PROF(7);
+  LTM_PROF(8);
+  float* hp = a->sticky ? a->hist_part : nullptr;
+  if (kvh) {
+    const uint16_t* Kh = reinterpret_cast<const uint16_t*>(a->KV);
+    if (tc512)
+      rc = ltm_cont_attn_rect_tc16_split(q, Kh, Kh + D, 2 * D, a->X16, a->W, a->W_out, a->jb, a->tb, ctx, a->scores,
+                                         a->attn_part, hp, a->Bv, a->Q, a->N, a->H, a->d, stream);
+    else
+      rc = ltm_cont_attn_rect_tc16(q, Kh, Kh + D, 2 * D, a->X16, a->W, a->W_out, a->c_none, a->jb, a->tb, ctx,
+                                   a->scores, hp, a->Bv, a->Q, a->N, a->H, a->d, stream);
+  } else if (tcp && tc512)
+    rc = ltm_cont_attn_rect_tc_split(q, a->KV, a->KV + D, 2 * D, a->X, a->W, a->W_out, a->jb, a->tb, ctx, a->scores,
+                                     a->attn_part, hp, a->Bv, a->Q, a->N, a->H, a->d, stream);
+  else if (tcp)
+    rc = ltm_cont_attn_rect_tc(q, a->KV, a->KV + D, 2 * D, a->X, a->W, a->W_out, a->c_none, a->jb, a->tb, ctx,
+                               a->scores, hp, a->Bv, a->Q, a->N, a->H, a->d, stream);
+  else if (fast)
+    rc = ltm_cont_attn_rect_t(q, a->Kt, a->V, D, a->W, a->W_out, a->jb, a->tb, ctx, a->scores, hp, a->Bv, a->Q, a->N,
+                              a->H, a->d, stream);
+  else
+    rc = ltm_cont_attn_rect(q, a->KV, a->W, a->W_out, a->jb, a->tb, ctx, a->scores, hp, a->Bv, a->Q, a->N, a->H, a->d,
+                            stream);
+  if (rc) return rc;
+  LTM_PROF(9);
 #undef LTM_PROF
   if (ragged && a->n_idle > 0) {
     // idle videos: the consolidation copied their coefficients into B_new, and the projection and attention ran over
@@ -236,50 +214,6 @@ extern "C" int ltm_rect_step(const ltm_rect_step_args* a, const float* k, const 
   return rc;
 }
 
-#ifdef LTM_BRINGUP
-// bring-up: a persistent kernel with a chosen footprint (threads, <= 96 registers, dynamic shared memory) that only
-// spins for `us` microseconds: measures what a co-resident footprint alone costs the streaming kernels beside it
-__global__ void __maxnreg__(96) footprint_spin_kernel(unsigned long long ns, float* sink) {
-  extern __shared__ float fs[];
-  unsigned long long t0, t1;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-  if (threadIdx.x == 0) fs[0] = 1.f;
-  do {
-    __nanosleep(200);
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-  } while (t1 - t0 < ns);
-  if (sink != nullptr && threadIdx.x == 0 && fs[0] == 2.f) sink[0] = 1.f;
-}
-extern "C" int ltm_debug_footprint_spin(int ctas, int threads, int smem_bytes, int us, void* stream) {
-  using namespace ltm;
-  LTM_CUDA(cudaFuncSetAttribute(footprint_spin_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-  footprint_spin_kernel<<<ctas, threads, smem_bytes, (cudaStream_t)stream>>>((unsigned long long)us * 1000ull, nullptr);
-  LTM_CHECK_LAUNCH("footprint_spin");
-  return 0;
-}
-
-// bring-up: host time spent in the sections of ltm_rect_step_overlap (sum and max, seconds)
-static double g_ov_sum[6] = {0, 0, 0, 0, 0, 0}, g_ov_max[6] = {0, 0, 0, 0, 0, 0};
-static inline double now_s() {
-  timespec ts;
-  clock_gettime(CLOCK_MONOTONIC, &ts);
-  return (double)ts.tv_sec + 1e-9 * (double)ts.tv_nsec;
-}
-extern "C" void ltm_debug_overlap_times(double* sum6, double* max6, int reset) {
-  for (int i = 0; i < 6; ++i) {
-    if (sum6) sum6[i] = g_ov_sum[i];
-    if (max6) max6[i] = g_ov_max[i];
-    if (reset) g_ov_sum[i] = g_ov_max[i] = 0.0;
-  }
-}
-#define LTM_OV_MARK(i) do { const double t_ = now_s(); const double d_ = t_ - t_prev; g_ov_sum[i] += d_; \
-                            if (d_ > g_ov_max[i]) g_ov_max[i] = d_; t_prev = t_; } while (0)
-#define LTM_OV_START() double t_prev = now_s()
-#else
-#define LTM_OV_MARK(i) do { } while (0)
-#define LTM_OV_START() do { } while (0)
-#endif
-
 extern "C" int ltm_rect_step_overlap(const ltm_rect_step_args* a, const ltm_overlap* o, const float* q,
                                      const double* u, const uint8_t* new_doc, float* ctx) {
   using namespace ltm;
@@ -287,13 +221,11 @@ extern "C" int ltm_rect_step_overlap(const ltm_rect_step_args* a, const ltm_over
   LTM_REQUIRE(o->ev_fork && o->ev_join, "rect_step_overlap: fork / join events missing");
   cudaStream_t ms = (cudaStream_t)o->main_stream, ss = (cudaStream_t)o->side_stream,
                cs = (cudaStream_t)o->compute_stream;
-  LTM_OV_START();
   if (o->k_next != nullptr) {
     LTM_REQUIRE(o->xpart_next && o->ev_fork_pool && o->ev_pooled_next, "rect_step_overlap: prefetch target missing");
     // the target buffer was last read by work already queued on the main stream
     LTM_CUDA(cudaEventRecord((cudaEvent_t)o->ev_fork_pool, ms));
     LTM_CUDA(cudaStreamWaitEvent(ss, (cudaEvent_t)o->ev_fork_pool, 0));
-    LTM_OV_MARK(0);
     if (a->prof_events[0]) cudaEventRecord((cudaEvent_t)a->prof_events[0], ss);
     LTM_REQUIRE(!o->next_lengths || (o->next_offs && !o->next_binned), "rect_step_overlap: ragged next chunk");
     const bool ragged_next = o->next_lengths != nullptr;
@@ -301,20 +233,15 @@ extern "C" int ltm_rect_step_overlap(const ltm_rect_step_args* a, const ltm_over
                         ragged_next ? o->next_splits : a->splits, o->next_binned != 0, o->pool_ctas, ss);
     if (rc) return rc;
     if (a->prof_events[1]) cudaEventRecord((cudaEvent_t)a->prof_events[1], ss);
-    LTM_OV_MARK(1);
     LTM_CUDA(cudaEventRecord((cudaEvent_t)o->ev_pooled_next, ss));
-    LTM_OV_MARK(2);
   }
   LTM_CUDA(cudaEventRecord((cudaEvent_t)o->ev_fork, ms));
   LTM_CUDA(cudaStreamWaitEvent(cs, (cudaEvent_t)o->ev_fork, 0));
   if (o->ev_pooled_cur) LTM_CUDA(cudaStreamWaitEvent(cs, (cudaEvent_t)o->ev_pooled_cur, 0));
-  LTM_OV_MARK(3);
   int rc = ltm_rect_step(a, nullptr, q, u, new_doc, ctx, cs);
   if (rc) return rc;
-  LTM_OV_MARK(4);
   LTM_CUDA(cudaEventRecord((cudaEvent_t)o->ev_join, cs));
   LTM_CUDA(cudaStreamWaitEvent(ms, (cudaEvent_t)o->ev_join, 0));
-  LTM_OV_MARK(5);
   return 0;
 }
 

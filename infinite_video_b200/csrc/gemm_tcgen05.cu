@@ -55,29 +55,19 @@ struct GemmDev {
   int c_half;                               // C is fp16 storage (row-major path only)
   void* C_lo;                               // fp16 output only: second array for the residual x - float(half(x))
   int max_ctas;                             // bound of the persistent grid (0 = one CTA per SM)
-  int dbg;                                  // bring-up builds only (-DLTM_BRINGUP): 1 = no global stores, 2 = no TMA loads
 };
-// The bring-up switches exist only in builds made with -DLTM_BRINGUP (scripts/*_probe.py); the product library
-// neither exports the setters nor carries the branches.
-#ifdef LTM_BRINGUP
-#define LTM_DBG(g) ((g).dbg)
-#else
-#define LTM_DBG(g) 0
-#endif
 
-// Work item -> tile origin.  CLUSTER == 1: items are tiles, n fastest.  CLUSTER == 2: a cluster of two CTAs takes
-// two vertically adjacent tiles (same n, rows m0 and m0 + 128) so that the B tile is fetched once and multicast.
-template <int CLUSTER, int BN_>
-__device__ __forceinline__ void decode_work(int w, int tiles_n, int tiles_m, int rank, int& n0, int& m0, int& bz) {
-  const int groups_m = (tiles_m + CLUSTER - 1) / CLUSTER;
+// Work item -> tile origin: items are tiles, n fastest.
+template <int BN_>
+__device__ __forceinline__ void decode_work(int w, int tiles_n, int tiles_m, int& n0, int& m0, int& bz) {
   n0 = (w % tiles_n) * BN_;
-  m0 = (((w / tiles_n) % groups_m) * CLUSTER + rank) * 128;
-  bz = w / (tiles_n * groups_m);
+  m0 = ((w / tiles_n) % tiles_m) * 128;
+  bz = w / (tiles_n * tiles_m);
 }
 // MN-major descriptor parameters.  For 32-bit (tf32) MN-major operands the only legal canonical layout is
 // the 128-byte swizzle with 32-byte atoms (TMA: SWIZZLE_128B_ATOM_32B): atoms of [4 k][32 mn], i.e. the
 // K groups are 4 rows = 512 B apart (SBO), the 32-wide MN atoms one slab = 4096 B apart (LBO), and one
-// MMA (K = 8) advances two K groups = 1024 B.  Kept in a struct so a bring-up harness can override them.
+// MMA (K = 8) advances two K groups = 1024 B.  fp16 operands use other values (set on the host per call).
 struct MnDesc { uint32_t layout, lbo, sbo, kadv; };
 // K-major tile [rows][32 fp32], SWIZZLE_128B: 8-row groups 1024 B apart (SBO); K advances 32 B inside the
 // swizzle row.  MN-major tile [mn/32 slabs][32 k][32 fp32]: see MnDesc.
@@ -105,10 +95,7 @@ __device__ __forceinline__ DescWords operand_desc_words(int kmajor, const MnDesc
 // tile, before the wait for the accumulator.  The first version did that arithmetic per store on 4 warps:
 // ~28 k cycles per 128 x 256 tile, 2.3x the tile's MMA time, and that -- not shared-memory bandwidth -- was what
 // held the kernel at 47 % tensor-pipe activity.
-#ifndef LTM_GEMM_EPI_WARPS
-#define LTM_GEMM_EPI_WARPS 8
-#endif
-constexpr int EPI_WARPS = LTM_GEMM_EPI_WARPS;          // 4 or 8 (each TMEM lane quarter is served by EPI_WARPS / 4 warps)
+constexpr int EPI_WARPS = 8;                           // each TMEM lane quarter is served by EPI_WARPS / 4 warps
 constexpr int EPI_SPLIT = EPI_WARPS / 4;
 constexpr int EPI_THREADS = EPI_WARPS * 32;
 constexpr int EPI_COLS = 32;
@@ -195,14 +182,13 @@ __device__ __forceinline__ void epilogue_tile(const GemmDev& g, uint32_t tmem_ac
         : "r"(taddr)
         : "memory");
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-    if (LTM_DBG(g) & 1) continue;
     if (g.CT != nullptr && n0 + c0 < g.ct_cols) {
       // transposed store (keys per head): lanes are consecutive rows of one group -> 128-byte coalesced
       float* dst = tbase + (size_t)(n0 + c0) * g.ct_group;
 #pragma unroll
       for (int i = 0; i < 32; ++i) {
         const float b = __shfl_sync(0xffffffffu, btr[j], i);             // all lanes take part
-        if (tbase != nullptr && !(LTM_DBG(g) & 4)) dst[(size_t)i * g.ct_group] = __uint_as_float(r[i]) + b;
+        if (tbase != nullptr) dst[(size_t)i * g.ct_group] = __uint_as_float(r[i]) + b;
       }
       continue;
     }
@@ -274,7 +260,7 @@ __device__ __forceinline__ void epilogue_tile(const GemmDev& g, uint32_t tmem_ac
       float4 v = *reinterpret_cast<const float4*>(stg + srow * EPI_COLS + ((lchunk ^ (srow & 7)) << 2));
       v.x += bv.x; v.y += bv.y; v.z += bv.z; v.w += bv.w;
       if (g.round_tf32) v = make_float4(tf32_rna(v.x), tf32_rna(v.y), tf32_rna(v.z), tf32_rna(v.w));
-      if (rok[i] && !(LTM_DBG(g) & 4)) {
+      if (rok[i]) {
         float* dst = cbase_ptr + roff[i] + ccol;
         if (vec) {
           *reinterpret_cast<float4*>(dst) = v;
@@ -312,7 +298,7 @@ struct Cfg {
 //   warp 1      TMEM owner + tcgen05.mma issuer (one lane)
 //   warps 2-9   epilogue (see epilogue_tile)
 //   warps 10-17 (precision 3 only) operand splitter hi/lo
-template <int BN, int STAGES, bool SPLIT, int CLUSTER, bool HOUT>
+template <int BN, int STAGES, bool SPLIT, bool HOUT>
 __global__ void __maxnreg__(GEMM_MAX_REGS)
 gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
                  const __grid_constant__ CUtensorMap mapB2, const GemmDev g) {
@@ -335,9 +321,8 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
   const int num_kb = (g.K + bke - 1) / bke;
   const int tiles_n = (g.Nc + BN - 1) / BN, tiles_m = (g.M + BM - 1) / BM;
   // static work list shared by all roles (see decode_work)
-  const int crank = (CLUSTER > 1) ? (int)(blockIdx.x % CLUSTER) : 0;
-  const int w_first = blockIdx.x / CLUSTER, w_stride = gridDim.x / CLUSTER;
-  const int num_work = tiles_n * ((tiles_m + CLUSTER - 1) / CLUSTER) * g.batch;
+  const int w_first = blockIdx.x, w_stride = gridDim.x;
+  const int num_work = tiles_n * tiles_m * g.batch;
 
   if (threadIdx.x == 0) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapA)) : "memory");
@@ -345,7 +330,7 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
     if (g.has_b2) asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapB2)) : "memory");
     for (int s = 0; s < STAGES; ++s) {
       mbar_init(full_bar(s), 1);
-      mbar_init(empty_bar(s), CLUSTER);  // the MMA warps of every CTA that received a multicast into this slot
+      mbar_init(empty_bar(s), 1);        // tcgen05.commit once the MMAs have read the slot
       mbar_init(split_bar(s), C_::SPLIT_THREADS);   // every splitter thread arrives after its proxy fence
     }
     mbar_init(lofree_bar(0), 1);         // MMAs of a k-block done with their lo buffer (two, alternating)
@@ -364,7 +349,6 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
   }
   tcgen05_fence_before();
   __syncthreads();
-  if (CLUSTER > 1) cluster_sync_all();    // peers' barriers are initialised before any multicast / remote arrive
   tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
@@ -374,13 +358,12 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
       uint32_t it = 0;
       for (int w = w_first; w < num_work; w += w_stride) {
         int n0, m0, bz;
-        decode_work<CLUSTER, BN>(w, tiles_n, tiles_m, crank, n0, m0, bz);
+        decode_work<BN>(w, tiles_n, tiles_m, n0, m0, bz);
         const int za = g.a_batched ? bz : 0;
         for (int kb = 0; kb < num_kb; ++kb, ++it) {
           const int s = it % STAGES;
           const uint32_t ph = (it / STAGES) & 1u;
           mbar_wait(empty_bar(s), ph ^ 1u);
-          if (LTM_DBG(g) & 2) { mbar_arrive(full_bar(s)); continue; }
           mbar_arrive_expect_tx(full_bar(s), A_BYTES + C_::B_BYTES);
           const uint32_t sa = smem_base + s * C_::STAGE_BYTES;
           const uint32_t sb = sa + A_BYTES;
@@ -399,13 +382,7 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
           const CUtensorMap* mb = seg2 ? &mapB2 : &mapB;
           const int kk = seg2 ? k0 - g.K1 : k0;
           const int zb = seg2 ? (g.b2_batched ? bz : 0) : (g.b_batched ? bz : 0);
-          if (CLUSTER > 1) {
-            // K-major B only (host-checked): this CTA fetches its 1/CLUSTER share of the B tile rows and
-            // multicasts it to every CTA of the cluster; the peers deliver the other shares
-            constexpr int SHARE = BN / CLUSTER;
-            tma_load_3d_mc(mb, sb + crank * (SHARE * BK * 4), full_bar(s), kk, n0 + crank * SHARE, zb,
-                           (uint16_t)((1u << CLUSTER) - 1u));
-          } else if (g.b_kmajor) {
+          if (g.b_kmajor) {
             tma_load_3d(mb, sb, full_bar(s), kk, n0, zb);
           } else if (g.ab_half) {
             // 16-bit MN-major: slabs of [64 k rows][64 n halves = 128 B], one per 64 columns of the tile
@@ -460,9 +437,7 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
             da += wa.kstep; db += wb.kstep;
           }
           if (SPLIT) tcgen05_commit(lofree_bar(it & 1u));  // the splitter may overwrite this lo buffer
-          // frees the stage once these MMAs have read it (in every CTA that multicasts into this slot)
-          if (CLUSTER > 1) tcgen05_commit_mc(empty_bar(s), (uint16_t)((1u << CLUSTER) - 1u));
-          else tcgen05_commit(empty_bar(s));
+          tcgen05_commit(empty_bar(s));            // frees the stage once these MMAs have read it
         }
         tcgen05_commit(tfull_bar(buf));          // accumulator of this tile complete
       }
@@ -475,7 +450,7 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
     uint32_t tc = 0;
     for (int w = w_first; w < num_work; w += w_stride, ++tc) {
       int n0, m0, bz;
-      decode_work<CLUSTER, BN>(w, tiles_n, tiles_m, crank, n0, m0, bz);
+      decode_work<BN>(w, tiles_n, tiles_m, n0, m0, bz);
       const uint32_t buf = tc & 1u, tph = (tc >> 1) & 1u;
       epilogue_tile<BN, HOUT>(g, tmem_base + buf * BN, ew, warp & 3, lane, stg, m0, n0, bz, tfull_bar(buf), tph);
       tcgen05_fence_before();
@@ -505,7 +480,7 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
             h.w = __uint_as_float(__float_as_uint(x.w) & 0xFFFFE000u);
             l.x = x.x - h.x; l.y = x.y - h.y; l.z = x.z - h.z; l.w = x.w - h.w;
             // `hi` stays as loaded: the tensor core itself truncates fp32 -> tf32 (measured on B200: rewriting
-            // the masked value gives bit-identical products, scripts/split_probe.py)
+            // the masked value gives bit-identical products)
             lo[f] = l;
           }
           asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic writes -> async proxy (UMMA)
@@ -517,327 +492,16 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
 
   tcgen05_fence_before();
   __syncthreads();
-  if (CLUSTER > 1) cluster_sync_all();    // no CTA may exit while a peer can still multicast into it / arrive on it
   if (warp == 1) {
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)C_::TMEM_COLS)
                  : "memory");
   }
 }
 
-#ifdef LTM_BRINGUP   // the CTA-pair and multicast variants measured no robust gain (DESIGN.md): bring-up builds only
-// ================================================================================================
-// CTA-pair variant: tcgen05.mma.cta_group::2.  Two CTAs on one TPC compute a 256 x BN tile together:
-// CTA r holds rows [m0 + 128 r, +128) of A and rows [n0 + BN/2 r, +BN/2) of B in its shared memory, the
-// leader (rank 0) issues one M = 256 MMA that reads both CTAs' operands, and each CTA's TMEM receives its own
-// 128 accumulator rows.  Per SM this halves the B bytes that have to be ingested and it lifts the
-// single-CTA MMA rate limit (measured: cta_group::1 TF32 tops out near 550 TFLOP/s).
-//   full[s]   (leader)   precision 1: armed by the leader for both CTAs' TMA bytes (the peer's loads use the
-//                        .cta_group::2 form and signal the leader's barrier); precision 3: each CTA's own
-//   split[s]  (leader)   precision 3: 2 x 256 splitter threads (the peer's arrive remotely)
-//   empty[s], lofree, tfull[b] (both CTAs)  tcgen05.commit.cta_group::2 multicast from the leader
-//   tempty[b] (leader)   2 x 128 epilogue threads (the peer's arrive remotely)
-// ================================================================================================
-__device__ __forceinline__ uint32_t mapa_rank(uint32_t local, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ uint32_t mbar_try_wait_cluster(uint32_t bar, uint32_t parity) {
-  uint32_t done;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(done)
-      : "r"(bar), "r"(parity)
-      : "memory");
-  return done;
-}
-// bounded wait with cluster-scope acquire (barriers that receive arrivals from the peer CTA)
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
-  if (mbar_try_wait_cluster(bar, parity)) return;
-  unsigned long long t0;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-  uint32_t spins = 0;
-  while (!mbar_try_wait_cluster(bar, parity)) {
-    if ((++spins & 0x3fffu) == 0) {
-      unsigned long long t1;
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-      if (t1 - t0 > 2000000000ull) {
-        printf("libinfltm gemm(pair): mbarrier wait timed out (block %d thread %d)\n", blockIdx.x, threadIdx.x);
-        asm volatile("trap;");
-      }
-    }
-  }
-}
-__device__ __forceinline__ void tma_load_3d_pair(const CUtensorMap* map, uint32_t dst, uint32_t bar_cluster, int c0,
-                                                 int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar_cluster), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tcgen05_mma_tf32_pair(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo,
-                                                      uint32_t b_hi, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-      "setp.ne.b32 p, %6, 0;\n\t"
-      "mov.b64 da, {%1, %2};\n\t"
-      "mov.b64 db, {%3, %4};\n\t"
-      "tcgen05.mma.cta_group::2.kind::tf32 [%0], da, db, %5, p;\n\t}"
-      ::"r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void tcgen05_mma_f16_pair(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo,
-                                                     uint32_t b_hi, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-      "setp.ne.b32 p, %6, 0;\n\t"
-      "mov.b64 da, {%1, %2};\n\t"
-      "mov.b64 db, {%3, %4};\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %5, p;\n\t}"
-      ::"r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void tcgen05_commit_pair(uint32_t bar) {     // arrives in both CTAs of the pair
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"((uint16_t)3) : "memory");
-}
-
-template <int BN, int STAGES, bool SPLIT>
-struct PairCfg {
-  static constexpr int BH = BN / 2;                            // B rows held by each CTA
-  static constexpr int B_BYTES = BH * BK * 4;
-  static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  static constexpr int LO_BYTES = SPLIT ? 2 * STAGE_BYTES : 0;
-  static constexpr int RING_BYTES = STAGES * STAGE_BYTES + LO_BYTES;
-  static constexpr int BAR_BYTES = 256;
-  static constexpr int SMEM_BYTES = RING_BYTES + STG_BYTES + BAR_BYTES + 1024;
-  static constexpr int TMEM_COLS = 2 * BN;
-  static constexpr int SPLIT_THREADS = 256;
-  static constexpr int THREADS = SPLIT ? ROLE_THREADS + SPLIT_THREADS : ROLE_THREADS;
-  static_assert(TMEM_COLS == 256 || TMEM_COLS == 512, "TMEM allocation must be a power of two <= 512");
-};
-
-template <int BN, int STAGES, bool SPLIT>
-__global__ void __maxnreg__(GEMM_MAX_REGS)
-gemm_tf32_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
-                      const __grid_constant__ CUtensorMap mapB2, const GemmDev g) {
-  using C_ = PairCfg<BN, STAGES, SPLIT>;
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* smem_al = smem_raw + (smem_base - smem_u32(smem_raw));
-  float* staging = reinterpret_cast<float*>(smem_al + C_::RING_BYTES);
-  const uint32_t bars = smem_base + C_::RING_BYTES + STG_BYTES;
-  auto full_bar = [&](int s) { return bars + 8u * s; };
-  auto empty_bar = [&](int s) { return bars + 8u * (STAGES + s); };
-  auto split_bar = [&](int s) { return bars + 8u * (2 * STAGES + s); };
-  auto tfull_bar = [&](int b) { return bars + 8u * (3 * STAGES + b); };
-  auto tempty_bar = [&](int b) { return bars + 8u * (3 * STAGES + 2 + b); };
-  auto lofree_bar = [&](uint32_t b) { return bars + 8u * (3 * STAGES + 4 + b); };
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem_al + C_::RING_BYTES + STG_BYTES + 8 * (3 * STAGES + 6));
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t crank = blockIdx.x & 1u;
-  const bool leader = crank == 0;
-  const int bke = g.ab_half ? 2 * BK : BK;        // K-elements per 128-byte swizzle row
-  const int num_kb = (g.K + bke - 1) / bke;
-  const int tiles_n = (g.Nc + BN - 1) / BN, tiles_m = (g.M + BM - 1) / BM;
-  const int w_first = blockIdx.x >> 1, w_stride = gridDim.x >> 1;
-  const int num_work = tiles_n * ((tiles_m + 1) / 2) * g.batch;
-
-  if (threadIdx.x == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapA)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapB)) : "memory");
-    if (g.has_b2) asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapB2)) : "memory");
-    for (int s = 0; s < STAGES; ++s) {
-      mbar_init(full_bar(s), 1);
-      mbar_init(empty_bar(s), 1);
-      mbar_init(split_bar(s), 2 * C_::SPLIT_THREADS);
-    }
-    mbar_init(lofree_bar(0), 1);
-    mbar_init(lofree_bar(1), 1);
-    for (int b = 0; b < 2; ++b) {
-      mbar_init(tfull_bar(b), 1);
-      mbar_init(tempty_bar(b), 2 * EPI_THREADS);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"((uint32_t)C_::TMEM_COLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  tcgen05_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  tcgen05_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0) {
-    // ------------------------------------------------------------------ TMA producer (both CTAs)
-    if (lane == 0) {
-      uint32_t it = 0;
-      for (int w = w_first; w < num_work; w += w_stride) {
-        int n0, m0, bz;
-        decode_work<2, BN>(w, tiles_n, tiles_m, (int)crank, n0, m0, bz);
-        const int nb0 = n0 + (int)crank * C_::BH;                       // this CTA's half of the B tile
-        const int za = g.a_batched ? bz : 0;
-        for (int kb = 0; kb < num_kb; ++kb, ++it) {
-          const int s = it % STAGES;
-          const uint32_t ph = (it / STAGES) & 1u;
-          mbar_wait(empty_bar(s), ph ^ 1u);
-          if (LTM_DBG(g) & 2) { if (SPLIT || leader) mbar_arrive(full_bar(s)); continue; }
-          uint32_t bar;                                                 // shared::cluster address of the barrier
-          if (SPLIT) {
-            mbar_arrive_expect_tx(full_bar(s), C_::STAGE_BYTES);        // own barrier: the splitter waits on it
-            bar = mapa_rank(full_bar(s), crank);
-          } else {
-            if (leader) mbar_arrive_expect_tx(full_bar(s), 2 * C_::STAGE_BYTES);
-            bar = mapa_rank(full_bar(s), 0);                            // both CTAs' bytes land on the leader's
-          }
-          const uint32_t sa = smem_base + s * C_::STAGE_BYTES;
-          const uint32_t sb = sa + A_BYTES;
-          const int k0 = kb * bke;
-          if (g.a_kmajor) {
-            tma_load_3d_pair(&mapA, sa, bar, k0, m0, za);
-          } else {
-#pragma unroll
-            for (int i = 0; i < BM / 32; ++i) tma_load_3d_pair(&mapA, sa + i * SLAB_BYTES, bar, m0 + 32 * i, k0, za);
-          }
-          const bool seg2 = g.has_b2 && (k0 >= g.K1);
-          const CUtensorMap* mb = seg2 ? &mapB2 : &mapB;
-          const int kk = seg2 ? k0 - g.K1 : k0;
-          const int zb = seg2 ? (g.b2_batched ? bz : 0) : (g.b_batched ? bz : 0);
-          if (g.b_kmajor) {
-            tma_load_3d_pair(mb, sb, bar, kk, nb0, zb);
-          } else {
-#pragma unroll
-            for (int i = 0; i < C_::BH / 32; ++i) tma_load_3d_pair(mb, sb + i * SLAB_BYTES, bar, nb0 + 32 * i, kk, zb);
-          }
-        }
-      }
-    }
-    __syncwarp();
-  } else if (warp == 1) {
-    // ------------------------------------------------------------------ MMA issuer (leader CTA only)
-    if (leader && lane == 0) {
-      const uint32_t fmt = g.ab_half ? 0u : 2u;         // operand format: 0 = f16 (kind::f16), 2 = tf32
-      const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((g.a_kmajor ? 0u : 1u) << 15) |
-                             ((g.b_kmajor ? 0u : 1u) << 16) | ((uint32_t)(BN >> 3) << 17) |
-                             ((uint32_t)((2 * BM) >> 4) << 24);                       // M = 256 across the pair
-      const MnDesc mn{g.mn_layout, g.mn_lbo, g.mn_sbo, g.mn_kadv};
-      const DescWords wa = operand_desc_words(g.a_kmajor, mn), wb = operand_desc_words(g.b_kmajor, mn);
-      const uint32_t da0 = wa.lo0 + ((smem_base & 0x3FFFFu) >> 4), db0 = wb.lo0 + (((smem_base + A_BYTES) & 0x3FFFFu) >> 4);
-      const uint32_t dal0 = da0 + STAGES * (C_::STAGE_BYTES >> 4), dbl0 = db0 + STAGES * (C_::STAGE_BYTES >> 4);
-      uint32_t it = 0, tc = 0;
-      for (int w = w_first; w < num_work; w += w_stride, ++tc) {
-        const uint32_t buf = tc & 1u, tph = (tc >> 1) & 1u;
-        mbar_wait_cluster(tempty_bar(buf), tph ^ 1u);          // both CTAs' epilogues have drained the accumulator
-        tcgen05_fence_after();
-        const uint32_t tmem_acc = tmem_base + buf * BN;
-        for (int kb = 0; kb < num_kb; ++kb, ++it) {
-          const int s = it % STAGES;
-          const uint32_t ph = (it / STAGES) & 1u;
-          if (SPLIT) mbar_wait_cluster(split_bar(s), ph); else mbar_wait_cluster(full_bar(s), ph);
-          tcgen05_fence_after();
-          uint32_t da = da0 + s * (C_::STAGE_BYTES >> 4), db = db0 + s * (C_::STAGE_BYTES >> 4);
-          const uint32_t lob = (it & 1u) * (C_::STAGE_BYTES >> 4);     // lo buffer [A_lo | B_lo] of this k-block
-          uint32_t dal = dal0 + lob, dbl = dbl0 + lob;
-#pragma unroll
-          for (int k = 0; k < BK / UMMA_K; ++k) {
-            if (g.ab_half) tcgen05_mma_f16_pair(tmem_acc, da, wa.hi, db, wb.hi, idesc, (kb | k) != 0 ? 1u : 0u);
-            else tcgen05_mma_tf32_pair(tmem_acc, da, wa.hi, db, wb.hi, idesc, (kb | k) != 0 ? 1u : 0u);
-            if (SPLIT) {
-              tcgen05_mma_tf32_pair(tmem_acc, dal, wa.hi, db, wb.hi, idesc, 1u);
-              tcgen05_mma_tf32_pair(tmem_acc, da, wa.hi, dbl, wb.hi, idesc, 1u);
-              dal += wa.kstep; dbl += wb.kstep;
-            }
-            da += wa.kstep; db += wb.kstep;
-          }
-          if (SPLIT) tcgen05_commit_pair(lofree_bar(it & 1u));
-          tcgen05_commit_pair(empty_bar(s));
-        }
-        tcgen05_commit_pair(tfull_bar(buf));
-      }
-    }
-    __syncwarp();
-  } else if (warp < 2 + EPI_WARPS) {
-    // ------------------------------------------------------------------ epilogue warps (both CTAs, own rows)
-    const int ew = warp - 2;
-    float* stg = staging + ew * STG_WARP_FLOATS;
-    uint32_t tc = 0;
-    for (int w = w_first; w < num_work; w += w_stride, ++tc) {
-      int n0, m0, bz;
-      decode_work<2, BN>(w, tiles_n, tiles_m, (int)crank, n0, m0, bz);
-      const uint32_t buf = tc & 1u, tph = (tc >> 1) & 1u;
-      epilogue_tile<BN, false>(g, tmem_base + buf * BN, ew, warp & 3, lane, stg, m0, n0, bz, tfull_bar(buf), tph);
-      tcgen05_fence_before();
-      mbar_arrive_remote(mapa_rank(tempty_bar(buf), 0));      // 2 x EPI_THREADS arrivals on the leader's barrier
-    }
-  } else {
-    // ------------------------------------------------------------------ operand splitter (precision 3, both CTAs)
-    if (SPLIT) {
-      const int et = threadIdx.x - ROLE_THREADS;
-      constexpr int NV = C_::STAGE_BYTES / 16;
-      uint32_t it = 0;
-      for (int w = w_first; w < num_work; w += w_stride) {
-        for (int kb = 0; kb < num_kb; ++kb, ++it) {
-          const int s = it % STAGES;
-          const uint32_t ph = (it / STAGES) & 1u;
-          mbar_wait(full_bar(s), ph);
-          mbar_wait(lofree_bar(it & 1u), ((it >> 1) & 1u) ^ 1u);
-          const float4* hi = reinterpret_cast<const float4*>(smem_al + s * C_::STAGE_BYTES);
-          float4* lo = reinterpret_cast<float4*>(smem_al + (STAGES + (it & 1u)) * C_::STAGE_BYTES);
-#pragma unroll 4
-          for (int f = et; f < NV; f += C_::SPLIT_THREADS) {
-            const float4 x = hi[f];
-            float4 l;
-            l.x = x.x - __uint_as_float(__float_as_uint(x.x) & 0xFFFFE000u);
-            l.y = x.y - __uint_as_float(__float_as_uint(x.y) & 0xFFFFE000u);
-            l.z = x.z - __uint_as_float(__float_as_uint(x.z) & 0xFFFFE000u);
-            l.w = x.w - __uint_as_float(__float_as_uint(x.w) & 0xFFFFE000u);
-            lo[f] = l;
-          }
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-          mbar_arrive_remote(mapa_rank(split_bar(s), 0));    // 2 x 256 arrivals on the leader's barrier
-        }
-      }
-    }
-  }
-
-  tcgen05_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)C_::TMEM_COLS)
-                 : "memory");
-  }
-}
-
-#endif  // LTM_BRINGUP
-
 // ------------------------------------------------------------------------------------------ host
 static PFN_cuTensorMapEncodeTiled_v12000 g_encode = nullptr;
-// bring-up override of the MN-major layout parameters: {layout, lbo, sbo, kadv, tma swizzle enum}
-// 2 enables the 2-CTA multicast variant.  Measured on B200 (profiles/r1e): no gain over unicast -- the kernel is
-// bound by per-SM ingest (~38 B/clk/SM), not by L2 reads -- so it is off by default and kept as a tested option.
-#ifdef LTM_BRINGUP
-static int g_cluster = 1;
-// CTA-pair (tcgen05 cta_group::2) kernel for problems with at least two row tiles: 0 = off (default), 1 = always,
-// -1 = for single-pass TF32 only.  Measured on two B200s: 130 vs 135 us (pair wins) on one, 152 vs 146 us (pair
-// loses) on the other -- no robust winner, so the simpler single-CTA kernel stays the default.
-static int g_pair = 0;
-static int g_dbg = 0;
-#else
-constexpr int g_cluster = 1, g_pair = 0, g_dbg = 0;
-#endif
-static unsigned g_mn_desc[5] = {1u, (unsigned)SLAB_BYTES, 512u, 1024u, (unsigned)CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B};
+// MN-major tf32 operands: UMMA descriptor parameters (see MnDesc); their TMA maps use SWIZZLE_128B_ATOM_32B
+constexpr MnDesc MN_TF32 = {1u, (uint32_t)SLAB_BYTES, 512u, 1024u};
 
 static int resolve_encode() {
   if (g_encode) return 0;
@@ -883,7 +547,7 @@ static int encode_operand(CUtensorMap* map, const float* base, int rows, int K, 
   cuuint32_t estr[3] = {1u, 1u, 1u};
   CUresult r = g_encode(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(base), dims, strides, box, estr,
                         CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        kmajor ? CU_TENSOR_MAP_SWIZZLE_128B : (CUtensorMapSwizzle)g_mn_desc[4],
+                        kmajor ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B,
                         CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   LTM_REQUIRE(r == CUDA_SUCCESS, "gemm: cuTensorMapEncodeTiled(%s) failed with CUresult %d", what, (int)r);
@@ -908,76 +572,22 @@ int tma_encode_2d(CUtensorMap* map, const float* base, unsigned long long inner,
   return 0;
 }
 
-template <int BN, int STAGES, bool SPLIT, int CLUSTER = 1, bool HOUT = false>
+template <int BN, int STAGES, bool SPLIT, bool HOUT = false>
 static int launch_cfg(const CUtensorMap& mA, const CUtensorMap& mB, const CUtensorMap& mB2, const GemmDev& d,
                       int batch, cudaStream_t stream) {
   using C_ = Cfg<BN, STAGES, SPLIT>;
   static PerDevice pd = {};
   int num_sms = 0;
-  if (int rc = kernel_setup(gemm_tf32_kernel<BN, STAGES, SPLIT, CLUSTER, HOUT>, (size_t)C_::SMEM_BYTES, pd, &num_sms))
+  if (int rc = kernel_setup(gemm_tf32_kernel<BN, STAGES, SPLIT, HOUT>, (size_t)C_::SMEM_BYTES, pd, &num_sms))
     return rc;
   const long long tiles = (long long)((d.Nc + BN - 1) / BN) * ((d.M + BM - 1) / BM) * batch;
   LTM_REQUIRE(tiles < (1ll << 31), "gemm: too many tiles");
-  if (CLUSTER > 1) {
-    // persistent clusters: CLUSTER CTAs on adjacent SMs share every B tile through TMA multicast
-    const long long tm = (d.M + BM - 1) / BM;
-    const long long work = (long long)((d.Nc + BN - 1) / BN) * ((tm + CLUSTER - 1) / CLUSTER) * batch;
-    long long clusters = num_sms / CLUSTER;
-    if (work < clusters) clusters = work;
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3((unsigned)(clusters * CLUSTER));
-    cfg.blockDim = dim3(C_::THREADS);
-    cfg.dynamicSmemBytes = C_::SMEM_BYTES;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = CLUSTER;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    LTM_CUDA(cudaLaunchKernelEx(&cfg, gemm_tf32_kernel<BN, STAGES, SPLIT, CLUSTER, HOUT>, mA, mB, mB2, d));
-    return 0;
-  }
   unsigned grid = (unsigned)(tiles < num_sms ? tiles : num_sms);     // persistent: one CTA per SM
   if (d.max_ctas > 0 && (unsigned)d.max_ctas < grid) grid = (unsigned)d.max_ctas;   // ... or fewer (ltm_gemm_args.max_ctas)
-  gemm_tf32_kernel<BN, STAGES, SPLIT, 1, HOUT><<<grid, C_::THREADS, C_::SMEM_BYTES, stream>>>(mA, mB, mB2, d);
+  gemm_tf32_kernel<BN, STAGES, SPLIT, HOUT><<<grid, C_::THREADS, C_::SMEM_BYTES, stream>>>(mA, mB, mB2, d);
   LTM_CHECK_LAUNCH("gemm(tcgen05)");
   return 0;
 }
-
-#ifdef LTM_BRINGUP
-template <int BN, int STAGES, bool SPLIT>
-static int launch_pair(const CUtensorMap& mA, const CUtensorMap& mB, const CUtensorMap& mB2, const GemmDev& d,
-                       int batch, cudaStream_t stream) {
-  using C_ = PairCfg<BN, STAGES, SPLIT>;
-  static PerDevice pd = {};
-  int num_sms = 0;
-  if (int rc = kernel_setup(gemm_tf32_pair_kernel<BN, STAGES, SPLIT>, (size_t)C_::SMEM_BYTES, pd, &num_sms)) return rc;
-  const long long tm = (d.M + BM - 1) / BM;
-  const long long work = (long long)((d.Nc + BN - 1) / BN) * ((tm + 1) / 2) * batch;
-  LTM_REQUIRE(work < (1ll << 31), "gemm: too many tiles");
-  long long pairs = num_sms / 2;
-  if (work < pairs) pairs = work;
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)(pairs * 2));
-  cfg.blockDim = dim3(C_::THREADS);
-  cfg.dynamicSmemBytes = C_::SMEM_BYTES;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  LTM_CUDA(cudaLaunchKernelEx(&cfg, gemm_tf32_pair_kernel<BN, STAGES, SPLIT>, mA, mB, mB2, d));
-  return 0;
-}
-
-#endif
 
 static int gemm_tcgen05_launch(const ltm_gemm_args& a, cudaStream_t stream) {
   if (resolve_encode()) return -1;
@@ -1014,12 +624,9 @@ static int gemm_tcgen05_launch(const ltm_gemm_args& a, cudaStream_t stream) {
                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     LTM_REQUIRE(r == CUDA_SUCCESS, "gemm: cuTensorMapEncodeTiled(grouped A) failed with CUresult %d", (int)r);
   } else if (encode_operand(&mA, a.A, a.M, a.K, a.lda, a.strideA, a.batch, a.a_kmajor, BM, "A", half)) return -1;
-  const bool pair = (g_pair > 0 || (g_pair < 0 && !split)) && a.M > BM && a.a_group == 0 && !a.c_fp16;
-  const bool mc_pre = !pair && g_cluster >= 2 && a.b_kmajor && !two && a.M > BM && !a.c_fp16;
-  const int b_box = (pair || mc_pre) ? bn / 2 : bn;             // B rows fetched per TMA box
-  if (encode_operand(&mB, a.B, a.Nc, K1, a.ldb, a.strideB, a.batch, a.b_kmajor, b_box, "B", half)) return -1;
+  if (encode_operand(&mB, a.B, a.Nc, K1, a.ldb, a.strideB, a.batch, a.b_kmajor, bn, "B", half)) return -1;
   if (two) {
-    if (encode_operand(&mB2, a.B2, a.Nc, a.K - K1, a.ldb2, a.strideB2, a.batch, a.b_kmajor, b_box, "B2", half)) return -1;
+    if (encode_operand(&mB2, a.B2, a.Nc, a.K - K1, a.ldb2, a.strideB2, a.batch, a.b_kmajor, bn, "B2", half)) return -1;
   } else {
     mB2 = mB;
   }
@@ -1029,13 +636,12 @@ static int gemm_tcgen05_launch(const ltm_gemm_args& a, cudaStream_t stream) {
   d.a_kmajor = a.a_kmajor ? 1 : 0; d.b_kmajor = a.b_kmajor ? 1 : 0;
   d.CT = a.CT; d.ct_cols = a.ct_cols; d.ct_group = a.ct_group;
   d.c_group = a.c_group; d.c_group_stride = a.c_group_stride; d.bias_stride = a.bias_stride;
-  d.mn_layout = g_mn_desc[0]; d.mn_lbo = g_mn_desc[1]; d.mn_sbo = g_mn_desc[2]; d.mn_kadv = g_mn_desc[3];
+  d.mn_layout = MN_TF32.layout; d.mn_lbo = MN_TF32.lbo; d.mn_sbo = MN_TF32.sbo; d.mn_kadv = MN_TF32.kadv;
   if (half) {
     // 16-bit MN-major SWIZZLE_128B: atoms of [8 k][64 mn], MN atoms one 8 KB slab apart (LBO), 8-row k groups 1024 B
     // apart (SBO); one MMA (K = 16) advances two groups
     d.mn_layout = 2u; d.mn_lbo = 64u * 128u; d.mn_sbo = 1024u; d.mn_kadv = 2048u;
   }
-  d.dbg = g_dbg;
   d.round_tf32 = a.round_tf32;
   d.ab_half = half;
   d.c_vec = (a.ldc % 4 == 0 && a.strideC % 4 == 0 && a.c_group_stride % 4 == 0 && aligned16(a.C) &&
@@ -1051,26 +657,11 @@ static int gemm_tcgen05_launch(const ltm_gemm_args& a, cudaStream_t stream) {
   LTM_REQUIRE(a.C_lo == nullptr || (a.c_fp16 && aligned16(a.C_lo)), "gemm: C_lo needs c_fp16 and 16-byte alignment");
   LTM_REQUIRE(!a.c_fp16 || a.CT == nullptr, "gemm: fp16 output has no transposed store");
   d.a_batched = a.strideA != 0; d.b_batched = a.strideB != 0; d.b2_batched = a.strideB2 != 0; d.has_b2 = two ? 1 : 0;
-#ifdef LTM_BRINGUP
-  if (pair) {
-    if (split) return bn == 256 ? launch_pair<256, 4, true>(mA, mB, mB2, d, a.batch, stream)
-                                : launch_pair<128, 6, true>(mA, mB, mB2, d, a.batch, stream);
-    return bn == 256 ? launch_pair<256, 6, false>(mA, mB, mB2, d, a.batch, stream)
-                     : launch_pair<128, 8, false>(mA, mB, mB2, d, a.batch, stream);
-  }
-  // 2-CTA clusters with a multicast B tile: K-major single-segment B and at least two row tiles
-  if (mc_pre) {
-    if (split && bn == 256) return launch_cfg<256, 2, true, 2>(mA, mB, mB2, d, a.batch, stream);
-    if (split) return launch_cfg<128, 4, true, 2>(mA, mB, mB2, d, a.batch, stream);
-    if (bn == 256) return launch_cfg<256, 4, false, 2>(mA, mB, mB2, d, a.batch, stream);
-    return launch_cfg<128, 6, false, 2>(mA, mB, mB2, d, a.batch, stream);
-  }
-#endif
   if (d.c_half) {           // fp16 output (the projected-memory K|V; Qt of the short-term attention)
-    if (split) return bn == 256 ? launch_cfg<256, 2, true, 1, true>(mA, mB, mB2, d, a.batch, stream)
-                                : launch_cfg<128, 4, true, 1, true>(mA, mB, mB2, d, a.batch, stream);
-    return bn == 256 ? launch_cfg<256, 4, false, 1, true>(mA, mB, mB2, d, a.batch, stream)
-                     : launch_cfg<128, 6, false, 1, true>(mA, mB, mB2, d, a.batch, stream);
+    if (split) return bn == 256 ? launch_cfg<256, 2, true, true>(mA, mB, mB2, d, a.batch, stream)
+                                : launch_cfg<128, 4, true, true>(mA, mB, mB2, d, a.batch, stream);
+    return bn == 256 ? launch_cfg<256, 4, false, true>(mA, mB, mB2, d, a.batch, stream)
+                     : launch_cfg<128, 6, false, true>(mA, mB, mB2, d, a.batch, stream);
   }
   if (split && bn == 256) return launch_cfg<256, 2, true>(mA, mB, mB2, d, a.batch, stream);
   if (split) return launch_cfg<128, 4, true>(mA, mB, mB2, d, a.batch, stream);
@@ -1079,19 +670,6 @@ static int gemm_tcgen05_launch(const ltm_gemm_args& a, cudaStream_t stream) {
 }
 
 }  // namespace ltm
-
-// Bring-up hooks (not part of include/infltm.h, compiled only with -DLTM_BRINGUP): kernel variant selection,
-// store / load suppression, override of the MN-major descriptor parameters.
-#ifdef LTM_BRINGUP
-extern "C" void ltm_debug_set_cluster(int c) { ltm::g_cluster = c; }
-extern "C" void ltm_debug_set_pair(int v) { ltm::g_pair = v; }
-extern "C" void ltm_debug_set_gemm_flags(int v) { ltm::g_dbg = v; }
-
-extern "C" void ltm_debug_set_mn_desc(unsigned layout, unsigned lbo, unsigned sbo, unsigned kadv, unsigned swz) {
-  ltm::g_mn_desc[0] = layout; ltm::g_mn_desc[1] = lbo; ltm::g_mn_desc[2] = sbo; ltm::g_mn_desc[3] = kadv;
-  ltm::g_mn_desc[4] = swz;
-}
-#endif
 
 extern "C" int ltm_gemm(const ltm_gemm_args* args, void* stream) {
   using namespace ltm;

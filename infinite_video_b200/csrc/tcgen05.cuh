@@ -67,24 +67,6 @@ __device__ __forceinline__ void tcgen05_fence_after() { asm volatile("tcgen05.fe
 __device__ __forceinline__ void tcgen05_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
-// commit that arrives on the barrier at the same shared-memory offset in every CTA of `mask` (cluster)
-__device__ __forceinline__ void tcgen05_commit_mc(uint32_t bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"(mask) : "memory");
-}
-// TMA load delivered to the same shared-memory offset (and mbarrier) of every CTA in `mask`
-__device__ __forceinline__ void tma_load_3d_mc(const CUtensorMap* map, uint32_t dst, uint32_t bar, int c0, int c1,
-                                               int c2, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%3, %4, %5}], [%2], %6;"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "h"(mask)
-      : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
 // The descriptors are passed as (low word, high word): only the low word (start address | LBO) changes from MMA
 // to MMA, by a constant step, so the issuing thread spends one add per operand instead of rebuilding 64-bit
 // descriptors (the first version's ~40 instructions per MMA on a single thread cost more than the MMA's 128 cycles).

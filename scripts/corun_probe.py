@@ -45,17 +45,3 @@ for name, f in (("gemm", gemm), ("attention", attn)):
     torch.cuda.synchronize()
     tpc, txc = p0.elapsed_time(p1), c0.elapsed_time(c1) / reps
     print(f"{name:10s}: alone {tx:.3f} ms | beside pool {txc:.3f} ms ({txc/tx:.2f}x) | pool beside it {tpc:.3f} ms (speed {tp/tpc:.2f})")
-# ---- footprint only: a spinning persistent kernel with the GEMM's threads / registers and varying shared memory
-import ctypes as C
-from infinite_video_b200 import _capi
-lib = _capi.lib()
-lib.ltm_debug_footprint_spin.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]; lib.ltm_debug_footprint_spin.restype = C.c_int
-for threads, smem in ((320, 214 * 1024), (320, 150 * 1024), (320, 100 * 1024), (320, 16 * 1024), (576, 214 * 1024), (128, 214 * 1024)):
-    torch.cuda.synchronize()
-    p0, p1 = torch.cuda.Event(True), torch.cuda.Event(True)
-    with torch.cuda.stream(comp):
-        lib.ltm_debug_footprint_spin(148, threads, smem, 3000, C.c_void_p(comp.cuda_stream))
-    with torch.cuda.stream(side):
-        p0.record(); ops.pool_mean(k, 1); p1.record()
-    torch.cuda.synchronize()
-    print(f"spin footprint {threads} thr x 96 regs, {smem//1024} KB smem: pool {p0.elapsed_time(p1):.3f} ms (speed {tp/p0.elapsed_time(p1):.2f})")

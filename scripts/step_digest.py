@@ -39,7 +39,6 @@ CONFIGS = [
     ("generic_no_kv_state_proj_tf32x3", dict(fast_attn=False, kv_state=False, proj_precision="tf32x3"), SMALL, "fp32",
      LOCKSTEP),
     ("n512", {}, dict(Bv=2, L=32, N=512), "fp32", LOCKSTEP + RAGGED),
-    ("video_block32", dict(video_block=32), BIG, "fp32", LOCKSTEP[:4] + RAGGED),
     ("bin_pool_true", dict(bin_pool=True), dict(Bv=2, L=256, N=256), "fp32", LOCKSTEP),
     ("bin_pool_false", dict(bin_pool=False), dict(Bv=2, L=256, N=256), "fp32", LOCKSTEP),
     ("not_sticky", dict(sticky=False), SMALL, "fp32", LOCKSTEP + RAGGED),
@@ -164,12 +163,9 @@ def main():
         for i, (name, kw, shape, dtype, entries) in enumerate(CONFIGS):
             if only is not None and name not in only:
                 continue
-            kw = dict(kw)
-            vb = kw.pop("video_block", 0)
             ks = qs = us = None
             for entry in entries:
                 eng = BatchedRectLTM(shape["N"], 0.75, *w, device=dev, **kw)
-                eng.video_block = vb
                 if ks is None:
                     ks, qs, us, nds = _inputs(torch, dev, name, shape, dtype, eng.S, 100 + i)
                 rag = _ragged_schedule(np, shape["Bv"], shape["L"], 200 + i) if entry.startswith("ragged") else None

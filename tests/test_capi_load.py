@@ -63,16 +63,18 @@ def test_version_and_error_convention(lib):
 def test_ctypes_structs_match_c_layout(tmp_path):
     prog = tmp_path / "sz.c"
     prog.write_text('#include <stdio.h>\n#include <stddef.h>\n#include "infltm.h"\n'
-                    'int main(){printf("%zu %zu %zu %zu %zu %zu %zu %zu %zu\\n", sizeof(ltm_gemm_args), offsetof(ltm_gemm_args, C),'
+                    'int main(){printf("%zu %zu %zu %zu %zu %zu %zu %zu %zu %zu %zu\\n", sizeof(ltm_gemm_args), offsetof(ltm_gemm_args, C),'
                     ' offsetof(ltm_gemm_args, impl), sizeof(ltm_rect_step_args), offsetof(ltm_rect_step_args, W_out),'
                     ' offsetof(ltm_rect_step_args, ctx_dev), offsetof(ltm_gemm_args, round_tf32),'
-                    ' offsetof(ltm_rect_step_args, X), offsetof(ltm_rect_step_args, c_none));return 0;}\n')
+                    ' offsetof(ltm_rect_step_args, X), offsetof(ltm_rect_step_args, c_none),'
+                    ' offsetof(ltm_rect_step_args, attn_part), offsetof(ltm_rect_step_args, hist_keep));return 0;}\n')
     exe = tmp_path / "sz"
     subprocess.check_call(["gcc", "-I", os.path.join(ROOT, "include"), str(prog), "-o", str(exe)])
     got = [int(x) for x in subprocess.check_output([str(exe)], text=True).split()]
     want = [C.sizeof(_capi.GemmArgs), _capi.GemmArgs.C.offset, _capi.GemmArgs.impl.offset,
             C.sizeof(_capi.RectStepArgs), _capi.RectStepArgs.W_out.offset, _capi.RectStepArgs.ctx_dev.offset,
-            _capi.GemmArgs.round_tf32.offset, _capi.RectStepArgs.X.offset, _capi.RectStepArgs.c_none.offset]
+            _capi.GemmArgs.round_tf32.offset, _capi.RectStepArgs.X.offset, _capi.RectStepArgs.c_none.offset,
+            _capi.RectStepArgs.attn_part.offset, _capi.RectStepArgs.hist_keep.offset]
     assert got == want
 
 

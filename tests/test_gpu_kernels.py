@@ -467,9 +467,9 @@ GEMM_CASES = [
     (128, 128, 256, 1, True, True, False, True),
     (256, 1536, 768, 1, True, True, False, True),      # K/V projection shape (per 256 coefficient rows)
     (100, 72, 40, 1, True, True, False, False),        # ragged tails everywhere
-    (384, 1536, 768, 1, True, True, False, True),      # odd number of row tiles (2-CTA multicast clusters)
-    (300, 520, 64, 2, True, True, False, True),        # ragged + batched through the cluster path
-    (1152, 256, 96, 1, False, True, False, False),     # A MN-major, B K-major multicast
+    (384, 1536, 768, 1, True, True, False, True),      # odd number of row tiles
+    (300, 520, 64, 2, True, True, False, True),        # ragged tails in M and N, batched, bias
+    (1152, 256, 96, 1, False, True, False, False),     # A MN-major, B K-major, nine row tiles
     (128, 768, 256, 3, True, False, False, False),     # Psi_tab @ B_past[v]   (B MN-major, batched)
     (256, 768, 544, 2, True, False, True, False),      # G_inf^T [xm ; k]      (two K segments)
     (64, 768, 8, 2, True, False, False, False),        # G0^T k with Lk = 8
@@ -478,30 +478,9 @@ GEMM_CASES = [
 ]
 
 
-@pytest.fixture(params=["pair", "single", "multicast"])
-def gemm_cluster(request):
-    """Runs the GEMM tests through the three kernel variants: CTA pairs (tcgen05 cta_group::2), single-CTA (the default), and single-CTA MMAs with 2-CTA TMA multicast (bring-up hooks)."""
-    import ctypes
-    from infinite_video_b200 import _capi
-    lib = _capi.lib()
-    if not hasattr(lib, "ltm_debug_set_pair"):
-        # product build: the variant kernels and their selection hooks are compiled only with INFLTM_BRINGUP=1
-        if request.param != "single":
-            pytest.skip("kernel variant exists in bring-up builds only")
-        yield request.param
-        return
-    for f in (lib.ltm_debug_set_cluster, lib.ltm_debug_set_pair):
-        f.argtypes, f.restype = [ctypes.c_int], None
-    lib.ltm_debug_set_pair(1 if request.param == "pair" else 0)
-    lib.ltm_debug_set_cluster(2 if request.param == "multicast" else 1)
-    yield request.param
-    lib.ltm_debug_set_pair(0)                  # back to the default
-    lib.ltm_debug_set_cluster(1)
-
-
 @pytest.mark.parametrize("M,N,K,batch,akm,bkm,two,bias", GEMM_CASES)
 @pytest.mark.parametrize("precision", ["tf32", "tf32x3"])
-def test_gemm_tcgen05(dev, gemm_cluster, M, N, K, batch, akm, bkm, two, bias, precision):
+def test_gemm_tcgen05(dev, M, N, K, batch, akm, bkm, two, bias, precision):
     ops = _ops()
     g = torch.Generator().manual_seed(M * 7 + N + K)
     A = torch.randn(*((M, K) if akm else (K, M)), generator=g)                  # shared across the batch
@@ -568,7 +547,7 @@ def test_tensor_core_attention_shapes(dev, Bv, N, Q, H, L):
 
 
 @pytest.mark.parametrize("M,N,K", [(512, 1536, 768), (300, 200, 136), (128, 256, 64)])
-def test_gemm_fp16_operands(dev, gemm_cluster, M, N, K):
+def test_gemm_fp16_operands(dev, M, N, K):
     """kind::f16 path of the tcgen05 GEMM: fp16 operands are exact inputs, products accumulate in fp32."""
     ops = _ops()
     g = torch.Generator().manual_seed(M + N + K)

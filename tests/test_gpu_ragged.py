@@ -360,3 +360,17 @@ def test_errors(dev):
             eng.step(k, q, u)                                               # lock-step continue of an empty slot
         with pytest.raises(RuntimeError):
             eng.x_past()
+
+
+def test_video_block_is_refused(dev):
+    """The step in blocks of videos was removed: a non-zero `video_block` set on the engine is an error, not a no-op."""
+    eng, _ = _engine(dev, 64)
+    k, q, _u = (t.to(dev) for t in _chunk(torch.Generator().manual_seed(43), 3, 8))
+    eng.video_block = 2
+    with torch.no_grad():
+        for run in (lambda: eng.step(k, q, new_doc=True), lambda: eng.step_overlapped(k, q, new_doc=True),
+                    lambda: eng.step(k, q, new_doc=True, lengths=[8, 8, 8])):
+            with pytest.raises(ValueError, match="video_block"):
+                run()
+        eng.video_block = 0
+        assert bool(torch.isfinite(eng.step(k, q, new_doc=True)).all())
