@@ -65,6 +65,13 @@ int ltm_pool_mean_16(const void* k, int is_bf16, float* xpart, int Bv, int L, in
  * dtype: 0 fp32, 1 fp16, 2 bfloat16 (16-bit: e % 8 == 0, ltm_pool_mean_16's summation). */
 int ltm_pool_mean_ragged(const void* k, int dtype, float* xpart, const int32_t* offs, int Bv, int L, int T, int e,
                          int splits, int frames, int max_ctas, void* stream);
+/* ragged twin of ltm_pool_mean_convert (fp32 chunk k[Bv, L, T, e], lengths as offs[Bv+1] above): xpart as
+ * ltm_pool_mean_ragged writes it for the same splits, and the chunk as IEEE fp16 padded per video,
+ * k16[Bv, ld16, e] (ld16 % 64 == 0, ld16 >= L*T): with n_v = lengths[v]*T, tokens [0, n_v) of video v hold the
+ * round-to-nearest-even cast, tokens [n_v, roundup64(n_v)) hold +0.0, and nothing past that is written -- the zero
+ * tail lets the short-term GEMMs run whole 64-token k-blocks (ltm_gemm_extents).  Only the frames listed are read. */
+int ltm_pool_mean_convert_ragged(const float* k, float* xpart, void* k16, const int32_t* offs, int Bv, int L, int T,
+                                 int e, int splits, int frames, int ld16, void* stream);
 
 /* ---- R6: sticky histogram of the previous call's density.  gibbs:196-203 (+score :224-230,
  * compute_probability :232-249).  scores[Bv,H,Q,N] -> hist_part[Bv,H,127] (sum over q; the sum
@@ -191,6 +198,12 @@ typedef struct {
   int max_ctas;
 } ltm_gemm_args;
 int ltm_gemm(const ltm_gemm_args* args, void* stream);
+/* ltm_gemm with per-batch extents (device int32 arrays of `batch` entries, each optional = NULL): the tiles of batch b
+ * whose first column is >= n_ext[b] are skipped (a tile that straddles n_ext[b] is computed and stored in full, up to
+ * Nc), and batch b accumulates over its first k_ext[b] K-elements only (a multiple of 64, the fp16 k-block; the
+ * operands must hold zeros in [K_b, roundup64) if K_b itself is not).  A batch with either extent 0 gets no tiles: its
+ * C is not written.  Supported: ab_fp16 with precision 1 and fp32 C (no B2, CT, c_fp16 or a_group). */
+int ltm_gemm_extents(const ltm_gemm_args* args, const int32_t* n_ext, const int32_t* k_ext, void* stream);
 
 /* ---- R9: K/V projection.  gibbs:312-313  keys=proj_key(B), values=proj_value(B).
  * KV[M, 2D] = Bcoef[M, e] * Wkv[2D, e]^T + bkv   (M = Bv*N; Wkv = [W_key ; W_value]). */
@@ -409,6 +422,13 @@ int ltm_blend(const float* a, const float* b, float alpha, float* out, int64_t n
  * fp32 -> fp16 conversion (round to nearest even) of the chunk tokens: operands of the kind::f16 short-term GEMMs */
 int ltm_softmax_rows_h(float* S, const float* mask, void* P16, int rows, int n, int rows_per_mask, float scale,
                        void* stream);
+/* the fp16 softmax of a ragged batch: S[rows, ld] and P16[rows, ld] (ld % 64 == 0); row r belongs to video
+ * v = r / rows_per_len and spans its first n_v = n_len[v] columns (n_len: device int32, rows / rows_per_len entries,
+ * n_v <= ld), softmax(S * scale + mask[v, :n_v]) with mask rows of pitch mask_ld (may be NULL).  A row of n_v
+ * columns is reduced in the order ltm_softmax_rows_h reduces a row of n = n_v.  P columns [n_v, roundup64(n_v)) are
+ * written as 0, nothing beyond; columns >= n_v of S and of the mask are not read; rows with n_v = 0 are not touched. */
+int ltm_softmax_rows_h_len(const float* S, const float* mask, void* P16, const int32_t* n_len, int rows, int ld,
+                           int mask_ld, int rows_per_len, float scale, void* stream);
 int ltm_to_half(const float* src, void* dst, int64_t n, void* stream);
 /* fp32 [rows, K] -> fp16 [rows, 3K], x ~ hi + lo in three K segments per row: side 0 (A operand) [hi | lo | hi], side 1
  * (B operand) [hi | hi | lo].  A plain fp16 ltm_gemm (ab_fp16) over K' = 3K then computes a_hi b_hi + a_lo b_hi +

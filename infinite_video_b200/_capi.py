@@ -91,6 +91,7 @@ _SIGS = {
     "ltm_pool_mean_16": (C.c_int, [_P, _I, _P, _I, _I, _I, _I, _I, _P]),
     "ltm_pool_mean_grid": (C.c_int, [_P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "ltm_pool_mean_ragged": (C.c_int, [_P, _I, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "ltm_pool_mean_convert_ragged": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "ltm_sticky_hist_rect": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "ltm_sticky_hist_rect_tiles": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "ltm_density_rect": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),
@@ -101,6 +102,7 @@ _SIGS = {
     "ltm_consolidate_rect_kv": (C.c_int, [_P, _P, _P, _L, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I,
                                           _I, _I, _I, _I, _I, _I, _P]),
     "ltm_gemm": (C.c_int, [C.POINTER(GemmArgs), _P]),
+    "ltm_gemm_extents": (C.c_int, [C.POINTER(GemmArgs), _P, _P, _P]),
     "ltm_project_kv": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "ltm_project_kv_t": (C.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "ltm_project_kv_r": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
@@ -125,6 +127,7 @@ _SIGS = {
     "ltm_gather_rows": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _P]),
     "ltm_softmax_rows": (C.c_int, [_P, _P, _I, _I, _I, _F, _P]),
     "ltm_softmax_rows_h": (C.c_int, [_P, _P, _P, _I, _I, _I, _F, _P]),
+    "ltm_softmax_rows_h_len": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _F, _P]),
     "ltm_to_half": (C.c_int, [_P, _P, _L, _P]),
     "ltm_blend": (C.c_int, [_P, _P, _F, _P, _L, _P]),
     "ltm_event_create": (C.c_int, [C.POINTER(C.c_void_p)]),

@@ -672,7 +672,9 @@ class BatchedRectLTM(_BatchedBase):
         (pooled, k16[Bv, L*T, e]) -- the operand of the caller's short-term attention (SURVEY 8f N1).
         `lengths` (ragged chunk, see `step`): only the first lengths[v] frames of video v are pooled and read; the
         result is packed video after video, [sum(lengths), splits, e] with splits = `_splits(sum(lengths))`, and is
-        handed to `step(..., pooled=..., lengths=...)` with the same lengths."""
+        handed to `step(..., pooled=..., lengths=...)` with the same lengths.  With `with_half` (fp32 chunks) it comes
+        with k16[Bv, ld16, e], ld16 = L*T rounded up to 64 tokens: video v's first n_v = lengths[v]*T tokens as fp16,
+        zeros up to roundup64(n_v), the rest unwritten (ltm_pool_mean_convert_ragged)."""
         require_cuda(k)
         k = k.contiguous()
         Bv, LT, e = k.shape
@@ -681,11 +683,14 @@ class BatchedRectLTM(_BatchedBase):
         L = LT // self.T
         if lengths is not None:
             dtype = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}.get(k.dtype)
-            if with_half or dtype is None:
-                raise ValueError("a ragged chunk is pooled from float32 / float16 / bfloat16 storage, without with_half")
+            if dtype is None or (with_half and dtype != 0):
+                raise ValueError("a ragged chunk is pooled from float32 / float16 / bfloat16 storage (with_half: float32)")
             lens = _as_lengths(lengths, Bv, L)
             frames = sum(lens)
             splits = self._splits(frames)
+            if with_half:
+                return ops.pool_mean_convert_ragged(k.view(Bv, L, self.T, e), self._lengths_dev(lens)[1], frames, splits,
+                                                    (LT + 63) // 64 * 64)
             out = torch.empty(frames, splits, e, device=self.device, dtype=torch.float32)
             if frames:
                 self._pool_launch(k, out, Bv, L, splits, 0, stream_ptr(self.device), offs=self._lengths_dev(lens)[1],

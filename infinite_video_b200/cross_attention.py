@@ -18,11 +18,18 @@ small streaming kernels.  The key/value projections are the ones the LTM shares 
 """
 import math
 
+import numpy as np
 import torch
 import torch.nn as nn
 
 from . import ops
+from .batched import _as_lengths
 from .ltm import LongTermAttention
+
+
+class RaggedUnsupported(NotImplementedError, ValueError):
+    """Per-video lengths with a configuration that has no ragged path (the Gaussian LTM variant): an unsupported
+    feature (NotImplementedError) and an invalid argument combination (ValueError), raised before any launch."""
 
 
 def encoder_mask_rows(mask, B, LT, device=None):
@@ -97,16 +104,35 @@ class CrossAttentionLTM(nn.Module):
         return ops.gemm_raw(x, K, 0, True, w, K, 0, True, out, lin.out_features, 0, M, lin.out_features, K, 1,
                             bias=b, precision=precision)
 
+    def _ragged_lengths(self, B, LT, e, lengths):
+        """Validated per-video lengths (frames) of a ragged call, before anything is launched."""
+        if self.operands != "fp16":
+            raise ValueError("per-video lengths need operands='fp16' (the fp32 path reads the padding of the chunk)")
+        T = self.long_term_attention.tokens_per_frame
+        if e % 8:
+            raise ValueError(f"per-video lengths need a token width that is a multiple of 8, got {e}")
+        if LT % T or LT // T < 2:
+            raise ValueError(f"the chunk has {LT} tokens: a ragged chunk is padded to L*{T} tokens, L >= 2")
+        return _as_lengths(lengths, B, LT // T)
+
     @torch.no_grad()
-    def short_term(self, q, enc, mask=None, enc16=None):
+    def short_term(self, q, enc, mask=None, enc16=None, lengths=None):
         """softmax(q_h K_h^T / sqrt(d) + mask) V_h for all heads.  q[B,Q,D] (already projected), enc[B,LT,e] fp32,
         mask: additive, one row per video ([B, LT], [B, 1, LT] or [B, 1, 1, LT], `encoder_mask_rows`) or None; enc16:
         the chunk as float16 when the caller already has it (the pooling pass of the LTM writes it,
-        `LongTermAttention.pool_for_caller`).  Returns [B,Q,D]."""
+        `LongTermAttention.pool_for_caller`).  Returns [B,Q,D].
+        lengths: per-video chunk lengths in frames (host ints, 0 = idle, else in [2, L]); video v attends over its
+        first n_v = lengths[v] * T tokens only -- the rest of its chunk and of its mask row is never read -- and the
+        rows of idle videos are zero.  enc16 is then the padded fp16 chunk [B, ld16, e] of `pool_for_caller(enc,
+        lengths)` (ld16 = L*T rounded up to 64 tokens)."""
         B, Q, D = q.shape
         LT, e = enc.shape[1], enc.shape[2]
         H, d = self.H, self.d
         dev = q.device
+        if lengths is not None:
+            lens = self._ragged_lengths(B, LT, e, lengths)
+            mask = encoder_mask_rows(mask, B, LT, dev)
+            return self._short_term_ragged(q, enc, mask, enc16, lens)
         mask = encoder_mask_rows(mask, B, LT, dev)
         wk = self.key.weight.detach().float().contiguous()          # [D, e]
         wv = self.value.weight.detach().float().contiguous()
@@ -160,20 +186,90 @@ class CrossAttentionLTM(nn.Module):
                          bias=bv, bias_stride=d, precision="tf32x3", c_offset=v0 * Q * D)
         return out
 
+    def _short_term_ragged(self, q, enc, mask, enc16, lens):
+        """The short-term half of a ragged batch on the fp16 path.  Per video v, n_v = lengths[v] * T tokens:
+        scores through the GEMM with column extents n_v (S rows of pitch ld16), the softmax over the first n_v columns
+        with a zero tail up to roundup64(n_v), the values GEMM over roundup64(n_v) tokens (k16 and P hold zeros past
+        n_v), then the per-head GEMM as in the lock-step path.  Idle videos get no tiles and zero rows."""
+        B, Q, D = q.shape
+        LT, e = enc.shape[1], enc.shape[2]
+        H, d = self.H, self.d
+        T = self.long_term_attention.tokens_per_frame
+        dev = q.device
+        ld16 = (LT + 63) // 64 * 64
+        n = np.asarray(lens, np.int64) * T
+        idle = np.flatnonzero(n == 0)
+        # one upload: n_v [B] | roundup64(n_v) [B] | frame offsets [B+1] | idle videos
+        host = np.concatenate([n, (n + 63) // 64 * 64, np.concatenate([[0], np.cumsum(lens)]), idle]).astype(np.int32)
+        ext = torch.from_numpy(host).pin_memory().to(dev, non_blocking=True)
+        n_dev, k_dev, offs = ext[:B], ext[B:2 * B], ext[2 * B:3 * B + 1]
+        if enc16 is None:
+            L = LT // T
+            enc16 = ops.pool_mean_convert_ragged(enc.contiguous().view(B, L, T, e), offs, int(sum(lens)), 1, ld16)[1]
+        elif enc16.dtype != torch.float16 or tuple(enc16.shape) != (B, ld16, e) or not enc16.is_contiguous():
+            raise ValueError(f"enc16 of a ragged call must be a contiguous float16 [{B}, {ld16}, {e}] tensor")
+        wk = self.key.weight.detach().float().contiguous()          # [D, e]
+        wv = self.value.weight.detach().float().contiguous()
+        bv = self.value.bias.detach().float().contiguous() if self.value.bias is not None else None
+        out = torch.empty(B, Q, D, device=dev, dtype=torch.float32)
+        for v0 in range(0, B, self.videos_per_pass):
+            nb = min(self.videos_per_pass, B - v0)
+            if not any(lens[v0:v0 + nb]):
+                continue                                 # every video of the pass idle: rows zeroed below
+            qv = q[v0:v0 + nb].contiguous()
+            e16 = enc16[v0:v0 + nb]
+            ne, ke = n_dev[v0:v0 + nb], k_dev[v0:v0 + nb]
+            Qt = torch.empty(nb, H, Q, e, device=dev, dtype=torch.float16)
+            ops.gemm_raw(qv, D, d, True, wk, e, d * e, False, Qt, e, Q * e, nb * Q, e, d, H,
+                         c_group=Q, c_group_stride=H * Q * e, precision="tf32x3", c_fp16=True)
+            # scores: tiles of video v with a first column >= n_v are skipped
+            S = torch.empty(nb, H * Q, ld16, device=dev, dtype=torch.float32)
+            ops.gemm_raw(Qt, e, H * Q * e, True, e16, e, ld16 * e, True, S, ld16, H * Q * ld16, H * Q, LT, e, nb,
+                         precision="tf32", ab_fp16=True, n_ext=ne)
+            m = None if mask is None else mask[v0:v0 + nb]
+            P = ops.softmax_rows_half_len(S, ne, H * Q, 1.0 / math.sqrt(d), m)
+            # values over the first roundup64(n_v) tokens of video v (P and k16 are zero past n_v)
+            Yh = torch.empty(H, nb, Q, e, device=dev, dtype=torch.float32)
+            ops.gemm_raw(P, ld16, H * Q * ld16, True, e16, e, ld16 * e, False, Yh, e, Q * e, H * Q, e, ld16, nb,
+                         c_group=Q, c_group_stride=nb * Q * e, precision="tf32", ab_fp16=True, k_ext=ke)
+            ops.gemm_raw(Yh, e, nb * Q * e, True, wv, e, d * e, True, out, D, d, nb * Q, d, e, H,
+                         bias=bv, bias_stride=d, precision="tf32x3", c_offset=v0 * Q * D)
+        if len(idle):
+            # (Yh of an idle video is never written: its rows of `out` are garbage until here)
+            out.index_fill_(0, ext[3 * B + 1:].long(), 0.0)
+        return out
+
     @torch.no_grad()
     def forward(self, hidden_states, encoder_hidden_states, new_video=False, layer=None,
-                encoder_attention_mask=None, u=None):
-        """Returns the blended context layer [B,Q,D] (what `BertSelfAttention.forward` returns as outputs[0])."""
+                encoder_attention_mask=None, u=None, lengths=None):
+        """Returns the blended context layer [B,Q,D] (what `BertSelfAttention.forward` returns as outputs[0]).
+        lengths: per-video chunk lengths in frames of a ragged batch (host ints, 0 = idle, else in [2, L]; the
+        chunk is padded to L frames and its padding is never read).  new_video is then a bool or one host flag per
+        video; idle videos keep their memory and get zero rows.  Needs operands='fp16' and the 'gibbs' LTM variant."""
         if not hidden_states.is_cuda:
             raise RuntimeError("CrossAttentionLTM runs on CUDA tensors only (no CPU fallback)")
         B, Q, _ = hidden_states.shape
         # HF additive mask [B,1,1,LT] -> [B,LT], validated before anything is launched
         enc = encoder_hidden_states
         mask = encoder_mask_rows(encoder_attention_mask, B, enc.shape[1], enc.device)
+        ltm = self.long_term_attention
+        if lengths is not None:
+            lens = self._ragged_lengths(B, enc.shape[1], enc.shape[2], lengths)
+            if self.alpha != 1.0:
+                if ltm.variant != "gibbs":
+                    raise RaggedUnsupported("per-video lengths exist for the 'gibbs' LTM variant only")
+                ltm.check_ragged(enc, lens, new_video, Q)
+            enc = enc.float().contiguous()
+            q = self._linear(hidden_states.float().reshape(B * Q, -1).contiguous(), self.query, "tf32x3").view(B, Q, -1)
+            enc16 = ltm.pool_for_caller(enc, lens) if (self.alpha != 1.0 and ltm.share_pooling) else None
+            ctx = self._short_term_ragged(q, enc, mask, enc16, lens)
+            if self.alpha == 1.0:
+                return ctx.to(hidden_states.dtype)
+            a_long = ltm(enc, q, new_doc=new_video, layer_n=layer, u=u, lengths=lens)
+            return ops.blend(ctx, a_long.float(), self.alpha).to(hidden_states.dtype)
         enc = enc.float().contiguous()
         q = self._linear(hidden_states.float().reshape(B * Q, -1).contiguous(), self.query, "tf32x3")
         q = q.view(B, Q, -1)
-        ltm = self.long_term_attention
         enc16 = None
         if (self.alpha != 1.0 and self.operands == "fp16" and ltm.variant == "gibbs" and ltm.share_pooling
                 and enc.dtype == torch.float32 and enc.is_contiguous() and enc.shape[2] % 8 == 0 and enc.shape[1] % 8 == 0

@@ -55,6 +55,8 @@ struct GemmDev {
   int c_half;                               // C is fp16 storage (row-major path only)
   void* C_lo;                               // fp16 output only: second array for the residual x - float(half(x))
   int max_ctas;                             // bound of the persistent grid (0 = one CTA per SM)
+  const int32_t* n_ext;                     // EXT instances: per-batch column bound (NULL = Nc) ...
+  const int32_t* k_ext;                     // ... and K bound, a multiple of the 64-element fp16 k-block (NULL = K)
 };
 
 // Work item -> tile origin: items are tiles, n fastest.
@@ -63,6 +65,28 @@ __device__ __forceinline__ void decode_work(int w, int tiles_n, int tiles_m, int
   n0 = (w % tiles_n) * BN_;
   m0 = ((w / tiles_n) % tiles_m) * 128;
   bz = w / (tiles_n * tiles_m);
+}
+// k-blocks of a tile of batch bz: all of them, or (EXT with k_ext) k_ext[bz] / 64 of them (fp16 k-blocks)
+template <bool EXT>
+__device__ __forceinline__ int tile_kb(const GemmDev& g, int bz, int num_kb) {
+  if (!EXT || g.k_ext == nullptr) return num_kb;
+  const int kb = __ldg(g.k_ext + bz) / 64;
+  return kb < num_kb ? kb : num_kb;
+}
+// First work item >= w of this CTA's static list that has work: without EXT, w itself; with EXT, tiles whose first
+// column lies at or past n_ext[bz], or whose batch runs no k-block, are skipped.  Every role walks the list through
+// this function, so producer, MMA issuer and epilogue agree on the tiles they skip.
+template <bool EXT, int BN_>
+__device__ __forceinline__ int next_work(const GemmDev& g, int w, int stride, int num_work, int tiles_n, int tiles_m,
+                                         int num_kb) {
+  if (EXT) {
+    for (; w < num_work; w += stride) {
+      int n0, m0, bz;
+      decode_work<BN_>(w, tiles_n, tiles_m, n0, m0, bz);
+      if ((g.n_ext == nullptr || n0 < __ldg(g.n_ext + bz)) && tile_kb<true>(g, bz, num_kb) > 0) break;
+    }
+  }
+  return w;
 }
 // MN-major descriptor parameters.  For 32-bit (tf32) MN-major operands the only legal canonical layout is
 // the 128-byte swizzle with 32-byte atoms (TMA: SWIZZLE_128B_ATOM_32B): atoms of [4 k][32 mn], i.e. the
@@ -298,7 +322,8 @@ struct Cfg {
 //   warp 1      TMEM owner + tcgen05.mma issuer (one lane)
 //   warps 2-9   epilogue (see epilogue_tile)
 //   warps 10-17 (precision 3 only) operand splitter hi/lo
-template <int BN, int STAGES, bool SPLIT, bool HOUT>
+//   EXT: per-batch extents (n_ext / k_ext, see next_work and tile_kb)
+template <int BN, int STAGES, bool SPLIT, bool HOUT, bool EXT>
 __global__ void __maxnreg__(GEMM_MAX_REGS)
 gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
                  const __grid_constant__ CUtensorMap mapB2, const GemmDev g) {
@@ -356,11 +381,13 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
     // ------------------------------------------------------------------ TMA producer
     if (lane == 0) {
       uint32_t it = 0;
-      for (int w = w_first; w < num_work; w += w_stride) {
+      for (int w = next_work<EXT, BN>(g, w_first, w_stride, num_work, tiles_n, tiles_m, num_kb); w < num_work;
+           w = next_work<EXT, BN>(g, w + w_stride, w_stride, num_work, tiles_n, tiles_m, num_kb)) {
         int n0, m0, bz;
         decode_work<BN>(w, tiles_n, tiles_m, n0, m0, bz);
         const int za = g.a_batched ? bz : 0;
-        for (int kb = 0; kb < num_kb; ++kb, ++it) {
+        const int nkb = tile_kb<EXT>(g, bz, num_kb);
+        for (int kb = 0; kb < nkb; ++kb, ++it) {
           const int s = it % STAGES;
           const uint32_t ph = (it / STAGES) & 1u;
           mbar_wait(empty_bar(s), ph ^ 1u);
@@ -412,12 +439,16 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
       const uint32_t da0 = wa.lo0 + ((smem_base & 0x3FFFFu) >> 4), db0 = wb.lo0 + (((smem_base + A_BYTES) & 0x3FFFFu) >> 4);
       const uint32_t dal0 = da0 + STAGES * (C_::STAGE_BYTES >> 4), dbl0 = db0 + STAGES * (C_::STAGE_BYTES >> 4);
       uint32_t it = 0, tc = 0;
-      for (int w = w_first; w < num_work; w += w_stride, ++tc) {
+      for (int w = next_work<EXT, BN>(g, w_first, w_stride, num_work, tiles_n, tiles_m, num_kb); w < num_work;
+           w = next_work<EXT, BN>(g, w + w_stride, w_stride, num_work, tiles_n, tiles_m, num_kb), ++tc) {
+        int n0, m0, bz;
+        decode_work<BN>(w, tiles_n, tiles_m, n0, m0, bz);
+        const int nkb = tile_kb<EXT>(g, bz, num_kb);
         const uint32_t buf = tc & 1u, tph = (tc >> 1) & 1u;
         mbar_wait(tempty_bar(buf), tph ^ 1u);                 // epilogue has drained this accumulator
         tcgen05_fence_after();
         const uint32_t tmem_acc = tmem_base + buf * BN;
-        for (int kb = 0; kb < num_kb; ++kb, ++it) {
+        for (int kb = 0; kb < nkb; ++kb, ++it) {
           const int s = it % STAGES;
           const uint32_t ph = (it / STAGES) & 1u;
           mbar_wait(SPLIT ? split_bar(s) : full_bar(s), ph);
@@ -448,7 +479,8 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
     const int ew = warp - 2;
     float* stg = staging + ew * STG_WARP_FLOATS;
     uint32_t tc = 0;
-    for (int w = w_first; w < num_work; w += w_stride, ++tc) {
+    for (int w = next_work<EXT, BN>(g, w_first, w_stride, num_work, tiles_n, tiles_m, num_kb); w < num_work;
+         w = next_work<EXT, BN>(g, w + w_stride, w_stride, num_work, tiles_n, tiles_m, num_kb), ++tc) {
       int n0, m0, bz;
       decode_work<BN>(w, tiles_n, tiles_m, n0, m0, bz);
       const uint32_t buf = tc & 1u, tph = (tc >> 1) & 1u;
@@ -462,8 +494,12 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
       const int et = threadIdx.x - ROLE_THREADS;  // 0..SPLIT_THREADS-1
       constexpr int NV = (A_BYTES + C_::B_BYTES) / 16;      // float4 count of [A | B]
       uint32_t it = 0;
-      for (int w = w_first; w < num_work; w += w_stride) {
-        for (int kb = 0; kb < num_kb; ++kb, ++it) {
+      for (int w = next_work<EXT, BN>(g, w_first, w_stride, num_work, tiles_n, tiles_m, num_kb); w < num_work;
+           w = next_work<EXT, BN>(g, w + w_stride, w_stride, num_work, tiles_n, tiles_m, num_kb)) {
+        int n0, m0, bz;
+        decode_work<BN>(w, tiles_n, tiles_m, n0, m0, bz);
+        const int nkb = tile_kb<EXT>(g, bz, num_kb);
+        for (int kb = 0; kb < nkb; ++kb, ++it) {
           const int s = it % STAGES;
           const uint32_t ph = (it / STAGES) & 1u;
           mbar_wait(full_bar(s), ph);
@@ -572,24 +608,25 @@ int tma_encode_2d(CUtensorMap* map, const float* base, unsigned long long inner,
   return 0;
 }
 
-template <int BN, int STAGES, bool SPLIT, bool HOUT = false>
+template <int BN, int STAGES, bool SPLIT, bool HOUT = false, bool EXT = false>
 static int launch_cfg(const CUtensorMap& mA, const CUtensorMap& mB, const CUtensorMap& mB2, const GemmDev& d,
                       int batch, cudaStream_t stream) {
   using C_ = Cfg<BN, STAGES, SPLIT>;
   static PerDevice pd = {};
   int num_sms = 0;
-  if (int rc = kernel_setup(gemm_tf32_kernel<BN, STAGES, SPLIT, HOUT>, (size_t)C_::SMEM_BYTES, pd, &num_sms))
+  if (int rc = kernel_setup(gemm_tf32_kernel<BN, STAGES, SPLIT, HOUT, EXT>, (size_t)C_::SMEM_BYTES, pd, &num_sms))
     return rc;
   const long long tiles = (long long)((d.Nc + BN - 1) / BN) * ((d.M + BM - 1) / BM) * batch;
   LTM_REQUIRE(tiles < (1ll << 31), "gemm: too many tiles");
   unsigned grid = (unsigned)(tiles < num_sms ? tiles : num_sms);     // persistent: one CTA per SM
   if (d.max_ctas > 0 && (unsigned)d.max_ctas < grid) grid = (unsigned)d.max_ctas;   // ... or fewer (ltm_gemm_args.max_ctas)
-  gemm_tf32_kernel<BN, STAGES, SPLIT, HOUT><<<grid, C_::THREADS, C_::SMEM_BYTES, stream>>>(mA, mB, mB2, d);
+  gemm_tf32_kernel<BN, STAGES, SPLIT, HOUT, EXT><<<grid, C_::THREADS, C_::SMEM_BYTES, stream>>>(mA, mB, mB2, d);
   LTM_CHECK_LAUNCH("gemm(tcgen05)");
   return 0;
 }
 
-static int gemm_tcgen05_launch(const ltm_gemm_args& a, cudaStream_t stream) {
+static int gemm_tcgen05_launch(const ltm_gemm_args& a, cudaStream_t stream, const int32_t* n_ext = nullptr,
+                               const int32_t* k_ext = nullptr) {
   if (resolve_encode()) return -1;
   const bool two = a.B2 != nullptr && a.K1 < a.K;
   const int half = a.ab_fp16 ? 1 : 0;
@@ -657,6 +694,11 @@ static int gemm_tcgen05_launch(const ltm_gemm_args& a, cudaStream_t stream) {
   LTM_REQUIRE(a.C_lo == nullptr || (a.c_fp16 && aligned16(a.C_lo)), "gemm: C_lo needs c_fp16 and 16-byte alignment");
   LTM_REQUIRE(!a.c_fp16 || a.CT == nullptr, "gemm: fp16 output has no transposed store");
   d.a_batched = a.strideA != 0; d.b_batched = a.strideB != 0; d.b2_batched = a.strideB2 != 0; d.has_b2 = two ? 1 : 0;
+  if (n_ext != nullptr || k_ext != nullptr) {      // ltm_gemm_extents: fp16 operands, precision 1, fp32 C (checked there)
+    d.n_ext = n_ext; d.k_ext = k_ext;
+    return bn == 256 ? launch_cfg<256, 4, false, false, true>(mA, mB, mB2, d, a.batch, stream)
+                     : launch_cfg<128, 6, false, false, true>(mA, mB, mB2, d, a.batch, stream);
+  }
   if (d.c_half) {           // fp16 output (the projected-memory K|V; Qt of the short-term attention)
     if (split) return bn == 256 ? launch_cfg<256, 2, true, true>(mA, mB, mB2, d, a.batch, stream)
                                 : launch_cfg<128, 4, true, true>(mA, mB, mB2, d, a.batch, stream);
@@ -671,7 +713,7 @@ static int gemm_tcgen05_launch(const ltm_gemm_args& a, cudaStream_t stream) {
 
 }  // namespace ltm
 
-extern "C" int ltm_gemm(const ltm_gemm_args* args, void* stream) {
+static int gemm_checked(const ltm_gemm_args* args, const int32_t* n_ext, const int32_t* k_ext, void* stream) {
   using namespace ltm;
   LTM_REQUIRE(args != nullptr, "gemm: null argument block");
   const ltm_gemm_args& a = *args;
@@ -687,7 +729,21 @@ extern "C" int ltm_gemm(const ltm_gemm_args* args, void* stream) {
   LTM_REQUIRE(!(a.c_fp16 && a.impl == 1), "gemm: fp16 output exists in the tcgen05 kernel only");
   if (a.impl == 1) return gemm_simt_launch(a, (cudaStream_t)stream);
   LTM_REQUIRE(a.impl == 0, "gemm: unknown impl %d", a.impl);
-  return gemm_tcgen05_launch(a, (cudaStream_t)stream);
+  return gemm_tcgen05_launch(a, (cudaStream_t)stream, n_ext, k_ext);
+}
+
+extern "C" int ltm_gemm(const ltm_gemm_args* args, void* stream) { return gemm_checked(args, nullptr, nullptr, stream); }
+
+extern "C" int ltm_gemm_extents(const ltm_gemm_args* args, const int32_t* n_ext, const int32_t* k_ext, void* stream) {
+  using namespace ltm;
+  LTM_REQUIRE(args != nullptr, "gemm_extents: null argument block");
+  const ltm_gemm_args& a = *args;
+  LTM_REQUIRE(a.ab_fp16 && a.precision == 1 && a.impl == 0,
+              "gemm_extents: only fp16 operands with precision 1 on tcgen05 (ab_fp16=%d precision=%d impl=%d)", a.ab_fp16,
+              a.precision, a.impl);
+  LTM_REQUIRE((a.B2 == nullptr || a.K1 >= a.K) && a.CT == nullptr && !a.c_fp16 && a.a_group == 0,
+              "gemm_extents: B2, the transposed store, fp16 output and grouped A rows are not supported");
+  return gemm_checked(args, n_ext, k_ext, stream);
 }
 
 extern "C" int ltm_project_kv_t(const float* Bcoef, const float* Wkv, const float* bkv, float* Kt, float* V, int M,

@@ -94,17 +94,15 @@ pool_bins_kernel(const float4* __restrict__ k, float4* __restrict__ xbin, const 
 // Frame pooling that also leaves an fp16 copy of the chunk behind (round to nearest even): the short-term attention of
 // the caller (Qformer.py:224-304) reads the same tokens as kind::f16 tensor-core operands, so the chunk is streamed
 // from HBM once for both (SURVEY 8f N1: "sharing the pass with frame pooling").  Same summation order as pool_unit.
-__global__ void __launch_bounds__(256)
-pool_mean_convert_kernel(const float4* __restrict__ k, float4* __restrict__ xpart, uint2* __restrict__ k16, int T,
-                         int e4, int splits, float Tf) {
-  const uint64_t pol = policy_evict_first();
-  const unsigned work = blockIdx.x;
-  const int unit = work / splits;
-  const int sp = work - unit * splits;
+// One (frame, token-split) item: token split sp of frame `src` of the chunk is pooled into row (unit * splits + sp) of
+// xpart and converted to the fp16 rows starting at token row `dst16` of k16.
+__device__ __forceinline__ void pool_convert_unit_at(const float4* __restrict__ k, float4* __restrict__ xpart,
+                                                     uint2* __restrict__ k16, int T, int e4, int splits, float Tf,
+                                                     int unit, int sp, size_t src, size_t dst16, uint64_t pol) {
   const int r0 = (int)(((long long)T * sp) / splits);
   const int r1 = (int)(((long long)T * (sp + 1)) / splits);
-  const float4* base = k + (size_t)unit * T * e4;
-  uint2* base16 = k16 + (size_t)unit * T * e4;
+  const float4* base = k + src * T * e4;
+  uint2* base16 = k16 + dst16 * e4;
   // lane pairs (c, c ^ 1) share 16-byte stores when every lane of the warp has a partner inside the row
   // (whole warps only: the exchange is a full-mask shuffle)
   const bool paired = (e4 % 32 == 0) && (reinterpret_cast<uintptr_t>(k16) & 15u) == 0;
@@ -159,6 +157,16 @@ pool_mean_convert_kernel(const float4* __restrict__ k, float4* __restrict__ xpar
     o.x = __fdiv_rn(o.x, Tf); o.y = __fdiv_rn(o.y, Tf); o.z = __fdiv_rn(o.z, Tf); o.w = __fdiv_rn(o.w, Tf);
     xpart[((size_t)unit * splits + sp) * e4 + c] = o;
   }
+}
+
+__global__ void __launch_bounds__(256)
+pool_mean_convert_kernel(const float4* __restrict__ k, float4* __restrict__ xpart, uint2* __restrict__ k16, int T,
+                         int e4, int splits, float Tf) {
+  const uint64_t pol = policy_evict_first();
+  const unsigned work = blockIdx.x;
+  const int unit = work / splits;
+  const int sp = work - unit * splits;
+  pool_convert_unit_at(k, xpart, k16, T, e4, splits, Tf, unit, sp, (size_t)unit, (size_t)unit * T, pol);
 }
 
 // one CTA per (frame, split)
@@ -276,6 +284,29 @@ pool_ragged_kernel(const void* __restrict__ k, float4* __restrict__ xpart, const
   }
 }
 
+// Ragged twin of pool_mean_convert_kernel, one CTA per (frame, token-split) item of pool_ragged_kernel: xpart packed
+// as there, the fp16 tokens of video v at rows [0, n_v) of its k16 block of ld16 rows (n_v = lengths[v] * T).  The
+// last item of a video also zeroes rows [n_v, roundup64(n_v)), so that GEMMs over whole 64-token k-blocks read zeros
+// past the video's end; nothing further is written.
+__global__ void __launch_bounds__(256)
+pool_convert_ragged_kernel(const float4* __restrict__ k, float4* __restrict__ xpart, uint2* __restrict__ k16,
+                           const int32_t* __restrict__ offs, int Bv, int L, int T, int e4, int splits, float Tf,
+                           long long ld16) {
+  const unsigned work = blockIdx.x;
+  const unsigned f = work / splits;
+  const int sp = (int)(work - f * splits);
+  const size_t src = ragged_src(offs, Bv, L, f);
+  const int v = (int)(src / L), l = (int)(src - (size_t)v * L);
+  pool_convert_unit_at(k, xpart, k16, T, e4, splits, Tf, (int)f, sp, src, (size_t)v * ld16 + (size_t)l * T,
+                       policy_evict_first());
+  uint2* v16 = k16 + (size_t)v * ld16 * e4;
+  if (sp == splits - 1 && f + 1 == (unsigned)__ldg(offs + v + 1)) {
+    const int n = (l + 1) * T, n64 = (n + 63) & ~63;
+    for (long long i = threadIdx.x; i < (long long)(n64 - n) * e4; i += blockDim.x)
+      v16[(size_t)n * e4 + i] = make_uint2(0u, 0u);
+  }
+}
+
 template <int DT>
 static void launch_pool_ragged(const void* k, float* xpart, const int32_t* offs, int Bv, int L, int T, int ev,
                                int splits, float Tf, unsigned total, int max_ctas, cudaStream_t st) {
@@ -311,6 +342,30 @@ extern "C" int ltm_pool_mean_ragged(const void* k, int dtype, float* xpart, cons
   else
     launch_pool_ragged<2>(k, xpart, offs, Bv, L, T, ev, splits, (float)T, (unsigned)units, max_ctas, st);
   LTM_CHECK_LAUNCH("pool_mean_ragged");
+  return 0;
+}
+
+extern "C" int ltm_pool_mean_convert_ragged(const float* k, float* xpart, void* k16, const int32_t* offs, int Bv, int L,
+                                            int T, int e, int splits, int frames, int ld16, void* stream) {
+  using namespace ltm;
+  LTM_REQUIRE(k && k16 && offs, "pool_mean_convert_ragged: null pointer");
+  LTM_REQUIRE(Bv > 0 && L > 0 && T > 0 && e > 0 && e % 4 == 0 && frames >= 0 && frames <= (long long)Bv * L,
+              "pool_mean_convert_ragged: bad shape Bv=%d L=%d T=%d e=%d frames=%d", Bv, L, T, e, frames);
+  LTM_REQUIRE(ld16 % 64 == 0 && ld16 >= (long long)L * T,
+              "pool_mean_convert_ragged: ld16=%d must be a multiple of 64 and >= L*T=%lld", ld16, (long long)L * T);
+  LTM_REQUIRE(splits >= 1 && splits <= T, "pool_mean_convert_ragged: splits=%d out of range [1,%d]", splits, T);
+  const long long units = (long long)frames * splits;
+  LTM_REQUIRE(units < (1ll << 31), "pool_mean_convert_ragged: too many frames");
+  if (units == 0) return 0;                        // every video idle: nothing to read, pool or write (xpart may be NULL)
+  LTM_REQUIRE(xpart != nullptr, "pool_mean_convert_ragged: null pointer");
+  LTM_REQUIRE(aligned16(k) && aligned16(xpart) && (reinterpret_cast<uintptr_t>(k16) & 7u) == 0,
+              "pool_mean_convert_ragged: pointer alignment");
+  const int e4 = e / 4;
+  const int threads = e4 >= 256 ? 256 : ((e4 + 31) / 32) * 32;
+  pool_convert_ragged_kernel<<<(unsigned)units, threads, 0, (cudaStream_t)stream>>>(
+      reinterpret_cast<const float4*>(k), reinterpret_cast<float4*>(xpart), reinterpret_cast<uint2*>(k16), offs, Bv, L,
+      T, e4, splits, (float)T, (long long)ld16);
+  LTM_CHECK_LAUNCH("pool_mean_convert_ragged");
   return 0;
 }
 

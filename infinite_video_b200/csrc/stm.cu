@@ -176,6 +176,121 @@ softmax_rows_reg_kernel(const float* __restrict__ S, const float* __restrict__ m
   }
 }
 
+// Columns 4i .. 4i+3 of a score row of n valid columns, scaled and masked; -inf past n (adds nothing to the max and
+// exp() = +0 to the sum).  Columns >= n of S and of the mask are not read.  With a mask, s * scale + m is one fused
+// multiply-add (one rounding), as the lock-step kernels compile `v *= scale; v += mm`.
+__device__ __forceinline__ float score_len(float s, const float* __restrict__ m, int c, float scale) {
+  return m ? __fmaf_rn(s, scale, __ldg(m + c)) : s * scale;
+}
+__device__ __forceinline__ float4 score4_len(const float* __restrict__ s, const float* __restrict__ m, int i, int n,
+                                             float scale) {
+  const int c = 4 * i;
+  float4 v;
+  if (c + 4 <= n) {
+    asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];"
+                 : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(s + c));
+    v.x = score_len(v.x, m, c, scale);
+    v.y = score_len(v.y, m, c + 1, scale);
+    v.z = score_len(v.z, m, c + 2, scale);
+    v.w = score_len(v.w, m, c + 3, scale);
+  } else {
+    v.x = score_len(__ldg(s + c), m, c, scale);
+    v.y = c + 1 < n ? score_len(__ldg(s + c + 1), m, c + 1, scale) : -INFINITY;
+    v.z = c + 2 < n ? score_len(__ldg(s + c + 2), m, c + 2, scale) : -INFINITY;
+    v.w = c + 3 < n ? score_len(__ldg(s + c + 3), m, c + 3, scale) : -INFINITY;
+  }
+  return v;
+}
+
+__device__ __forceinline__ uint2 half4_scaled(const float4& w, float inv) {
+  const __half2 lo = __floats2half2_rn(w.x * inv, w.y * inv), hi = __floats2half2_rn(w.z * inv, w.w * inv);
+  return make_uint2(*reinterpret_cast<const uint32_t*>(&lo), *reinterpret_cast<const uint32_t*>(&hi));
+}
+
+// Row softmax of a ragged batch with fp16 output: row r belongs to video r / rows_per_len and spans that video's first
+// n = n_len[video] columns.  The arithmetic (scale and mask in one FFMA, score4_len) and the reduction order are
+// those of softmax_rows_reg_kernel / softmax_rows_kernel on a row of n columns, so a row whose n is a multiple of 4
+// gets the same bits, with or without a mask; P columns
+// [n, roundup64(n)) are written as +0 (the value GEMM reads whole 64-column k-blocks), nothing beyond.  Rows with
+// n = 0 are not touched.  REG: the row (<= 8192 columns) stays in registers; otherwise S is read three times.
+template <bool REG>
+__global__ void __launch_bounds__(256)
+softmax_rows_len_kernel(const float* __restrict__ S, const float* __restrict__ mask, const int32_t* __restrict__ n_len,
+                        __half* __restrict__ P16, long long ld, long long mask_ld, int rows_per_len, float scale) {
+  constexpr int ITEMS = 8;
+  __shared__ float red[8];
+  const int row = blockIdx.x, vid = row / rows_per_len;
+  const int n = __ldg(n_len + vid);
+  if (n <= 0) return;
+  const float* s = S + (size_t)row * ld;
+  const float* m = mask ? mask + (size_t)vid * mask_ld : nullptr;
+  const int nq = (n + 3) >> 2, n64q = ((n + 63) & ~63) >> 2, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  float4 v[REG ? ITEMS : 1];
+  float mx = -INFINITY;
+  if (REG) {
+#pragma unroll
+    for (int k = 0; k < ITEMS; ++k) {
+      const int i = tid + 256 * k;
+      v[k] = make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY);
+      if (i < nq) {
+        v[k] = score4_len(s, m, i, n, scale);
+        mx = fmaxf(mx, fmaxf(fmaxf(v[k].x, v[k].y), fmaxf(v[k].z, v[k].w)));
+      }
+    }
+  } else {
+    for (int i = tid; i < nq; i += 256) {
+      const float4 w = score4_len(s, m, i, n, scale);
+      mx = fmaxf(mx, fmaxf(fmaxf(w.x, w.y), fmaxf(w.z, w.w)));
+    }
+  }
+  mx = warp_max(mx);
+  if (lane == 0) red[warp] = mx;
+  __syncthreads();
+  mx = red[0];
+#pragma unroll
+  for (int w = 1; w < 8; ++w) mx = fmaxf(mx, red[w]);
+  __syncthreads();
+  float sum = 0.f;
+  if (REG) {
+#pragma unroll
+    for (int k = 0; k < ITEMS; ++k) {
+      if (tid + 256 * k < nq) {
+        v[k].x = expf(v[k].x - mx); v[k].y = expf(v[k].y - mx); v[k].z = expf(v[k].z - mx); v[k].w = expf(v[k].w - mx);
+        sum += (v[k].x + v[k].y) + (v[k].z + v[k].w);
+      }
+    }
+  } else {
+    for (int i = tid; i < nq; i += 256) {
+      float4 w = score4_len(s, m, i, n, scale);
+      w.x = expf(w.x - mx); w.y = expf(w.y - mx); w.z = expf(w.z - mx); w.w = expf(w.w - mx);
+      sum += (w.x + w.y) + (w.z + w.w);
+    }
+  }
+  sum = warp_sum(sum);
+  if (lane == 0) red[warp] = sum;
+  __syncthreads();
+  sum = ((red[0] + red[1]) + (red[2] + red[3])) + ((red[4] + red[5]) + (red[6] + red[7]));
+  const float inv = 1.0f / sum;
+  uint2* p2 = reinterpret_cast<uint2*>(P16 + (size_t)row * ld);
+  if (REG) {
+#pragma unroll
+    for (int k = 0; k < ITEMS; ++k) {
+      const int i = tid + 256 * k;
+      if (i < n64q) p2[i] = i < nq ? half4_scaled(v[k], inv) : make_uint2(0u, 0u);   // then the zero tail
+    }
+  } else {
+    for (int i = tid; i < n64q; i += 256) {
+      uint2 pk = make_uint2(0u, 0u);
+      if (i < nq) {
+        float4 w = score4_len(s, m, i, n, scale);
+        w.x = expf(w.x - mx); w.y = expf(w.y - mx); w.z = expf(w.z - mx); w.w = expf(w.w - mx);
+        pk = half4_scaled(w, inv);
+      }
+      p2[i] = pk;
+    }
+  }
+}
+
 __global__ void blend_kernel(const float4* __restrict__ a, const float4* __restrict__ b, float alpha,
                              float4* __restrict__ out, long long n4) {
   const float beta = 1.0f - alpha;
@@ -215,6 +330,25 @@ extern "C" int ltm_softmax_rows_h(float* S, const float* mask, void* P16, int ro
     softmax_rows_kernel<<<rows, 256, 0, (cudaStream_t)stream>>>(S, mask, n, rows_per_mask > 0 ? rows_per_mask : 1, scale,
                                                                 reinterpret_cast<__half*>(P16));
   LTM_CHECK_LAUNCH("softmax_rows_h");
+  return 0;
+}
+
+extern "C" int ltm_softmax_rows_h_len(const float* S, const float* mask, void* P16, const int32_t* n_len, int rows, int ld,
+                                      int mask_ld, int rows_per_len, float scale, void* stream) {
+  using namespace ltm;
+  LTM_REQUIRE(S != nullptr && P16 != nullptr && n_len != nullptr, "softmax_rows_h_len: null pointer");
+  LTM_REQUIRE(rows > 0 && ld > 0 && ld % 64 == 0 && rows_per_len > 0 && rows % rows_per_len == 0,
+              "softmax_rows_h_len: bad shape rows=%d ld=%d rows_per_len=%d (ld %% 64 == 0, rows %% rows_per_len == 0)",
+              rows, ld, rows_per_len);
+  LTM_REQUIRE(mask == nullptr || mask_ld > 0, "softmax_rows_h_len: mask_ld must be positive");
+  LTM_REQUIRE(aligned16(S) && aligned16(P16), "softmax_rows_h_len: 16-byte alignment");
+  if (ld <= 8192)   // every row fits the registers of one CTA
+    softmax_rows_len_kernel<true><<<rows, 256, 0, (cudaStream_t)stream>>>(
+        S, mask, n_len, reinterpret_cast<__half*>(P16), ld, mask_ld, rows_per_len, scale);
+  else
+    softmax_rows_len_kernel<false><<<rows, 256, 0, (cudaStream_t)stream>>>(
+        S, mask, n_len, reinterpret_cast<__half*>(P16), ld, mask_ld, rows_per_len, scale);
+  LTM_CHECK_LAUNCH("softmax_rows_h_len");
   return 0;
 }
 

@@ -21,11 +21,12 @@ Differences that are deliberate (DESIGN.md section "boundary"):
 """
 import weakref
 
+import numpy as np
 import torch
 import torch.nn as nn
 
 from . import tables
-from .batched import BatchedGaussLTM, BatchedRectLTM
+from .batched import BatchedGaussLTM, BatchedRectLTM, _as_lengths
 
 
 class LongTermAttention(nn.Module):
@@ -162,10 +163,47 @@ class LongTermAttention(nn.Module):
         torch.rand(self.nb_samples, dtype=torch.float64, generator=generator)
         return u
 
+    def check_ragged(self, k, lengths, new_doc, Q):
+        """Host-side validation of a ragged call with Q queries per video, before anything is launched: lengths (host
+        ints, each 0 or in [2, L]), new_doc (a bool or one host flag per video), that every present video that does not
+        start a new document has memory to continue, and that no video holding memory sees its number of query tiles
+        change without new_doc (the checks `BatchedRectLTM.step` makes).  Returns (lengths tuple, bool ndarray of
+        new_doc flags)."""
+        if self.variant != "gibbs":
+            raise NotImplementedError("per-video lengths exist for variant 'gibbs' only")
+        bsz, LT = k.shape[0], k.shape[1]
+        if LT % self.tokens_per_frame or LT // self.tokens_per_frame < 2:
+            raise ValueError(f"k has {LT} tokens: a ragged chunk is padded to L*{self.tokens_per_frame} tokens, L >= 2")
+        lens = _as_lengths(lengths, bsz, LT // self.tokens_per_frame)
+        if isinstance(new_doc, (bool, int)):
+            nd = np.full(bsz, bool(new_doc))
+        else:
+            t = torch.as_tensor(new_doc)
+            if t.device.type != "cpu" or t.numel() != bsz:
+                raise ValueError("with lengths, new_doc is a bool or one host flag per video")
+            nd = t.reshape(-1).to(torch.bool).numpy()
+        eng = self._engine
+        same = eng is not None and eng.has_state and eng.Bv == bsz
+        mem = (eng._slots if eng._slots is not None else np.ones(bsz, bool)) if same else np.zeros(bsz, bool)
+        hist = getattr(eng, "_hist", None)
+        if same and hist is not None and hist.shape[1] != eng.H * ((Q + 31) // 32) and (mem & ~nd).any():
+            raise ValueError(f"the number of queries changed inside a video ({Q} now): pass new_doc=True or keep Q")
+        bad = (np.asarray(lens) > 0) & ~nd & ~mem
+        if bad.any():
+            raise ValueError(f"video slot(s) {np.flatnonzero(bad).tolist()} hold no memory and receive a chunk without "
+                             "new_doc: pass new_doc for their first chunk")
+        return lens, nd
+
     @torch.no_grad()
-    def forward(self, k, q, new_doc, layer_n=None, u=None, generator=None):
+    def forward(self, k, q, new_doc, layer_n=None, u=None, generator=None, lengths=None):
+        """lengths (variant 'gibbs'): per-video chunk lengths in frames (host ints, 0 = idle, else in [2, L]) of a
+        ragged batch whose chunk k is padded to L frames; new_doc is then a bool or one host flag per video and is
+        applied per slot (BatchedRectLTM.step), idle videos keep their memory and get zero rows."""
         if not k.is_cuda:
             raise RuntimeError("infinite_video_b200.LongTermAttention runs on CUDA tensors only (no CPU fallback)")
+        lens = None
+        if lengths is not None:
+            lens, new_doc = self.check_ragged(k, lengths, new_doc, q.shape[1])
         self.device = k.device
         eng = self._get_engine(k.device)
         out_dtype = q.dtype
@@ -177,7 +215,7 @@ class LongTermAttention(nn.Module):
         bsz = k32.size(0)
         if self.variant == "gibbs":
             self.length = k32.size(1) // self.tokens_per_frame            # gibbs:291-292
-        if new_doc:
+        if lens is None and new_doc:
             eng.reset()                                                    # gibbs:300-302
             sp = LongTermAttention._shared_pool
             if sp["key"] is None or sp["key"][0]() is not k:               # do not keep the last video's frames alive
@@ -191,19 +229,24 @@ class LongTermAttention(nn.Module):
         else:
             u = None
         pooled = None
-        if self.variant == "gibbs" and self.share_pooling:
+        # (a batch of idle videos has no frames: the step takes its empty chunk itself, no zero-size pooled tensor)
+        if self.variant == "gibbs" and self.share_pooling and (lens is None or any(lens)):
             # identity of the tensor OBJECT (a weak reference) + its version counter: a data pointer alone is not
             # a key, the caching allocator hands the same address to the next chunk
             sp = LongTermAttention._shared_pool
             ref = sp["key"]
             hit = (ref is not None and ref[0]() is k and ref[1] == k._version and ref[2] == self.tokens_per_frame
-                   and sp["x"] is not None and sp["x"].device == k.device)
+                   and ref[3] == lens and sp["x"] is not None and sp["x"].device == k.device)
             if not hit:
-                sp["x"], sp["k16"] = eng.pool(k32), None
-                sp["key"] = (weakref.ref(k), k._version, self.tokens_per_frame)
+                sp["x"], sp["k16"] = eng.pool(k32, lengths=lens), None
+                sp["key"] = (weakref.ref(k), k._version, self.tokens_per_frame, lens)
             pooled = sp["x"]
-        ctx = eng.step(k32, q32, u=u, new_doc=False, pooled=pooled) if pooled is not None else \
-            eng.step(k32, q32, u=u, new_doc=False)
+        if lens is not None:
+            ctx = eng.step(k32, q32, u=u, new_doc=torch.from_numpy(new_doc), pooled=pooled, lengths=lens)
+        elif pooled is not None:
+            ctx = eng.step(k32, q32, u=u, new_doc=False, pooled=pooled)
+        else:
+            ctx = eng.step(k32, q32, u=u, new_doc=False)
         if self.output_density and self.variant == "gibbs":
             self.alphas = eng.density()
             if self.dump_path is not None:
@@ -215,20 +258,27 @@ class LongTermAttention(nn.Module):
             return ctx.to(out_dtype), self.kl_reg
         return ctx.to(out_dtype)
 
-    def pool_for_caller(self, k):
+    def pool_for_caller(self, k, lengths=None):
         """One pass over an fp32 chunk for both halves of the caller's cross-attention branch: pools the frames for
         this (and every other) LTM layer -- the result is parked in the shared-pooling slot, so the following
         `forward(k, ...)` does not stream the chunk again -- and returns the chunk as float16 for the short-term
         attention GEMMs (cross_attention.py).  Every cross-attention layer of a Q-former is handed the same chunk: the
-        second and later layers find both results in the slot."""
+        second and later layers find both results in the slot.  `lengths` (ragged chunk): the frames are packed and
+        the fp16 chunk is k16[Bv, ld16, e] padded per video (`BatchedRectLTM.pool`); the slot is keyed on the lengths
+        too, so `forward(k, ..., lengths=)` with the same lengths finds it."""
+        lens = None
+        if lengths is not None:
+            if self.variant != "gibbs":
+                raise NotImplementedError("per-video lengths exist for variant 'gibbs' only")
+            lens = _as_lengths(lengths, k.shape[0], k.shape[1] // self.tokens_per_frame)
         sp = LongTermAttention._shared_pool
         ref = sp["key"]
         if (ref is not None and ref[0]() is k and ref[1] == k._version and ref[2] == self.tokens_per_frame
-                and sp["x"] is not None and sp["k16"] is not None and sp["x"].device == k.device):
+                and ref[3] == lens and sp["x"] is not None and sp["k16"] is not None and sp["x"].device == k.device):
             return sp["k16"]
         eng = self._get_engine(k.device)
-        pooled, k16 = eng.pool(k.contiguous(), with_half=True)
-        sp.update(key=(weakref.ref(k), k._version, self.tokens_per_frame), x=pooled, k16=k16)
+        pooled, k16 = eng.pool(k.contiguous(), with_half=True, lengths=lens)
+        sp.update(key=(weakref.ref(k), k._version, self.tokens_per_frame, lens), x=pooled, k16=k16)
         return k16
 
     def extra_repr(self):

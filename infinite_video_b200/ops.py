@@ -56,6 +56,21 @@ def pool_mean_convert(k, splits=1):
     return out, k16
 
 
+def pool_mean_convert_ragged(k, offs, frames, splits, ld16):
+    """Ragged `pool_mean_convert`: k[Bv,L,T,e] fp32 padded, offs int32 [Bv+1] device frame offsets (exclusive prefix sum
+    of the lengths, `frames` = offs[Bv]) -> (xpart[frames, splits, e] packed video after video, k16[Bv, ld16, e]).
+    k16 rows [0, n_v) of video v hold its first lengths[v] * T tokens as fp16, rows [n_v, roundup64(n_v)) are zero and
+    the rest is left unwritten (ld16 % 64 == 0, ld16 >= L*T)."""
+    require_cuda(k, offs)
+    k = _f32c(k)
+    Bv, L, T, e = k.shape
+    out = torch.empty(frames, splits, e, device=k.device, dtype=torch.float32)
+    k16 = torch.empty(Bv, ld16, e, device=k.device, dtype=torch.float16)
+    check(lib().ltm_pool_mean_convert_ragged(ptr(k), ptr(out), ptr(k16), ptr(offs), Bv, L, T, e, splits, frames, ld16,
+                                             stream_ptr(k.device)), "pool_mean_convert_ragged")
+    return out, k16
+
+
 def pool_bins(k, fbin_ptr, rows):
     """Per-bin pooling of an update chunk: k[Bv,L,T,e] fp32, fbin_ptr int32 [rows+1] -> xbin[Bv,rows,e], the sum of the
     pooled frames [fbin_ptr[r], fbin_ptr[r+1]) (tables.RectTables.fbin_ptr)."""
@@ -226,11 +241,17 @@ def gemm(A, B, *, a_kmajor=True, b_kmajor=True, B2=None, bias=None, out=None, pr
 def gemm_raw(A, lda, strideA, a_kmajor, B, ldb, strideB, b_kmajor, C_, ldc, strideC, M, Nc, K, batch, *, bias=None,
              bias_stride=0, c_group=0, c_group_stride=0, precision="tf32", impl="tcgen05", a_offset=0, b_offset=0,
              c_offset=0, round_tf32=False, a_group=0, a_group_stride=0, bias_offset=0, c_fp16=False, ab_fp16=False,
-             C_lo=None, max_ctas=0):
+             C_lo=None, max_ctas=0, n_ext=None, k_ext=None):
     """ltm_gemm with every pitch / batch stride spelled out (elements).  A, B, C_ are the base tensors; *_offset
     shifts the start (elements).  Used where operands are strided views that tensor shapes cannot express
-    (per-head column blocks, per-head / per-video output layouts)."""
-    require_cuda(A, B, C_, bias)
+    (per-head column blocks, per-head / per-video output layouts).
+    n_ext / k_ext: optional contiguous device int32 [batch] extents (ltm_gemm_extents, fp16 operands only): tiles of
+    batch b starting at column >= n_ext[b] are skipped, batch b runs k_ext[b] (a multiple of 64) K-elements; a batch
+    with an extent of 0 leaves its C unwritten."""
+    require_cuda(A, B, C_, bias, n_ext, k_ext)
+    for ext in (n_ext, k_ext):
+        if ext is not None and (ext.dtype != torch.int32 or not ext.is_contiguous() or ext.numel() != batch):
+            raise ValueError(f"gemm extents must be contiguous int32 tensors of {batch} entries")
     g = GemmArgs()
     esz = 2 if ab_fp16 else 4                     # (ab_fp16: A and B are float16 tensors, offsets in elements)
     g.A, g.lda, g.strideA, g.a_kmajor = A.data_ptr() + esz * a_offset, lda, strideA, int(a_kmajor)
@@ -249,6 +270,9 @@ def gemm_raw(A, lda, strideA, a_kmajor, B, ldb, strideB, b_kmajor, C_, ldc, stri
     g.c_group, g.c_group_stride = c_group, c_group_stride
     g.round_tf32 = int(bool(round_tf32))
     g.a_group, g.a_group_stride = a_group, a_group_stride
+    if n_ext is not None or k_ext is not None:
+        check(lib().ltm_gemm_extents(C.byref(g), ptr(n_ext), ptr(k_ext), stream_ptr(A.device)), "gemm_extents")
+        return C_
     check(lib().ltm_gemm(C.byref(g), stream_ptr(A.device)), "gemm")
     return C_
 
@@ -312,6 +336,33 @@ def softmax_rows_half(S, scale=1.0, mask=None, rows_per_mask=1):
     P = torch.empty(S.shape, device=S.device, dtype=torch.float16)
     check(lib().ltm_softmax_rows_h(ptr(S), ptr(mask), ptr(P), rows, n, rows_per_mask, float(scale),
                                    stream_ptr(S.device)), "softmax_rows_h")
+    return P
+
+
+def softmax_rows_half_len(S, n_len, rows_per_len, scale=1.0, mask=None):
+    """Ragged `softmax_rows_half`: S[..., ld] fp32 (ld % 64 == 0), n_len device int32 [rows / rows_per_len]: row r spans
+    the first n_len[r // rows_per_len] <= ld columns.  Returns P fp16 of S's shape: softmax(S * scale + mask) on those
+    columns, zeros up to the next multiple of 64, the rest unwritten (rows with n = 0 entirely).  mask: float32 rows
+    [rows / rows_per_len, mask_ld] (only their first n columns are read) or None."""
+    require_cuda(S, n_len, mask)
+    if not S.is_contiguous() or S.dtype != torch.float32:
+        raise ValueError("softmax_rows_half_len needs a contiguous float32 tensor")
+    ld = S.shape[-1]
+    rows = S.numel() // ld
+    if rows_per_len <= 0 or rows % rows_per_len:
+        raise ValueError(f"softmax_rows_half_len: rows_per_len={rows_per_len} must divide rows={rows}")
+    if n_len.dtype != torch.int32 or not n_len.is_contiguous() or n_len.numel() != rows // rows_per_len:
+        raise ValueError(f"softmax_rows_half_len: n_len must be contiguous int32 with {rows // rows_per_len} entries")
+    mask_ld = 0
+    if mask is not None:
+        if mask.dtype != torch.float32 or not mask.is_contiguous() or mask.device != S.device or mask.dim() != 2 \
+                or mask.shape[0] != rows // rows_per_len:
+            raise ValueError(f"softmax_rows_half_len: the mask must be contiguous float32 [{rows // rows_per_len}, n] "
+                             f"on {S.device}")
+        mask_ld = mask.shape[1]
+    P = torch.empty(S.shape, device=S.device, dtype=torch.float16)
+    check(lib().ltm_softmax_rows_h_len(ptr(S), ptr(mask), ptr(P), ptr(n_len), rows, ld, mask_ld, rows_per_len,
+                                       float(scale), stream_ptr(S.device)), "softmax_rows_h_len")
     return P
 
 
