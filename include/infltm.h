@@ -57,6 +57,11 @@ int ltm_pool_bins(const float* k, float* xbin, const int32_t* fbin_ptr, int Bv, 
  * autocast): 128-bit loads of 8 elements, fp32 accumulation, fp32 output.  e % 8 == 0. */
 int ltm_pool_mean_16(const void* k, int is_bf16, float* xpart, int Bv, int L, int T, int e, int splits,
                      void* stream);
+/* same with a bounded (persistent) grid of max_ctas CTAs (0 = one CTA per frame-split, i.e. ltm_pool_mean_16): the
+ * pooling of the next 16-bit chunk beside the current step.  Every frame-split is pooled by the same code for any
+ * max_ctas, so xpart carries the same bits. */
+int ltm_pool_mean_16_grid(const void* k, int is_bf16, float* xpart, int Bv, int L, int T, int e, int splits,
+                          int max_ctas, void* stream);
 
 /* ---- frame pooling of a ragged batch: k[Bv, L, T, e] is padded, video v uses its first lengths[v] frames
  * (0 = none), given as offs[Bv+1] = the exclusive prefix sum of the lengths (frames = offs[Bv]).
@@ -339,7 +344,7 @@ typedef struct {
   float* p;                             /* [Bv,127] */
   float* scores;                        /* optional [Bv,H,Q,N] */
   /* device staging for the *_host entry point */
-  float* k_dev; float* q_dev; double* u_dev; uint8_t* new_doc_dev; float* ctx_dev;
+  void* k_dev; float* q_dev; double* u_dev; uint8_t* new_doc_dev; float* ctx_dev;
   /* optional cudaEvent_t pairs recorded on `stream` around each stage (NULL = skip):
    * [0,1] pool  [2,3] re-sample  [4,5] consolidate  [6,7] K/V projection  [8,9] attention */
   void* prof_events[10];
@@ -385,10 +390,14 @@ typedef struct {
   const int32_t *bank_seg_ptr0, *bank_seg_mem0; const float* bank_g0;
   const int32_t *bank_seg_ptr1, *bank_seg_mem1; const float* bank_g1;
   float* hist_keep;
+  /* storage of the chunk: k of ltm_rect_step, k_host and k_dev of ltm_rect_step_host.  0 fp32, 1 fp16, 2 bfloat16.
+   * A 16-bit chunk (e % 8 == 0) is pooled per frame from its own storage with fp32 accumulation, in the summation
+   * order of ltm_pool_mean_16 (lock-step) or ltm_pool_mean_ragged (ragged); it is never pooled per bin (binned == 0). */
+  int k_dtype;
 } ltm_rect_step_args;
-int ltm_rect_step(const ltm_rect_step_args* a, const float* k, const float* q, const double* u,
+int ltm_rect_step(const ltm_rect_step_args* a, const void* k, const float* q, const double* u,
                   const uint8_t* new_doc, float* ctx, void* stream);
-int ltm_rect_step_host(const ltm_rect_step_args* a, const float* k_host, const float* q_host,
+int ltm_rect_step_host(const ltm_rect_step_args* a, const void* k_host, const float* q_host,
                        const double* u_host, const uint8_t* new_doc_host, float* ctx_host, void* stream);
 
 /* ---- the same step with the frame pooling of the NEXT chunk issued beside it (two-stream schedule in one call):
@@ -403,11 +412,12 @@ int ltm_rect_step_host(const ltm_rect_step_args* a, const float* k_host, const f
 typedef struct {
   void *main_stream, *side_stream, *compute_stream;
   void *ev_fork_pool, *ev_pooled_cur, *ev_pooled_next, *ev_fork, *ev_join;
-  const float* k_next; float* xpart_next; int pool_ctas;
+  const void* k_next; float* xpart_next; int pool_ctas;
   int next_binned;     /* pool k_next with ltm_pool_bins (the call that consumes it must set args.binned) */
   /* ragged next chunk (next_lengths != NULL): pool the first next_lengths[v] frames of each video of k_next (padded
    * to args.L frames) into xpart_next packed as [next_frames, next_splits, e] (ltm_pool_mean_ragged) */
   const int32_t* next_lengths; const int32_t* next_offs; int next_frames; int next_splits;
+  int next_dtype;      /* storage of k_next, as ltm_rect_step_args.k_dtype (16-bit: next_binned == 0) */
 } ltm_overlap;
 int ltm_rect_step_overlap(const ltm_rect_step_args* a, const ltm_overlap* o, const float* q, const double* u,
                           const uint8_t* new_doc, float* ctx);

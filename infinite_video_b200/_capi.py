@@ -63,6 +63,7 @@ class RectStepArgs(C.Structure):
         ("bank_seg_ptr0", C.c_void_p), ("bank_seg_mem0", C.c_void_p), ("bank_g0", C.c_void_p),
         ("bank_seg_ptr1", C.c_void_p), ("bank_seg_mem1", C.c_void_p), ("bank_g1", C.c_void_p),
         ("hist_keep", C.c_void_p),
+        ("k_dtype", C.c_int),
     ]
 
 
@@ -74,6 +75,7 @@ class Overlap(C.Structure):
         ("k_next", C.c_void_p), ("xpart_next", C.c_void_p), ("pool_ctas", C.c_int),
         ("next_binned", C.c_int),
         ("next_lengths", C.c_void_p), ("next_offs", C.c_void_p), ("next_frames", C.c_int), ("next_splits", C.c_int),
+        ("next_dtype", C.c_int),
     ]
 
 
@@ -89,6 +91,7 @@ _SIGS = {
     "ltm_split_half3": (C.c_int, [_P, _P, _L, _I, _I, _P]),
     "ltm_pool_bins": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "ltm_pool_mean_16": (C.c_int, [_P, _I, _P, _I, _I, _I, _I, _I, _P]),
+    "ltm_pool_mean_16_grid": (C.c_int, [_P, _I, _P, _I, _I, _I, _I, _I, _I, _P]),
     "ltm_pool_mean_grid": (C.c_int, [_P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "ltm_pool_mean_ragged": (C.c_int, [_P, _I, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "ltm_pool_mean_convert_ragged": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),

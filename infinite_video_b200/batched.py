@@ -70,6 +70,10 @@ def _as_lengths(lengths, Bv, Lmax):
     return vals
 
 
+# storage of a chunk k as the library takes it (ltm_rect_step_args.k_dtype, ltm_overlap.next_dtype)
+_CHUNK_DTYPES = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
+
+
 def _pad_rows(m):
     """Copy a 2-D matrix into storage whose row pitch is a multiple of 4 floats (TMA: 16-byte pitches)."""
     r, c = m.shape
@@ -236,14 +240,25 @@ class BatchedRectLTM(_BatchedBase):
         # (at most T/8 splits: the partial sums are written and read back, T/splits rows of input per row of output)
         return 1 if units >= want or units == 0 else max(1, min(max(1, self.T // 8), -(-want // units)))
 
-    def _bin_ok(self, Bv, L, tab):
-        """Whether an update chunk of this shape is pooled per bin (see `bin_pool`)."""
-        if self.bin_pool is False or tab.xb_rows <= 0:
+    def _bin_ok(self, Bv, L, tab, k_dtype=0):
+        """Whether an update chunk of this shape and storage (k_dtype, see `_chunk_dtype`) is pooled per bin (see
+        `bin_pool`).  A 16-bit chunk never is: it is pooled per frame, as `step` always pooled it."""
+        if k_dtype or self.bin_pool is False or tab.xb_rows <= 0:
             return False
         if self.bin_pool:
             return True
         # (measured: 4 frames per bin +0.4 % burst / +1.1 % sustained at the NExT-QA shape; 2 per bin -2 % at num_basis 512)
         return L >= 3 * tab.xb_rows and Bv * tab.xb_rows >= 4 * 8 * self.sm_count
+
+    def _chunk_dtype(self, k, name="k"):
+        """Storage code of chunk k (0 float32, 1 float16, 2 bfloat16); ValueError for any other dtype, and for a 16-bit
+        chunk whose width is not a multiple of 8 (it is read as 128-bit vectors of 8 elements)."""
+        dt = _CHUNK_DTYPES.get(k.dtype)
+        if dt is None:
+            raise ValueError(f"{name} must be float32, float16 or bfloat16, not {k.dtype}")
+        if dt and k.shape[-1] % 8:
+            raise ValueError(f"a 16-bit {name} needs a width that is a multiple of 8, not {k.shape[-1]}")
+        return dt
 
     def reset(self):
         """Forget every video (new_doc for all) and every pending prefetch."""
@@ -297,7 +312,8 @@ class BatchedRectLTM(_BatchedBase):
         ws["xi"] = (1 - ws["xi"]) if (1 - ws["xi"]) not in held else ws["xi"]
         if ws["xi"] in held:
             self._pref[:] = [e for e in self._pref if e["buf"] != ws["xi"]]
-        ws["xtag"][ws["xi"]] = update and self._bin_ok(k.shape[0], k.shape[1] // self.T, tab)
+        ws["xtag"][ws["xi"]] = update and self._bin_ok(k.shape[0], k.shape[1] // self.T, tab,
+                                                       _CHUNK_DTYPES.get(k.dtype, 0))
         return None
 
     def _state(self, Bv, Q):
@@ -316,7 +332,7 @@ class BatchedRectLTM(_BatchedBase):
         return self._B[self._cur] if (self._B is not None and self.has_state) else None
 
     # ------------------------------------------------------------------ one chunk
-    def _args(self, Bv, L, Q, ws, tab, tdev, beside_pool=False, rag=None):
+    def _args(self, Bv, L, Q, ws, tab, tdev, beside_pool=False, rag=None, k_dtype=0):
         # the argument block is built once per workspace / table set / weights and only its per-call fields are
         # rewritten afterwards (the ~40 ctypes assignments were a third of the host time of a chunk)
         sig = (id(tdev), self.Wkv.data_ptr(), self.bkv.data_ptr(), self._hist.data_ptr(), self.sticky,
@@ -331,6 +347,7 @@ class BatchedRectLTM(_BatchedBase):
         a.B_new = self._B[1 - self._cur].data_ptr()
         a.xpart = ws["xbufs"][ws["xi"]].data_ptr()
         a.binned = 1 if ws["xtag"][ws["xi"]] else 0
+        a.k_dtype = k_dtype
         # (only where the pooling is the long pole of the step: a chunk of at least 16 tokens per basis function; with
         # 8 frames x 32 tokens on 64 bins the chain of this stream is, and a narrower projection would lengthen it)
         bound = beside_pool and L * self.T >= self.gemm_ctas_min_ratio * self.N
@@ -559,17 +576,21 @@ class BatchedRectLTM(_BatchedBase):
 
         Frame pooling (gibbs:304) does not depend on the memory state, and it is the HBM-bound 93 % of a
         call's bytes, while regression / projection / attention of the current chunk are compute-bound; issuing
-        it one chunk ahead lets the two overlap.  The following `step(k_next, ...)` must pass the same tensor."""
+        it one chunk ahead lets the two overlap.  The following `step(k_next, ...)` must pass the same tensor.
+        A 16-bit chunk (float16 / bfloat16) is pooled per frame from its own storage, never per bin."""
         require_cuda(k_next)
+        dt = self._chunk_dtype(k_next, "k_next")
         if not k_next.is_contiguous():
             raise ValueError("prefetch needs a contiguous chunk (the following step must be given the same tensor)")
         Bv, LT, e = k_next.shape
+        if e != self.e or LT % self.T:
+            raise ValueError(f"k_next must be [Bv, L*{self.T}, {self.e}]")
         L = LT // self.T
+        lens = None if lengths is None else _as_lengths(lengths, Bv, L)
         ws = self._workspace(Bv, L, Q)
-        lens = offs = None
+        offs = None
         frames, splits = 0, ws["splits"]
-        if lengths is not None:
-            lens = _as_lengths(lengths, Bv, L)
+        if lens is not None:
             self._ragged_ws(ws, Bv, L)
             offs = self._lengths_dev(lens)[1]
             frames = sum(lens)
@@ -594,11 +615,11 @@ class BatchedRectLTM(_BatchedBase):
         if events is not None:
             check(lib().ltm_event_record(events[0], sp), "event_record")
         tab = tables.rect_tables(L, self.N, self.tau, self.S, spacing=self.spacing)
-        binned = lens is None and bool(update) and self._bin_ok(Bv, L, tab)
+        binned = lens is None and bool(update) and self._bin_ok(Bv, L, tab, dt)
         if offs is not None:
             offs.record_stream(self._side)
         self._pool_launch(k_next, ws["xbufs"][b], Bv, L, splits, int(self.pool_ctas), sp, offs=offs, frames=frames,
-                          bins=tab if binned else None)
+                          bins=tab if binned else None, dtype=dt)
         if events is not None:
             check(lib().ltm_event_record(events[1], sp), "event_record")
         check(lib().ltm_event_record(ev["pooled"][b], sp), "event_record")
@@ -607,14 +628,18 @@ class BatchedRectLTM(_BatchedBase):
 
     def _pool_launch(self, k, out, Bv, L, splits, max_ctas, stream, offs=None, frames=0, bins=None, dtype=0):
         """Pool chunk k[Bv, L*T, e] into `out` on `stream`: the packed frames of a ragged chunk (offs: device frame
-        offsets, `frames` in all; dtype 0 / 1 / 2: float32 / float16 / bfloat16 storage), the per-bin sums of an update
-        chunk (bins: its tables) or per-frame means.  max_ctas bounds the grid (0 = one CTA per unit)."""
+        offsets, `frames` in all), the per-bin sums of an update chunk (bins: its tables; float32 only) or per-frame
+        means.  dtype 0 / 1 / 2: float32 / float16 / bfloat16 storage.  max_ctas bounds the grid (0 = one CTA per
+        unit)."""
         if offs is not None:
             check(lib().ltm_pool_mean_ragged(ptr(k), dtype, ptr(out), ptr(offs), Bv, L, self.T, self.e, splits, frames,
                                              max_ctas, stream), "pool_mean_ragged")
         elif bins is not None:
             check(lib().ltm_pool_bins(ptr(k), ptr(out), ptr(bins.to(self.device)["fbin_ptr"]), Bv, L, self.T, self.e,
                                       bins.xb_rows, stream), "pool_bins")
+        elif dtype:
+            check(lib().ltm_pool_mean_16_grid(ptr(k), int(dtype == 2), ptr(out), Bv, L, self.T, self.e, splits,
+                                              max_ctas, stream), "pool_mean_16_grid")
         else:
             check(lib().ltm_pool_mean_grid(ptr(k), ptr(out), Bv, L, self.T, self.e, splits, max_ctas, stream),
                   "pool_mean")
@@ -703,7 +728,8 @@ class BatchedRectLTM(_BatchedBase):
 
     @_on_device
     def step(self, k, q, u=None, new_doc=False, pooled=None, beside_pooling=False, lengths=None):
-        """k[Bv, L*T, e], q[Bv,Q,D] fp32 CUDA; u[Bv,S] fp64 uniforms (needed from the second chunk on when
+        """k[Bv, L*T, e] float32 / float16 / bfloat16 (16-bit: e % 8 == 0, pooled per frame from its own storage),
+        q[Bv,Q,D] float32, CUDA; u[Bv,S] fp64 uniforms (needed from the second chunk on when
         sticky); new_doc: bool or per-video flags; pooled: result of `pool(k)` (then `k` is only used for its
         shape); beside_pooling: the caller pools another chunk on a second stream while this step runs (the K/V
         projection then keeps to part of the SMs, see `gemm_ctas_overlap`).  Returns ctx[Bv,Q,D].
@@ -714,10 +740,9 @@ class BatchedRectLTM(_BatchedBase):
         cleared instead).  new_doc is then a bool or host flags; a slot without memory must receive new_doc with its
         first chunk.  Passing lengths always takes the ragged kernels, even when all lengths are equal."""
         require_cuda(k, q, u)
-        if k.dtype in (torch.float16, torch.bfloat16) and pooled is None:
-            pooled = self.pool(k, lengths=lengths)  # 16-bit chunk: pooled straight from its 16-bit storage
-        if (k.dtype != torch.float32 and pooled is None) or q.dtype != torch.float32:
-            raise ValueError("k must be float32 / float16 / bfloat16 and q float32")
+        kdt = self._chunk_dtype(k) if pooled is None else 0       # (with `pooled`, k only gives the shape)
+        if q.dtype != torch.float32:
+            raise ValueError("q must be float32")
         k, q = k.contiguous(), q.contiguous()
         Bv, L, Q, tab, tdev, flags, u, rag = self._prepare(k, q, new_doc, u, lengths, pooled)
         ws = self._workspace(Bv, L, Q)
@@ -739,7 +764,7 @@ class BatchedRectLTM(_BatchedBase):
                 check(lib().ltm_stream_wait_event(rp, hit["event"]), "stream_wait_event")
         # (a pending prefetch = the next chunk is being pooled on the side stream while this step runs)
         beside = bool(beside_pooling) or (pooled is None and bool(self._pref))
-        a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=beside, rag=rag)
+        a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=beside, rag=rag, k_dtype=kdt)
         if pooled is not None:
             a.xpart, a.splits, a.binned = pooled.data_ptr(), pooled.shape[-2], 0
         if rag is not None and run is not main:
@@ -763,10 +788,18 @@ class BatchedRectLTM(_BatchedBase):
         `step`, bit for bit.  `next_new_doc=True` says that `k_next` will start new documents (then it is pooled per
         frame; a chunk expected to continue the videos may be pooled per bin, see `bin_pool`).
         `lengths` / `next_lengths`: per-video lengths of `k` / `k_next` (ragged chunks, see `step`); `k` is matched
-        with its prefetch by lengths too."""
+        with its prefetch by lengths too.  `k` and `k_next` are float32, float16 or bfloat16, each on its own (see
+        `step`); `q` is float32."""
         require_cuda(k, q, u, k_next)
-        if k.dtype != torch.float32 or q.dtype != torch.float32 or (k_next is not None and k_next.dtype != torch.float32):
-            raise ValueError("step_overlapped takes float32 tensors")
+        kdt = self._chunk_dtype(k)
+        ndt = self._chunk_dtype(k_next, "k_next") if k_next is not None else 0
+        if q.dtype != torch.float32:
+            raise ValueError("q must be float32")
+        if k_next is not None and (not k_next.is_contiguous() or tuple(k_next.shape) != tuple(k.shape)):
+            raise ValueError("k_next must be contiguous and have the shape of k")
+        nl = None
+        if k_next is not None and next_lengths is not None:
+            nl = _as_lengths(next_lengths, k.shape[0], k.shape[1] // self.T)
         k, q = k.contiguous(), q.contiguous()
         Bv, L, Q, tab, tdev, flags, u, rag = self._prepare(k, q, new_doc, u, lengths)
         ws = self._workspace(Bv, L, Q)
@@ -782,12 +815,8 @@ class BatchedRectLTM(_BatchedBase):
         o.ev_pooled_cur = hit["event"] if (hit["captured"] or not capturing) else None
         o.pool_ctas = int(self.pool_ctas)
         if k_next is not None:
-            if not k_next.is_contiguous() or tuple(k_next.shape) != tuple(k.shape):
-                raise ValueError("k_next must be contiguous and have the shape of k")
             b = self._pref_buffer(ws)
-            nl = None
-            if next_lengths is not None:
-                nl = _as_lengths(next_lengths, Bv, L)
+            if nl is not None:
                 nl_dev, noffs_dev = self._lengths_dev(nl)
                 nl_dev.record_stream(self._side)
                 nf = sum(nl)
@@ -795,14 +824,15 @@ class BatchedRectLTM(_BatchedBase):
                 o.next_frames, o.next_splits = nf, self._splits(nf)
                 nb = False
             else:
-                nb = (not next_new_doc) and self._bin_ok(Bv, L, tab)
+                nb = (not next_new_doc) and self._bin_ok(Bv, L, tab, ndt)
             o.k_next, o.xpart_next, o.next_binned = k_next.data_ptr(), ws["xbufs"][b].data_ptr(), int(nb)
+            o.next_dtype = ndt
             o.ev_fork_pool, o.ev_pooled_next = ev["fork_pool"][b], ev["pooled"][b]
             k_next.record_stream(self._side)
             self._pref.append(dict(ref=weakref.ref(k_next), ver=k_next._version, buf=b, event=ev["pooled"][b],
                                    captured=capturing, binned=nb, lens=nl))
         ctx = torch.empty(Bv, Q, self.D, device=self.device, dtype=torch.float32)   # main joins the compute stream
-        a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=k_next is not None, rag=rag)
+        a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=k_next is not None, rag=rag, k_dtype=kdt)
         if rag is not None:
             rag["lens_dev"].record_stream(self._compute)
         check(lib().ltm_rect_step_overlap(C.byref(a), C.byref(o), ptr(q), ptr(u), ptr(flags), ptr(ctx)),
@@ -814,16 +844,20 @@ class BatchedRectLTM(_BatchedBase):
     def step_host(self, k_host, q_host, u_host=None, new_doc=False, out=None):
         """Same as `step` but through HOST buffers (ideally pinned): the C entry point enqueues the H2D copies,
         the kernels and the D2H copy of ctx on the current stream.  Returns the host ctx tensor; the caller
-        synchronises the stream before reading it."""
+        synchronises the stream before reading it.  k_host is float32, float16 or bfloat16 (a 16-bit chunk is copied
+        as it is: half the H2D bytes); q_host float32."""
         if k_host.is_cuda or q_host.is_cuda:
             raise ValueError("step_host takes host tensors")
-        if k_host.dtype != torch.float32 or q_host.dtype != torch.float32:
-            raise ValueError("step_host takes float32 k and q")
+        kdt = self._chunk_dtype(k_host, "k_host")
+        if q_host.dtype != torch.float32:
+            raise ValueError("step_host takes float32 q")
         Bv, L, Q, tab, tdev, flags, u_host, _ = self._prepare(k_host, q_host, new_doc, u_host, u_name="u_host")
         ws = self._workspace(Bv, L, Q)
         dev = self.device
-        if ws["k_dev"] is None:
-            ws["k_dev"] = torch.empty(Bv, L * self.T, self.e, device=dev, dtype=torch.float32)
+        if ws["k_dev"] is None or ws["k_dev"].dtype != k_host.dtype:
+            # staging buffer in the chunk's own storage: the H2D copy moves 2 bytes per element for a 16-bit chunk
+            ws["k_dev"] = torch.empty(Bv, L * self.T, self.e, device=dev, dtype=k_host.dtype)
+        if ws["q_dev"] is None:
             ws["q_dev"] = torch.empty(Bv, Q, self.D, device=dev, dtype=torch.float32)
             ws["u_dev"] = torch.empty(Bv, self.S, device=dev, dtype=torch.float64)
             ws["nd_dev"] = torch.empty(Bv, device=dev, dtype=torch.uint8)
@@ -831,7 +865,8 @@ class BatchedRectLTM(_BatchedBase):
         if out is None:
             out = torch.empty(Bv, Q, self.D, dtype=torch.float32, pin_memory=True)
         ws["xtag"][ws["xi"]] = False          # the host path pools per frame
-        a = self._args(Bv, L, Q, ws, tab, tdev)
+        a = self._args(Bv, L, Q, ws, tab, tdev, k_dtype=kdt)
+        a.k_dev = ws["k_dev"].data_ptr()      # (the cached block may hold a staging buffer of another dtype)
         nd_host = None
         if flags is not None:
             nd_host = torch.as_tensor(new_doc).to(torch.uint8).contiguous()

@@ -41,23 +41,36 @@ extern "C" int ltm_device_check(void) {
   return 0;
 }
 
+// Storage of a chunk (ltm_rect_step_args.k_dtype, ltm_overlap.next_dtype): 0 fp32, 1 fp16, 2 bfloat16.  A 16-bit chunk
+// is read as 128-bit vectors of 8 elements and is never pooled per bin.
+static int check_chunk_dtype(const char* who, const char* field, int dtype, int e, bool binned) {
+  LTM_REQUIRE(dtype >= 0 && dtype <= 2, "%s: %s=%d (0 fp32, 1 fp16, 2 bfloat16)", who, field, dtype);
+  LTM_REQUIRE(dtype == 0 || e % 8 == 0, "%s: a 16-bit chunk needs e %% 8 == 0 (e=%d)", who, e);
+  LTM_REQUIRE(dtype == 0 || !binned, "%s: a 16-bit chunk is not pooled per bin", who);
+  return 0;
+}
+
 // Frame pooling of one chunk of the geometry of `a` into xpart: packed frames of a ragged chunk (offs != NULL: frame
-// offsets, `frames` in all), per-bin sums (binned) or per-frame means.  max_ctas bounds the grid (0 = one CTA per unit).
-static int pool_chunk(const ltm_rect_step_args* a, const float* k, float* xpart, const int32_t* offs, int frames,
-                      int splits, bool binned, int max_ctas, void* stream) {
-  if (offs) return ltm_pool_mean_ragged(k, 0, xpart, offs, a->Bv, a->L, a->T, a->e, splits, frames, max_ctas, stream);
-  if (binned) return ltm_pool_bins(k, xpart, a->fbin_ptr, a->Bv, a->L, a->T, a->e, a->xb_rows, stream);
-  return ltm_pool_mean_grid(k, xpart, a->Bv, a->L, a->T, a->e, splits, max_ctas, stream);
+// offsets, `frames` in all), per-bin sums (binned, fp32 chunks) or per-frame means.  dtype: storage of k, as checked
+// by check_chunk_dtype.  max_ctas bounds the grid (0 = one CTA per unit).
+static int pool_chunk(const ltm_rect_step_args* a, const void* k, int dtype, float* xpart, const int32_t* offs,
+                      int frames, int splits, bool binned, int max_ctas, void* stream) {
+  if (offs)
+    return ltm_pool_mean_ragged(k, dtype, xpart, offs, a->Bv, a->L, a->T, a->e, splits, frames, max_ctas, stream);
+  if (binned) return ltm_pool_bins((const float*)k, xpart, a->fbin_ptr, a->Bv, a->L, a->T, a->e, a->xb_rows, stream);
+  if (dtype) return ltm_pool_mean_16_grid(k, dtype == 2, xpart, a->Bv, a->L, a->T, a->e, splits, max_ctas, stream);
+  return ltm_pool_mean_grid((const float*)k, xpart, a->Bv, a->L, a->T, a->e, splits, max_ctas, stream);
 }
 
 // ------------------------------------------------------------------------------------------------
 // One chunk of variant R for Bv videos:  pool -> (re-sample) -> consolidate -> project K,V ->
 // continuous attention (+ next call's sticky histogram).  long_term_attention_gibbs.py:288-346.
 // ------------------------------------------------------------------------------------------------
-extern "C" int ltm_rect_step(const ltm_rect_step_args* a, const float* k, const float* q, const double* u,
+extern "C" int ltm_rect_step(const ltm_rect_step_args* a, const void* k, const float* q, const double* u,
                              const uint8_t* new_doc, float* ctx, void* stream) {
   using namespace ltm;
   LTM_REQUIRE(a && q && ctx, "rect_step: null pointer");
+  if (int rc = check_chunk_dtype("rect_step", "k_dtype", a->k_dtype, a->e, a->binned != 0)) return rc;
   const int D = a->H * a->d;
   const int qtiles = (a->Q + 31) / 32;
   cudaStream_t st_ = (cudaStream_t)stream;
@@ -86,7 +99,8 @@ extern "C" int ltm_rect_step(const ltm_rect_step_args* a, const float* k, const 
   }
   if (k != nullptr) {          // k == NULL: a->xpart was already filled (frame pooling is stateless and may be
     LTM_PROF(0);               // issued ahead of time on another stream, see BatchedRectLTM.prefetch)
-    rc = pool_chunk(a, k, a->xpart, ragged ? a->frame_offs : nullptr, a->frames, a->splits, binned, 0, stream);
+    rc = pool_chunk(a, k, a->k_dtype, a->xpart, ragged ? a->frame_offs : nullptr, a->frames, a->splits, binned, 0,
+                    stream);
     if (rc) return rc;
     LTM_PROF(1);
   }
@@ -219,18 +233,24 @@ extern "C" int ltm_rect_step_overlap(const ltm_rect_step_args* a, const ltm_over
   using namespace ltm;
   LTM_REQUIRE(a && o && q && ctx, "rect_step_overlap: null pointer");
   LTM_REQUIRE(o->ev_fork && o->ev_join, "rect_step_overlap: fork / join events missing");
+  if (int rc = check_chunk_dtype("rect_step_overlap", "k_dtype", a->k_dtype, a->e, a->binned != 0)) return rc;
+  if (o->k_next != nullptr) {
+    if (int rc = check_chunk_dtype("rect_step_overlap", "next_dtype", o->next_dtype, a->e, o->next_binned != 0))
+      return rc;
+    LTM_REQUIRE(o->xpart_next && o->ev_fork_pool && o->ev_pooled_next, "rect_step_overlap: prefetch target missing");
+    LTM_REQUIRE(!o->next_lengths || (o->next_offs && !o->next_binned), "rect_step_overlap: ragged next chunk");
+  }
   cudaStream_t ms = (cudaStream_t)o->main_stream, ss = (cudaStream_t)o->side_stream,
                cs = (cudaStream_t)o->compute_stream;
   if (o->k_next != nullptr) {
-    LTM_REQUIRE(o->xpart_next && o->ev_fork_pool && o->ev_pooled_next, "rect_step_overlap: prefetch target missing");
     // the target buffer was last read by work already queued on the main stream
     LTM_CUDA(cudaEventRecord((cudaEvent_t)o->ev_fork_pool, ms));
     LTM_CUDA(cudaStreamWaitEvent(ss, (cudaEvent_t)o->ev_fork_pool, 0));
     if (a->prof_events[0]) cudaEventRecord((cudaEvent_t)a->prof_events[0], ss);
-    LTM_REQUIRE(!o->next_lengths || (o->next_offs && !o->next_binned), "rect_step_overlap: ragged next chunk");
     const bool ragged_next = o->next_lengths != nullptr;
-    int rc = pool_chunk(a, o->k_next, o->xpart_next, ragged_next ? o->next_offs : nullptr, o->next_frames,
-                        ragged_next ? o->next_splits : a->splits, o->next_binned != 0, o->pool_ctas, ss);
+    int rc = pool_chunk(a, o->k_next, o->next_dtype, o->xpart_next, ragged_next ? o->next_offs : nullptr,
+                        o->next_frames, ragged_next ? o->next_splits : a->splits, o->next_binned != 0, o->pool_ctas,
+                        ss);
     if (rc) return rc;
     if (a->prof_events[1]) cudaEventRecord((cudaEvent_t)a->prof_events[1], ss);
     LTM_CUDA(cudaEventRecord((cudaEvent_t)o->ev_pooled_next, ss));
@@ -289,15 +309,16 @@ extern "C" int ltm_event_destroy(void* ev) {
   return 0;
 }
 
-extern "C" int ltm_rect_step_host(const ltm_rect_step_args* a, const float* k_host, const float* q_host,
+extern "C" int ltm_rect_step_host(const ltm_rect_step_args* a, const void* k_host, const float* q_host,
                                   const double* u_host, const uint8_t* new_doc_host, float* ctx_host, void* stream) {
   using namespace ltm;
   LTM_REQUIRE(a && k_host && q_host && ctx_host, "rect_step_host: null pointer");
   LTM_REQUIRE(a->k_dev && a->q_dev && a->ctx_dev, "rect_step_host: device staging buffers missing");
+  if (int rc = check_chunk_dtype("rect_step_host", "k_dtype", a->k_dtype, a->e, a->binned != 0)) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const size_t D = (size_t)a->H * a->d;
-  LTM_CUDA(cudaMemcpyAsync(a->k_dev, k_host, sizeof(float) * (size_t)a->Bv * a->L * a->T * a->e,
-                           cudaMemcpyHostToDevice, st));
+  const size_t elem = a->k_dtype ? 2 : 4;           // k_host and k_dev hold the chunk in its own storage
+  LTM_CUDA(cudaMemcpyAsync(a->k_dev, k_host, elem * (size_t)a->Bv * a->L * a->T * a->e, cudaMemcpyHostToDevice, st));
   LTM_CUDA(cudaMemcpyAsync(a->q_dev, q_host, sizeof(float) * (size_t)a->Bv * a->Q * D, cudaMemcpyHostToDevice, st));
   const double* u_dev = nullptr;
   if (u_host) {

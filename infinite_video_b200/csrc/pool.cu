@@ -186,7 +186,8 @@ pool_mean_persistent_kernel(const float4* __restrict__ k, float4* __restrict__ x
 
 // ---- 16-bit inputs (VideoChat2 runs the Q-former under fp16 autocast, videochat2_it_mistral.py:187): the chunk is
 // read as 128-bit vectors of 8 halves / bfloat16s and accumulated in fp32 -- half the HBM bytes of the fp32 path
-// and no up-cast pass.  One thread per 8 columns.
+// and no up-cast pass.  One thread per 8 columns.  Every entry point of the step (plain, prefetched, overlapped, host
+// buffers, ragged) pools a 16-bit chunk per frame through pool_unit16_at, so they all give the same bits.
 template <bool BF16>
 __device__ __forceinline__ void unpack8(const uint4& v, float* f) {
   const uint32_t w[4] = {v.x, v.y, v.z, v.w};
@@ -247,11 +248,35 @@ __device__ __forceinline__ void pool_unit16_at(const uint4* __restrict__ k, floa
   }
 }
 
-template <bool BF16>
+// one CTA per (frame, split); PERSIST: bounded grid walking the `total` items (the side-stream pooling of the
+// overlapped step), each pooled by the same pool_unit16_at call, so the bits do not depend on the grid
+template <bool BF16, bool PERSIST>
 __global__ void __launch_bounds__(256)
-pool_mean16_kernel(const uint4* __restrict__ k, float4* __restrict__ xpart, int T, int e8, int splits, float Tf) {
-  const unsigned unit = blockIdx.x / splits;
-  pool_unit16_at<BF16>(k, xpart, T, e8, splits, Tf, unit, (int)(blockIdx.x - unit * splits), unit, policy_evict_first());
+pool_mean16_kernel(const uint4* __restrict__ k, float4* __restrict__ xpart, int T, int e8, int splits, float Tf,
+                   unsigned total) {
+  if constexpr (!PERSIST) {
+    const unsigned unit = blockIdx.x / splits;
+    pool_unit16_at<BF16>(k, xpart, T, e8, splits, Tf, unit, (int)(blockIdx.x - unit * splits), unit,
+                         policy_evict_first());
+  } else {
+    const uint64_t pol = policy_evict_first();
+    for (unsigned work = blockIdx.x; work < total; work += gridDim.x) {
+      const unsigned unit = work / splits;
+      pool_unit16_at<BF16>(k, xpart, T, e8, splits, Tf, unit, (int)(work - unit * splits), unit, pol);
+    }
+  }
+}
+
+template <bool BF16>
+static void launch_pool_mean16(const void* k, float* xpart, int T, int e8, int splits, unsigned total, int max_ctas,
+                               cudaStream_t st) {
+  const int threads = e8 >= 256 ? 256 : ((e8 + 31) / 32) * 32;
+  const uint4* k4 = reinterpret_cast<const uint4*>(k);
+  float4* x = reinterpret_cast<float4*>(xpart);
+  if (max_ctas > 0 && (unsigned)max_ctas < total)
+    pool_mean16_kernel<BF16, true><<<(unsigned)max_ctas, threads, 0, st>>>(k4, x, T, e8, splits, (float)T, total);
+  else
+    pool_mean16_kernel<BF16, false><<<total, threads, 0, st>>>(k4, x, T, e8, splits, (float)T, total);
 }
 
 // ---- ragged batch: the grid covers exactly the (frame, token-split) items of the frames in use, packed video after
@@ -371,23 +396,26 @@ extern "C" int ltm_pool_mean_convert_ragged(const float* k, float* xpart, void* 
 
 extern "C" int ltm_pool_mean_16(const void* k, int is_bf16, float* xpart, int Bv, int L, int T, int e, int splits,
                                 void* stream) {
+  return ltm_pool_mean_16_grid(k, is_bf16, xpart, Bv, L, T, e, splits, 0, stream);
+}
+
+extern "C" int ltm_pool_mean_16_grid(const void* k, int is_bf16, float* xpart, int Bv, int L, int T, int e, int splits,
+                                     int max_ctas, void* stream) {
   using namespace ltm;
-  LTM_REQUIRE(k && xpart, "pool_mean_16: null pointer");
-  LTM_REQUIRE(Bv > 0 && L > 0 && T > 0 && e > 0, "pool_mean_16: bad shape Bv=%d L=%d T=%d e=%d", Bv, L, T, e);
-  LTM_REQUIRE(e % 8 == 0, "pool_mean_16: e=%d must be a multiple of 8 (128-bit access of 16-bit elements)", e);
-  LTM_REQUIRE(splits >= 1 && splits <= T, "pool_mean_16: splits=%d out of range [1,%d]", splits, T);
-  LTM_REQUIRE(aligned16(k) && aligned16(xpart), "pool_mean_16: pointers must be 16-byte aligned");
+  LTM_REQUIRE(k && xpart, "pool_mean_16_grid: null pointer");
+  LTM_REQUIRE(Bv > 0 && L > 0 && T > 0 && e > 0, "pool_mean_16_grid: bad shape Bv=%d L=%d T=%d e=%d", Bv, L, T, e);
+  LTM_REQUIRE(e % 8 == 0, "pool_mean_16_grid: e=%d must be a multiple of 8 (128-bit access of 16-bit elements)", e);
+  LTM_REQUIRE(splits >= 1 && splits <= T, "pool_mean_16_grid: splits=%d out of range [1,%d]", splits, T);
+  LTM_REQUIRE(max_ctas >= 0, "pool_mean_16_grid: max_ctas=%d must be >= 0", max_ctas);
+  LTM_REQUIRE(aligned16(k) && aligned16(xpart), "pool_mean_16_grid: pointers must be 16-byte aligned");
   const long long units = (long long)Bv * L * splits;
-  LTM_REQUIRE(units < (1ll << 31), "pool_mean_16: too many frames");
-  const int e8 = e / 8;
-  const int threads = e8 >= 256 ? 256 : ((e8 + 31) / 32) * 32;
+  LTM_REQUIRE(units < (1ll << 31), "pool_mean_16_grid: too many frames");
+  cudaStream_t st = (cudaStream_t)stream;
   if (is_bf16)
-    pool_mean16_kernel<true><<<(unsigned)units, threads, 0, (cudaStream_t)stream>>>(
-        reinterpret_cast<const uint4*>(k), reinterpret_cast<float4*>(xpart), T, e8, splits, (float)T);
+    launch_pool_mean16<true>(k, xpart, T, e / 8, splits, (unsigned)units, max_ctas, st);
   else
-    pool_mean16_kernel<false><<<(unsigned)units, threads, 0, (cudaStream_t)stream>>>(
-        reinterpret_cast<const uint4*>(k), reinterpret_cast<float4*>(xpart), T, e8, splits, (float)T);
-  LTM_CHECK_LAUNCH("pool_mean_16");
+    launch_pool_mean16<false>(k, xpart, T, e / 8, splits, (unsigned)units, max_ctas, st);
+  LTM_CHECK_LAUNCH("pool_mean_16_grid");
   return 0;
 }
 

@@ -44,8 +44,10 @@ CONFIGS = [
     ("not_sticky", dict(sticky=False), SMALL, "fp32", LOCKSTEP + RAGGED),
     ("mixed_new_doc", {}, SMALL, "fp32", LOCKSTEP),
     ("mixed_new_doc_bins", dict(bin_pool=True), dict(Bv=2, L=256, N=256), "fp32", LOCKSTEP),   # stale per-bin prefetch
-    ("fp16_chunk", {}, SMALL, "fp16", ("step", "pool+step", "ragged_step", "ragged_pool+step")),
-    ("bf16_chunk", {}, SMALL, "bf16", ("step", "pool+step", "ragged_step", "ragged_pool+step")),
+    # 16-bit chunks: every entry point must print the digest of `step` on the same chunks
+    ("fp16_chunk", {}, SMALL, "fp16", LOCKSTEP + ("ragged_step", "ragged_pool+step", "ragged_overlapped")),
+    ("bf16_chunk", {}, SMALL, "bf16", LOCKSTEP + ("ragged_step", "ragged_pool+step", "ragged_overlapped")),
+    ("production_fp16", {}, BIG, "fp16", LOCKSTEP[:4] + RAGGED),
 ]
 
 
