@@ -270,7 +270,7 @@ int ltm_cont_attn_rect_tc_split(const float* q, const float* K, const float* V, 
                                 const float* W, float W_out, const int32_t* jb, const float* tb,
                                 float* ctx, float* scores_ws, float* part_ws, float* hist_part,
                                 int Bv, int Q, int N, int H, int d, void* stream);
-/* the same two entry points for K|V stored as IEEE fp16 (csrc/attn_tc16.cu: kind::f16 UMMAs, the same 11-bit
+/* the same two entry points for K|V stored as IEEE fp16 (csrc/attn_tc.cu, KvF16: kind::f16 UMMAs, the same 11-bit
  * significand as the tf32 grid at half the bytes).  K, V: fp16 [Bv*N, ldkv] (ldkv in halves, % 8 == 0; e.g. the two
  * halves of an fp16 KV[Bv,N,2D] from ltm_gemm c_fp16 / ltm_consolidate_rect_kv round_tf32 == 2); X16: fp16 [N,64]
  * (columns 0..2 = 1, hi, lo of c_j / W_j; infinite_video_b200/tables.py).  q, W, outputs as above (fp32). */

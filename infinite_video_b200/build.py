@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libinfltm.so")
-SOURCES = ["pool.cu", "consolidate.cu", "sticky.cu", "attn.cu", "attn_fast.cu", "attn_tc.cu", "attn_tc16.cu", "attn_g16.cu", "gemm_simt.cu", "gemm_tcgen05.cu", "ridge.cu", "stm.cu",
+SOURCES = ["pool.cu", "consolidate.cu", "sticky.cu", "attn.cu", "attn_fast.cu", "attn_tc.cu", "attn_g16.cu", "gemm_simt.cu", "gemm_tcgen05.cu", "ridge.cu", "stm.cu",
            "capi.cu"]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC"]

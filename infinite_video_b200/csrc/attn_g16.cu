@@ -1,8 +1,9 @@
 // Continuous attention of variant G (Gaussian RBF bases) on the tensor cores (G4, long_term_attention.py:286-325).
 //
-// Same pipeline and work decomposition as attn_tc16.cu (read that file's header first): persistent CTAs walk the work
-// items (query tile, head, video); per item one thread issues  S^T = K_h q_h^T  and  D = V_h^T r  as kind::f16 UMMAs
-// with fp32 accumulation in TMEM while eight compute warps turn the scores into the weights r.  What differs:
+// Same pipeline and work decomposition as the fp16 path of attn_tc.cu (read that file's header first): persistent CTAs
+// walk the work items (query tile, head, video); per item one thread issues  S^T = K_h q_h^T  and  D = V_h^T r  as
+// kind::f16 UMMAs with fp32 accumulation in TMEM while eight compute warps turn the scores into the weights r.  What
+// differs:
 //
 //   * precision.  softmax(20 S) amplifies score errors twenty-fold and the weights r_j reach ~80 with the coefficients
 //     of an ill-conditioned ridge regression behind V, so single-pass fp16 / tf32 products are not enough (measured:
@@ -25,10 +26,6 @@
 #include "tcgen05.cuh"
 
 namespace ltm {
-
-int tma_encode_2d_f16(CUtensorMap* map, const void* base, unsigned long long inner, unsigned long long outer,
-                      unsigned long long pitch_elems, unsigned box_outer, const char* what);
-
 namespace g16 {
 
 constexpr int DH = 64;

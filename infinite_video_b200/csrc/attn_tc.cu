@@ -22,6 +22,23 @@
 // and issue slots stay almost free (288 threads), which is what lets the frame pooling of the next chunk run
 // beside it (BatchedRectLTM.prefetch).  K and V must already be tf32-rounded (ltm_gemm round_tf32) so that the
 // tensor core's own fp32 -> tf32 truncation does not bias the scores.
+//
+// K|V stored as fp16 (KvF16, the default) run the same kernel with another operand format: K|V come in as IEEE fp16
+// -- the same 11-bit significand as the tf32 grid, at half the bytes -- the queries and the attention weights are
+// written as fp16 by the CTA, and both contractions run as kind::f16 UMMAs (K = 16 per instruction) with fp32
+// accumulation in TMEM:
+//
+//   S^T[j, q] = K_h[j, :] . q_h[q, :]     A = K_h  (TMA, K-major SWIZZLE_128B: one row of 64 halves = 128 B per basis)
+//                                          B = q_h / sqrt(d) as fp16, written by the CTA ([32 q][64 d], K-major)
+//   D[m, q]   = sum_j A2[m, j] e[j, q]    A2 = [V_h^T ; X^T] (TMA, MN-major SWIZZLE_128B: atoms of 8 j-rows x 64 halves;
+//                                          the 64 value columns and the 64-column table X are the two MN atoms, so
+//                                          M = 128 exactly), B = e^T as fp16 ([NB/64 k-blocks][32 q][64 j], K-major)
+//
+// The fp16 weights are scaled by 256 (e' = 256 W_j exp(S - m), W_j ~ 1/256: the largest weight is ~1) so that weights
+// down to e^{-9.7} of the largest stay fp16-normal; the factor cancels in every ratio that leaves the kernel.
+// Shared memory per CTA at num_basis 256: K 32 KB + V 32 KB + X 32 KB + e^T 16 KB + q 4 KB (fp32 K|V: 200 KB).
+#include <cuda_fp16.h>
+
 #include "rect_hist.cuh"
 #include "tcgen05.cuh"
 
@@ -54,23 +71,55 @@ struct Params {
 };
 constexpr int PART_ROWS = 68;
 
-template <int NB>
+// Storage formats of K|V.  ROW: elements in one 128-byte swizzle row, so that every UMMA consumes 32 bytes of K
+// (ROW / 4 elements); V_SBO / V_LAYOUT: UMMA descriptor of the MN-major A2 operand.
+struct KvTf32 {                          // fp32 on the tf32 grid: kind::tf32, A2 in SWIZZLE_128B_BASE32B
+  static constexpr bool HALF = false;
+  static constexpr int ROW = 32;
+  static constexpr uint32_t IDESC_AB = (2u << 7) | (2u << 10);
+  static constexpr uint32_t V_SBO = 512, V_LAYOUT = 1;
+  static constexpr float WSCALE = 1.f;
+  static constexpr const char* NAME = "cont_attn_rect_tc";
+};
+struct KvF16 {                           // IEEE fp16: kind::f16, A2 in 16-bit SWIZZLE_128B (atoms of [8 j][64 mn])
+  static constexpr bool HALF = true;
+  static constexpr int ROW = 64;
+  static constexpr uint32_t IDESC_AB = 0u;
+  static constexpr uint32_t V_SBO = 1024, V_LAYOUT = 2;
+  static constexpr float WSCALE = 256.f; // weights are formed as 256 W_j exp(S - m): fp16-normal down to e^{-9.7}
+  static constexpr const char* NAME = "cont_attn_rect_tc16";
+};
+
+template <int NB, class KV>
 struct Lay {
-  static constexpr int SLAB = NB * 128;              // NB rows x 32 floats
-  static constexpr int K_OFF = 0;                    // 2 slabs: d 0..31 | d 32..63        (K-major rows = j)
-  static constexpr int V_OFF = 2 * SLAB;             // 3 slabs: V d 0..31 | V d 32..63 | X (MN-major rows = j)
-  static constexpr int R_OFF = 5 * SLAB;             // e^T: [NB/32 k-blocks][32 q][32 j]; also "slab 3" of A2
-  static constexpr int Q_OFF = 6 * SLAB;             // q tile: [2 k-blocks][32 q][32 d]
-  static constexpr int MISC_OFF = Q_OFF + 2 * 4096;
+  static constexpr int SLAB = NB * 128;              // NB rows x 128 B: 32 floats or 64 halves
+  static constexpr int KSLABS = DH / KV::ROW;        // slabs of one K|V row: 2 (d 0..31 | d 32..63) or 1
+  static constexpr int K_OFF = 0;                    // KSLABS slabs: K_h                 (K-major rows = j)
+  static constexpr int V_OFF = KSLABS * SLAB;        // KSLABS + 1 slabs: V_h | X         (MN-major rows = j)
+  static constexpr int R_OFF = V_OFF + (KSLABS + 1) * SLAB;   // e^T: [NB/ROW k-blocks][32 q][ROW j]; fp32: also
+                                                              // "slab 3" of A2
+  static constexpr int R_BYTES = ((NB + KV::ROW - 1) / KV::ROW) * 4096;   // (fp16, NB = 64: one block)
+  static constexpr int Q_OFF = R_OFF + R_BYTES;      // q tile: [KSLABS k-blocks][32 q][ROW d]
+  static constexpr int MISC_OFF = Q_OFF + KSLABS * 4096;
   static constexpr int MISC_FLOATS = 8 * 32 + 4 * 32 + 96 + NB + 32;
   static constexpr int BYTES = MISC_OFF + MISC_FLOATS * 4 + 64 + 1024;   // + 6 barriers, TMEM slot, alignment slack
 };
 
+template <class KV>
+__device__ __forceinline__ void mma(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi,
+                                    uint32_t idesc, uint32_t accumulate) {
+  if constexpr (KV::HALF)
+    tcgen05_mma_f16(tmem_d, a_lo, a_hi, b_lo, b_hi, idesc, accumulate);
+  else
+    tcgen05_mma_tf32(tmem_d, a_lo, a_hi, b_lo, b_hi, idesc, accumulate);
+}
+
 __device__ __forceinline__ void cw_sync() { asm volatile("bar.sync 1, 256;" ::: "memory"); }   // the 8 compute warps
 
-// q tile of one work item, scaled by 1/sqrt(d) (gibbs:226; a power of two, exact) and rounded to tf32, in the
-// K-major SWIZZLE_128B layout: element (q, d) at [d >> 5][q][((d & 31) >> 2) ^ (q & 7)][d & 3].  256 threads; the
-// global loads are issued one item ahead (load_q) so that their latency is off the item's critical path.
+// q tile of one work item, scaled by 1/sqrt(d) (gibbs:226; a power of two, exact) and rounded to the operand format,
+// in the K-major SWIZZLE_128B layout.  tf32: element (q, d) at [d >> 5][q][((d & 31) >> 2) ^ (q & 7)][d & 3]; fp16:
+// row q = 64 halves = 128 B, 16-byte chunk (d >> 3) at position (d >> 3) ^ (q & 7).  256 threads, 8 consecutive d
+// each; the global loads are issued one item ahead (load_q) so that their latency is off the item's critical path.
 struct QRegs { float4 a, b; };
 __device__ __forceinline__ QRegs load_q(const float* qbase, int rows, int D, int tid) {
   const int qq = tid >> 3, dch = tid & 7;                          // 8 consecutive d per thread
@@ -88,15 +137,26 @@ __device__ __forceinline__ QRegs load_q(const float* qbase, int rows, int D, int
   }
   return r;
 }
+__device__ __forceinline__ uint32_t pack_h2(float lo, float hi) {
+  const __half2 h = __floats2half2_rn(lo, hi);
+  return *reinterpret_cast<const uint32_t*>(&h);
+}
+template <class KV>
 __device__ __forceinline__ void store_q_tile(uint8_t* dstq, const QRegs& r, int tid) {
   const int qq = tid >> 3, dch = tid & 7;
   const float sc = 0.125f;
-  const float4 a = make_float4(tf32_rna(r.a.x * sc), tf32_rna(r.a.y * sc), tf32_rna(r.a.z * sc), tf32_rna(r.a.w * sc));
-  const float4 b = make_float4(tf32_rna(r.b.x * sc), tf32_rna(r.b.y * sc), tf32_rna(r.b.z * sc), tf32_rna(r.b.w * sc));
-  uint8_t* row = dstq + (dch >> 2) * 4096 + qq * 128;
-  const int c0 = (dch & 3) * 2;
-  *reinterpret_cast<float4*>(row + (((c0) ^ (qq & 7)) << 4)) = a;
-  *reinterpret_cast<float4*>(row + (((c0 + 1) ^ (qq & 7)) << 4)) = b;
+  if constexpr (KV::HALF) {
+    const uint4 v = make_uint4(pack_h2(r.a.x * sc, r.a.y * sc), pack_h2(r.a.z * sc, r.a.w * sc),
+                               pack_h2(r.b.x * sc, r.b.y * sc), pack_h2(r.b.z * sc, r.b.w * sc));
+    *reinterpret_cast<uint4*>(dstq + qq * 128 + ((dch ^ (qq & 7)) << 4)) = v;
+  } else {
+    const float4 a = make_float4(tf32_rna(r.a.x * sc), tf32_rna(r.a.y * sc), tf32_rna(r.a.z * sc), tf32_rna(r.a.w * sc));
+    const float4 b = make_float4(tf32_rna(r.b.x * sc), tf32_rna(r.b.y * sc), tf32_rna(r.b.z * sc), tf32_rna(r.b.w * sc));
+    uint8_t* row = dstq + (dch >> 2) * 4096 + qq * 128;
+    const int c0 = (dch & 3) * 2;
+    *reinterpret_cast<float4*>(row + (((c0) ^ (qq & 7)) << 4)) = a;
+    *reinterpret_cast<float4*>(row + (((c0 + 1) ^ (qq & 7)) << 4)) = b;
+  }
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 }
 
@@ -107,12 +167,14 @@ __device__ __forceinline__ void store_q_tile(uint8_t* dstq, const QRegs& r, int 
 //   bar_k / bar_v   TMA bytes of this item's K / V (+ X once)            bar_s / bar_pv   tcgen05.commit
 //   bar_q           256 arrivals: q tile of the next item is in place (and S has been read out of TMEM)
 //   bar_r           256 arrivals: e^T is in place (and D of the previous item has been read out of TMEM)
-template <int NB>
+template <int NB, class KV>
 __global__ void __maxnreg__(TC_MAX_REGS)
 cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_constant__ CUtensorMap mapV,
                     const __grid_constant__ CUtensorMap mapX, const Params p, const int q_tiles, const int total) {
   static_assert(NB == 64 || NB == 128 || NB == 256, "the tensor-core path covers num_basis 64 / 128 / 256");
-  using L_ = Lay<NB>;
+  using L_ = Lay<NB, KV>;
+  constexpr int KSLABS = L_::KSLABS;
+  constexpr int MMA_K = KV::ROW / 4;         // elements of K per UMMA: 32 bytes, a quarter of a swizzle row
   constexpr int HALVES = (NB + 127) / 128;   // score MMAs (M = 128 each); NB = 64: the upper 64 rows read past the
                                              // K tile (finite or not, they only reach accumulator rows nobody reads)
   constexpr int JWARPS = NB / 32;            // compute warps that own a basis (the others only help with the outputs)
@@ -163,13 +225,13 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
       asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
       int qt, h, v;
       decode(w0, qt, h, v);
-      mbar_arrive_expect_tx(bar_k, 2 * L_::SLAB);
+      mbar_arrive_expect_tx(bar_k, KSLABS * L_::SLAB);
       tma_load_2d(&mapK, sK, bar_k, h * DH, jrow(w0, v));
-      tma_load_2d(&mapK, sK + L_::SLAB, bar_k, h * DH + 32, jrow(w0, v));
-      mbar_arrive_expect_tx(bar_v, 3 * L_::SLAB);
+      if constexpr (KSLABS == 2) tma_load_2d(&mapK, sK + L_::SLAB, bar_k, h * DH + 32, jrow(w0, v));
+      mbar_arrive_expect_tx(bar_v, (KSLABS + 1) * L_::SLAB);
       tma_load_2d(&mapV, sV, bar_v, h * DH, jrow(w0, v));
-      tma_load_2d(&mapV, sV + L_::SLAB, bar_v, h * DH + 32, jrow(w0, v));
-      tma_load_2d(&mapX, sV + 2 * L_::SLAB, bar_v, 0, (w0 % halves) * NB);
+      if constexpr (KSLABS == 2) tma_load_2d(&mapV, sV + L_::SLAB, bar_v, h * DH + 32, jrow(w0, v));
+      tma_load_2d(&mapX, sV + KSLABS * L_::SLAB, bar_v, 0, (w0 % halves) * NB);
     }
     __syncwarp();
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
@@ -182,17 +244,19 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
   tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
-  // instruction descriptors: D=f32 [4,6)=1, A=tf32 [7,10)=2, B=tf32 [10,13)=2, a_major bit 15 (1 = MN-major),
-  // N>>3 [17,23), M>>4 [24,29)
-  constexpr uint32_t IDESC_S = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(QT >> 3) << 17) | ((128u >> 4) << 24);
+  // instruction descriptors: D=f32 [4,6)=1, A [7,10) and B [10,13) = KV::IDESC_AB (tf32 2, f16 0), a_major bit 15
+  // (1 = MN-major), N>>3 [17,23), M>>4 [24,29)
+  constexpr uint32_t IDESC_S = (1u << 4) | KV::IDESC_AB | ((uint32_t)(QT >> 3) << 17) | ((128u >> 4) << 24);
   constexpr uint32_t IDESC_PV = IDESC_S | (1u << 15);
 
   if (warp == 8) {
     // ------------------------------------------------------------------ TMA + MMA issue (one lane)
     if (lane == 0) {
       // descriptor words: only the start-address field of the low word changes between MMAs (compile-time offsets)
+      // K-major SWIZZLE_128B: 8-row groups 1024 B apart; MN-major A2: the MN atoms one slab apart (LBO), the 8-row j
+      // groups KV::V_SBO apart; an MMA of K = MMA_K consumes MMA_K rows of j
       const uint64_t dK = umma_desc(sK, 16, 1024, 2u), dQ = umma_desc(sQ, 16, 1024, 2u);
-      const uint64_t dV = umma_desc(sV, L_::SLAB, 512, 1u), dR = umma_desc(sR, 16, 1024, 2u);
+      const uint64_t dV = umma_desc(sV, L_::SLAB, KV::V_SBO, KV::V_LAYOUT), dR = umma_desc(sR, 16, 1024, 2u);
       const uint32_t dk_lo = (uint32_t)dK, dk_hi = (uint32_t)(dK >> 32), dq_lo = (uint32_t)dQ;
       const uint32_t dv_lo = (uint32_t)dV, dv_hi = (uint32_t)(dV >> 32), dr_lo = (uint32_t)dR;
       auto issue_scores = [&](uint32_t ph) {            // S^T of the item whose K tile / q tile carry parity ph
@@ -202,11 +266,10 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
 #pragma unroll
         for (int hf = 0; hf < HALVES; ++hf) {
 #pragma unroll
-          for (int ks = 0; ks < DH / 8; ++ks)
-            tcgen05_mma_tf32(tmem_base + hf * QT,
-                             dk_lo + (uint32_t)(((ks >> 2) * L_::SLAB + hf * (128 * 128) + (ks & 3) * 32) >> 4), dk_hi,
-                             dq_lo + (uint32_t)(((ks >> 2) * 4096 + (ks & 3) * 32) >> 4), dk_hi, IDESC_S,
-                             ks != 0 ? 1u : 0u);
+          for (int ks = 0; ks < DH / MMA_K; ++ks)      // (ks >> 2: second slab of K / k-block of q, fp32 only)
+            mma<KV>(tmem_base + hf * QT,
+                    dk_lo + (uint32_t)(((ks >> 2) * L_::SLAB + hf * (128 * 128) + (ks & 3) * 32) >> 4), dk_hi,
+                    dq_lo + (uint32_t)(((ks >> 2) * 4096 + (ks & 3) * 32) >> 4), dk_hi, IDESC_S, ks != 0 ? 1u : 0u);
         }
         tcgen05_commit(bar_s);
       };
@@ -219,9 +282,9 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
         if (wn < total) decode(wn, qtn, hn, vn);
         mbar_wait(bar_s, ph);                          // the K buffer has been read
         if (wn < total) {
-          mbar_arrive_expect_tx(bar_k, 2 * L_::SLAB);
+          mbar_arrive_expect_tx(bar_k, KSLABS * L_::SLAB);
           tma_load_2d(&mapK, sK, bar_k, hn * DH, jrow(wn, vn));
-          tma_load_2d(&mapK, sK + L_::SLAB, bar_k, hn * DH + 32, jrow(wn, vn));
+          if constexpr (KSLABS == 2) tma_load_2d(&mapK, sK + L_::SLAB, bar_k, hn * DH + 32, jrow(wn, vn));
         }
         mbar_wait(bar_r, ph);                          // e^T written, D free
         mbar_wait(bar_v, ph);
@@ -229,10 +292,9 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
         // this warp contracts the first half of the basis range into D0, warp 9 the second half into D1: the issue
         // of 32 small MMAs by one thread (~33 ns each) was 1.05 us of the item's 4.7 us
 #pragma unroll
-        for (int ks = 0; ks < NB / 16; ++ks)
-          tcgen05_mma_tf32(tmem_base + 64, dv_lo + (uint32_t)((ks * 1024) >> 4), dv_hi,
-                           dr_lo + (uint32_t)(((ks >> 2) * 4096 + (ks & 3) * 32) >> 4), dk_hi, IDESC_PV,
-                           ks != 0 ? 1u : 0u);
+        for (int ks = 0; ks < NB / (2 * MMA_K); ++ks)
+          mma<KV>(tmem_base + 64, dv_lo + (uint32_t)((ks * MMA_K * 128) >> 4), dv_hi,
+                  dr_lo + (uint32_t)(((ks >> 2) * 4096 + (ks & 3) * 32) >> 4), dk_hi, IDESC_PV, ks != 0 ? 1u : 0u);
         tcgen05_commit(bar_pv);
         // the next item's scores go out right behind: its keys landed during this item's weight phase, so S is
         // ready by the time the compute warps have written this item's outputs
@@ -240,10 +302,10 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
         mbar_wait(bar_pv, ph);                         // the V buffer (and e^T) have been read
         if (wn < total) {
           // (the per-basis operand rows X change with the basis half: re-fetched with V when there are two)
-          mbar_arrive_expect_tx(bar_v, (halves > 1 ? 3 : 2) * L_::SLAB);
+          mbar_arrive_expect_tx(bar_v, (halves > 1 ? KSLABS + 1 : KSLABS) * L_::SLAB);
           tma_load_2d(&mapV, sV, bar_v, hn * DH, jrow(wn, vn));
-          tma_load_2d(&mapV, sV + L_::SLAB, bar_v, hn * DH + 32, jrow(wn, vn));
-          if (halves > 1) tma_load_2d(&mapX, sV + 2 * L_::SLAB, bar_v, 0, (wn % halves) * NB);
+          if constexpr (KSLABS == 2) tma_load_2d(&mapV, sV + L_::SLAB, bar_v, hn * DH + 32, jrow(wn, vn));
+          if (halves > 1) tma_load_2d(&mapX, sV + KSLABS * L_::SLAB, bar_v, 0, (wn % halves) * NB);
         }
       }
     }
@@ -251,7 +313,7 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
   } else if (warp == 9) {
     // ------------------------------------------------------------------ second MMA issuer (one lane)
     if (lane == 0) {
-      const uint64_t dV = umma_desc(sV, L_::SLAB, 512, 1u), dR = umma_desc(sR, 16, 1024, 2u);
+      const uint64_t dV = umma_desc(sV, L_::SLAB, KV::V_SBO, KV::V_LAYOUT), dR = umma_desc(sR, 16, 1024, 2u);
       const uint32_t dv_lo = (uint32_t)dV, dv_hi = (uint32_t)(dV >> 32), dr_lo = (uint32_t)dR, dr_hi = (uint32_t)(dR >> 32);
       uint32_t it = 0;
       for (int w = w0; w < total; w += wstride, ++it) {
@@ -260,10 +322,10 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
         mbar_wait(bar_v, ph);
         tcgen05_fence_after();
 #pragma unroll
-        for (int ks = NB / 16; ks < NB / 8; ++ks)
-          tcgen05_mma_tf32(tmem_base + 96, dv_lo + (uint32_t)((ks * 1024) >> 4), dv_hi,
-                           dr_lo + (uint32_t)(((ks >> 2) * 4096 + (ks & 3) * 32) >> 4), dr_hi, IDESC_PV,
-                           ks != NB / 16 ? 1u : 0u);
+        for (int ks = NB / (2 * MMA_K); ks < NB / MMA_K; ++ks)
+          mma<KV>(tmem_base + 96, dv_lo + (uint32_t)((ks * MMA_K * 128) >> 4), dv_hi,
+                  dr_lo + (uint32_t)(((ks >> 2) * 4096 + (ks & 3) * 32) >> 4), dr_hi, IDESC_PV,
+                  ks != NB / (2 * MMA_K) ? 1u : 0u);
         tcgen05_commit(bar_pv);
       }
     }
@@ -273,7 +335,7 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
     const bool active = warp < JWARPS;
     const int j = (warp >> 2) * 128 + (warp & 3) * 32 + lane;      // this thread's basis in the weight phase
     const int quarter = warp & 3, chalf = warp >> 2;
-    float Wj = active ? __ldg(p.W + (w0 % halves) * NB + j) : 0.f;
+    float Wj = active ? KV::WSCALE * __ldg(p.W + (w0 % halves) * NB + j) : 0.f;
     float rWj = active ? 1.0f / Wj : 0.f;
     // histogram bin of this thread (tid < 127): p_i = dt_{i+1}/2 (G[jb_{i+1}] + G[jb_{i+2}])
     int hja = NB, hjb = NB;
@@ -288,7 +350,7 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
       int qt, h, v;
       decode(w0, qt, h, v);
       const QRegs qr = load_q(p.q + ((size_t)v * Q + qt * QT) * D + h * DH, min(QT, Q - qt * QT), D, tid);
-      store_q_tile(sm + L_::Q_OFF, qr, tid);
+      store_q_tile<KV>(sm + L_::Q_OFF, qr, tid);
       mbar_arrive(bar_q);
     }
     QRegs qnext;                                       // queries of item it + 1, fetched during item it - 1
@@ -310,7 +372,7 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
       const int wn = w + wstride;
       const int jhalf = (w % halves) * NB;               // first basis of this item's half
       if (halves > 1 && active) {
-        Wj = __ldg(p.W + jhalf + j);
+        Wj = KV::WSCALE * __ldg(p.W + jhalf + j);
         rWj = 1.0f / Wj;
       }
       mbar_wait(bar_s, ph);
@@ -333,7 +395,7 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
         for (int c = 0; c < 32; ++c) e[c] = __uint_as_float(r[c]);
       }
       // the score MMAs are complete (bar_s): the q tile can take the next item's queries
-      if (wn < total) store_q_tile(sm + L_::Q_OFF, qnext, tid);
+      if (wn < total) store_q_tile<KV>(sm + L_::Q_OFF, qnext, tid);
       tcgen05_fence_before();
       mbar_arrive(bar_q);
       if (active) {
@@ -358,13 +420,25 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
 #pragma unroll
         for (int ww = 0; ww < JWARPS; ++ww) M = fmaxf(M, wmax[ww * 32 + lane]);
         if (warp == 0) mcol[lane] = M;
-        uint8_t* rblk = sm + L_::R_OFF + (j >> 5) * 4096 + (lane & 3) * 4;
+        if constexpr (KV::HALF) {
+          // e^T element (q = c, j) as fp16: k-block j >> 6, row c, 16-byte chunk ((j & 63) >> 3) ^ (c & 7), half j & 7
+          uint8_t* rblk = sm + L_::R_OFF + (j >> 6) * 4096 + (lane & 7) * 2;
+          const int jchunk = (j & 63) >> 3;
 #pragma unroll
-        for (int c = 0; c < 32; ++c) {
-          const float m = __shfl_sync(0xffffffffu, M, c);
-          e[c] = Wj * __expf(e[c] - m);
-          // e^T element (q = c, j): row c of k-block j >> 5, chunk ((j & 31) >> 2) ^ (c & 7)
-          *reinterpret_cast<float*>(rblk + c * 128 + ((((lane >> 2) ^ (c & 7))) << 4)) = tf32_rna(e[c]);
+          for (int c = 0; c < 32; ++c) {
+            const float m = __shfl_sync(0xffffffffu, M, c);
+            e[c] = Wj * __expf(e[c] - m);
+            *reinterpret_cast<__half*>(rblk + c * 128 + ((jchunk ^ (c & 7)) << 4)) = __float2half_rn(e[c]);
+          }
+        } else {
+          uint8_t* rblk = sm + L_::R_OFF + (j >> 5) * 4096 + (lane & 3) * 4;
+#pragma unroll
+          for (int c = 0; c < 32; ++c) {
+            const float m = __shfl_sync(0xffffffffu, M, c);
+            e[c] = Wj * __expf(e[c] - m);
+            // e^T element (q = c, j): row c of k-block j >> 5, chunk ((j & 31) >> 2) ^ (c & 7)
+            *reinterpret_cast<float*>(rblk + c * 128 + ((((lane >> 2) ^ (c & 7))) << 4)) = tf32_rna(e[c]);
+          }
         }
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
       }
@@ -428,8 +502,8 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
         if (lane < 16) {
           const int c = chalf * 16 + lane;
           const float em = expf(-mcol[c]);
-          zq[c] = 1.0f / (sc[lane] + p.W_out * em);
-          const float rz = (c < rows) ? 1.0f / (sc[16 + lane] + sc[32 + lane] + p.c_none * em) : 0.f;
+          zq[c] = 1.0f / (sc[lane] + KV::WSCALE * p.W_out * em);
+          const float rz = (c < rows) ? 1.0f / (sc[16 + lane] + sc[32 + lane] + KV::WSCALE * p.c_none * em) : 0.f;
           rzh[c] = rz;
           ems[c] = em * rz;
         }
@@ -473,6 +547,7 @@ cont_attn_tc_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_const
 
 // Merge of the two basis halves of num_basis = 512: ctx = (D_0 s_0 + D_1 s_1) / (Z_0 s_0 + Z_1 s_1 + W_out e^{-m}),
 // m = max(m_0, m_1), s_i = e^{m_i - m}.  One CTA per (query tile, head, video); thread -> (q, d) with d fastest.
+// W_out is the quadrature weight on the scale of the stored sums (KV::WSCALE * W_out).
 __global__ void __launch_bounds__(256)
 attn_tc_combine_kernel(const float* __restrict__ part, float* __restrict__ ctx, float W_out, int Q, int H,
                        int q_tiles, int nvid) {
@@ -499,28 +574,66 @@ attn_tc_combine_kernel(const float* __restrict__ part, float* __restrict__ ctx, 
   }
 }
 
-template <int NB>
+template <int NB, class KV>
 static int launch(const CUtensorMap& mK, const CUtensorMap& mV, const CUtensorMap& mX, const Params& p, int Bv,
                   cudaStream_t stream) {
+  using L_ = Lay<NB, KV>;
   static PerDevice pd = {};
   int num_sms = 0;
-  if (int rc = kernel_setup(cont_attn_tc_kernel<NB>, (size_t)Lay<NB>::BYTES, pd, &num_sms)) return rc;
+  if (int rc = kernel_setup(cont_attn_tc_kernel<NB, KV>, (size_t)L_::BYTES, pd, &num_sms)) return rc;
   const int q_tiles = (p.Q + QT - 1) / QT;
   const long long total = (long long)q_tiles * p.H * Bv * p.halves;
   LTM_REQUIRE(total < (1ll << 31), "cont_attn_rect_tc: too many work items");
   // persistent CTAs: one per SM for num_basis 256 (209 KB of shared memory), two for 64 / 128 (60 / 106 KB; 2 x 320
   // threads x 96 registers and 2 x 128 TMEM columns fit): an item costs ~3 us of mostly latency whatever its size, so
   // the small shapes (cfg1, cfg3: 12 k / 2.3 k items of 64 bases) gain from a second CTA filling the bubbles
-  constexpr int PER_SM = (2 * Lay<NB>::BYTES <= 227 * 1024) ? 2 : 1;
+  constexpr int PER_SM = (2 * L_::BYTES <= 227 * 1024) ? 2 : 1;
   const long long slots = (long long)num_sms * PER_SM;
   const unsigned grid = (unsigned)(total < slots ? total : slots);
-  cont_attn_tc_kernel<NB><<<grid, THREADS, Lay<NB>::BYTES, stream>>>(mK, mV, mX, p, q_tiles, (int)total);
+  cont_attn_tc_kernel<NB, KV><<<grid, THREADS, L_::BYTES, stream>>>(mK, mV, mX, p, q_tiles, (int)total);
   LTM_CHECK_LAUNCH("cont_attn_rect_tc");
   if (p.halves > 1) {
-    attn_tc_combine_kernel<<<(unsigned)(total / 2), 256, 0, stream>>>(p.part, p.ctx, p.W_out, p.Q, p.H, q_tiles, Bv);
+    attn_tc_combine_kernel<<<(unsigned)(total / 2), 256, 0, stream>>>(p.part, p.ctx, KV::WSCALE * p.W_out, p.Q, p.H,
+                                                                       q_tiles, Bv);
     LTM_CHECK_LAUNCH("attn_tc_combine");
   }
   return 0;
+}
+
+// K, V, X: fp32 (KvTf32) or fp16 (KvF16) rows; see include/infltm.h
+template <class KV>
+static int cont_attn_rect_tc_impl(const float* q, const void* K, const void* V, int64_t ldkv, const void* X,
+                                  const float* W, float W_out, float c_none, const int32_t* jb, const float* tb,
+                                  float* ctx, float* scores_out, float* hist_part, float* part, int Bv, int Q, int N,
+                                  int H, int d, void* stream) {
+  const int halves = part != nullptr ? 2 : 1;
+  const int NBk = N / halves;                        // basis functions per work item
+  LTM_REQUIRE(q && K && V && X && W && ctx, "%s: null pointer", KV::NAME);
+  LTM_REQUIRE(hist_part == nullptr || (jb && tb), "%s: histogram requested without edge tables", KV::NAME);
+  LTM_REQUIRE(Bv > 0 && Bv <= 65535 && Q > 0 && H > 0 && H <= 65535 && ldkv % (KV::HALF ? 8 : 4) == 0 &&
+                  ldkv >= (int64_t)H * d,
+              "%s: bad shape", KV::NAME);
+  LTM_REQUIRE(aligned16(q) && aligned16(ctx) && aligned16(part), "%s: 16-byte alignment", KV::NAME);
+  CUtensorMap mK, mV, mX;
+  const unsigned long long rows = (unsigned long long)Bv * N, hd = (unsigned long long)H * d;
+  if constexpr (KV::HALF) {
+    if (tma_encode_2d_f16(&mK, K, hd, rows, (unsigned long long)ldkv, (unsigned)NBk, "attn16 K")) return -1;
+    if (tma_encode_2d_f16(&mV, V, hd, rows, (unsigned long long)ldkv, (unsigned)NBk, "attn16 V")) return -1;
+    if (tma_encode_2d_f16(&mX, X, 64, (unsigned long long)N, 64, (unsigned)NBk, "attn16 X")) return -1;
+  } else {
+    const float *Kf = static_cast<const float*>(K), *Vf = static_cast<const float*>(V);
+    const float* Xf = static_cast<const float*>(X);
+    if (tma_encode_2d(&mK, Kf, hd, rows, (unsigned long long)ldkv, 32, (unsigned)NBk, 0, "attn K")) return -1;
+    if (tma_encode_2d(&mV, Vf, hd, rows, (unsigned long long)ldkv, 32, (unsigned)NBk, 1, "attn V")) return -1;
+    if (tma_encode_2d(&mX, Xf, 32, (unsigned long long)N, 32, 32, (unsigned)NBk, 1, "attn X")) return -1;
+  }
+  Params p{};
+  p.q = q; p.W = W; p.tb = tb; p.jb = jb; p.W_out = W_out; p.c_none = c_none; p.ctx = ctx;
+  p.scores_out = scores_out; p.hist_part = hist_part; p.Q = Q; p.H = H;
+  p.halves = halves; p.NT = N; p.part = part;
+  if (NBk == 256) return launch<256, KV>(mK, mV, mX, p, Bv, (cudaStream_t)stream);
+  if (NBk == 128) return launch<128, KV>(mK, mV, mX, p, Bv, (cudaStream_t)stream);
+  return launch<64, KV>(mK, mV, mX, p, Bv, (cudaStream_t)stream);
 }
 
 }  // namespace tc
@@ -532,42 +645,14 @@ extern "C" int64_t ltm_attn_tc_split_workspace_floats(int Bv, int Q, int H) {
   return (int64_t)Bv * H * ((Q + ltm::tc::QT - 1) / ltm::tc::QT) * 2 * ltm::tc::PART_ROWS * ltm::tc::QT;
 }
 
-static int cont_attn_rect_tc_impl(const float* q, const float* K, const float* V, int64_t ldkv, const float* X,
-                                  const float* W, float W_out, float c_none, const int32_t* jb, const float* tb,
-                                  float* ctx, float* scores_out, float* hist_part, float* part, int Bv, int Q, int N,
-                                  int H, int d, void* stream) {
-  using namespace ltm;
-  const int halves = part != nullptr ? 2 : 1;
-  const int NBk = N / halves;                        // basis functions per work item
-  LTM_REQUIRE(q && K && V && X && W && ctx, "cont_attn_rect_tc: null pointer");
-  LTM_REQUIRE(hist_part == nullptr || (jb && tb), "cont_attn_rect_tc: histogram requested without edge tables");
-  LTM_REQUIRE(Bv > 0 && Bv <= 65535 && Q > 0 && H > 0 && H <= 65535 && ldkv % 4 == 0 && ldkv >= (int64_t)H * d,
-              "cont_attn_rect_tc: bad shape");
-  LTM_REQUIRE(aligned16(q) && aligned16(ctx) && aligned16(part), "cont_attn_rect_tc: 16-byte alignment");
-  CUtensorMap mK, mV, mX;
-  const unsigned long long rows = (unsigned long long)Bv * N;
-  if (tma_encode_2d(&mK, K, (unsigned long long)H * d, rows, (unsigned long long)ldkv, 32, (unsigned)NBk, 0, "attn K"))
-    return -1;
-  if (tma_encode_2d(&mV, V, (unsigned long long)H * d, rows, (unsigned long long)ldkv, 32, (unsigned)NBk, 1, "attn V"))
-    return -1;
-  if (tma_encode_2d(&mX, X, 32, (unsigned long long)N, 32, 32, (unsigned)NBk, 1, "attn X")) return -1;
-  tc::Params p{};
-  p.q = q; p.W = W; p.tb = tb; p.jb = jb; p.W_out = W_out; p.c_none = c_none; p.ctx = ctx;
-  p.scores_out = scores_out; p.hist_part = hist_part; p.Q = Q; p.H = H;
-  p.halves = halves; p.NT = N; p.part = part;
-  if (NBk == 256) return tc::launch<256>(mK, mV, mX, p, Bv, (cudaStream_t)stream);
-  if (NBk == 128) return tc::launch<128>(mK, mV, mX, p, Bv, (cudaStream_t)stream);
-  return tc::launch<64>(mK, mV, mX, p, Bv, (cudaStream_t)stream);
-}
-
 extern "C" int ltm_cont_attn_rect_tc(const float* q, const float* K, const float* V, int64_t ldkv, const float* X,
                                      const float* W, float W_out, float c_none, const int32_t* jb, const float* tb,
                                      float* ctx, float* scores_out, float* hist_part, int Bv, int Q, int N, int H,
                                      int d, void* stream) {
   using namespace ltm;
   LTM_REQUIRE(ltm_attn_tc_supported(N, d), "cont_attn_rect_tc: unsupported num_basis=%d / head_size=%d", N, d);
-  return cont_attn_rect_tc_impl(q, K, V, ldkv, X, W, W_out, c_none, jb, tb, ctx, scores_out, hist_part, nullptr, Bv, Q,
-                                N, H, d, stream);
+  return tc::cont_attn_rect_tc_impl<tc::KvTf32>(q, K, V, ldkv, X, W, W_out, c_none, jb, tb, ctx, scores_out, hist_part,
+                                                nullptr, Bv, Q, N, H, d, stream);
 }
 
 // num_basis 512: two work items per (query tile, head, video), merged by attn_tc_combine_kernel; the sticky
@@ -582,8 +667,33 @@ extern "C" int ltm_cont_attn_rect_tc_split(const float* q, const float* K, const
   LTM_REQUIRE(ltm_attn_tc_split_supported(N, d), "cont_attn_rect_tc_split: unsupported num_basis=%d / head_size=%d", N, d);
   LTM_REQUIRE(part_ws != nullptr && (hist_part == nullptr || scores_ws != nullptr),
               "cont_attn_rect_tc_split: workspaces missing");
-  int rc = cont_attn_rect_tc_impl(q, K, V, ldkv, X, W, W_out, 0.f, jb, tb, ctx, scores_ws, nullptr, part_ws, Bv, Q, N,
-                                  H, d, stream);
+  int rc = tc::cont_attn_rect_tc_impl<tc::KvTf32>(q, K, V, ldkv, X, W, W_out, 0.f, jb, tb, ctx, scores_ws, nullptr,
+                                                  part_ws, Bv, Q, N, H, d, stream);
+  if (rc || hist_part == nullptr) return rc;
+  return ltm_sticky_hist_rect_tiles(scores_ws, jb, tb, hist_part, Bv, H, Q, N, stream);
+}
+
+extern "C" int ltm_cont_attn_rect_tc16(const float* q, const void* K, const void* V, int64_t ldkv, const void* X,
+                                       const float* W, float W_out, float c_none, const int32_t* jb, const float* tb,
+                                       float* ctx, float* scores_out, float* hist_part, int Bv, int Q, int N, int H,
+                                       int d, void* stream) {
+  using namespace ltm;
+  LTM_REQUIRE(ltm_attn_tc_supported(N, d), "cont_attn_rect_tc16: unsupported num_basis=%d / head_size=%d", N, d);
+  return tc::cont_attn_rect_tc_impl<tc::KvF16>(q, K, V, ldkv, X, W, W_out, c_none, jb, tb, ctx, scores_out, hist_part,
+                                               nullptr, Bv, Q, N, H, d, stream);
+}
+
+extern "C" int ltm_cont_attn_rect_tc16_split(const float* q, const void* K, const void* V, int64_t ldkv,
+                                             const void* X, const float* W, float W_out, const int32_t* jb,
+                                             const float* tb, float* ctx, float* scores_ws, float* part_ws,
+                                             float* hist_part, int Bv, int Q, int N, int H, int d, void* stream) {
+  using namespace ltm;
+  LTM_REQUIRE(ltm_attn_tc_split_supported(N, d), "cont_attn_rect_tc16_split: unsupported num_basis=%d / head_size=%d",
+              N, d);
+  LTM_REQUIRE(part_ws != nullptr && (hist_part == nullptr || scores_ws != nullptr),
+              "cont_attn_rect_tc16_split: workspaces missing");
+  int rc = tc::cont_attn_rect_tc_impl<tc::KvF16>(q, K, V, ldkv, X, W, W_out, 0.f, jb, tb, ctx, scores_ws, nullptr,
+                                                 part_ws, Bv, Q, N, H, d, stream);
   if (rc || hist_part == nullptr) return rc;
   return ltm_sticky_hist_rect_tiles(scores_ws, jb, tb, hist_part, Bv, H, Q, N, stream);
 }

@@ -608,6 +608,22 @@ int tma_encode_2d(CUtensorMap* map, const float* base, unsigned long long inner,
   return 0;
 }
 
+int tma_encode_2d_f16(CUtensorMap* map, const void* base, unsigned long long inner, unsigned long long outer,
+                      unsigned long long pitch_elems, unsigned box_outer, const char* what) {
+  if (resolve_encode()) return -1;
+  LTM_REQUIRE(aligned16(base) && pitch_elems % 8 == 0 && pitch_elems >= inner && box_outer >= 1 && box_outer <= 256,
+              "%s: fp16 tensor map needs a 16-byte aligned base, a pitch that is a multiple of 8 halves, box <= 256", what);
+  cuuint64_t dims[2] = {(cuuint64_t)inner, (cuuint64_t)outer};
+  cuuint64_t strides[1] = {(cuuint64_t)pitch_elems * 2ull};
+  cuuint32_t box[2] = {64u, box_outer};
+  cuuint32_t estr[2] = {1u, 1u};
+  CUresult r = g_encode(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
+                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  LTM_REQUIRE(r == CUDA_SUCCESS, "%s: cuTensorMapEncodeTiled failed with CUresult %d", what, (int)r);
+  return 0;
+}
+
 template <int BN, int STAGES, bool SPLIT, bool HOUT = false, bool EXT = false>
 static int launch_cfg(const CUtensorMap& mA, const CUtensorMap& mB, const CUtensorMap& mB2, const GemmDev& d,
                       int batch, cudaStream_t stream) {

@@ -12,6 +12,10 @@ namespace ltm {
 int tma_encode_2d(CUtensorMap* map, const float* base, unsigned long long inner, unsigned long long outer,
                   unsigned long long pitch_elems, unsigned box_inner, unsigned box_outer, int swizzle32b_atom,
                   const char* what);
+// Host: 2-D fp16 tensor map {inner halves, outer rows} with row pitch `pitch_elems` halves, box {64, box_outer},
+// SWIZZLE_128B.
+int tma_encode_2d_f16(CUtensorMap* map, const void* base, unsigned long long inner, unsigned long long outer,
+                      unsigned long long pitch_elems, unsigned box_outer, const char* what);
 
 #ifdef __CUDACC__
 // ------------------------------------------------------------------------------------------ PTX

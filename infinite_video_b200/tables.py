@@ -143,7 +143,7 @@ class RectTables:
     W: np.ndarray = None             # fp32 [N]
     W_out: float = 0.0
     X: np.ndarray = None             # fp32 [N,32] extra operand rows of the tensor-core attention (or None)
-    X16: np.ndarray = None           # fp16 [N,64] the same table for the fp16 attention (csrc/attn_tc16.cu)
+    X16: np.ndarray = None           # fp16 [N,64] the same table for the fp16 attention (csrc/attn_tc.cu)
     c_none: float = 0.0              # trapezoid node weight of the sticky edges outside every basis
     # uniform (non-sticky) resampling table: basis index of sample s (-1 none)  (gibbs:152-157,:212)
     idx_uniform: np.ndarray = None   # int32 [S]

@@ -4,7 +4,7 @@
 # usage: scripts/ncu_all.sh [kernel-name-regex ...]
 OUT=gpurun_out
 mkdir -p $OUT
-KERNELS=${@:-"pool_mean_kernel pool_bins_kernel pool_mean_convert_kernel softmax_rows_reg_kernel resample_kernel consolidate gemm_tf32_kernel cont_attn_tc16_kernel cont_attn_tc_kernel attn_tc_combine sticky_hist_rect_kernel cont_attn_fast_kernel cont_attn_kernel sticky_hist_gauss_kernel cont_attn_g16_kernel split_half3_kernel fold_sample_columns_kernel rbf_eval_kernel gather_rows_kernel density_rect_kernel ridge"}
+KERNELS=${@:-"pool_mean_kernel pool_bins_kernel pool_mean_convert_kernel softmax_rows_reg_kernel resample_kernel consolidate gemm_tf32_kernel cont_attn_tc_kernel attn_tc_combine sticky_hist_rect_kernel cont_attn_fast_kernel cont_attn_kernel sticky_hist_gauss_kernel cont_attn_g16_kernel split_half3_kernel fold_sample_columns_kernel rbf_eval_kernel gather_rows_kernel density_rect_kernel ridge"}
 for k in $KERNELS; do
   which=rect
   case $k in sticky_hist_gauss*|rbf_eval*|gather_rows*|ridge*|cont_attn_g16*|split_half3*|fold_sample*) which=gauss;; pool_bins*) which=bins;;

@@ -48,6 +48,8 @@ CONFIGS = [
     ("fp16_chunk", {}, SMALL, "fp16", LOCKSTEP + ("ragged_step", "ragged_pool+step", "ragged_overlapped")),
     ("bf16_chunk", {}, SMALL, "bf16", LOCKSTEP + ("ragged_step", "ragged_pool+step", "ragged_overlapped")),
     ("production_fp16", {}, BIG, "fp16", LOCKSTEP[:4] + RAGGED),
+    # num_basis 512 with K|V on the tf32 grid: the fp32 two-half attention (ltm_cont_attn_rect_tc_split)
+    ("n512_kv_fp32", dict(kv_dtype="fp32"), dict(Bv=2, L=32, N=512), "fp32", LOCKSTEP + RAGGED),
 ]
 
 

@@ -69,13 +69,13 @@ def _assert_gemm_256(M, Nc, batch):
 
 
 def _attn_slots(sms, nb_item):
-    # attn_tc.cu:538 / attn_tc16.cu:535  PER_SM = (2 * Lay<NB>::BYTES <= 227 KB) ? 2 : 1 -- two CTAs per SM for 64 / 128
+    # attn_tc.cu launch()  PER_SM = (2 * Lay<NB, KV>::BYTES <= 227 KB) ? 2 : 1 -- two CTAs per SM for 64 / 128
     # bases per item (60 / 106 KB of shared memory), one for 256 (209 KB);  grid = min(items, num_sms * PER_SM)
     return sms * (2 if nb_item < 256 else 1)
 
 
 def _assert_multi_item(items, slots):
-    # attn_tc.cu:540 / attn_tc16.cu:537 / attn_g16.cu:467  grid = min(total, slots): CTA b runs items b, b + grid, ...
+    # attn_tc.cu launch() / attn_g16.cu launch()  grid = min(total, slots): CTA b runs items b, b + grid, ...
     assert items >= 2 * slots and items % slots != 0, (items, slots)
 
 
