@@ -70,10 +70,6 @@ def _as_lengths(lengths, Bv, Lmax):
     return vals
 
 
-# storage of a chunk k as the library takes it (ltm_rect_step_args.k_dtype, ltm_overlap.next_dtype)
-_CHUNK_DTYPES = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
-
-
 def _pad_rows(m):
     """Copy a 2-D matrix into storage whose row pitch is a multiple of 4 floats (TMA: 16-byte pitches)."""
     r, c = m.shape
@@ -253,7 +249,7 @@ class BatchedRectLTM(_BatchedBase):
     def _chunk_dtype(self, k, name="k"):
         """Storage code of chunk k (0 float32, 1 float16, 2 bfloat16); ValueError for any other dtype, and for a 16-bit
         chunk whose width is not a multiple of 8 (it is read as 128-bit vectors of 8 elements)."""
-        dt = _CHUNK_DTYPES.get(k.dtype)
+        dt = ops.CHUNK_DTYPES.get(k.dtype)
         if dt is None:
             raise ValueError(f"{name} must be float32, float16 or bfloat16, not {k.dtype}")
         if dt and k.shape[-1] % 8:
@@ -313,7 +309,7 @@ class BatchedRectLTM(_BatchedBase):
         if ws["xi"] in held:
             self._pref[:] = [e for e in self._pref if e["buf"] != ws["xi"]]
         ws["xtag"][ws["xi"]] = update and self._bin_ok(k.shape[0], k.shape[1] // self.T, tab,
-                                                       _CHUNK_DTYPES.get(k.dtype, 0))
+                                                       ops.CHUNK_DTYPES.get(k.dtype, 0))
         return None
 
     def _state(self, Bv, Q):
@@ -618,31 +614,13 @@ class BatchedRectLTM(_BatchedBase):
         binned = lens is None and bool(update) and self._bin_ok(Bv, L, tab, dt)
         if offs is not None:
             offs.record_stream(self._side)
-        self._pool_launch(k_next, ws["xbufs"][b], Bv, L, splits, int(self.pool_ctas), sp, offs=offs, frames=frames,
-                          bins=tab if binned else None, dtype=dt)
+        ops.pool_into(k_next, ws["xbufs"][b], L, self.T, splits, int(self.pool_ctas), sp, offs=offs, frames=frames,
+                      fbin_ptr=tab.to(self.device)["fbin_ptr"] if binned else None, rows=tab.xb_rows)
         if events is not None:
             check(lib().ltm_event_record(events[1], sp), "event_record")
         check(lib().ltm_event_record(ev["pooled"][b], sp), "event_record")
         self._pref.append(dict(ref=weakref.ref(k_next), ver=k_next._version, buf=b, event=ev["pooled"][b],
                                captured=torch.cuda.is_current_stream_capturing(), binned=binned, lens=lens))
-
-    def _pool_launch(self, k, out, Bv, L, splits, max_ctas, stream, offs=None, frames=0, bins=None, dtype=0):
-        """Pool chunk k[Bv, L*T, e] into `out` on `stream`: the packed frames of a ragged chunk (offs: device frame
-        offsets, `frames` in all), the per-bin sums of an update chunk (bins: its tables; float32 only) or per-frame
-        means.  dtype 0 / 1 / 2: float32 / float16 / bfloat16 storage.  max_ctas bounds the grid (0 = one CTA per
-        unit)."""
-        if offs is not None:
-            check(lib().ltm_pool_mean_ragged(ptr(k), dtype, ptr(out), ptr(offs), Bv, L, self.T, self.e, splits, frames,
-                                             max_ctas, stream), "pool_mean_ragged")
-        elif bins is not None:
-            check(lib().ltm_pool_bins(ptr(k), ptr(out), ptr(bins.to(self.device)["fbin_ptr"]), Bv, L, self.T, self.e,
-                                      bins.xb_rows, stream), "pool_bins")
-        elif dtype:
-            check(lib().ltm_pool_mean_16_grid(ptr(k), int(dtype == 2), ptr(out), Bv, L, self.T, self.e, splits,
-                                              max_ctas, stream), "pool_mean_16_grid")
-        else:
-            check(lib().ltm_pool_mean_grid(ptr(k), ptr(out), Bv, L, self.T, self.e, splits, max_ctas, stream),
-                  "pool_mean")
 
     def _sync_events(self):
         if self._evs is None:
@@ -707,8 +685,7 @@ class BatchedRectLTM(_BatchedBase):
             raise ValueError(f"k must be [Bv, L*{self.T}, {self.e}]")
         L = LT // self.T
         if lengths is not None:
-            dtype = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}.get(k.dtype)
-            if dtype is None or (with_half and dtype != 0):
+            if k.dtype not in ops.CHUNK_DTYPES or (with_half and k.dtype != torch.float32):
                 raise ValueError("a ragged chunk is pooled from float32 / float16 / bfloat16 storage (with_half: float32)")
             lens = _as_lengths(lengths, Bv, L)
             frames = sum(lens)
@@ -718,8 +695,7 @@ class BatchedRectLTM(_BatchedBase):
                                                     (LT + 63) // 64 * 64)
             out = torch.empty(frames, splits, e, device=self.device, dtype=torch.float32)
             if frames:
-                self._pool_launch(k, out, Bv, L, splits, 0, stream_ptr(self.device), offs=self._lengths_dev(lens)[1],
-                                  frames=frames, dtype=dtype)
+                ops.pool_into(k, out, L, self.T, splits, offs=self._lengths_dev(lens)[1], frames=frames)
             return out
         if with_half:
             x, k16 = ops.pool_mean_convert(k.view(Bv, L, self.T, e), self._splits(Bv * L))

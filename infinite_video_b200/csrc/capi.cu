@@ -55,11 +55,9 @@ static int check_chunk_dtype(const char* who, const char* field, int dtype, int 
 // by check_chunk_dtype.  max_ctas bounds the grid (0 = one CTA per unit).
 static int pool_chunk(const ltm_rect_step_args* a, const void* k, int dtype, float* xpart, const int32_t* offs,
                       int frames, int splits, bool binned, int max_ctas, void* stream) {
-  if (offs)
-    return ltm_pool_mean_ragged(k, dtype, xpart, offs, a->Bv, a->L, a->T, a->e, splits, frames, max_ctas, stream);
-  if (binned) return ltm_pool_bins((const float*)k, xpart, a->fbin_ptr, a->Bv, a->L, a->T, a->e, a->xb_rows, stream);
-  if (dtype) return ltm_pool_mean_16_grid(k, dtype == 2, xpart, a->Bv, a->L, a->T, a->e, splits, max_ctas, stream);
-  return ltm_pool_mean_grid((const float*)k, xpart, a->Bv, a->L, a->T, a->e, splits, max_ctas, stream);
+  LTM_REQUIRE(!binned || a->fbin_ptr, "frame pooling: per-bin pooling without fbin_ptr");
+  return ltm::pool_frames("frame pooling", k, dtype, xpart, a->Bv, a->L, a->T, a->e, binned ? 1 : splits, max_ctas,
+                          stream, offs, frames, nullptr, 0, binned ? a->fbin_ptr : nullptr, a->xb_rows);
 }
 
 // ------------------------------------------------------------------------------------------------

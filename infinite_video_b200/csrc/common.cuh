@@ -39,6 +39,16 @@ void set_error(const char* fmt, ...);
 
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
+// Frame pooling behind every ltm_pool_* entry point and the step: checks the arguments (`who` names the caller in the
+// error text), picks the kernel, thread count and grid.  k[Bv, L, T, e], dtype 0 fp32, 1 fp16, 2 bfloat16, is pooled
+// into xpart as the frame means in `splits` partial sums, [Bv*L, splits, e]; offs != NULL: only the `frames` frames of
+// a ragged chunk (ltm_pool_mean_ragged), packed; fbin_ptr != NULL: the per-bin sums [Bv, rows, e] instead
+// (ltm_pool_bins); k16 != NULL: the chunk as fp16 as well (ltm_pool_mean_convert, ld16 rows per video when ragged).
+// max_ctas > 0 bounds the grid of the per-frame means (0 = one CTA per (frame, token-split)).
+int pool_frames(const char* who, const void* k, int dtype, float* xpart, int Bv, int L, int T, int e, int splits,
+                int max_ctas, void* stream, const int32_t* offs = nullptr, int frames = 0, void* k16 = nullptr,
+                int ld16 = 0, const int32_t* fbin_ptr = nullptr, int rows = 0);
+
 // ---- ragged batches (ltm_rect_step_args.lengths), internal to the library
 // ltm_consolidate_rect_kv with per-video lengths (0 = idle) and frame offsets; NULL lengths = lock-step
 int consolidate_rect_ragged(const float* B_past, const float* xpart, const int32_t* idx, int64_t idx_stride,

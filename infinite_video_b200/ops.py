@@ -29,18 +29,39 @@ def _rowmajor(t):
     return t
 
 
+# storage of a chunk k as the library takes it (ltm_rect_step_args.k_dtype, ltm_overlap.next_dtype)
+CHUNK_DTYPES = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
+
+
+def pool_into(k, out, L, T, splits, max_ctas=0, stream=None, offs=None, frames=0, fbin_ptr=None, rows=0):
+    """Frame pooling of a contiguous chunk k of Bv videos of L frames of T tokens of width e (float32 / float16 /
+    bfloat16) into `out`, on `stream` (default: torch's current stream).  With offs (int32 [Bv+1] device frame
+    offsets, `frames` in all): the packed frames of a ragged chunk, [frames, splits, e].  With fbin_ptr (float32
+    chunks, tables.RectTables.fbin_ptr): the per-bin sums of an update chunk, [Bv, rows, e].  Otherwise the frame
+    means as `splits` partial sums, [Bv, L, splits, e].  max_ctas > 0 bounds the grid (0: one CTA per frame-split)."""
+    Bv, e = k.shape[0], k.shape[-1]
+    dt = CHUNK_DTYPES[k.dtype]
+    st = stream_ptr(k.device) if stream is None else stream
+    if offs is not None:
+        check(lib().ltm_pool_mean_ragged(ptr(k), dt, ptr(out), ptr(offs), Bv, L, T, e, splits, frames, max_ctas, st),
+              "pool_mean_ragged")
+    elif fbin_ptr is not None:
+        check(lib().ltm_pool_bins(ptr(k), ptr(out), ptr(fbin_ptr), Bv, L, T, e, rows, st), "pool_bins")
+    elif dt:
+        check(lib().ltm_pool_mean_16_grid(ptr(k), int(dt == 2), ptr(out), Bv, L, T, e, splits, max_ctas, st),
+              "pool_mean_16_grid")
+    else:
+        check(lib().ltm_pool_mean_grid(ptr(k), ptr(out), Bv, L, T, e, splits, max_ctas, st), "pool_mean")
+
+
 def pool_mean(k, splits=1):
     """k[Bv,L,T,e] -> xpart[Bv,L,splits,e] (frame means as `splits` partial sums).  gibbs:304."""
     require_cuda(k)
     Bv, L, T, e = k.shape
     out = torch.empty(Bv, L, splits, e, device=k.device, dtype=torch.float32)
-    if k.dtype in (torch.float16, torch.bfloat16):        # 16-bit chunk: read as is, accumulate in fp32
-        k = k.contiguous()
-        check(lib().ltm_pool_mean_16(ptr(k), int(k.dtype == torch.bfloat16), ptr(out), Bv, L, T, e, splits,
-                                     stream_ptr(k.device)), "pool_mean_16")
-        return out
-    k = _f32c(k)
-    check(lib().ltm_pool_mean(ptr(k), ptr(out), Bv, L, T, e, splits, stream_ptr(k.device)), "pool_mean")
+    # a 16-bit chunk is read as is and accumulated in fp32
+    k = k.contiguous() if k.dtype in (torch.float16, torch.bfloat16) else _f32c(k)
+    pool_into(k, out, L, T, splits)
     return out
 
 
@@ -78,7 +99,7 @@ def pool_bins(k, fbin_ptr, rows):
     k = _f32c(k)
     Bv, L, T, e = k.shape
     out = torch.empty(Bv, rows, e, device=k.device, dtype=torch.float32)
-    check(lib().ltm_pool_bins(ptr(k), ptr(out), ptr(fbin_ptr), Bv, L, T, e, rows, stream_ptr(k.device)), "pool_bins")
+    pool_into(k, out, L, T, 1, fbin_ptr=fbin_ptr, rows=rows)
     return out
 
 

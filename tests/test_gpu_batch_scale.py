@@ -519,7 +519,7 @@ def test_pool_mean_bounded_grid(dev, splits):
     units = Bv * L * splits
     full = ops.pool_mean(k, splits)
     for max_ctas in (7, 296):
-        # pool.cu:280  max_ctas > 0 && max_ctas < units -> pool_mean_persistent_kernel
+        # pool.cu:307  max_ctas > 0 && max_ctas < units -> pool_mean_kernel<F32, LockStep, true>
         assert 0 < max_ctas < units and units % max_ctas != 0
         out = torch.full_like(full, SENT)
         ca.check(ca.lib().ltm_pool_mean_grid(ca.ptr(k), ca.ptr(out), Bv, L, T_, e, splits, max_ctas,
