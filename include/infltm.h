@@ -70,6 +70,15 @@ int ltm_pool_mean_16_grid(const void* k, int is_bf16, float* xpart, int Bv, int 
  * dtype: 0 fp32, 1 fp16, 2 bfloat16 (16-bit: e % 8 == 0, ltm_pool_mean_16's summation). */
 int ltm_pool_mean_ragged(const void* k, int dtype, float* xpart, const int32_t* offs, int Bv, int L, int T, int e,
                          int splits, int frames, int max_ctas, void* stream);
+/* ltm_pool_mean_ragged with each video's chunk at its own address: ptrs[Bv] (device) holds the base address of video
+ * v's tokens, and frame l of video v is read at ptrs[v] + l*T*e elements, for l < offs[v+1] - offs[v].  The videos may
+ * be separate tensors, views into one tensor holding a whole video, or views into one packed tensor; nothing is copied
+ * into a padded chunk first.  xpart[frames, splits, e] is bit-identical to ltm_pool_mean_ragged over the same frames.
+ * The caller guarantees what the library cannot check without reading the table: the pointer of every video with
+ * frames is 16-byte aligned and its lengths[v]*T rows of e elements are dense (row pitch e).  The pointers of idle
+ * videos are not read.  dtype, e, splits and max_ctas as ltm_pool_mean_ragged. */
+int ltm_pool_mean_ptrs(const void* const* ptrs, int dtype, float* xpart, const int32_t* offs, int Bv, int L, int T,
+                       int e, int splits, int frames, int max_ctas, void* stream);
 /* ragged twin of ltm_pool_mean_convert (fp32 chunk k[Bv, L, T, e], lengths as offs[Bv+1] above): xpart as
  * ltm_pool_mean_ragged writes it for the same splits, and the chunk as IEEE fp16 padded per video,
  * k16[Bv, ld16, e] (ld16 % 64 == 0, ld16 >= L*T): with n_v = lengths[v]*T, tokens [0, n_v) of video v hold the
@@ -394,6 +403,11 @@ typedef struct {
    * A 16-bit chunk (e % 8 == 0) is pooled per frame from its own storage with fp32 accumulation, in the summation
    * order of ltm_pool_mean_16 (lock-step) or ltm_pool_mean_ragged (ragged); it is never pooled per bin (binned == 0). */
   int k_dtype;
+  /* chunk given per video (NULL = off): k_ptrs[Bv] (device) holds the base address of video v's tokens, pooled as
+   * ltm_pool_mean_ptrs pools them; the ragged fields above must be set (lengths, frame_offs, frames) and k must be
+   * NULL.  Not with binned.  The step pools the chunk from the table whenever it is set (ltm_rect_step_overlap: on the
+   * compute stream, before the rest of the step). */
+  const void* const* k_ptrs;
 } ltm_rect_step_args;
 int ltm_rect_step(const ltm_rect_step_args* a, const void* k, const float* q, const double* u,
                   const uint8_t* new_doc, float* ctx, void* stream);
@@ -407,7 +421,7 @@ int ltm_rect_step_host(const ltm_rect_step_args* a, const void* k_host, const fl
  *   main:     wait(compute)
  * Frame pooling does not depend on the memory state and is the HBM-bound 93 % of a call's bytes; the other kernels
  * are tensor- / latency-bound.  Streams and (timing-disabled) events are the caller's; the events are re-recorded
- * on every call.  k_next == NULL issues no pooling; ev_pooled_cur == NULL waits for nothing.  The pooling of the
+ * on every call.  k_next == next_ptrs == NULL issues no pooling; ev_pooled_cur == NULL waits for nothing.  The pooling of the
  * next chunk is bracketed by a->prof_events[0,1] when those are set. */
 typedef struct {
   void *main_stream, *side_stream, *compute_stream;
@@ -418,6 +432,9 @@ typedef struct {
    * to args.L frames) into xpart_next packed as [next_frames, next_splits, e] (ltm_pool_mean_ragged) */
   const int32_t* next_lengths; const int32_t* next_offs; int next_frames; int next_splits;
   int next_dtype;      /* storage of k_next, as ltm_rect_step_args.k_dtype (16-bit: next_binned == 0) */
+  /* next chunk given per video, as ltm_rect_step_args.k_ptrs (NULL = off): needs next_lengths / next_offs, k_next must
+   * be NULL and next_binned 0 */
+  const void* const* next_ptrs;
 } ltm_overlap;
 int ltm_rect_step_overlap(const ltm_rect_step_args* a, const ltm_overlap* o, const float* q, const double* u,
                           const uint8_t* new_doc, float* ctx);

@@ -64,6 +64,7 @@ class RectStepArgs(C.Structure):
         ("bank_seg_ptr1", C.c_void_p), ("bank_seg_mem1", C.c_void_p), ("bank_g1", C.c_void_p),
         ("hist_keep", C.c_void_p),
         ("k_dtype", C.c_int),
+        ("k_ptrs", C.c_void_p),
     ]
 
 
@@ -76,6 +77,7 @@ class Overlap(C.Structure):
         ("next_binned", C.c_int),
         ("next_lengths", C.c_void_p), ("next_offs", C.c_void_p), ("next_frames", C.c_int), ("next_splits", C.c_int),
         ("next_dtype", C.c_int),
+        ("next_ptrs", C.c_void_p),
     ]
 
 
@@ -94,6 +96,7 @@ _SIGS = {
     "ltm_pool_mean_16_grid": (C.c_int, [_P, _I, _P, _I, _I, _I, _I, _I, _I, _P]),
     "ltm_pool_mean_grid": (C.c_int, [_P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "ltm_pool_mean_ragged": (C.c_int, [_P, _I, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "ltm_pool_mean_ptrs": (C.c_int, [_P, _I, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "ltm_pool_mean_convert_ragged": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "ltm_sticky_hist_rect": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "ltm_sticky_hist_rect_tiles": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),

@@ -70,6 +70,31 @@ def _as_lengths(lengths, Bv, Lmax):
     return vals
 
 
+class _Entries:
+    """A chunk given per video (see `BatchedRectLTM.step`), validated: the entries (None = idle), their lengths in
+    frames, the storage code of the present ones, their base addresses, one entry per distinct storage (the tensors to
+    `record_stream` on a stream that reads them) and `shape` = (Bv, L*T, e), the padded chunk it stands for."""
+    __slots__ = ("entries", "lens", "code", "ptrs", "stores", "shape")
+
+
+def _chunk_refs(k):
+    """Identity of a chunk for prefetch matching: per tensor (one for a padded chunk, one per entry of a list) a weak
+    reference and its version counter.  A data pointer is not a key: the caching allocator hands the same address to
+    the next chunk, and an in-place write changes the contents behind an unchanged pointer."""
+    ts = k.entries if isinstance(k, _Entries) else (k,)
+    return tuple(None if t is None else (weakref.ref(t), t._version) for t in ts)
+
+
+def _refs_match(refs, k):
+    ts = k.entries if isinstance(k, _Entries) else (k,)
+    return len(refs) == len(ts) and all(
+        (t is None) if r is None else (t is not None and r[0]() is t and r[1] == t._version) for r, t in zip(refs, ts))
+
+
+def _refs_alive(refs):
+    return all(r is None or r[0]() is not None for r in refs)
+
+
 def _pad_rows(m):
     """Copy a 2-D matrix into storage whose row pitch is a multiple of 4 floats (TMA: 16-byte pitches)."""
     r, c = m.shape
@@ -256,6 +281,52 @@ class BatchedRectLTM(_BatchedBase):
             raise ValueError(f"a 16-bit {name} needs a width that is a multiple of 8, not {k.shape[-1]}")
         return dt
 
+    def _entries(self, k, chunk_frames, lengths=None, name="k"):
+        """A chunk given as a list of Bv entries (see `step`) -> `_Entries`; a tensor (or an `_Entries`) is returned
+        as it is.  Every entry is checked before any state changes, and nothing is copied: a silent `.contiguous()`
+        would bring back the copy this form exists to avoid, and break prefetch matching."""
+        if not isinstance(k, (list, tuple)):
+            if chunk_frames is not None and not isinstance(k, _Entries):
+                raise ValueError(f"chunk_frames applies to a chunk given as a list, and {name} is a tensor")
+            return k
+        if lengths is not None:
+            raise ValueError(f"{name} given as a list carries its own lengths: do not pass lengths as well")
+        if chunk_frames is None:
+            raise ValueError(f"{name} given as a list needs chunk_frames= (the padded chunk length L)")
+        L, T, e = int(chunk_frames), self.T, self.e
+        if L < 2 or not k:
+            raise ValueError(f"{name} given as a list needs chunk_frames >= 2 and at least one entry")
+        lens, ptrs, stores, dtype = [], [], {}, None
+        for v, t in enumerate(k):
+            if t is None:
+                lens.append(0)
+                ptrs.append(0)
+                continue
+            if not isinstance(t, torch.Tensor) or t.device != self.device:
+                raise ValueError(f"{name}[{v}] must be None or a tensor on {self.device}")
+            if dtype is None:
+                dtype = t.dtype
+                code = self._chunk_dtype(t, f"{name}[{v}]")
+            elif t.dtype != dtype:
+                raise ValueError(f"{name}[{v}] is {t.dtype}, the entries before it {dtype}: one dtype per chunk")
+            if t.dim() != 2 or t.shape[1] != e:
+                raise ValueError(f"{name}[{v}] must be [n*{T}, {e}], not {list(t.shape)}")
+            n = t.shape[0]
+            if n % T or not 2 <= n // T <= L:
+                raise ValueError(f"{name}[{v}] has {n} tokens: a multiple of {T} for 2 to {L} frames (None = idle)")
+            if t.stride() != (e, 1):
+                raise ValueError(f"{name}[{v}] must have dense rows, strides ({e}, 1), not {t.stride()}")
+            p = t.data_ptr()
+            if p % 16:
+                raise ValueError(f"{name}[{v}] must start at a 16-byte aligned address")
+            lens.append(n // T)
+            ptrs.append(p)
+            stores.setdefault(t.untyped_storage().data_ptr(), t)
+        c = _Entries()
+        c.entries, c.lens, c.code, c.ptrs = tuple(k), tuple(lens), (code if dtype is not None else 0), ptrs
+        c.stores, c.shape = tuple(stores.values()), (len(k), L * T, e)
+        return c
+
     def reset(self):
         """Forget every video (new_doc for all) and every pending prefetch."""
         super().reset()
@@ -266,19 +337,18 @@ class BatchedRectLTM(_BatchedBase):
         """Drop the chunks pooled ahead of time that were never consumed by a `step`."""
         self._pref.clear()
 
-    # pending prefetches are identified by the tensor OBJECT (weak reference) and its version counter: a data pointer
-    # is not a key, the caching allocator hands the same address to the next chunk (and an in-place write changes
-    # the contents behind an unchanged pointer)
+    # pending prefetches are identified by the tensor OBJECTS (weak references) and their version counters
+    # (`_chunk_refs`), and by the lengths
     def _pref_take(self, k, lens=None):
         for i, ent in enumerate(self._pref):
-            if ent["ref"]() is k and ent["ver"] == k._version and ent["lens"] == lens:
+            if ent["lens"] == lens and _refs_match(ent["refs"], k):
                 return self._pref.pop(i)
         return None
 
     def _pref_buffer(self, ws):
         """Buffer for the next prefetch: one that no pending prefetch holds, preferably not the one the most recent
         step consumes.  An abandoned prefetch (tensor gone, or never stepped) is evicted, oldest first."""
-        self._pref[:] = [e for e in self._pref if e["ref"]() is not None]
+        self._pref[:] = [e for e in self._pref if _refs_alive(e["refs"])]
         while len(self._pref) >= 2:
             self._pref.pop(0)
         held = {e["buf"] for e in self._pref}
@@ -298,7 +368,10 @@ class BatchedRectLTM(_BatchedBase):
         if hit is not None and hit["binned"] and not update:
             hit = None                                   # pooled per bin for an update that did not come: pool again
         if hit is None and prefetch:
-            self.prefetch(k, Q, lengths=lens, update=update)
+            if isinstance(k, _Entries):
+                self.prefetch(k, Q)
+            else:
+                self.prefetch(k, Q, lengths=lens, update=update)
             hit = self._pref_take(k, lens)
         if hit is not None:
             ws["xi"] = hit["buf"]
@@ -343,7 +416,7 @@ class BatchedRectLTM(_BatchedBase):
         a.B_new = self._B[1 - self._cur].data_ptr()
         a.xpart = ws["xbufs"][ws["xi"]].data_ptr()
         a.binned = 1 if ws["xtag"][ws["xi"]] else 0
-        a.k_dtype = k_dtype
+        a.k_dtype, a.k_ptrs = k_dtype, None
         # (only where the pooling is the long pole of the step: a chunk of at least 16 tokens per basis function; with
         # 8 frames x 32 tokens on 64 bins the chain of this stream is, and a narrower projection would lengthen it)
         bound = beside_pool and L * self.T >= self.gemm_ctas_min_ratio * self.N
@@ -415,7 +488,7 @@ class BatchedRectLTM(_BatchedBase):
             setattr(a, f, ws[n].data_ptr() if ws[n] is not None else None)
         return a
 
-    def _prepare(self, k, q, new_doc, u, lengths=None, pooled=None, u_name="u"):
+    def _prepare(self, k, q, new_doc, u, lengths=None, pooled=None, u_name="u", ptrs=None):
         """Host side of a step: validation, per-slot bookkeeping, tables.  Every ValueError fires before any state
         changes.  Returns (Bv, L, Q, tab, tdev, flags, u, rag): the device new_doc flags the step applies (None: none),
         the contiguous uniforms (None: the step reads none) and, for a ragged step, its table bank and device lengths /
@@ -496,8 +569,9 @@ class BatchedRectLTM(_BatchedBase):
             if getattr(self, "_hist_keep", None) is None or self._hist_keep.shape != self._hist.shape:
                 self._hist_keep = torch.empty_like(self._hist)
             hist_keep = self._hist_keep
-        lens_dev, offs_dev = self._lengths_dev(ln)
-        rag = dict(lens=tuple(ln.tolist()), lens_dev=lens_dev, offs_dev=offs_dev, bank=bdev, frames=frames,
+        lens_dev, offs_dev, ptrs_dev = self._lengths_dev(ln, ptrs)
+        rag = dict(lens=tuple(ln.tolist()), lens_dev=lens_dev, offs_dev=offs_dev, ptrs_dev=ptrs_dev, bank=bdev,
+                   frames=frames,
                    splits=self._splits(frames), n_idle=n_idle,
                    jf=int(bank.jf[ln[cont]].min()) if (keep and cont.any()) else self.N, hist_keep=hist_keep,
                    slots=np.where(nd, present, mem))
@@ -514,14 +588,19 @@ class BatchedRectLTM(_BatchedBase):
             bank = self._banks[L] = tables.RectBank(L, self.N, self.tau, self.S, spacing=self.spacing)
         return bank
 
-    def _lengths_dev(self, lens):
-        """(lengths [Bv], exclusive prefix sum [Bv+1]): int32 views of one device buffer, copied on the current stream."""
+    def _lengths_dev(self, lens, ptrs=None):
+        """(lengths [Bv], exclusive prefix sum [Bv+1], pointer table [Bv] or None): views of one device buffer, copied
+        on the current stream in one upload -- the int64 entry addresses of a list chunk, then the int32 lengths and
+        offsets."""
         Bv = len(lens)
-        host = np.zeros(2 * Bv + 1, np.int32)
-        host[:Bv] = lens
-        np.cumsum(host[:Bv], out=host[Bv + 1:])
+        p = 0 if ptrs is None else 2 * Bv
+        host = np.zeros(p + 2 * Bv + 1, np.int32)
+        if ptrs is not None:
+            host[:p].view(np.int64)[:] = ptrs
+        host[p:p + Bv] = lens
+        np.cumsum(host[p:p + Bv], out=host[p + Bv + 1:])
         t = torch.from_numpy(host).pin_memory().to(self.device, non_blocking=True)
-        return t[:Bv], t[Bv:]
+        return t[p:p + Bv], t[p + Bv:], (t[:p] if ptrs is not None else None)
 
     def _ragged_ws(self, ws, Bv, L):
         """Packed pooled frames of a ragged step take sum(lengths) * splits rows: at most Bv * L (one split) or, when
@@ -564,7 +643,7 @@ class BatchedRectLTM(_BatchedBase):
         self.last = dict(b=ws["b_draw"], ts=ws["ts"], idx=ws["idx"], p=ws["p"], scores=ws["scores"], V=V, KV=kv)
 
     @_on_device
-    def prefetch(self, k_next, Q, lengths=None, events=None, update=False):
+    def prefetch(self, k_next, Q, lengths=None, events=None, update=False, chunk_frames=None):
         """Pool the frames of the NEXT chunk now, on a side stream, into the alternate buffer.
         `update=True`: the chunk will continue every video (no new_doc), so it may be pooled per bin (`bin_pool`); a
         step that turns out to start a new document pools it again.  `lengths`: the chunk is ragged (see `step`); the
@@ -573,22 +652,29 @@ class BatchedRectLTM(_BatchedBase):
         Frame pooling (gibbs:304) does not depend on the memory state, and it is the HBM-bound 93 % of a
         call's bytes, while regression / projection / attention of the current chunk are compute-bound; issuing
         it one chunk ahead lets the two overlap.  The following `step(k_next, ...)` must pass the same tensor.
-        A 16-bit chunk (float16 / bfloat16) is pooled per frame from its own storage, never per bin."""
-        require_cuda(k_next)
-        dt = self._chunk_dtype(k_next, "k_next")
-        if not k_next.is_contiguous():
-            raise ValueError("prefetch needs a contiguous chunk (the following step must be given the same tensor)")
+        A 16-bit chunk (float16 / bfloat16) is pooled per frame from its own storage, never per bin.
+        `k_next` may be a list of per-video entries with `chunk_frames` (see `step`); the step that consumes it must
+        be handed the same tensor objects."""
+        k_next = self._entries(k_next, chunk_frames, lengths, "k_next")
+        lst = isinstance(k_next, _Entries)
+        if lst:
+            dt, lengths = k_next.code, k_next.lens
+        else:
+            require_cuda(k_next)
+            dt = self._chunk_dtype(k_next, "k_next")
+            if not k_next.is_contiguous():
+                raise ValueError("prefetch needs a contiguous chunk (the following step must be given the same tensor)")
         Bv, LT, e = k_next.shape
         if e != self.e or LT % self.T:
             raise ValueError(f"k_next must be [Bv, L*{self.T}, {self.e}]")
         L = LT // self.T
         lens = None if lengths is None else _as_lengths(lengths, Bv, L)
         ws = self._workspace(Bv, L, Q)
-        offs = None
+        offs = table = None
         frames, splits = 0, ws["splits"]
         if lens is not None:
             self._ragged_ws(ws, Bv, L)
-            offs = self._lengths_dev(lens)[1]
+            _, offs, table = self._lengths_dev(lens, k_next.ptrs if lst else None)
             frames = sum(lens)
             splits = self._splits(frames)
         if self._side is None:
@@ -607,19 +693,23 @@ class BatchedRectLTM(_BatchedBase):
         # those per chunk-step the host enqueue time of a step varied between 0.9 and 8 ms from run to run
         check(lib().ltm_event_record(ev["fork_pool"][b], mp), "event_record")
         check(lib().ltm_stream_wait_event(sp, ev["fork_pool"][b]), "stream_wait_event")
-        k_next.record_stream(self._side)
+        for t in (k_next.stores if lst else (k_next,)):
+            t.record_stream(self._side)
         if events is not None:
             check(lib().ltm_event_record(events[0], sp), "event_record")
         tab = tables.rect_tables(L, self.N, self.tau, self.S, spacing=self.spacing)
         binned = lens is None and bool(update) and self._bin_ok(Bv, L, tab, dt)
         if offs is not None:
-            offs.record_stream(self._side)
-        ops.pool_into(k_next, ws["xbufs"][b], L, self.T, splits, int(self.pool_ctas), sp, offs=offs, frames=frames,
-                      fbin_ptr=tab.to(self.device)["fbin_ptr"] if binned else None, rows=tab.xb_rows)
+            offs.record_stream(self._side)          # (the table shares its buffer)
+        if lst:
+            ops.pool_ptrs(table, dt, ws["xbufs"][b], offs, Bv, L, self.T, e, splits, frames, int(self.pool_ctas), sp)
+        else:
+            ops.pool_into(k_next, ws["xbufs"][b], L, self.T, splits, int(self.pool_ctas), sp, offs=offs, frames=frames,
+                          fbin_ptr=tab.to(self.device)["fbin_ptr"] if binned else None, rows=tab.xb_rows)
         if events is not None:
             check(lib().ltm_event_record(events[1], sp), "event_record")
         check(lib().ltm_event_record(ev["pooled"][b], sp), "event_record")
-        self._pref.append(dict(ref=weakref.ref(k_next), ver=k_next._version, buf=b, event=ev["pooled"][b],
+        self._pref.append(dict(refs=_chunk_refs(k_next), buf=b, event=ev["pooled"][b],
                                captured=torch.cuda.is_current_stream_capturing(), binned=binned, lens=lens))
 
     def _sync_events(self):
@@ -666,7 +756,7 @@ class BatchedRectLTM(_BatchedBase):
         return ops.density_rect(sc, td["jd"], td["wd"])
 
     @_on_device
-    def pool(self, k, with_half=False, lengths=None):
+    def pool(self, k, with_half=False, lengths=None, chunk_frames=None):
         """Frame pooling alone (gibbs:304): k[Bv, L*T, e] -> pooled frames [Bv, L, splits, e].  The result can be
         handed to `step(..., pooled=...)` of SEVERAL engines: every LTM layer of a Q-former receives the same
         `encoder_hidden_states` per chunk (2 layers in Video-LLaMA, 6 in VideoChat2; SURVEY section 8f N2), so the
@@ -677,7 +767,21 @@ class BatchedRectLTM(_BatchedBase):
         result is packed video after video, [sum(lengths), splits, e] with splits = `_splits(sum(lengths))`, and is
         handed to `step(..., pooled=..., lengths=...)` with the same lengths.  With `with_half` (fp32 chunks) it comes
         with k16[Bv, ld16, e], ld16 = L*T rounded up to 64 tokens: video v's first n_v = lengths[v]*T tokens as fp16,
-        zeros up to roundup64(n_v), the rest unwritten (ltm_pool_mean_convert_ragged)."""
+        zeros up to roundup64(n_v), the rest unwritten (ltm_pool_mean_convert_ragged).
+        `k` may be a list of per-video entries with `chunk_frames` (see `step`): the packed frames as for `lengths`,
+        read from each entry where it lives (no `with_half`)."""
+        k = self._entries(k, chunk_frames, lengths)
+        if isinstance(k, _Entries):
+            if with_half:
+                raise ValueError("with_half: a chunk given as a list is pooled without the fp16 copy")
+            Bv, LT, e = k.shape
+            frames = sum(k.lens)
+            splits = self._splits(frames)
+            out = torch.empty(frames, splits, e, device=self.device, dtype=torch.float32)
+            if frames:
+                _, offs, table = self._lengths_dev(k.lens, k.ptrs)
+                ops.pool_ptrs(table, k.code, out, offs, Bv, LT // self.T, self.T, e, splits, frames)
+            return out
         require_cuda(k)
         k = k.contiguous()
         Bv, LT, e = k.shape
@@ -703,7 +807,7 @@ class BatchedRectLTM(_BatchedBase):
         return ops.pool_mean(k.view(Bv, L, self.T, e), self._splits(Bv * L))
 
     @_on_device
-    def step(self, k, q, u=None, new_doc=False, pooled=None, beside_pooling=False, lengths=None):
+    def step(self, k, q, u=None, new_doc=False, pooled=None, beside_pooling=False, lengths=None, chunk_frames=None):
         """k[Bv, L*T, e] float32 / float16 / bfloat16 (16-bit: e % 8 == 0, pooled per frame from its own storage),
         q[Bv,Q,D] float32, CUDA; u[Bv,S] fp64 uniforms (needed from the second chunk on when
         sticky); new_doc: bool or per-video flags; pooled: result of `pool(k)` (then `k` is only used for its
@@ -714,13 +818,23 @@ class BatchedRectLTM(_BatchedBase):
         its padded chunk (the rest is never read and may hold anything); lengths[v] == 0 leaves video v idle: its
         memory is kept bit for bit, its row of u is not read and its ctx rows are zero (with new_doc[v] the slot is
         cleared instead).  new_doc is then a bool or host flags; a slot without memory must receive new_doc with its
-        first chunk.  Passing lengths always takes the ragged kernels, even when all lengths are equal."""
-        require_cuda(k, q, u)
-        kdt = self._chunk_dtype(k) if pooled is None else 0       # (with `pooled`, k only gives the shape)
+        first chunk.  Passing lengths always takes the ragged kernels, even when all lengths are equal.
+
+        k as a list (per-video chunks, no padded copy): Bv entries, each None (the slot is idle, length 0) or a CUDA
+        tensor [n_v*T, e] with 2 <= n_v <= chunk_frames, dense rows (strides (e, 1)) and a 16-byte aligned start --
+        separate tensors, chunk views of whole-video tensors (`video.split_videos`) or views into one packed tensor.
+        The present entries share one dtype (float32 / float16 / bfloat16).  chunk_frames (required) is the padded
+        length L that selects the tables and workspace; the lengths follow from the entries (passing `lengths` too is
+        a ValueError).  Everything else is the ragged step above, bit for bit: each frame is pooled where it lives."""
+        k = self._entries(k, chunk_frames, lengths)
+        lst = isinstance(k, _Entries)
+        require_cuda(q, u, None if lst else k)
+        kdt = (k.code if lst else self._chunk_dtype(k)) if pooled is None else 0   # (with `pooled`, k gives the shape)
         if q.dtype != torch.float32:
             raise ValueError("q must be float32")
-        k, q = k.contiguous(), q.contiguous()
-        Bv, L, Q, tab, tdev, flags, u, rag = self._prepare(k, q, new_doc, u, lengths, pooled)
+        k, q = (k if lst else k.contiguous()), q.contiguous()
+        Bv, L, Q, tab, tdev, flags, u, rag = self._prepare(k, q, new_doc, u, k.lens if lst else lengths, pooled,
+                                                           ptrs=k.ptrs if lst else None)
         ws = self._workspace(Bv, L, Q)
         if rag is not None:
             self._ragged_ws(ws, Bv, L)
@@ -746,8 +860,10 @@ class BatchedRectLTM(_BatchedBase):
         if rag is not None and run is not main:
             rag["lens_dev"].record_stream(run)
         pool_here = pooled is None and hit is None
-        check(lib().ltm_rect_step(C.byref(a), ptr(k) if pool_here else None, ptr(q), ptr(u), ptr(flags), ptr(ctx),
-                                  C.c_void_p(run.cuda_stream)), "rect_step")
+        if pool_here and lst:
+            a.k_ptrs = rag["ptrs_dev"].data_ptr()
+        check(lib().ltm_rect_step(C.byref(a), ptr(k) if pool_here and not lst else None, ptr(q), ptr(u), ptr(flags),
+                                  ptr(ctx), C.c_void_p(run.cuda_stream)), "rect_step")
         if hit is not None:
             check(lib().ltm_event_record(ev["join"], rp), "event_record")
             check(lib().ltm_stream_wait_event(mp, ev["join"]), "stream_wait_event")
@@ -756,7 +872,7 @@ class BatchedRectLTM(_BatchedBase):
 
     @_on_device
     def step_overlapped(self, k, q, u=None, new_doc=False, k_next=None, next_new_doc=False, lengths=None,
-                        next_lengths=None):
+                        next_lengths=None, chunk_frames=None):
         """`step(k, ...)` with the frame pooling of `k_next` issued beside it, in ONE library call
         (`ltm_rect_step_overlap`: side stream pools the next chunk, a high-priority stream runs this chunk's
         regression / projection / attention, the current stream joins both).  `k` must be the tensor handed over as
@@ -765,21 +881,33 @@ class BatchedRectLTM(_BatchedBase):
         frame; a chunk expected to continue the videos may be pooled per bin, see `bin_pool`).
         `lengths` / `next_lengths`: per-video lengths of `k` / `k_next` (ragged chunks, see `step`); `k` is matched
         with its prefetch by lengths too.  `k` and `k_next` are float32, float16 or bfloat16, each on its own (see
-        `step`); `q` is float32."""
-        require_cuda(k, q, u, k_next)
-        kdt = self._chunk_dtype(k)
-        ndt = self._chunk_dtype(k_next, "k_next") if k_next is not None else 0
+        `step`); `q` is float32.  `k` and `k_next` may each be a list of per-video entries (see `step`), with
+        `chunk_frames` = L; a padded `k` or `k_next` then has L*T tokens."""
+        listed = [isinstance(x, (list, tuple)) for x in (k, k_next)]
+        if chunk_frames is not None and not any(listed):
+            raise ValueError("chunk_frames applies to a chunk given as a list")
+        k = self._entries(k, chunk_frames if listed[0] else None, lengths)
+        k_next = self._entries(k_next, chunk_frames if listed[1] else None, next_lengths, "k_next")
+        lst, nlst = isinstance(k, _Entries), isinstance(k_next, _Entries)
+        require_cuda(q, u, None if lst else k, None if (nlst or k_next is None) else k_next)
+        kdt = k.code if lst else self._chunk_dtype(k)
+        ndt = 0 if k_next is None else k_next.code if nlst else self._chunk_dtype(k_next, "k_next")
         if q.dtype != torch.float32:
             raise ValueError("q must be float32")
-        if k_next is not None and (not k_next.is_contiguous() or tuple(k_next.shape) != tuple(k.shape)):
-            raise ValueError("k_next must be contiguous and have the shape of k")
+        if chunk_frames is not None and k.shape[1] != int(chunk_frames) * self.T:
+            raise ValueError(f"k has {k.shape[1]} tokens, chunk_frames={chunk_frames} means {int(chunk_frames) * self.T}")
+        if k_next is not None and ((not nlst and not k_next.is_contiguous()) or tuple(k_next.shape) != tuple(k.shape)):
+            raise ValueError("k_next must be contiguous and have the shape of k (a list: as many entries as k has "
+                             "videos)")
         nl = None
-        if k_next is not None and next_lengths is not None:
+        if nlst:
+            nl = k_next.lens
+        elif k_next is not None and next_lengths is not None:
             nl = _as_lengths(next_lengths, k.shape[0], k.shape[1] // self.T)
-        k, q = k.contiguous(), q.contiguous()
-        Bv, L, Q, tab, tdev, flags, u, rag = self._prepare(k, q, new_doc, u, lengths)
+        k, q = (k if lst else k.contiguous()), q.contiguous()
+        Bv, L, Q, tab, tdev, flags, u, rag = self._prepare(k, q, new_doc, u, k.lens if lst else lengths)
         ws = self._workspace(Bv, L, Q)
-        if rag is not None or next_lengths is not None:
+        if rag is not None or nl is not None:
             self._ragged_ws(ws, Bv, L)
         hit = self._frames_source(k, Q, ws, tab, flags, rag, prefetch=True)
         ev = self._sync_events()
@@ -793,20 +921,23 @@ class BatchedRectLTM(_BatchedBase):
         if k_next is not None:
             b = self._pref_buffer(ws)
             if nl is not None:
-                nl_dev, noffs_dev = self._lengths_dev(nl)
-                nl_dev.record_stream(self._side)
+                nl_dev, noffs_dev, ntab = self._lengths_dev(nl, k_next.ptrs if nlst else None)
+                nl_dev.record_stream(self._side)        # (with the table: one buffer)
                 nf = sum(nl)
                 o.next_lengths, o.next_offs = nl_dev.data_ptr(), noffs_dev.data_ptr()
                 o.next_frames, o.next_splits = nf, self._splits(nf)
+                o.next_ptrs = ntab.data_ptr() if nlst else None
                 nb = False
             else:
                 nb = (not next_new_doc) and self._bin_ok(Bv, L, tab, ndt)
-            o.k_next, o.xpart_next, o.next_binned = k_next.data_ptr(), ws["xbufs"][b].data_ptr(), int(nb)
+            o.k_next = None if nlst else k_next.data_ptr()
+            o.xpart_next, o.next_binned = ws["xbufs"][b].data_ptr(), int(nb)
             o.next_dtype = ndt
             o.ev_fork_pool, o.ev_pooled_next = ev["fork_pool"][b], ev["pooled"][b]
-            k_next.record_stream(self._side)
-            self._pref.append(dict(ref=weakref.ref(k_next), ver=k_next._version, buf=b, event=ev["pooled"][b],
-                                   captured=capturing, binned=nb, lens=nl))
+            for t in (k_next.stores if nlst else (k_next,)):
+                t.record_stream(self._side)
+            self._pref.append(dict(refs=_chunk_refs(k_next), buf=b, event=ev["pooled"][b], captured=capturing,
+                                   binned=nb, lens=nl))
         ctx = torch.empty(Bv, Q, self.D, device=self.device, dtype=torch.float32)   # main joins the compute stream
         a = self._args(Bv, L, Q, ws, tab, tdev, beside_pool=k_next is not None, rag=rag, k_dtype=kdt)
         if rag is not None:

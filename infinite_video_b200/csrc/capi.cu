@@ -50,14 +50,25 @@ static int check_chunk_dtype(const char* who, const char* field, int dtype, int 
   return 0;
 }
 
+// A chunk given per video (table: ltm_rect_step_args.k_ptrs, ltm_overlap.next_ptrs) is ragged, comes without a chunk
+// pointer and is never pooled per bin.
+static int check_chunk_table(const char* who, const char* field, const void* table, const void* k,
+                             const int32_t* lengths, bool binned) {
+  if (!table) return 0;
+  LTM_REQUIRE(!k, "%s: %s and a chunk pointer are both set", who, field);
+  LTM_REQUIRE(lengths, "%s: %s needs per-video lengths", who, field);
+  LTM_REQUIRE(!binned, "%s: a chunk given per video (%s) is not pooled per bin", who, field);
+  return 0;
+}
+
 // Frame pooling of one chunk of the geometry of `a` into xpart: packed frames of a ragged chunk (offs != NULL: frame
-// offsets, `frames` in all), per-bin sums (binned, fp32 chunks) or per-frame means.  dtype: storage of k, as checked
-// by check_chunk_dtype.  max_ctas bounds the grid (0 = one CTA per unit).
-static int pool_chunk(const ltm_rect_step_args* a, const void* k, int dtype, float* xpart, const int32_t* offs,
-                      int frames, int splits, bool binned, int max_ctas, void* stream) {
+// offsets, `frames` in all; from the per-video table ptrs when set), per-bin sums (binned, fp32 chunks) or per-frame
+// means.  dtype: storage of k, as checked by check_chunk_dtype.  max_ctas bounds the grid (0 = one CTA per unit).
+static int pool_chunk(const ltm_rect_step_args* a, const void* k, const void* const* ptrs, int dtype, float* xpart,
+                      const int32_t* offs, int frames, int splits, bool binned, int max_ctas, void* stream) {
   LTM_REQUIRE(!binned || a->fbin_ptr, "frame pooling: per-bin pooling without fbin_ptr");
   return ltm::pool_frames("frame pooling", k, dtype, xpart, a->Bv, a->L, a->T, a->e, binned ? 1 : splits, max_ctas,
-                          stream, offs, frames, nullptr, 0, binned ? a->fbin_ptr : nullptr, a->xb_rows);
+                          stream, offs, frames, nullptr, 0, binned ? a->fbin_ptr : nullptr, a->xb_rows, ptrs);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -69,6 +80,7 @@ extern "C" int ltm_rect_step(const ltm_rect_step_args* a, const void* k, const f
   using namespace ltm;
   LTM_REQUIRE(a && q && ctx, "rect_step: null pointer");
   if (int rc = check_chunk_dtype("rect_step", "k_dtype", a->k_dtype, a->e, a->binned != 0)) return rc;
+  if (int rc = check_chunk_table("rect_step", "k_ptrs", a->k_ptrs, k, a->lengths, a->binned != 0)) return rc;
   const int D = a->H * a->d;
   const int qtiles = (a->Q + 31) / 32;
   cudaStream_t st_ = (cudaStream_t)stream;
@@ -95,9 +107,9 @@ extern "C" int ltm_rect_step(const ltm_rect_step_args* a, const void* k, const f
       if (rc) return rc;
     }
   }
-  if (k != nullptr) {          // k == NULL: a->xpart was already filled (frame pooling is stateless and may be
-    LTM_PROF(0);               // issued ahead of time on another stream, see BatchedRectLTM.prefetch)
-    rc = pool_chunk(a, k, a->k_dtype, a->xpart, ragged ? a->frame_offs : nullptr, a->frames, a->splits, binned, 0,
+  if (k != nullptr || a->k_ptrs != nullptr) {  // neither: a->xpart was already filled (frame pooling is stateless
+    LTM_PROF(0);               // and may be issued ahead of time on another stream, see BatchedRectLTM.prefetch)
+    rc = pool_chunk(a, k, a->k_ptrs, a->k_dtype, a->xpart, ragged ? a->frame_offs : nullptr, a->frames, a->splits, binned, 0,
                     stream);
     if (rc) return rc;
     LTM_PROF(1);
@@ -232,7 +244,13 @@ extern "C" int ltm_rect_step_overlap(const ltm_rect_step_args* a, const ltm_over
   LTM_REQUIRE(a && o && q && ctx, "rect_step_overlap: null pointer");
   LTM_REQUIRE(o->ev_fork && o->ev_join, "rect_step_overlap: fork / join events missing");
   if (int rc = check_chunk_dtype("rect_step_overlap", "k_dtype", a->k_dtype, a->e, a->binned != 0)) return rc;
-  if (o->k_next != nullptr) {
+  if (int rc = check_chunk_table("rect_step_overlap", "k_ptrs", a->k_ptrs, nullptr, a->lengths, a->binned != 0))
+    return rc;
+  if (int rc = check_chunk_table("rect_step_overlap", "next_ptrs", o->next_ptrs, o->k_next, o->next_lengths,
+                                 o->next_binned != 0))
+    return rc;
+  const bool pool_next = o->k_next != nullptr || o->next_ptrs != nullptr;
+  if (pool_next) {
     if (int rc = check_chunk_dtype("rect_step_overlap", "next_dtype", o->next_dtype, a->e, o->next_binned != 0))
       return rc;
     LTM_REQUIRE(o->xpart_next && o->ev_fork_pool && o->ev_pooled_next, "rect_step_overlap: prefetch target missing");
@@ -240,13 +258,13 @@ extern "C" int ltm_rect_step_overlap(const ltm_rect_step_args* a, const ltm_over
   }
   cudaStream_t ms = (cudaStream_t)o->main_stream, ss = (cudaStream_t)o->side_stream,
                cs = (cudaStream_t)o->compute_stream;
-  if (o->k_next != nullptr) {
+  if (pool_next) {
     // the target buffer was last read by work already queued on the main stream
     LTM_CUDA(cudaEventRecord((cudaEvent_t)o->ev_fork_pool, ms));
     LTM_CUDA(cudaStreamWaitEvent(ss, (cudaEvent_t)o->ev_fork_pool, 0));
     if (a->prof_events[0]) cudaEventRecord((cudaEvent_t)a->prof_events[0], ss);
     const bool ragged_next = o->next_lengths != nullptr;
-    int rc = pool_chunk(a, o->k_next, o->next_dtype, o->xpart_next, ragged_next ? o->next_offs : nullptr,
+    int rc = pool_chunk(a, o->k_next, o->next_ptrs, o->next_dtype, o->xpart_next, ragged_next ? o->next_offs : nullptr,
                         o->next_frames, ragged_next ? o->next_splits : a->splits, o->next_binned != 0, o->pool_ctas,
                         ss);
     if (rc) return rc;

@@ -43,11 +43,12 @@ static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t
 // error text), picks the kernel, thread count and grid.  k[Bv, L, T, e], dtype 0 fp32, 1 fp16, 2 bfloat16, is pooled
 // into xpart as the frame means in `splits` partial sums, [Bv*L, splits, e]; offs != NULL: only the `frames` frames of
 // a ragged chunk (ltm_pool_mean_ragged), packed; fbin_ptr != NULL: the per-bin sums [Bv, rows, e] instead
-// (ltm_pool_bins); k16 != NULL: the chunk as fp16 as well (ltm_pool_mean_convert, ld16 rows per video when ragged).
-// max_ctas > 0 bounds the grid of the per-frame means (0 = one CTA per (frame, token-split)).
+// (ltm_pool_bins); k16 != NULL: the chunk as fp16 as well (ltm_pool_mean_convert, ld16 rows per video when ragged);
+// ptrs != NULL (with offs, k == NULL): the ragged chunk of video v read from ptrs[v] instead of k[v]
+// (ltm_pool_mean_ptrs).  max_ctas > 0 bounds the grid of the per-frame means (0 = one CTA per (frame, token-split)).
 int pool_frames(const char* who, const void* k, int dtype, float* xpart, int Bv, int L, int T, int e, int splits,
                 int max_ctas, void* stream, const int32_t* offs = nullptr, int frames = 0, void* k16 = nullptr,
-                int ld16 = 0, const int32_t* fbin_ptr = nullptr, int rows = 0);
+                int ld16 = 0, const int32_t* fbin_ptr = nullptr, int rows = 0, const void* const* ptrs = nullptr);
 
 // ---- ragged batches (ltm_rect_step_args.lengths), internal to the library
 // ltm_consolidate_rect_kv with per-video lengths (0 = idle) and frame offsets; NULL lengths = lock-step

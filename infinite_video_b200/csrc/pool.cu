@@ -10,7 +10,7 @@
 // exists to fill the 148 SMs when Bv*L is small.
 //
 // Every kernel below pools a frame through the pool() of its element type (F32, F16, BF16), so a pooled frame carries
-// the same bits whichever kernel, frame map (LockStep, Ragged) or grid produced it.
+// the same bits whichever kernel, frame map (LockStep, Ragged, PerVideo) or grid produced it.
 #include <cuda_fp16.h>
 #include <type_traits>
 
@@ -142,24 +142,49 @@ using F16 = Half<false>;
 using BF16 = Half<true>;
 
 // ---- frame maps: the work items are the (frame, token-split) pairs of the pooled frames, frame f of them read from
-// frame src(f) of the chunk.  A kernel builds its map from its last three arguments: offs[Bv+1], Bv, L.  (Scalar
-// arguments rather than a struct: a struct argument is loaded whole and held in registers across the work loop.)
+// frame src(f) of the chunk, which starts at frame(k, src(f), T, ev).  A kernel builds its map from its last three
+// arguments: offs[Bv+1], Bv, L.  (Scalar arguments rather than a struct: a struct argument is loaded whole and held in
+// registers across the work loop.)
 struct LockStep {      // every video uses all L frames: frame v*L + l in and out
   static constexpr bool ragged = false;
   __device__ __forceinline__ LockStep(const int32_t*, int, int) {}
   __device__ __forceinline__ size_t src(unsigned f) const { return f; }
+  template <class In>
+  static __device__ __forceinline__ const In* frame(const In* k, size_t src, int T, int ev) { return k + src * T * ev; }
 };
 struct Ragged {        // frames packed video after video: frame f is frame f - offs[v] of video v, offs[v] <= f <
   static constexpr bool ragged = true;     // offs[v+1]; the padding of the chunk is never read
   const int32_t* offs;
   int Bv, L;
-  __device__ __forceinline__ size_t src(unsigned f) const {
+  __device__ __forceinline__ int video(unsigned f) const {
     int lo = 0, hi = Bv;                                  // offs[lo] <= f < offs[hi]
     while (hi - lo > 1) {
       const int mid = (lo + hi) >> 1;
       if ((unsigned)__ldg(offs + mid) <= f) lo = mid; else hi = mid;
     }
-    return (size_t)lo * L + (f - (unsigned)__ldg(offs + lo));
+    return lo;
+  }
+  __device__ __forceinline__ size_t src(unsigned f) const {
+    const int v = video(f);
+    return (size_t)v * L + (f - (unsigned)__ldg(offs + v));
+  }
+  template <class In>
+  static __device__ __forceinline__ const In* frame(const In* k, size_t src, int T, int ev) { return k + src * T * ev; }
+};
+// The work items of Ragged, each video's frames read from wherever its chunk lives: k is then a table of Bv 64-bit
+// base addresses, and frame l of video v starts at ptrs[v] + l*T*e.  src(f) packs (v, l) as v << 32 | l.  (The
+// offset in a video is a 32-bit product, L*T*ev < 2^32 is checked on the host: with a 64-bit one the bounded-grid
+// 16-bit kernels spill.)
+struct PerVideo : Ragged {
+  __device__ __forceinline__ PerVideo(const int32_t* o, int b, int l) : Ragged{o, b, l} {}
+  __device__ __forceinline__ size_t src(unsigned f) const {
+    const int v = video(f);
+    return (size_t)v << 32 | (f - (unsigned)__ldg(offs + v));
+  }
+  template <class In>
+  static __device__ __forceinline__ const In* frame(const In* k, size_t src, int T, int ev) {
+    const auto* ptrs = reinterpret_cast<const unsigned long long*>(k);
+    return reinterpret_cast<const In*>(__ldg(ptrs + (src >> 32))) + (size_t)((unsigned)src * (unsigned)(T * ev));
   }
 };
 
@@ -175,13 +200,13 @@ __device__ __forceinline__ WorkItem work_item(const Map& map, unsigned work, int
 }
 
 // Token split it.sp of chunk frame it.src, written to row (it.f * splits + it.sp) of xpart.
-template <class E, class Visit = NoVisit>
+template <class E, class Map, class Visit = NoVisit>
 __device__ __forceinline__ void pool_item(const typename E::In* __restrict__ k, float4* __restrict__ xpart, int T,
                                           int ev, int splits, float Tf, const WorkItem& it, uint64_t pol,
                                           const Visit& visit = {}) {
   const int r0 = (int)(((long long)T * it.sp) / splits);
   const int r1 = (int)(((long long)T * (it.sp + 1)) / splits);
-  const typename E::In* base = k + it.src * T * ev;
+  const typename E::In* base = Map::frame(k, it.src, T, ev);
   for (int c = threadIdx.x; c < ev; c += blockDim.x)
     E::pool(xpart, (size_t)it.f * splits + it.sp, base, r0, r1, ev, c, Tf, pol, visit);
 }
@@ -194,11 +219,11 @@ pool_mean_kernel(const typename E::In* __restrict__ k, float4* __restrict__ xpar
                  float Tf, unsigned total, const int32_t* offs, int Bv, int L) {
   const Map map{offs, Bv, L};
   if constexpr (!PERSIST) {
-    pool_item<E>(k, xpart, T, ev, splits, Tf, work_item(map, blockIdx.x, splits), policy_evict_first());
+    pool_item<E, Map>(k, xpart, T, ev, splits, Tf, work_item(map, blockIdx.x, splits), policy_evict_first());
   } else {
     const uint64_t pol = policy_evict_first();
     for (unsigned work = blockIdx.x; work < total; work += gridDim.x)
-      pool_item<E>(k, xpart, T, ev, splits, Tf, work_item(map, work, splits), pol);
+      pool_item<E, Map>(k, xpart, T, ev, splits, Tf, work_item(map, work, splits), pol);
   }
 }
 
@@ -296,7 +321,7 @@ pool_mean_convert_kernel(const float4* __restrict__ k, float4* __restrict__ xpar
         v16[(size_t)n * e4 + i] = make_uint2(0u, 0u);
     }
   }
-  pool_item<F32>(k, xpart, T, e4, splits, Tf, it, policy_evict_first(), StoreHalf{k16 + row16 * e4, e4, paired});
+  pool_item<F32, Map>(k, xpart, T, e4, splits, Tf, it, policy_evict_first(), StoreHalf{k16 + row16 * e4, e4, paired});
 }
 
 template <class Map, class E>
@@ -324,9 +349,11 @@ static void launch_mean(int dtype, const void* k, float* xpart, const int32_t* o
 
 int pool_frames(const char* who, const void* k, int dtype, float* xpart, int Bv, int L, int T, int e, int splits,
                 int max_ctas, void* stream, const int32_t* offs, int frames, void* k16, int ld16,
-                const int32_t* fbin_ptr, int rows) {
+                const int32_t* fbin_ptr, int rows, const void* const* ptrs) {
   const long long nf = offs ? frames : (long long)Bv * L, units = nf * splits;
-  LTM_REQUIRE(k && (xpart || units == 0), "%s: null pointer", who);
+  LTM_REQUIRE((k || ptrs) && (xpart || units == 0), "%s: null pointer", who);
+  LTM_REQUIRE(!ptrs || (offs && !k && !k16 && !fbin_ptr),
+              "%s: a chunk pointer table needs frame offsets and takes no chunk, fp16 copy or per-bin pooling", who);
   LTM_REQUIRE(Bv > 0 && L > 0 && T > 0 && e > 0 && nf >= 0 && nf <= (long long)Bv * L &&
               (!fbin_ptr || (rows > 0 && Bv <= 65535)),
               "%s: bad shape Bv=%d L=%d T=%d e=%d frames=%lld rows=%d", who, Bv, L, T, e, nf, rows);
@@ -337,9 +364,12 @@ int pool_frames(const char* who, const void* k, int dtype, float* xpart, int Bv,
               "%s: ld16=%d must be a multiple of 64 and >= L*T=%lld", who, ld16, (long long)L * T);
   LTM_REQUIRE(splits >= 1 && splits <= T, "%s: splits=%d out of range [1,%d]", who, splits, T);
   LTM_REQUIRE(max_ctas >= 0, "%s: max_ctas=%d must be >= 0", who, max_ctas);
-  LTM_REQUIRE(aligned16(k) && aligned16(xpart) && (reinterpret_cast<uintptr_t>(k16) & 7u) == 0,
-              "%s: pointers must be 16-byte aligned%s", who, k16 ? " (k16: 8-byte)" : "");
+  LTM_REQUIRE(aligned16(k) && aligned16(xpart) && (reinterpret_cast<uintptr_t>(k16) & 7u) == 0 &&
+              (reinterpret_cast<uintptr_t>(ptrs) & 7u) == 0,
+              "%s: pointers must be 16-byte aligned%s", who, k16 ? " (k16: 8-byte)" : ptrs ? " (ptrs: 8-byte)" : "");
   LTM_REQUIRE(units < (1ll << 31), "%s: too many frames", who);
+  LTM_REQUIRE(!ptrs || (long long)L * T * (e / w) < (1ll << 32), "%s: a video of L*T*e=%lld elements is too large for "
+              "the pointer table", who, (long long)L * T * e);
   if (units == 0) return 0;                  // every video of a ragged chunk idle: nothing to read, pool or write
   const int ev = e / w;
   const int threads = ev >= 256 ? 256 : ((ev + 31) / 32) * 32;
@@ -355,6 +385,8 @@ int pool_frames(const char* who, const void* k, int dtype, float* xpart, int Bv,
   else if (k16)
     pool_mean_convert_kernel<LockStep><<<(unsigned)units, threads, 0, st>>>(k4, x4, h, T, ev, splits, (float)T, 0,
                                                                              offs, Bv, L);
+  else if (ptrs)
+    launch_mean<PerVideo>(dtype, ptrs, xpart, offs, Bv, L, T, ev, splits, (unsigned)units, max_ctas, threads, st);
   else if (offs)
     launch_mean<Ragged>(dtype, k, xpart, offs, Bv, L, T, ev, splits, (unsigned)units, max_ctas, threads, st);
   else
@@ -388,6 +420,13 @@ extern "C" int ltm_pool_mean_ragged(const void* k, int dtype, float* xpart, cons
                                     int e, int splits, int frames, int max_ctas, void* stream) {
   LTM_REQUIRE(offs, "pool_mean_ragged: null pointer");
   return ltm::pool_frames("pool_mean_ragged", k, dtype, xpart, Bv, L, T, e, splits, max_ctas, stream, offs, frames);
+}
+
+extern "C" int ltm_pool_mean_ptrs(const void* const* ptrs, int dtype, float* xpart, const int32_t* offs, int Bv, int L,
+                                  int T, int e, int splits, int frames, int max_ctas, void* stream) {
+  LTM_REQUIRE(ptrs && offs, "pool_mean_ptrs: null pointer");
+  return ltm::pool_frames("pool_mean_ptrs", nullptr, dtype, xpart, Bv, L, T, e, splits, max_ctas, stream, offs, frames,
+                          nullptr, 0, nullptr, 0, ptrs);
 }
 
 extern "C" int ltm_pool_mean_convert(const float* k, float* xpart, void* k16, int Bv, int L, int T, int e, int splits,

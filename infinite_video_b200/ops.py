@@ -54,6 +54,17 @@ def pool_into(k, out, L, T, splits, max_ctas=0, stream=None, offs=None, frames=0
         check(lib().ltm_pool_mean_grid(ptr(k), ptr(out), Bv, L, T, e, splits, max_ctas, st), "pool_mean")
 
 
+def pool_ptrs(ptrs, dtype, out, offs, Bv, L, T, e, splits, frames, max_ctas=0, stream=None):
+    """`pool_into` of a ragged chunk whose videos live at their own addresses: ptrs int64 [Bv] device table of base
+    addresses (video v's lengths[v]*T dense rows of width e, 16-byte aligned; idle videos are not read), dtype a
+    `CHUNK_DTYPES` code, offs int32 [Bv+1] device frame offsets -> out[frames, splits, e] (any float32 storage of that
+    many elements), bit for bit what `pool_into` gives with offs for the same frames of a padded chunk."""
+    require_cuda(ptrs, out, offs)
+    st = stream_ptr(out.device) if stream is None else stream
+    check(lib().ltm_pool_mean_ptrs(ptr(ptrs), dtype, ptr(out), ptr(offs), Bv, L, T, e, splits, frames, max_ctas, st),
+          "pool_mean_ptrs")
+
+
 def pool_mean(k, splits=1):
     """k[Bv,L,T,e] -> xpart[Bv,L,splits,e] (frame means as `splits` partial sums).  gibbs:304."""
     require_cuda(k)
